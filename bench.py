@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — MCTS simulations/sec of the batched c21 search step (BASELINE.json's metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one NablaOptimizer::par_roll_out_episodes over the whole batch of roots
 (az-discrete-opt/src/nabla/optimizer/mod.rs:121-191): walks + pack + MLP forward + add_actions + argmin.
@@ -34,6 +34,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # no bytecode caches for the modules it imports from the tree (which may be read-only)
 
 METRIC = "mcts_simulations_per_sec"
 UNIT = "simulations/s"
@@ -137,6 +138,49 @@ def cpu_reference_run(n, roots, steps, warmup, seed, threads, budget_s=None):
     return k["n_live"] / dt, dt, k
 
 
+def dump_outputs(out_dir, h, capi, n_improved, seed, world=1, budget=64_000_000, row_budget=40_000_000, max_trees=32):
+    """Writes what the timed steps computed, as of their last step, to out_dir/<name>.npy in float32 or float64 (counts
+    and indices as exact integers): the step counters and improvement count, the argmin, and per tree the model's
+    priors, the state vectors it read, the walker's path length and the tree sizes, then the node records of a few
+    whole trees.  A tree whose root is exhausted did not expand in the step (path length 0): its prior and state rows
+    are zeros.  With `world` ranks each rank gets 1/world of both byte budgets, so the dumps of all ranks together stay
+    within them.  When all rows do not fit the row budget, a fixed sample of trees drawn from `seed` is written, in
+    tree order."""
+    budget //= world
+    row_budget //= world
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"counters": np.array([h.counters()[f] for f in capi.COUNTER_FIELDS], dtype=np.float64),
+           "n_improved": np.array([n_improved], dtype=np.float64)}
+    am = h.argmin()
+    out.update(argmin_eval=np.array([am["eval"]], dtype=np.float32), argmin_lambda1=np.array([am["lambda1"]]),
+               argmin_mu=np.array([am["mu"]], dtype=np.float64), argmin_parents=am["parents"].astype(np.float64),
+               argmin_permitted=am["permitted"].astype(np.float64))
+    k = min(h.b, row_budget // (4 * 3 * h.a + 8 * 4))
+    rows = np.arange(h.b) if k == h.b else np.sort(np.random.default_rng(seed).choice(h.b, k, replace=False))
+    priors, states = h.priors()[rows], h.state_vecs()[rows]
+    path_len = h.walkers()["path_len"][rows]
+    priors[path_len == 0] = 0.0
+    states[path_len == 0] = 0.0
+    out.update(priors=priors, state_vecs=states, walker_path_len=path_len.astype(np.float64),
+               tree_sizes=np.array([h.tree_sizes(int(i)) for i in rows], dtype=np.float64))
+    # whole trees, one record per node: tree, c, c*, n_t, exhausted children, prediction range lo, hi (include/azb.h);
+    # as many sampled trees as the byte budget leaves room for
+    used = sum(a.nbytes for a in out.values()) + 128 * (len(out) + 1)  # each .npy file adds a 128-byte header
+    nodes = []
+    for i in rows[np.linspace(0, len(rows) - 1, min(max_trees, len(rows))).astype(np.int64)]:
+        nd = h.dump_tree(int(i))["nodes"]
+        costs = np.ascontiguousarray(nd[:, :2]).view(np.float32)  # c and c* are stored as their f32 bit patterns
+        rec = np.concatenate([np.full((len(nd), 1), i, dtype=np.float64), costs.astype(np.float64),
+                              nd[:, 2:].astype(np.float64)], axis=1)
+        if used + rec.nbytes > budget:
+            break
+        nodes.append(rec)
+        used += rec.nbytes
+    out["tree_nodes"] = np.concatenate(nodes) if nodes else np.zeros((0, 7))
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def timed_config(capi, n, b, workers, steps, warmup, seed, rank, local_rank, prior_hash=False, mlp_mode=None):
     """K device-timed steps of another configuration on this rank's GPU (inputs resident, W warm-up steps first).
     Returns (simulations, ms, cost evals, device bytes)."""
@@ -179,7 +223,12 @@ def main():
     ap.add_argument("--cpu-baseline-seconds", type=float, default=20.0, help="time bound of the cpu_baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the same_priors / c3 / c4 objects")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what they computed to DIR/<name>.npy (rank r > 0: DIR/rank<r>/); "
+                         "the inputs depend only on the arguments, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     # stdout carries exactly ONE line, the JSON: everything else a library prints there (NCCL's version banner, ...) goes
@@ -304,12 +353,15 @@ def main():
     time.sleep(0.25)
     barrier()
     t0 = time.time()
-    ms, _ = h.step_timed(args.steps)
+    ms, n_improved = h.step_timed(args.steps)
     barrier()
     t1 = time.time()
     clocks = sampler.stop(t0, t1)
     launches = h.kernel_launches() - launches0
     k = h.counters()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs if rank == 0 else os.path.join(args.dump_outputs, f"rank{rank}"), h, capi,
+                     n_improved, args.seed, world=world)
     h.set_counter_mode(True)
     ms_max = allreduce(ms, dist.ReduceOp.MAX if world > 1 else None)
     sims = allreduce(float(k["n_live"]), dist.ReduceOp.SUM if world > 1 else None)
