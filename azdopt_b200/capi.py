@@ -19,6 +19,7 @@ MLP_FP32, MLP_TC, MLP_TC3 = 0, 1, 2
 MAX_TOL = 8
 ASYNC_AUTO = 0xFFFFFFFF
 ASYNC_SHARED = 0xFFFFFFFE  # every SM walks trees and serves the model with its last warpgroup (include/azb.h)
+SELECT_REFERENCE, SELECT_PUCT = 0, 1  # azb_config.selection: next_action, or PUCT (rule in include/azb.h; no reference)
 
 COUNTER_FIELDS = [
     "n_sel", "d_sel", "n_cur", "n_cand", "n_probe", "n_ins", "n_term", "n_hit", "n_arc", "n_pred",
@@ -33,7 +34,8 @@ class Config(C.Structure):
         ("n_as_tol", C.c_uint32 * MAX_TOL), ("n_as_tol_len", C.c_uint32), ("n_as_tol_default", C.c_uint32),
         ("mlp_hidden", C.c_uint32 * 3), ("mlp_mode", C.c_uint32), ("prior_mode", C.c_uint32),
         ("prior_seed", C.c_uint64), ("max_steps", C.c_uint32), ("cap_nodes", C.c_uint32), ("cap_preds", C.c_uint32),
-        ("cap_parents", C.c_uint32), ("max_episodes", C.c_uint32), ("n_groups", C.c_uint32), ("async_workers", C.c_uint32), ("reserved", C.c_uint32 * 5),
+        ("cap_parents", C.c_uint32), ("max_episodes", C.c_uint32), ("n_groups", C.c_uint32), ("async_workers", C.c_uint32),
+        ("selection", C.c_uint32), ("puct_c", C.c_float), ("reserved", C.c_uint32 * 3),
     ]
 
 

@@ -191,6 +191,8 @@ int azb_config_default(azb_config *cfg, uint32_t n_vertices, uint32_t n_roots) {
     cfg->max_steps = 800;
     cfg->max_episodes = 0;
     cfg->n_groups = 1;
+    cfg->selection = AZB_SELECT_REFERENCE;
+    cfg->puct_c = 1.0f;
     return AZB_OK;
 }
 
@@ -242,6 +244,8 @@ int azb_create(const azb_config *cfg_in, azb_handle **out) {
     if (cfg.n_vertices < 5 || cfg.n_vertices > AZB_MAX_VERTICES || cfg.n_roots == 0) return AZB_ERR_INVALID;
     if (cfg.n_as_tol_len > AZB_MAX_TOL) return AZB_ERR_INVALID;
     if (cfg.prior_mode > AZB_PRIOR_INJECTED || cfg.mlp_mode > AZB_MLP_TC3) return AZB_ERR_INVALID;
+    if (cfg.selection > AZB_SELECT_PUCT) return AZB_ERR_INVALID;
+    if (cfg.selection == AZB_SELECT_PUCT && !(std::isfinite(cfg.puct_c) && cfg.puct_c > 0.0f)) return AZB_ERR_INVALID;
     azb_handle *h = new azb_handle();
     memset((void *)h, 0, sizeof(*h));
     h->err[0] = 0;
@@ -347,6 +351,8 @@ int azb_create(const azb_config *cfg_in, azb_handle **out) {
     for (uint32_t i = 0; i < 8; ++i) L.tol[i] = cfg.n_as_tol[i];
     L.tol_len = cfg.n_as_tol_len;
     L.tol_default = cfg.n_as_tol_default;
+    L.selection = cfg.selection;
+    L.puct_c = cfg.puct_c;
     L.prior_mode = cfg.prior_mode;
     L.log_cap = 4096;
     L.frontier_cap = AZB_FRONTIER_CAP;
@@ -411,18 +417,30 @@ int azb_create(const azb_config *cfg_in, azb_handle **out) {
     {
         const int sb = (int)h->smem_bytes;
         const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-        switch (azb_stack_depth(N)) {
-            case 3:
+        switch (azb_stack_depth(N) * 2 + (cfg.selection == AZB_SELECT_PUCT ? 1 : 0)) {
+            case 6:
                 CK(cudaFuncSetAttribute(azb_tree_kernel<3, true>, attr, sb));
                 CK(cudaFuncSetAttribute(azb_tree_kernel<3, false>, attr, sb));
                 break;
-            case 4:
+            case 7:
+                CK(cudaFuncSetAttribute(azb_tree_kernel<3, true, true>, attr, sb));
+                CK(cudaFuncSetAttribute(azb_tree_kernel<3, false, true>, attr, sb));
+                break;
+            case 8:
                 CK(cudaFuncSetAttribute(azb_tree_kernel<4, true>, attr, sb));
                 CK(cudaFuncSetAttribute(azb_tree_kernel<4, false>, attr, sb));
                 break;
-            default:
+            case 9:
+                CK(cudaFuncSetAttribute(azb_tree_kernel<4, true, true>, attr, sb));
+                CK(cudaFuncSetAttribute(azb_tree_kernel<4, false, true>, attr, sb));
+                break;
+            case 10:
                 CK(cudaFuncSetAttribute(azb_tree_kernel<5, true>, attr, sb));
                 CK(cudaFuncSetAttribute(azb_tree_kernel<5, false>, attr, sb));
+                break;
+            default:
+                CK(cudaFuncSetAttribute(azb_tree_kernel<5, true, true>, attr, sb));
+                CK(cudaFuncSetAttribute(azb_tree_kernel<5, false, true>, attr, sb));
                 break;
         }
     }
@@ -654,9 +672,15 @@ static int launch_tree(azb_handle *h, uint32_t flags, uint32_t target_step, int 
     const uint32_t blocks = (tree_end - tree0 + AZB_WARPS_PER_BLOCK - 1) / AZB_WARPS_PER_BLOCK;
     const dim3 block(AZB_WARPS_PER_BLOCK * 32);
     const uint32_t me = h->cfg.max_episodes;
-#define AZB_LAUNCH_TREE(D, C)                                                                                       \
-    azb_tree_kernel<D, C><<<blocks, block, h->smem_bytes, stream>>>(L, flags, h->smem_words_per_warp, h->lcap, target_step, \
-                                                                    me, tree0, tree_end)
+#define AZB_LAUNCH_TREE(D, C)                                                                                             \
+    do {                                                                                                                  \
+        if (L.selection == AZB_SELECT_PUCT)                                                                               \
+            azb_tree_kernel<D, C, true><<<blocks, block, h->smem_bytes, stream>>>(L, flags, h->smem_words_per_warp, h->lcap, \
+                                                                                  target_step, me, tree0, tree_end);        \
+        else                                                                                                              \
+            azb_tree_kernel<D, C><<<blocks, block, h->smem_bytes, stream>>>(L, flags, h->smem_words_per_warp, h->lcap,     \
+                                                                            target_step, me, tree0, tree_end);              \
+    } while (0)
     switch (azb_stack_depth(h->N) * 2 + (h->count_full ? 1 : 0)) {
         case 6: AZB_LAUNCH_TREE(3, false); break;
         case 7: AZB_LAUNCH_TREE(3, true); break;
@@ -773,15 +797,17 @@ int azb_init_trees(azb_handle *h) {
 }  // extern "C"
 
 // ---- the asynchronous search kernel (azb_async.cuh): set-up and launch -------------------------------------------
-template <int D, bool C, bool PAIR>
+template <int D, bool C, bool PAIR, bool PUCT>
 static int async_prepare_one(azb_handle *h, int *blocks_per_sm) {
-    CK(cudaFuncSetAttribute(azb_async_kernel<D, C, PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->async_smem));
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, azb_async_kernel<D, C, PAIR>, AS_THREADS, h->async_smem));
+    CK(cudaFuncSetAttribute(azb_async_kernel<D, C, PAIR, PUCT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->async_smem));
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, azb_async_kernel<D, C, PAIR, PUCT>, AS_THREADS, h->async_smem));
     return AZB_OK;
 }
 template <int D, bool C>
 static int async_prepare_kernel(azb_handle *h, int *blocks_per_sm, bool pair) {
-    return pair ? async_prepare_one<D, C, true>(h, blocks_per_sm) : async_prepare_one<D, C, false>(h, blocks_per_sm);
+    if (h->cfg.selection == AZB_SELECT_PUCT)
+        return pair ? async_prepare_one<D, C, true, true>(h, blocks_per_sm) : async_prepare_one<D, C, false, true>(h, blocks_per_sm);
+    return pair ? async_prepare_one<D, C, true, false>(h, blocks_per_sm) : async_prepare_one<D, C, false, false>(h, blocks_per_sm);
 }
 
 static int async_create(azb_handle *h) {
@@ -952,8 +978,8 @@ static int async_create(azb_handle *h) {
     return AZB_OK;
 }
 
-template <int D, bool C>
-static cudaError_t async_launch(azb_handle *h) {
+template <int D, bool C, bool PUCT>
+static cudaError_t async_launch_sel(azb_handle *h) {
     void *args[] = {(void *)&h->L, (void *)&h->asP, (void *)&h->asM};
     if (h->asP.pair) {  // cooperative AND clustered: CTAs 2c and 2c + 1 land on the two SMs of one TPC
         cudaLaunchConfig_t cfg = {};
@@ -970,10 +996,14 @@ static cudaError_t async_launch(azb_handle *h) {
         at[1].val.clusterDim.z = 1;
         cfg.attrs = at;
         cfg.numAttrs = 2;
-        return cudaLaunchKernelExC(&cfg, (const void *)azb_async_kernel<D, C, true>, args);
+        return cudaLaunchKernelExC(&cfg, (const void *)azb_async_kernel<D, C, true, PUCT>, args);
     }
-    return cudaLaunchCooperativeKernel((const void *)azb_async_kernel<D, C, false>, dim3(h->async_grid), dim3(AS_THREADS), args,
+    return cudaLaunchCooperativeKernel((const void *)azb_async_kernel<D, C, false, PUCT>, dim3(h->async_grid), dim3(AS_THREADS), args,
                                        h->async_smem, h->stream);
+}
+template <int D, bool C>
+static cudaError_t async_launch(azb_handle *h) {
+    return h->cfg.selection == AZB_SELECT_PUCT ? async_launch_sel<D, C, true>(h) : async_launch_sel<D, C, false>(h);
 }
 
 // n_steps of every tree in ONE persistent cooperative kernel (tree CTAs + model CTAs), then one batched forward over

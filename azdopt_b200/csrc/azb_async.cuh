@@ -1564,7 +1564,7 @@ struct AsTreeTable {
 __device__ __forceinline__ uint32_t as_lds_volatile(const uint32_t *p) { return *reinterpret_cast<const volatile uint32_t *>(p); }
 __device__ __forceinline__ void as_sts_volatile(uint32_t *p, uint32_t v) { *reinterpret_cast<volatile uint32_t *>(p) = v; }
 
-template <int DEPTH, bool COUNT>
+template <int DEPTH, bool COUNT, bool PUCT>
 __device__ void async_tree_worker(const AzbLayout &L, const AzbAsyncParams &P, const uint32_t tree_cta,
                                   const uint32_t n_tree_ctas, uint32_t *smem, const uint32_t n_thr) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -1792,9 +1792,9 @@ __device__ void async_tree_worker(const AzbLayout &L, const AzbAsyncParams &P, c
             // warp for every tree; with several trees per warp it only lengthens the hot loop (32 768 roots: -11 %), so
             // those launches take the instantiation that submits after the walk.
             if (P.early)
-                tree_rollout<DEPTH>(L, cx, tree, 0u, submit);
+                tree_rollout<DEPTH, PUCT>(L, cx, tree, 0u, submit);
             else
-                tree_rollout<DEPTH>(L, cx, tree, 0u);
+                tree_rollout<DEPTH, PUCT>(L, cx, tree, 0u);
         }
         in_walk = false;
         uint32_t new_state = 0u;
@@ -1903,7 +1903,7 @@ __device__ void async_tree_worker(const AzbLayout &L, const AzbAsyncParams &P, c
 // PAIR: the CTA-pair form of the model CTAs (its own instantiation: a kernel that contains cta_group::2 code can only be
 // launched in clusters — the driver refuses anything else as a "cluster misconfiguration" — and a cooperative launch in
 // clusters fails under ncu, so the default form stays free of it and keeps its plain cooperative launch)
-template <int DEPTH, bool COUNT, bool PAIR>
+template <int DEPTH, bool COUNT, bool PAIR, bool PUCT = false>  // PUCT: azb_config.selection == AZB_SELECT_PUCT
 __global__ void __launch_bounds__(AS_THREADS, 1)
     azb_async_kernel(const AzbLayout L, const AzbAsyncParams P, const __grid_constant__ AzbAsyncMaps M) {
     extern __shared__ __align__(1024) uint8_t as_smem[];
@@ -1966,5 +1966,5 @@ __global__ void __launch_bounds__(AS_THREADS, 1)
             asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(AS_REGS_WIDE_TREE));
         }
     }
-    async_tree_worker<DEPTH, COUNT>(L, P, tree_cta, n_tree_ctas, reinterpret_cast<uint32_t *>(as_smem), n_thr);
+    async_tree_worker<DEPTH, COUNT, PUCT>(L, P, tree_cta, n_tree_ctas, reinterpret_cast<uint32_t *>(as_smem), n_thr);
 }

@@ -85,6 +85,8 @@ struct AzbLayout {
     float c_lower, slope;
     uint32_t tol[8];
     uint32_t tol_len, tol_default;
+    uint32_t selection;   // AZB_SELECT_*: 0 = next_action, 1 = PUCT (the kernels' PUCT instantiations)
+    float puct_c;
     uint32_t prior_mode, log_cap;
     uint32_t frontier_cap;  // entries of a cascade work list kept in shared memory (<= AZB_FRONTIER_CAP)
     unsigned long long first_root, prior_seed;

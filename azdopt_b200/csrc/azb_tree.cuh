@@ -478,6 +478,110 @@ __device__ __forceinline__ void step_done(const AzbLayout &L, WarpCtx &cx, uint3
     cx.err = __reduce_or_sync(0xffffffffu, cx.err);
 }
 
+// PUCT prior weight w_j = (1 - c_s) + g_j, or +0 where negative (azb.h, AZB_SELECT_PUCT step 2)
+__device__ __forceinline__ float puct_weight(float one_minus_c, uint32_t g_bits) {
+    const float x = __fadd_rn(one_minus_c, __uint_as_float(g_bits));
+    return x < 0.f ? 0.f : x;
+}
+__device__ __forceinline__ float puct_butterfly(float x) {  // every lane ends with the chunk sum of azb.h step 3
+#pragma unroll
+    for (int m = 16; m >= 1; m >>= 1) x = __fadd_rn(x, __shfl_xor_sync(0xffffffffu, x, m));
+    return x;
+}
+
+// AZB_SELECT_PUCT in place of next_action at the active node whose block header is the 16-byte unit lo2 (the rule is
+// in azb.h).  kd / pr are the first 32 kid entries / predictions, already loaded.  Returns j for Unvisited(j) with its
+// prediction word in y, or -1 for Visited with the chosen kid entry's first two words in w0 / w1; sets cx.err.
+// The kid of an arc'd prediction is found through the warp's scratch (cx.lbuf as u32: kid slot by action id).
+__device__ __forceinline__ int puct_select(const AzbLayout &L, WarpCtx &cx, uint32_t lo2, float c_s, uint32_t n_out,
+                                           uint32_t cnt, uint4 kd, uint2 pr, uint32_t &w0, uint32_t &w1, uint32_t &y) {
+    const int lane = cx.lane;
+    const uint32_t FULL = 0xffffffffu;
+    uint32_t *kslot = reinterpret_cast<uint32_t *>(cx.lbuf);
+    count(cx, CT_CUR, 1);
+    count(cx, CT_CAND, cnt);
+    // 1. N_s = 1 + sum_k (n_k + 1)
+    uint32_t ns = 1u;
+#pragma unroll 1
+    for (uint32_t base = 0; base < n_out; base += 32) {
+        if (base) kd = cx.blk4[lo2 + 1u + base + lane];
+        const uint32_t t = base + lane;
+        uint32_t v = 0u;
+        if (t < n_out) {
+            kslot[kd.x >> 20] = t;
+            v = kd.z + 1u;
+        }
+        ns += __reduce_add_sync(FULL, v);
+    }
+    __syncwarp();
+    if (ns >= (1u << 24)) {
+        cx.err = 3;
+        return -1;
+    }
+    const float sq = __fsqrt_rn(__uint2float_rn(ns));
+    // 2-3. Z: butterfly per chunk, chunks folded left to right
+    const float omc = __fsub_rn(1.f, c_s);
+    float z = 0.f;
+#pragma unroll 1
+    for (uint32_t base = 0; base < cnt; base += 32) {
+        if (base) pr = cx.blk[2u * lo2 - 1u - base - lane];
+        const float s = puct_butterfly(base + lane < cnt ? puct_weight(omc, pr.x) : 0.f);
+        z = base ? __fadd_rn(z, s) : s;
+    }
+    const float p0 = __fdiv_rn(1.f, __uint2float_rn(cnt));  // Z == 0
+    // 4-6. scores, first maximum in ascending j
+    float best = 0.f;
+    int bj = -1;
+    uint32_t by = 0u, bw0 = 0u, bw1 = 0u;
+#pragma unroll 1
+    for (uint32_t base = 0; base < cnt; base += 32) {
+        if (cnt > 32u) pr = cx.blk[2u * lo2 - 1u - base - lane];
+        const uint32_t j = base + lane;
+        bool cand = false;
+        float sc = 0.f;
+        uint32_t kx = 0u, ky = 0u;
+        if (j < cnt) {
+            const float p = z == 0.f ? p0 : __fdiv_rn(puct_weight(omc, pr.x), z);
+            float q = __uint_as_float(pr.x);
+            uint32_t n1 = 1u;  // 1 + n
+            cand = true;
+            if ((pr.y >> 11) & 1u) {
+                const uint4 kid = cx.blk4[lo2 + 1u + kslot[pr.y & 0x7ffu]];
+                cand = (kid.y >> 31) != 0u;
+                q = __fsub_rn(c_s, __uint_as_float(kid.w));
+                n1 = kid.z + 2u;
+                kx = kid.x;
+                ky = kid.y;
+            }
+            sc = __fadd_rn(q, __fdiv_rn(__fmul_rn(__fmul_rn(L.puct_c, p), sq), __uint2float_rn(n1)));
+            if (cand && sc != sc) cx.err = 4;
+        }
+        if (!__any_sync(FULL, cand)) continue;
+        const float red = azb_ord2f(__reduce_max_sync(FULL, cand ? azb_f2ord(sc) : 0u));
+        if (bj < 0 || red > best) {  // earlier chunks win ties
+            const int wl = __ffs(__ballot_sync(FULL, cand && sc == red)) - 1;
+            best = red;
+            bj = (int)base + wl;
+            by = __shfl_sync(FULL, pr.y, wl);
+            bw0 = __shfl_sync(FULL, kx, wl);
+            bw1 = __shfl_sync(FULL, ky, wl);
+        }
+    }
+    cx.err = __reduce_or_sync(FULL, cx.err);
+    if (cx.err) return -1;
+    if (bj < 0) {
+        cx.err = 6;
+        return -1;
+    }
+    if ((by >> 11) & 1u) {
+        w0 = bw0;
+        w1 = bw1;
+        return -1;
+    }
+    y = by;
+    return bj;
+}
+
 // `early(cx)` is called as soon as the step's new node is known to be non-terminal — BEFORE its cost is evaluated and the
 // node is inserted: the walker's state is final from that point on, so the asynchronous kernel hands the state vector to
 // the model there and the cost evaluation (~5 us) and the insert overlap the model's round trip.  The lock step passes a
@@ -485,7 +589,8 @@ __device__ __forceinline__ void step_done(const AzbLayout &L, WarpCtx &cx, uint3
 struct TreeNoEarly {
     __device__ __forceinline__ void operator()(WarpCtx &) const {}
 };
-template <int DEPTH, class Early = TreeNoEarly>
+// PUCT: AZB_SELECT_PUCT in place of next_action (azb.h); the default instantiations carry none of its code
+template <int DEPTH, bool PUCT = false, class Early = TreeNoEarly>
 __device__ void tree_rollout(const AzbLayout &L, WarpCtx &cx, uint32_t tree, uint32_t max_episodes, Early early = Early()) {
     const int lane = cx.lane;
     const uint32_t FULL = 0xffffffffu;
@@ -524,103 +629,109 @@ __device__ void tree_rollout(const AzbLayout &L, WarpCtx &cx, uint32_t tree, uin
         const uint32_t n_out = hd.y & 0xffffu, cnt = hd.y >> 16;
         count(cx, CT_SEL, 1);
         count(cx, CT_DSEL, n_out);
-        // ---- revisit_choice (next_action.rs:28-53): first minimum of (n_t, c*) over active children, newest first
-        unsigned long long best_key = ~0ull;
-        int best_t = -1;
-        uint32_t best_w0 = 0, best_w1 = 0;
-        for (uint32_t base = 0; base < n_out; base += 32) {
-            if (base) kd = cx.blk4[lo2 + 1u + base + lane];
-            const uint32_t t = base + lane;
-            bool act_t = false;
-            uint32_t oc = 0xffffffffu;
-            if (t < n_out) {
-                if (n_out > 32u) cx.lbuf[t] = __uint_as_float(kd.w);  // single-chunk nodes store only if curiosity runs
-                act_t = (kd.y >> 31) != 0u;
-                oc = azb_f2ord(__uint_as_float(kd.w));
-            }
-            const uint32_t ntmin = __reduce_min_sync(FULL, act_t ? kd.z : 0xffffffffu);
-            if (__any_sync(FULL, act_t)) {
-                const bool cand_t = act_t && kd.z == ntmin;
-                const uint32_t cmin = __reduce_min_sync(FULL, cand_t ? oc : 0xffffffffu);
-                const unsigned long long mk = ((unsigned long long)ntmin << 32) | cmin;
-                if (mk <= best_key) {  // a later chunk holds newer arcs: it wins ties
-                    const uint32_t bal = __ballot_sync(FULL, cand_t && oc == cmin);
-                    const int wl = 31 - __clz(bal);  // newest arc among equals
-                    best_key = mk;
-                    best_t = (int)base + wl;
-                    best_w0 = __shfl_sync(FULL, kd.x, wl);
-                    best_w1 = __shfl_sync(FULL, kd.y, wl);
-                }
-            }
-        }
-        __syncwarp();
-        PROF_ADD(cx, PH_SEL);
-        const bool have_r = best_t >= 0;
-        const uint32_t tol = depth < L.tol_len ? L.tol[depth] : L.tol_default;  // 04-c21-tree.rs:136-138
-        bool visit = have_r && (uint32_t)(best_key >> 32) < tol;               // next_action.rs:16-20
+        bool visit;
         int chosen_j = -1;
-        uint32_t chosen_y = 0;
-        if (!visit) {
-            // ---- max_curiosity (next_action.rs:55-88)
-            if (n_out <= 32u) {
-                if ((uint32_t)lane < n_out) cx.lbuf[lane] = __uint_as_float(kd.w);
-                __syncwarp();
-            }
-            count(cx, CT_CUR, 1);
-            count(cx, CT_CAND, cnt);
-#ifdef AZB_PROFILE
-            if (lane == 0) cx.ct[30] += cnt * n_out;
-#endif
-            const bool no_kids = n_out == 0;
-            uint32_t bk32 = 0u;
-            for (uint32_t base = 0; base < cnt; base += 32) {
-                if (base) pr = cx.blk[2u * lo2 - 1u - base - lane];
-                const uint32_t j = base + lane;
-                bool cand_j = false;
-                uint32_t ov = 0u;
-                if (j < cnt && ((pr.y >> 11) & 1u) == 0u) {  // no arc yet (:68-71)
-                    cand_j = true;
-                    const float v = __fsub_rn(c_s, __uint_as_float(pr.x));
-                    if (no_kids) {
-                        if (v != v) cx.err = 4;
-                        ov = azb_f2ord(v);
-                    } else {
-                        float cur = 0.f;
-#pragma unroll 2
-                        for (int t = (int)n_out - 1; t >= 0; --t)  // newest first, left fold (:79-82)
-                            cur = __fadd_rn(cur, __fsqrt_rn(fabsf(__fsub_rn(cx.lbuf[t], v))));
-                        if (cur != cur) cx.err = 4;
-                        ov = azb_f2ord(cur);
-                    }
-                }
-                if (!__any_sync(FULL, cand_j)) continue;
-                if (no_kids) {  // first minimum (:73-75): earlier chunks win ties
-                    const uint32_t red = __reduce_min_sync(FULL, cand_j ? ov : 0xffffffffu);
-                    if (chosen_j < 0 || red < bk32) {
-                        bk32 = red;
-                        const int wl = __ffs(__ballot_sync(FULL, cand_j && ov == red)) - 1;
-                        chosen_j = (int)base + wl;
-                        chosen_y = __shfl_sync(FULL, pr.y, wl);
-                    }
-                } else {  // last maximum (:85): later chunks win ties
-                    const uint32_t red = __reduce_max_sync(FULL, cand_j ? ov : 0u);
-                    if (chosen_j < 0 || red >= bk32) {
-                        bk32 = red;
-                        const int wl = 31 - __clz(__ballot_sync(FULL, cand_j && ov == red));
-                        chosen_j = (int)base + wl;
-                        chosen_y = __shfl_sync(FULL, pr.y, wl);
-                    }
-                }
-            }
-            cx.err = __reduce_or_sync(FULL, cx.err);
-            PROF_ADD(cx, PH_CUR);
+        uint32_t chosen_y = 0, best_w0 = 0, best_w1 = 0;
+        if constexpr (PUCT) {  // AZB_SELECT_PUCT: a kernel instantiation of its own
+            chosen_j = puct_select(L, cx, lo2, c_s, n_out, cnt, kd, pr, best_w0, best_w1, chosen_y);
             if (cx.err) break;
-            if (chosen_j < 0) {
-                if (have_r)
-                    visit = true;  // next_action.rs:24
-                else {
-                    cx.err = 6;
-                    break;
+            visit = chosen_j < 0;
+        } else {
+            // ---- revisit_choice (next_action.rs:28-53): first minimum of (n_t, c*) over active children, newest first
+            unsigned long long best_key = ~0ull;
+            int best_t = -1;
+            for (uint32_t base = 0; base < n_out; base += 32) {
+                if (base) kd = cx.blk4[lo2 + 1u + base + lane];
+                const uint32_t t = base + lane;
+                bool act_t = false;
+                uint32_t oc = 0xffffffffu;
+                if (t < n_out) {
+                    if (n_out > 32u) cx.lbuf[t] = __uint_as_float(kd.w);  // single-chunk nodes store only if curiosity runs
+                    act_t = (kd.y >> 31) != 0u;
+                    oc = azb_f2ord(__uint_as_float(kd.w));
+                }
+                const uint32_t ntmin = __reduce_min_sync(FULL, act_t ? kd.z : 0xffffffffu);
+                if (__any_sync(FULL, act_t)) {
+                    const bool cand_t = act_t && kd.z == ntmin;
+                    const uint32_t cmin = __reduce_min_sync(FULL, cand_t ? oc : 0xffffffffu);
+                    const unsigned long long mk = ((unsigned long long)ntmin << 32) | cmin;
+                    if (mk <= best_key) {  // a later chunk holds newer arcs: it wins ties
+                        const uint32_t bal = __ballot_sync(FULL, cand_t && oc == cmin);
+                        const int wl = 31 - __clz(bal);  // newest arc among equals
+                        best_key = mk;
+                        best_t = (int)base + wl;
+                        best_w0 = __shfl_sync(FULL, kd.x, wl);
+                        best_w1 = __shfl_sync(FULL, kd.y, wl);
+                    }
+                }
+            }
+            __syncwarp();
+            PROF_ADD(cx, PH_SEL);
+            const bool have_r = best_t >= 0;
+            const uint32_t tol = depth < L.tol_len ? L.tol[depth] : L.tol_default;  // 04-c21-tree.rs:136-138
+            visit = have_r && (uint32_t)(best_key >> 32) < tol;                    // next_action.rs:16-20
+            if (!visit) {
+                // ---- max_curiosity (next_action.rs:55-88)
+                if (n_out <= 32u) {
+                    if ((uint32_t)lane < n_out) cx.lbuf[lane] = __uint_as_float(kd.w);
+                    __syncwarp();
+                }
+                count(cx, CT_CUR, 1);
+                count(cx, CT_CAND, cnt);
+    #ifdef AZB_PROFILE
+                if (lane == 0) cx.ct[30] += cnt * n_out;
+    #endif
+                const bool no_kids = n_out == 0;
+                uint32_t bk32 = 0u;
+                for (uint32_t base = 0; base < cnt; base += 32) {
+                    if (base) pr = cx.blk[2u * lo2 - 1u - base - lane];
+                    const uint32_t j = base + lane;
+                    bool cand_j = false;
+                    uint32_t ov = 0u;
+                    if (j < cnt && ((pr.y >> 11) & 1u) == 0u) {  // no arc yet (:68-71)
+                        cand_j = true;
+                        const float v = __fsub_rn(c_s, __uint_as_float(pr.x));
+                        if (no_kids) {
+                            if (v != v) cx.err = 4;
+                            ov = azb_f2ord(v);
+                        } else {
+                            float cur = 0.f;
+    #pragma unroll 2
+                            for (int t = (int)n_out - 1; t >= 0; --t)  // newest first, left fold (:79-82)
+                                cur = __fadd_rn(cur, __fsqrt_rn(fabsf(__fsub_rn(cx.lbuf[t], v))));
+                            if (cur != cur) cx.err = 4;
+                            ov = azb_f2ord(cur);
+                        }
+                    }
+                    if (!__any_sync(FULL, cand_j)) continue;
+                    if (no_kids) {  // first minimum (:73-75): earlier chunks win ties
+                        const uint32_t red = __reduce_min_sync(FULL, cand_j ? ov : 0xffffffffu);
+                        if (chosen_j < 0 || red < bk32) {
+                            bk32 = red;
+                            const int wl = __ffs(__ballot_sync(FULL, cand_j && ov == red)) - 1;
+                            chosen_j = (int)base + wl;
+                            chosen_y = __shfl_sync(FULL, pr.y, wl);
+                        }
+                    } else {  // last maximum (:85): later chunks win ties
+                        const uint32_t red = __reduce_max_sync(FULL, cand_j ? ov : 0u);
+                        if (chosen_j < 0 || red >= bk32) {
+                            bk32 = red;
+                            const int wl = 31 - __clz(__ballot_sync(FULL, cand_j && ov == red));
+                            chosen_j = (int)base + wl;
+                            chosen_y = __shfl_sync(FULL, pr.y, wl);
+                        }
+                    }
+                }
+                cx.err = __reduce_or_sync(FULL, cx.err);
+                PROF_ADD(cx, PH_CUR);
+                if (cx.err) break;
+                if (chosen_j < 0) {
+                    if (have_r)
+                        visit = true;  // next_action.rs:24
+                    else {
+                        cx.err = 6;
+                        break;
+                    }
                 }
             }
         }
@@ -859,7 +970,7 @@ __device__ __forceinline__ void tree_pack(const AzbLayout &L, WarpCtx &cx, uint3
 #ifndef AZB_TREE_MIN_BLOCKS
 #define AZB_TREE_MIN_BLOCKS 7
 #endif
-template <int DEPTH, bool COUNT>
+template <int DEPTH, bool COUNT, bool PUCT = false>  // PUCT: azb_config.selection == AZB_SELECT_PUCT
 __global__ void __launch_bounds__(AZB_WARPS_PER_BLOCK * 32, AZB_TREE_MIN_BLOCKS)
     azb_tree_kernel(const AzbLayout L, const uint32_t flags, const uint32_t smem_words_per_warp, const uint32_t lcap,
                     const uint32_t target_step, const uint32_t max_episodes, const uint32_t tree0,
@@ -943,7 +1054,7 @@ __global__ void __launch_bounds__(AZB_WARPS_PER_BLOCK * 32, AZB_TREE_MIN_BLOCKS)
             if ((flags & AZB_F_ADD) && (cx.wk[WK_FLAGS] & 1u)) tree_add_actions<DEPTH == 5>(L, cx, tree);
             PROF_ADD(cx, PH_ADD);
             if ((flags & AZB_F_ROLLOUT) && cx.err == 0 && cx.wk[WK_STEP] < target_step && !(cx.wk[WK_FLAGS] & 1u)) {
-                tree_rollout<DEPTH>(L, cx, tree, max_episodes);
+                tree_rollout<DEPTH, PUCT>(L, cx, tree, max_episodes);
 #ifdef AZB_PROFILE
                 prof_t0 = clock64();
 #endif

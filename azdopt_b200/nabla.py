@@ -78,9 +78,12 @@ class NablaOptimizer:
     @classmethod
     def par_new(cls, space: ROTModifyParentsOnce, init_states, model, batch: int, *, n_as_tol=(200, 50, 50),
                 n_as_tol_default=25, device: int = 0, first_root: int = 0, max_steps: int = 800,
-                async_workers: Optional[int] = None) -> "NablaOptimizer":
+                async_workers: Optional[int] = None, selection: int = capi.SELECT_REFERENCE,
+                puct_c: float = 1.0) -> "NablaOptimizer":
         """optimizer/mod.rs:39-118.  ``init_states`` is either ``(parents[B,N] u8, permitted[B,W] u32)`` or a callable
-        ``i -> (parents[N], iterable of permitted action ids)`` (the reference's closure draws from thread_rng)."""
+        ``i -> (parents[N], iterable of permitted action ids)`` (the reference's closure draws from thread_rng).
+        ``selection=capi.SELECT_PUCT`` replaces the reference's next_action with PUCT at constant ``puct_c``
+        (include/azb.h; a rule of this library with no reference to check it against)."""
         self = object.__new__(cls)
         self.space, self.model, self.batch = space, model, batch
         self._tol = (tuple(n_as_tol), n_as_tol_default)
@@ -95,7 +98,7 @@ class NablaOptimizer:
         cfg = capi.default_config(space.n, batch, device=device, first_root=first_root, c_lower=space.c_lower,
                                   c_upper=space.c_upper, n_as_tol=n_as_tol, n_as_tol_default=n_as_tol_default,
                                   prior_mode=prior, mlp_mode=mlp, mlp_hidden=hidden, max_steps=max_steps,
-                                  async_workers=async_workers)
+                                  async_workers=async_workers, selection=selection, puct_c=puct_c)
         self.h = capi.Handle(cfg)
         if isinstance(model, ActionModel):
             if model.params is not None:

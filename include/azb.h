@@ -65,6 +65,29 @@ enum {
                              reference runs (nabla/model/dfdx.rs:69-84), at about three times the tensor work */
 };
 
+/* selection rule at an active node (azb_config.selection) */
+enum {
+    AZB_SELECT_REFERENCE = 0, /* next_action (next_action.rs:11-26): revisit_choice under n_as_tol, else max_curiosity */
+    AZB_SELECT_PUCT = 1       /* AlphaZero-style PUCT argmax; defined here, it has NO reference to be checked against */
+};
+/* AZB_SELECT_PUCT replaces next_action at an active node s; everything after the choice (Visited -> descend,
+ * Unvisited(j) -> probe, transposition, insert, cost, cascades, n_t, c*, argmin) is unchanged and n_as_tol is not
+ * consulted.  Every operation is f32, round-to-nearest, in the order written, nothing fused.  c_s = the node's c; kids
+ * k in creation order with action a_k, active_k, n_k (the child's n_t) and c*_k; predictions j = 0..cnt-1 in the node's
+ * prediction order with a_j, g_j = c_s - h_j and has_arc_j.
+ *   1. N_s = 1 + sum_k (n_k + 1) over all kids, active or not (an exact integer; AZB_ERR_CAPACITY at 2^24);
+ *      sq = sqrt((float)N_s).
+ *   2. w_j = (1 - c_s) + g_j, or +0 where that is negative (the model's predicted goodness 1 - h_j, up to rounding).
+ *   3. Z = sum_j w_j: each chunk of 32 predictions is summed as a warp's xor butterfly does it (lane i holds
+ *      w_{32c+i} or +0 beyond cnt; for m = 16, 8, 4, 2, 1: x[i] = x[i] + x[i^m]; the chunk sum is x[0]), then the
+ *      chunk sums are folded left to right starting from chunk 0's.  p_j = w_j / Z, or 1 / cnt when Z == 0.
+ *   4. A prediction without an arc has n = 0, q = g_j.  One with an arc to kid k (a_k == a_j) is skipped if the kid is
+ *      inactive, else n = n_k + 1, q = c_s - c*_k.
+ *   5. score_j = q + ((puct_c * p_j) * sq) / (float)(1 + n).
+ *   6. The first maximum of score_j in ascending j wins: Visited(k) if it has an arc, else Unvisited(j).  A NaN score
+ *      is AZB_ERR_NAN; no candidate at an active node is AZB_ERR_UNREACHABLE.
+ * Counters per selection: n_sel += 1, d_sel += kids, n_cur += 1, n_cand += cnt (n_visit as in the reference mode). */
+
 typedef struct azb_config {
     uint32_t struct_size;       /* sizeof(azb_config), for ABI growth */
     uint32_t n_vertices;        /* N, 5..64                                (04-c21-tree.rs:33) */
@@ -103,7 +126,9 @@ typedef struct azb_config {
                                    CTAs as CTA pairs of one cluster: tcgen05.mma.cta_group::2, even async_workers),
                                    AZB_ASYNC_STEAL=0/1 (tree scheduling inside a CTA), AZB_ASYNC_FLUSH_NS,
                                    AZB_ASYNC_TIMEOUT_MS (watchdog floor, default 2000). */
-    uint32_t reserved[5];
+    uint32_t selection;         /* AZB_SELECT_*; 0 = the reference's next_action */
+    float puct_c;               /* c_puct of AZB_SELECT_PUCT (finite, > 0; azb_config_default: 1); unused otherwise */
+    uint32_t reserved[3];
 } azb_config;
 
 typedef struct azb_counters {   /* workload counters; definitions in oracle/azb_oracle.h and DESIGN.md */

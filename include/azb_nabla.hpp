@@ -43,6 +43,13 @@ struct TrivialModel : NablaModel {
     void write_predictions(const std::vector<float> &, std::vector<float> &) override {}
 };
 
+// PUCT selection (azb.h AZB_SELECT_PUCT) on a config before par_new; the reference's next_action stays the default
+inline azb_config &with_puct(azb_config &cfg, float c_puct = 1.0f) {
+    cfg.selection = AZB_SELECT_PUCT;
+    cfg.puct_c = c_puct;
+    return cfg;
+}
+
 class NablaOptimizer {
    public:
     // par_new (optimizer/mod.rs:39-118).  model == nullptr selects the built-in device MLP (ActionModel,

@@ -53,6 +53,16 @@ pub enum Model<M> {
     Device { params: Vec<f32>, tensor_cores: bool },
 }
 
+/// The selection rule at an active node (`azb_config.selection`).
+#[derive(Clone, Copy, Debug, PartialEq)]
+pub enum Selection {
+    /// the reference's `next_action` (`nabla/tree/next_action.rs:11-26`)
+    Reference,
+    /// PUCT with constant `c_puct` (finite, > 0); the rule is this library's own (`include/azb.h`) and has no
+    /// reference to check it against
+    Puct { c_puct: f32 },
+}
+
 /// The only two things the example's `modify_root` reads from a `StateWeight` (whose constructor is `pub(crate)`):
 /// `c()` and `c_star()` (`nabla/tree/state_weight.rs:23-29`).
 #[derive(Clone, Copy, Debug)]
@@ -167,6 +177,19 @@ impl<const N: usize, M: NablaModel> B200Optimizer<N, M> {
         n_as_tol: impl Fn(usize) -> u32,
         max_steps_per_epoch: u32,
     ) -> Self {
+        Self::par_new_with_selection(space, init_states, model, batch, n_as_tol, max_steps_per_epoch, Selection::Reference)
+    }
+
+    /// `par_new` with a choice of selection rule (`Selection::Reference` is `par_new`).
+    pub fn par_new_with_selection(
+        space: Space<N>,
+        init_states: impl Fn() -> State<N> + Sync + Send,
+        model: Model<M>,
+        batch: usize,
+        n_as_tol: impl Fn(usize) -> u32,
+        max_steps_per_epoch: u32,
+        selection: Selection,
+    ) -> Self {
         assert!(N >= 5 && N <= sys::AZB_MAX_VERTICES as usize && batch > 0);
         let mut cfg: sys::azb_config = unsafe { std::mem::zeroed() };
         ck(std::ptr::null(), unsafe { sys::azb_config_default(&mut cfg, N as u32, batch as u32) });
@@ -179,6 +202,10 @@ impl<const N: usize, M: NablaModel> B200Optimizer<N, M> {
         cfg.n_as_tol_len = 8;
         cfg.n_as_tol_default = table[8];
         cfg.max_steps = max_steps_per_epoch;
+        if let Selection::Puct { c_puct } = selection {
+            cfg.selection = sys::AZB_SELECT_PUCT;
+            cfg.puct_c = c_puct;
+        }
         let (host_model, params) = match model {
             Model::Host(m) => {
                 cfg.prior_mode = sys::AZB_PRIOR_INJECTED;

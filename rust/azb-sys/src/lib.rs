@@ -26,6 +26,9 @@ pub const AZB_MLP_FP32: u32 = 0;
 pub const AZB_MLP_TC: u32 = 1;
 pub const AZB_MLP_TC3: u32 = 2;
 
+pub const AZB_SELECT_REFERENCE: u32 = 0;
+pub const AZB_SELECT_PUCT: u32 = 1;
+
 #[repr(C)]
 #[derive(Clone, Copy, Debug)]
 pub struct azb_config {
@@ -50,7 +53,9 @@ pub struct azb_config {
     pub max_episodes: u32,
     pub n_groups: u32,
     pub async_workers: u32,
-    pub reserved: [u32; 5],
+    pub selection: u32,
+    pub puct_c: f32,
+    pub reserved: [u32; 3],
 }
 
 #[repr(C)]
