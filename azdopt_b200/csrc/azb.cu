@@ -25,7 +25,6 @@
 #include "azb_tree.cuh"
 #include "azb_train.cuh"
 #include "azb_async.cuh"
-#include <unistd.h>
 
 #include <dlfcn.h>
 
@@ -702,15 +701,12 @@ static int read_globals(azb_handle *h, AzbGlobals *g) {
         CK(cudaMallocHost((void **)&h->pin_abort, 16));
     }
     CK(cudaMemcpyAsync(h->pin_rg, h->L.g, offsetof(AzbGlobals, argmin_state), cudaMemcpyDeviceToHost, h->stream));
-    h->pin_abort[0] = h->pin_abort[1] = 0u;
-    if (h->async_ran) CK(cudaMemcpyAsync(h->pin_abort, &h->asP.st->abort, 8, cudaMemcpyDeviceToHost, h->stream));  // abort, stuck
+    h->pin_abort[0] = 0u;
+    if (h->async_ran) CK(cudaMemcpyAsync(h->pin_abort, &h->asP.st->abort, 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     memcpy(g, h->pin_rg, offsetof(AzbGlobals, argmin_state));
     const uint32_t as_abort = h->pin_abort[0];
     h->async_ran = false;
-    if (as_abort == 1u && h->pin_abort[1])
-        return fail(h, AZB_ERR_CUDA, "async search kernel: watchdog expired (barrier wait %u of CTA %u never completed)", h->pin_abort[1] >> 16,
-                    h->pin_abort[1] & 0xffffu);
     if (as_abort == 1u) return fail(h, AZB_ERR_CUDA, "async search kernel: watchdog expired (no progress)");
     if (g->err)
         return fail(h, (int)g->err, "%s (tree %u, step %u)", azb_strerror((int)g->err), g->err_tree, g->err_step);
@@ -797,17 +793,15 @@ int azb_init_trees(azb_handle *h) {
 }  // extern "C"
 
 // ---- the asynchronous search kernel (azb_async.cuh): set-up and launch -------------------------------------------
-template <int D, bool C, bool PAIR, bool PUCT>
+template <int D, bool C, bool PUCT>
 static int async_prepare_one(azb_handle *h, int *blocks_per_sm) {
-    CK(cudaFuncSetAttribute(azb_async_kernel<D, C, PAIR, PUCT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->async_smem));
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, azb_async_kernel<D, C, PAIR, PUCT>, AS_THREADS, h->async_smem));
+    CK(cudaFuncSetAttribute(azb_async_kernel<D, C, PUCT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->async_smem));
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, azb_async_kernel<D, C, PUCT>, AS_THREADS, h->async_smem));
     return AZB_OK;
 }
 template <int D, bool C>
-static int async_prepare_kernel(azb_handle *h, int *blocks_per_sm, bool pair) {
-    if (h->cfg.selection == AZB_SELECT_PUCT)
-        return pair ? async_prepare_one<D, C, true, true>(h, blocks_per_sm) : async_prepare_one<D, C, false, true>(h, blocks_per_sm);
-    return pair ? async_prepare_one<D, C, true, false>(h, blocks_per_sm) : async_prepare_one<D, C, false, false>(h, blocks_per_sm);
+static int async_prepare_kernel(azb_handle *h, int *blocks_per_sm) {
+    return h->cfg.selection == AZB_SELECT_PUCT ? async_prepare_one<D, C, true>(h, blocks_per_sm) : async_prepare_one<D, C, false>(h, blocks_per_sm);
 }
 
 static int async_create(azb_handle *h) {
@@ -828,10 +822,6 @@ static int async_create(azb_handle *h) {
     if (shared_sm && azb_stack_depth(h->N) == 5)
         return fail(h, AZB_ERR_INVALID, "AZB_ASYNC_SHARED needs N <= 46 (larger trees take the whole SM's shared memory)");
     uint32_t group = shared_sm ? 8u : (B < 4096 ? 2u : 1u);  // pairs answer a tile faster; from 4096 roots on the model's throughput matters more
-    // CTA pairs (azb_async.cuh): two model CTAs of one cluster answer two tiles with one weight stream (cta_group::2)
-    bool pair = false;
-    if (const char *e = getenv("AZB_ASYNC_PAIR")) pair = atoi(e) != 0;
-    if (pair && !shared_sm) group = 1u;
     if (const char *e = getenv("AZB_ASYNC_GROUP")) group = (uint32_t)strtoul(e, nullptr, 10);
     if (group == 0) return fail(h, AZB_ERR_INVALID, "AZB_ASYNC_GROUP must be positive");
     if (shared_sm) W = 0;
@@ -839,7 +829,6 @@ static int async_create(azb_handle *h) {
     const size_t lut_bytes = azb_tables_bytes(h->A, h->N, h->W), per_warp = (size_t)h->smem_words_per_warp * 4;
     uint32_t tree_warps = (uint32_t)std::max<size_t>(4, std::min<size_t>(AS_WARPS, (160 * 1024 - lut_bytes) / per_warp));
     if (azb_stack_depth(h->N) == 5) tree_warps = std::min<uint32_t>(tree_warps, AS_WIDE_TREE_WARPS);  // see azb_async_kernel
-    if (const char *e = getenv("AZB_ASYNC_TREE_WARPS")) tree_warps = std::min<uint32_t>(tree_warps, std::max(1, atoi(e)));
     if (shared_sm) tree_warps = SH_TREE_WARPS;
     // a tree CTA's scheduling table (azb_async.cuh): one entry per tree it owns
     const uint32_t n_tree_ctas_est = (uint32_t)prop.multiProcessorCount - (shared_sm ? 0u : W);
@@ -868,13 +857,11 @@ static int async_create(azb_handle *h) {
         while (sh_stages > 2u && need(sh_stages) > (size_t)prop.sharedMemPerBlockOptin - 2048) --sh_stages;
         h->async_smem = need(sh_stages);
     }
-    if (const char *e = getenv("AZB_ASYNC_SMEM_PAD_KB"))  // experiment: shrink the L1 the walkers see
-        h->async_smem = std::min<size_t>(224 * 1024, h->async_smem + (size_t)atoi(e) * 1024);
     int nb = 0, nb2 = 0, rc;
     switch (azb_stack_depth(h->N)) {
-        case 3: rc = async_prepare_kernel<3, false>(h, &nb, pair); if (!rc) rc = async_prepare_kernel<3, true>(h, &nb2, pair); break;
-        case 4: rc = async_prepare_kernel<4, false>(h, &nb, pair); if (!rc) rc = async_prepare_kernel<4, true>(h, &nb2, pair); break;
-        default: rc = async_prepare_kernel<5, false>(h, &nb, pair); if (!rc) rc = async_prepare_kernel<5, true>(h, &nb2, pair); break;
+        case 3: rc = async_prepare_kernel<3, false>(h, &nb); if (!rc) rc = async_prepare_kernel<3, true>(h, &nb2); break;
+        case 4: rc = async_prepare_kernel<4, false>(h, &nb); if (!rc) rc = async_prepare_kernel<4, true>(h, &nb2); break;
+        default: rc = async_prepare_kernel<5, false>(h, &nb); if (!rc) rc = async_prepare_kernel<5, true>(h, &nb2); break;
     }
     if (rc) return rc;
     nb = std::min(nb, nb2);
@@ -902,19 +889,10 @@ static int async_create(azb_handle *h) {
     // free warps take over any runnable tree of their CTA
     P.steal = (B > 2u * NW || (azb_stack_depth(h->N) == 5 && B > NW)) ? 1u : 0u;
     if (const char *e = getenv("AZB_ASYNC_STEAL")) P.steal = atoi(e) != 0;
-    P.early = P.steal ? 0u : 1u;  // the tree's own latency chain is the bound: hand the state vector over before the cost evaluation
-    if (const char *e = getenv("AZB_ASYNC_EARLY")) P.early = atoi(e) != 0;
-    P.sweep_gap = AS_SWEEP_GAP;
-    if (const char *e = getenv("AZB_ASYNC_SWEEP_GAP")) P.sweep_gap = (uint32_t)strtoul(e, nullptr, 10);
     // worker SMs per tile
     P.group = group;
     if (W % P.group) return fail(h, AZB_ERR_INVALID, "async_workers must be a multiple of the group size %u", P.group);
     if (n_model_groups > AS_MAX_GROUPS) return fail(h, AZB_ERR_INVALID, "more than %u model groups", (unsigned)AS_MAX_GROUPS);
-    if (pair) {
-        if (shared_sm || group != 1u || (W & 1u) || (h->async_grid & 1) || nb != 1)
-            return fail(h, AZB_ERR_INVALID, "CTA pairs need whole model SMs, an even async_workers, group 1 and an even grid");
-        P.pair = 1u;
-    }
     P.smem_words_per_warp = h->smem_words_per_warp;
     P.wide = h->tc.split ? 2u : 1u;
     P.ring_ld = P.wide * h->tc.kpad[0];
@@ -922,12 +900,7 @@ static int async_create(azb_handle *h) {
     if (const char *e = getenv("AZB_ASYNC_TIMEOUT_MS")) h->async_timeout_base_ns = strtoull(e, nullptr, 10) * 1000000ull;
     P.timeout_ns = h->async_timeout_base_ns;
     P.flush_ns = 4000ull;
-    P.nap_count = 6;
-    P.nap_long_ns = 5000;
-    P.nap_short_ns = 1000;
-    if (const char *e = getenv("AZB_ASYNC_NAPS")) sscanf(e, "%u,%u,%u", &P.nap_count, &P.nap_long_ns, &P.nap_short_ns);
     if (const char *e = getenv("AZB_ASYNC_FLUSH_NS")) P.flush_ns = strtoull(e, nullptr, 10);
-    if (const char *e = getenv("AZB_ASYNC_DBG")) P.dbg_flags = (uint32_t)strtoul(e, nullptr, 10);
     for (int l = 0; l < 4; ++l) {
         P.kpad[l] = h->tc.kpad[l];
         P.npad[l] = h->tc.npad[l];
@@ -948,7 +921,7 @@ static int async_create(azb_handle *h) {
         auto up = [](size_t x) { return (x + 255) & ~(size_t)255; };
         const size_t o_cnt = up(sizeof(AzbAsyncState)), o_ret = o_cnt + up((size_t)P.NT * 4), o_flag = o_ret + up((size_t)P.NT * 4),
                      o_dbg = o_flag + up((size_t)B * 4);
-        h->async_zero_bytes = o_dbg + 64 * 8;
+        h->async_zero_bytes = o_dbg + 32 * 8;
         uint8_t *slab = nullptr;
         CK(alloc((void **)&slab, h->async_zero_bytes));
         P.st = reinterpret_cast<AzbAsyncState *>(slab);
@@ -981,24 +954,7 @@ static int async_create(azb_handle *h) {
 template <int D, bool C, bool PUCT>
 static cudaError_t async_launch_sel(azb_handle *h) {
     void *args[] = {(void *)&h->L, (void *)&h->asP, (void *)&h->asM};
-    if (h->asP.pair) {  // cooperative AND clustered: CTAs 2c and 2c + 1 land on the two SMs of one TPC
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(h->async_grid);
-        cfg.blockDim = dim3(AS_THREADS);
-        cfg.dynamicSmemBytes = h->async_smem;
-        cfg.stream = h->stream;
-        cudaLaunchAttribute at[2];
-        at[0].id = cudaLaunchAttributeCooperative;
-        at[0].val.cooperative = 1;
-        at[1].id = cudaLaunchAttributeClusterDimension;
-        at[1].val.clusterDim.x = 2;
-        at[1].val.clusterDim.y = 1;
-        at[1].val.clusterDim.z = 1;
-        cfg.attrs = at;
-        cfg.numAttrs = 2;
-        return cudaLaunchKernelExC(&cfg, (const void *)azb_async_kernel<D, C, true, PUCT>, args);
-    }
-    return cudaLaunchCooperativeKernel((const void *)azb_async_kernel<D, C, false, PUCT>, dim3(h->async_grid), dim3(AS_THREADS), args,
+    return cudaLaunchCooperativeKernel((const void *)azb_async_kernel<D, C, PUCT>, dim3(h->async_grid), dim3(AS_THREADS), args,
                                        h->async_smem, h->stream);
 }
 template <int D, bool C>
@@ -1027,25 +983,6 @@ static int run_async(azb_handle *h, uint32_t n_steps) {
         default: ce = async_launch<5, true>(h); break;
     }
     if (ce != cudaSuccess) return fail(h, AZB_ERR_CUDA, "async kernel launch: %s", cudaGetErrorString(ce));
-    if (getenv("AZB_ASYNC_PEEK")) {  // debugging aid: a launch that does not end within 15 s gets its progress markers printed
-        for (int i = 0; i < 1500 && cudaStreamQuery(h->stream) == cudaErrorNotReady; ++i) usleep(10000);
-        if (cudaStreamQuery(h->stream) == cudaErrorNotReady) {
-            cudaStream_t s2;
-            cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking);
-            unsigned long long d[64];
-            AzbAsyncState *st = (AzbAsyncState *)malloc(sizeof(AzbAsyncState));
-            cudaMemcpyAsync(d, P.dbg, sizeof(d), cudaMemcpyDeviceToHost, s2);
-            cudaMemcpyAsync(st, P.st, sizeof(AzbAsyncState), cudaMemcpyDeviceToHost, s2);
-            cudaError_t e2 = cudaStreamSynchronize(s2);
-            fprintf(stderr, "AZB_ASYNC_PEEK: kernel still running (%s); abort %u stuck %x row_tail %u tile_head %u tiles_done %u done_trees %u\n",
-                    cudaGetErrorString(e2), st->abort, st->stuck, st->row_tail, st->tile_head, st->tiles_done, st->done_trees);
-            for (int w = 0; w < 4; ++w)
-                fprintf(stderr, "  worker %d: producer %llx mma %llx epilogue %llx cta %llx\n", w, d[32 + w * 8], d[32 + w * 8 + 1], d[32 + w * 8 + 2],
-                        d[32 + w * 8 + 7]);
-            fflush(stderr);
-            _exit(3);
-        }
-    }
     h->launches += 1;
     h->async_ran = true;
     // (the rows of the last step are answered inside the kernel too: no batched forward behind it)
@@ -1071,7 +1008,7 @@ static int enqueue_steps(azb_handle *h, uint32_t n_steps, uint32_t flags) {
     const uint32_t target = h->steps_done + n_steps;
     if (h->cfg.async_workers && n_steps >= 2 && flags == (AZB_F_ADD | AZB_F_ROLLOUT)) return run_async(h, n_steps);
     if (h->cfg.prior_mode == AZB_PRIOR_HASH && h->cfg.max_episodes == 0 && h->n_groups <= 1 && n_steps >= 2 &&
-        flags == (AZB_F_ADD | AZB_F_ROLLOUT) && !getenv("AZB_HASH_LOCKSTEP")) {
+        flags == (AZB_F_ADD | AZB_F_ROLLOUT)) {
         // counter-hash priors need no model call, so nothing ties the trees together: ONE launch in which every warp takes
         // its tree through all n_steps steps (per-tree step clocks and cand[step][tree] as in the asynchronous kernel)
         int rc = launch_tree(h, flags | AZB_F_MULTI, target);

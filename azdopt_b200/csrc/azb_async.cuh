@@ -26,8 +26,6 @@
 // pass does not depend on which tile it rides in (same K order per dot product).  Per-tree step clocks and the
 // cand[step][tree] table (DESIGN.md §4.1) make the argmin pass indifferent to the interleaving.
 // Every spin loop has a watchdog on %globaltimer; on expiry the kernel sets `abort` and drains.
-// AZB_ASYNC_PAIR=1 selects the CTA-PAIR form of the model CTAs (template parameter PAIR, launched in clusters of two):
-// two CTAs of one TPC answer two tiles with ONE tcgen05.mma.cta_group::2 stream, see "CTA pairs" below.
 //
 // Round 1 also had a two-kernel form (tree kernel + model kernel on two streams, spinning on each other) and a
 // weight-stationary model pipeline kernel.  Both are gone: separately launched kernels that wait for each other are
@@ -57,35 +55,25 @@
 #define AS_ACC 2          // 128-column blocks per pass (one N = 256 MMA per k-step).  The 512 TMEM columns hold TWO passes:
                           // the epilogue drains one while the MMAs of the next run (4-block passes filled TMEM and
                           // serialised the two: MMA 24 us + epilogue 25 us per tile)
-#define AS_SWEEP_GAP 1000u  // cycles between two sweeps of a tree CTA's answer flags
+#define AS_SWEEP_GAP 1000u  // cycles between two sweeps of a tree CTA's answer flags (steal)
+// a warp whose own trees all wait for their priors (no steal): AS_NAP_COUNT sleeps of AS_NAP_LONG_NS, then AS_NAP_SHORT_NS
+// between polls; a warp without the sweep token (steal) naps AS_NAP_LONG_NS
+#define AS_NAP_COUNT 6u
+#define AS_NAP_LONG_NS 5000u
+#define AS_NAP_SHORT_NS 1000u
 #define AS_TILE 128
 #define AS_NONE 0xffffffffu
 #define AS_MAX_GROUPS 128
-// one acquire load of a flag after the relaxed polls have seen it (PTX memory model: what the flag guards is read or
-// overwritten afterwards).  It costs one L1 invalidation (CCTL.IVALL) per tree-step; -DAS_ACQUIRE=0 measures without.
-#ifndef AS_ACQUIRE
-#define AS_ACQUIRE 1
-#endif
 // cycle counters of the workers (tools/async_probe.py): only in the -DAZB_PROFILE flavour
 #ifdef AZB_PROFILE
 #define AS_CLK() clock64()
-#define AS_DBG(bit) ((P.dbg_flags & (bit)) != 0u)  // timing experiments (AZB_ASYNC_DBG): profile flavour only
 #else
 #define AS_CLK() 0ll
-#define AS_DBG(bit) false
-#endif
-
-// progress markers of the model CTAs (-DAS_MARKS; AZB_ASYNC_PEEK=1 prints them from the host while the kernel runs)
-#ifdef AS_MARKS
-#define AS_MARK(worker, role, v) do { if ((threadIdx.x & 31) == 0 && (worker) < 4u) *reinterpret_cast<volatile unsigned long long *>(P.dbg + 32 + (worker) * 8 + (role)) = (unsigned long long)(v); } while (0)
-#else
-#define AS_MARK(worker, role, v) do { } while (0)
 #endif
 
 struct AzbAsyncState {  // device memory, zeroed before every launch
     uint32_t abort;       // 1 watchdog, 2 tree error.  Polled by every waiting warp: alone in its 128-byte line, away
-    uint32_t stuck;       // from the counters the atomics below keep invalidating.  stuck: the first barrier wait that
-    uint32_t pad0[30];    // expired (code << 16 | CTA), 0 = none
+    uint32_t pad0[31];    // from the counters the atomics below keep invalidating
     uint32_t sm_flag[1024];  // first CTA to arrive on each SM (indexed by %smid)
     uint32_t mlp_claims, tree_claims;
     uint32_t row_tail;    // ring slots handed out
@@ -124,16 +112,12 @@ struct AzbAsyncParams {
     uint32_t tree_warps;     // tree warps per CTA (32 unless the per-warp shared memory of a large N does not fit)
     uint32_t tab_slots;      // entries of a tree CTA's scheduling table: the most trees any CTA owns
     uint32_t steal;          // 1: a free warp advances ANY runnable tree of its CTA (more trees than warps); 0: only its own
-    uint32_t sweep_gap;      // cycles between two sweeps of a tree CTA's answer flags (steal)
-    uint32_t early;          // 1: the state vector is handed to the model from inside the walk (before the cost evaluation)
-    uint32_t nap_count, nap_long_ns, nap_short_ns;  // a warp whose trees all wait: that many long sleeps, then short ones between polls
-    uint32_t pair;           // 1: model CTAs work as CTA pairs of one cluster (tcgen05.mma.cta_group::2): two 128-row tiles share every weight tile
+                             // (and hands the state vector to the model from inside the walk, before the cost evaluation)
     uint32_t shared_sm;      // 1: shared-SM form — every CTA walks trees with 28 warps and serves the model with its last warpgroup
     uint32_t sh_stages;      // shared-SM form: stages of a member's operand ring
     uint32_t cw[4];          // shared-SM form: output columns of layer l per group member (a multiple of 16, <= 256)
     unsigned long long timeout_ns, flush_ns;
-    uint32_t dbg_flags;       // timing experiments only (AZB_ASYNC_DBG): 1 skip activation stores, 2 skip the TMEM reads
-    unsigned long long *dbg;  // optional [16] cycle counters of the MLP workers (tools/async_probe.py); null = off
+    unsigned long long *dbg;  // optional [32] cycle counters of the workers (azb_debug_async, tools/async_probe.py); null = off
 };
 
 __device__ __forceinline__ unsigned long long as_now() {
@@ -144,7 +128,8 @@ __device__ __forceinline__ unsigned long long as_now() {
 // Polls use ld.volatile (served by L2, where the atomics land), never ld.acquire.gpu: an acquire load comes with
 // CCTL.IVALL — it invalidates the SM's whole L1 — and a waiting warp polls every microsecond beside 31 warps whose
 // walks live on L1 hits (ncu: 160 M CCTL per 100 steps; phase cycles of the walkers 1.6-2x the lock step's).  Once a
-// poll has seen its value, ONE as_ld_acquire of the same word orders what follows (AS_ACQUIRE).
+// poll has seen its value, ONE as_ld_acquire of the same word orders what follows (PTX memory model: what the word
+// guards is read or overwritten afterwards).
 __device__ __forceinline__ uint32_t as_ld_volatile(const uint32_t *p) {
     uint32_t v;
     asm volatile("ld.volatile.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
@@ -162,19 +147,6 @@ __device__ __forceinline__ void as_red_release_add(uint32_t *p, uint32_t v) {
 __device__ __forceinline__ void as_mbar_arrive(uint64_t *bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc_smem_u32(bar)) : "memory");
 }
-// CTA pairs (clusters of two): the same shared-memory offset in the pair's FIRST CTA — bit 24 of a shared::cluster address
-// is the CTA's rank within its pair
-#define AS_PEER_BIT_MASK 0xFEFFFFFFu
-__device__ __forceinline__ void as_mbar_arrive_leader(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(tc_smem_u32(bar) & AS_PEER_BIT_MASK) : "memory");
-}
-__device__ __forceinline__ void as_mbar_arrive_peer(uint64_t *bar) {  // the same barrier in the OTHER CTA of the pair
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(tc_smem_u32(bar) ^ ~AS_PEER_BIT_MASK) : "memory");
-}
-__device__ __forceinline__ void as_cluster_sync() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
 // spin on test_wait (no suspend): the worker owns its SM, and try_wait's suspend/wake-up costs more than the
 // wait itself at this granularity (one barrier round trip per 64-deep k-block)
 __device__ __forceinline__ void as_mbar_spin(uint64_t *bar, uint32_t parity) {
@@ -190,36 +162,6 @@ __device__ __forceinline__ void as_mbar_spin(uint64_t *bar, uint32_t parity) {
             : "r"(tc_smem_u32(bar)), "r"(parity)
             : "memory");
     } while (!done);
-}
-// The same with a watchdog, for the warps of a CTA pair (their barriers are fed from the peer CTA): a barrier of this
-// kernel completes within microseconds, so 2^26 polls (a second or more) mean a broken protocol.  The wait then records
-// which barrier it was, raises `abort` and RETURNS — every later wait of the launch returns after 2^16 polls once `abort`
-// is up, so the kernel drains (with garbage in the tiles in flight) and the host reports the watchdog instead of hanging.
-__device__ __noinline__ void as_mbar_stuck(AzbAsyncState *st, uint32_t code) {
-    atomicCAS(&st->stuck, 0u, (code << 16) | (blockIdx.x & 0xffffu));
-    atomicExch(&st->abort, 1u);
-}
-__device__ __forceinline__ void as_mbar_spin_wd(uint64_t *bar, uint32_t parity, AzbAsyncState *st, uint32_t code) {
-    uint32_t done, spins = 0;
-    for (;;) {
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-            "selp.u32 %0, 1, 0, p;\n"
-            "}\n"
-            : "=r"(done)
-            : "r"(tc_smem_u32(bar)), "r"(parity)
-            : "memory");
-        if (done) return;
-        if ((++spins & 0xffffu) == 0u) {
-            if (*reinterpret_cast<volatile uint32_t *>(&st->abort)) return;
-            if (spins >= (1u << 26)) {
-                as_mbar_stuck(st, code);
-                return;
-            }
-        }
-    }
 }
 __device__ __forceinline__ void as_named_bar(uint32_t id, uint32_t threads) {
     asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory");
@@ -271,12 +213,9 @@ __device__ __forceinline__ void as_fence_proxy_async() { asm volatile("fence.pro
 // Model CTA.  Roles: warp 0 TMA producer and tile taker, warp 1 MMA issuer and TMEM owner (warpgroup 0, 56 registers),
 // warps 4-11 epilogue (warpgroups 1-2, 168 registers).  Each role is its own function with its own copy of the loop
 // over tiles, so that no code is shared between register budgets; they meet at named barrier 1 (AS_MLP_THREADS).
-#define AS_PAIR_STAGES 4   // operand ring of a CTA pair: [A | half of B] per stage (see "CTA pairs" below)
-#define AS_MAX_STAGES (AS_STAGES > AS_PAIR_STAGES ? AS_STAGES : AS_PAIR_STAGES)
 struct AsWorkerShared {
-    uint64_t full_bar[AS_MAX_STAGES], empty_bar[AS_MAX_STAGES], acc_full[2], acc_empty[2], layer_bar, exit_bar;
+    uint64_t full_bar[AS_STAGES], empty_bar[AS_STAGES], acc_full[2], acc_empty[2], layer_bar;
     uint32_t tmem_slot, tile, epi_last;
-    uint32_t stored;  // pair form: (epilogue warp, pass) pairs of hidden layers whose activations are stored (monotonic over the launch)
     uint32_t bias_off[4];  // first entry of layer l's biases in the shared-memory copy
     uint32_t rowtree[AS_TILE];
 };
@@ -348,9 +287,7 @@ __device__ __forceinline__ uint32_t as_group_next_tile(const AzbLayout &L, const
                 break;
             }
         }
-#if AS_ACQUIRE
         if (q != AS_NONE) (void)as_ld_acquire(cnt_p);  // the tile's rows and owners are read after this
-#endif
         st->grp[grp].tile = q;
         __threadfence();
         atomicAdd(&st->grp[grp].seq, 1u);
@@ -360,9 +297,7 @@ __device__ __forceinline__ uint32_t as_group_next_tile(const AzbLayout &L, const
             if ((spins & 4095u) == 4095u && as_now() - t_start > P.timeout_ns) atomicExch(&st->abort, 1u);
             if (as_ld_volatile(&st->abort)) break;
         }
-#if AS_ACQUIRE
         (void)as_ld_acquire(&st->grp[grp].seq);
-#endif
         q = as_ld_volatile(&st->abort) ? AS_NONE : as_ld_volatile(&st->grp[grp].tile);
     }
     return q;
@@ -407,7 +342,7 @@ __device__ __forceinline__ void async_worker_producer(const AzbLayout &L, const 
         if (q == AS_NONE) break;
         const uint32_t ring_row0 = (q % P.NT) * AS_TILE;
         const uint32_t arrive_target = G * (seq + 1u);  // value of the group's counters once every member has arrived
-        if (!AS_DBG(16u) && tc_elect_one()) {
+        if (tc_elect_one()) {
             const long long tt0 = AS_CLK();
             d_tiles += 1;
             const uint64_t w_policy = as_policy_evict_last();
@@ -425,25 +360,22 @@ __device__ __forceinline__ void async_worker_producer(const AzbLayout &L, const 
                     // the weights do not depend on it: while the epilogue warps still drain the previous layer, the
                     // ring's stages are free, so the first stages' B tiles go out now and only their A tiles wait
                     const uint32_t np0 = min((uint32_t)AS_ACC, mine);
-                    if (!AS_DBG(4u))
-                        for (; np0 && pre < min((uint32_t)AS_STAGES, k_blocks); ++pre) {
-                            const uint32_t kc = kbc + pre, s = kc % AS_STAGES, ph = (kc / AS_STAGES) & 1u;
-                            as_mbar_spin(&S.empty_bar[s], ph ^ 1u);
-                            uint8_t *a_dst = smem + (size_t)s * AS_STAGE_BYTES;
-                            tc_mbar_expect_tx(&S.full_bar[s], (1u + np0) * AS_TILE_BYTES);
-                            for (uint32_t j = 0; j < np0; ++j)
-                                as_tma_load_2d_hint(a_dst + (1u + j) * AS_TILE_BYTES, &M.w[l], &S.full_bar[s], (int)(pre * TC_BK),
-                                                    (int)((mem + j * G) * 128u), w_policy);
-                        }
+                    for (; np0 && pre < min((uint32_t)AS_STAGES, k_blocks); ++pre) {
+                        const uint32_t kc = kbc + pre, s = kc % AS_STAGES, ph = (kc / AS_STAGES) & 1u;
+                        as_mbar_spin(&S.empty_bar[s], ph ^ 1u);
+                        uint8_t *a_dst = smem + (size_t)s * AS_STAGE_BYTES;
+                        tc_mbar_expect_tx(&S.full_bar[s], (1u + np0) * AS_TILE_BYTES);
+                        for (uint32_t j = 0; j < np0; ++j)
+                            as_tma_load_2d_hint(a_dst + (1u + j) * AS_TILE_BYTES, &M.w[l], &S.full_bar[s], (int)(pre * TC_BK),
+                                                (int)((mem + j * G) * 128u), w_policy);
+                    }
                     const long long tw = AS_CLK();
                     if (G == 1u) {  // a single worker: the layer boundary is a shared-memory barrier, not an L2 round trip
                         as_mbar_spin(&S.layer_bar, lbc & 1u);
                         ++lbc;
                     } else {
                         while (as_ld_volatile(&st->grp[grp].layer[l - 1]) < arrive_target && !as_ld_volatile(&st->abort)) {}
-#if AS_ACQUIRE
                         (void)as_ld_acquire(&st->grp[grp].layer[l - 1]);
-#endif
                     }
                     d_w1 += AS_CLK() - tw;
                     as_fence_proxy_async();
@@ -465,10 +397,6 @@ __device__ __forceinline__ void async_worker_producer(const AzbLayout &L, const 
                         const long long tw = AS_CLK();
                         as_mbar_spin(&S.empty_bar[s], ph ^ 1u);
                         d_w0 += AS_CLK() - tw;
-                        if (AS_DBG(4u)) {  // timing experiment: no loads, the MMAs run on stale operands
-                            as_mbar_arrive(&S.full_bar[s]);
-                            continue;
-                        }
                         tc_mbar_expect_tx(&S.full_bar[s], (1u + np) * AS_TILE_BYTES);
                         tc_tma_load_2d(a_dst, ma, &S.full_bar[s], a_col, arow);
                         for (uint32_t j = 0; j < np; ++j)
@@ -513,60 +441,57 @@ __device__ __forceinline__ void async_worker_mma(const AzbAsyncParams &P, const 
         as_named_bar(1, AS_MLP_THREADS);
         const uint32_t q = S.tile;
         if (q == AS_NONE) break;
-        if (!AS_DBG(16u))
-            for (uint32_t l = 0; l < 4; ++l) {
-                const uint32_t k_blocks = (P.wide == 2u ? 3u : 1u) * (P.kpad[l] / TC_BK);  // all k-segments
-                const uint32_t mine = as_blocks_of_member(P.npad[l], id);
-                for (uint32_t p0 = 0; p0 < mine; p0 += AS_ACC, ++ntc) {
-                    const uint32_t np = min((uint32_t)AS_ACC, mine - p0);
-                    long long tw = AS_CLK();
-                    const uint32_t slot = ntc & 1u, acc_ph = (ntc >> 1) & 1u;  // TMEM half of this pass, phase of its barriers
-                    as_mbar_spin(&S.acc_empty[slot], acc_ph ^ 1u);  // the epilogue has drained the pass before last
-                    d_w1 += AS_CLK() - tw;
-                    const uint32_t tmem_acc = tmem_base + slot * (AS_ACC * 128u);
+        for (uint32_t l = 0; l < 4; ++l) {
+            const uint32_t k_blocks = (P.wide == 2u ? 3u : 1u) * (P.kpad[l] / TC_BK);  // all k-segments
+            const uint32_t mine = as_blocks_of_member(P.npad[l], id);
+            for (uint32_t p0 = 0; p0 < mine; p0 += AS_ACC, ++ntc) {
+                const uint32_t np = min((uint32_t)AS_ACC, mine - p0);
+                long long tw = AS_CLK();
+                const uint32_t slot = ntc & 1u, acc_ph = (ntc >> 1) & 1u;  // TMEM half of this pass, phase of its barriers
+                as_mbar_spin(&S.acc_empty[slot], acc_ph ^ 1u);  // the epilogue has drained the pass before last
+                d_w1 += AS_CLK() - tw;
+                const uint32_t tmem_acc = tmem_base + slot * (AS_ACC * 128u);
+                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                for (uint32_t kb = 0; kb < k_blocks; ++kb, ++kbc) {
+                    const uint32_t s = kbc % AS_STAGES, ph = (kbc / AS_STAGES) & 1u;
+                    tw = AS_CLK();
+                    as_mbar_spin(&S.full_bar[s], ph);
+                    d_w0 += AS_CLK() - tw;
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                    for (uint32_t kb = 0; kb < k_blocks; ++kb, ++kbc) {
-                        const uint32_t s = kbc % AS_STAGES, ph = (kbc / AS_STAGES) & 1u;
-                        tw = AS_CLK();
-                        as_mbar_spin(&S.full_bar[s], ph);
-                        d_w0 += AS_CLK() - tw;
-                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                        if (tc_elect_one()) {
-                            const uint32_t a_addr = tc_smem_u32(smem + (size_t)s * AS_STAGE_BYTES);
-                            if (G == 1u) {
-                                // adjacent 128-column blocks are adjacent in the stage and in TMEM: one N <= 256 MMA per
-                                // pair reads the A tile once for both (a 128x128x16 SS-MMA is shared-memory bound)
-                                for (uint32_t j = 0; j < np; j += 2) {
-                                    const uint32_t nt = p0 + j;
-                                    const uint32_t bn = min(256u, P.npad[l] - nt * 128u);
-                                    const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((bn >> 3) << 17) | ((AS_TILE >> 4) << 24);
-                                    const uint32_t b_addr = a_addr + (1u + j) * AS_TILE_BYTES;
+                    if (tc_elect_one()) {
+                        const uint32_t a_addr = tc_smem_u32(smem + (size_t)s * AS_STAGE_BYTES);
+                        if (G == 1u) {
+                            // adjacent 128-column blocks are adjacent in the stage and in TMEM: one N <= 256 MMA per
+                            // pair reads the A tile once for both (a 128x128x16 SS-MMA is shared-memory bound)
+                            for (uint32_t j = 0; j < np; j += 2) {
+                                const uint32_t nt = p0 + j;
+                                const uint32_t bn = min(256u, P.npad[l] - nt * 128u);
+                                const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((bn >> 3) << 17) | ((AS_TILE >> 4) << 24);
+                                const uint32_t b_addr = a_addr + (1u + j) * AS_TILE_BYTES;
 #pragma unroll
-                                    for (uint32_t k = 0; k < TC_BK / 16; ++k)
-                                        if (!AS_DBG(8u))
-                                            tc_umma_f16(tmem_acc + j * 128u, tc_smem_desc(a_addr + k * 32u), tc_smem_desc(b_addr + k * 32u),
-                                                        idesc, (kb | k) != 0u ? 1u : 0u);
-                                }
-                            } else {
-                                for (uint32_t j = 0; j < np; ++j) {
-                                    const uint32_t nt = mem + (p0 + j) * G;
-                                    const uint32_t bn = min(128u, P.npad[l] - nt * 128u);
-                                    const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((bn >> 3) << 17) | ((AS_TILE >> 4) << 24);
-                                    const uint32_t b_addr = a_addr + (1u + j) * AS_TILE_BYTES;
-#pragma unroll
-                                    for (uint32_t k = 0; k < TC_BK / 16; ++k)
-                                        if (!AS_DBG(8u))  // timing experiment: loads only
-                                            tc_umma_f16(tmem_acc + j * 128u, tc_smem_desc(a_addr + k * 32u), tc_smem_desc(b_addr + k * 32u),
-                                                        idesc, (kb | k) != 0u ? 1u : 0u);
-                                }
+                                for (uint32_t k = 0; k < TC_BK / 16; ++k)
+                                    tc_umma_f16(tmem_acc + j * 128u, tc_smem_desc(a_addr + k * 32u), tc_smem_desc(b_addr + k * 32u),
+                                                idesc, (kb | k) != 0u ? 1u : 0u);
                             }
-                            tc_umma_commit(&S.empty_bar[s]);
-                            if (kb + 1 == k_blocks) tc_umma_commit(&S.acc_full[slot]);
+                        } else {
+                            for (uint32_t j = 0; j < np; ++j) {
+                                const uint32_t nt = mem + (p0 + j) * G;
+                                const uint32_t bn = min(128u, P.npad[l] - nt * 128u);
+                                const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((bn >> 3) << 17) | ((AS_TILE >> 4) << 24);
+                                const uint32_t b_addr = a_addr + (1u + j) * AS_TILE_BYTES;
+#pragma unroll
+                                for (uint32_t k = 0; k < TC_BK / 16; ++k)
+                                    tc_umma_f16(tmem_acc + j * 128u, tc_smem_desc(a_addr + k * 32u), tc_smem_desc(b_addr + k * 32u),
+                                                idesc, (kb | k) != 0u ? 1u : 0u);
+                            }
                         }
-                        __syncwarp();
+                        tc_umma_commit(&S.empty_bar[s]);
+                        if (kb + 1 == k_blocks) tc_umma_commit(&S.acc_full[slot]);
                     }
+                    __syncwarp();
                 }
             }
+        }
         as_named_bar(1, AS_MLP_THREADS);
     }
 #ifdef AZB_PROFILE
@@ -581,298 +506,7 @@ __device__ __forceinline__ void async_worker_mma(const AzbAsyncParams &P, const 
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
 }
 
-// ---------------------------------------------------------------------------------------------------------------
-// CTA pairs (P.pair).  A model SM moves ~87 GB/s through TMA whatever the schedule, and 2.75 of the 4.0 MB a 128-row tile
-// needs are weights.  Two model CTAs of one cluster (one TPC) therefore answer two tiles TOGETHER: every 256-column
-// weight tile is fetched once per pair — each CTA loads its own activation tile and HALF of the weight tile —, and ONE
-// tcgen05.mma.cta_group::2 (M = 256: rows 0-127 in the first CTA's TMEM, 128-255 in the second's) reads both halves
-// through the pair's shared memory.  Per CTA and k-block 16 + 16 KB arrive instead of 16 + 32; the ring has four stages.
-//  * full barriers live in the first CTA: both CTAs' TMA loads complete their bytes there (cta_group::2 loads, peer bit
-//    of the barrier address cleared), the first CTA's producer posts the expected bytes of both;
-//  * the first CTA's MMA warp issues; tcgen05.commit multicasts to the empty / accumulator-full barriers of both CTAs;
-//  * the epilogue warps of both CTAs arrive on the first CTA's accumulator-empty barriers;
-//  * each CTA runs its own epilogue, layer boundaries and answer flags for its own 128 rows (the code of a single worker).
-// A ticket is a double tile: ring tiles 2q and 2q + 1.
-#define AS_PAIR_STAGE_BYTES (2u * AS_TILE_BYTES)  // [A | B half]
-
-__device__ __forceinline__ void as_tma_load_2d_pair(void *dst, const CUtensorMap *map, uint64_t *bar, int c0, int c1, uint64_t policy) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(
-            tc_smem_u32(dst)),
-        "l"(map), "r"(tc_smem_u32(bar) & AS_PEER_BIT_MASK), "r"(c0), "r"(c1), "l"(policy)
-        : "memory");
-}
-__device__ __forceinline__ uint64_t as_policy_evict_first() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ void as_umma_f16_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "setp.ne.b32 p, %4, 0;\n"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n"
-        "}\n" ::"r"(tmem_d),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void as_umma_commit_pair(uint64_t *bar) {  // arrives on this barrier in BOTH CTAs of the pair
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(tc_smem_u32(bar)),
-                 "h"((uint16_t)3)
-                 : "memory");
-}
-
-// The double tile the pair answers next (AS_NONE: leave).  Lane 0 of the producer warp of each CTA; `rank` = CTA in the pair.
-__device__ __forceinline__ uint32_t as_pair_next_ticket(const AzbLayout &L, const AzbAsyncParams &P, const uint32_t worker, const uint32_t rank,
-                                                        const uint32_t seq, const unsigned long long t_start) {
-    AzbAsyncState *st = P.st;
-    AzbAsyncState::Group &box = st->grp[worker & ~1u];  // the pair's mailbox: the line of its first CTA
-    uint32_t q;
-    if (rank == 0) {
-        q = atomicAdd(&st->tile_head, 1u);  // tickets count double tiles here
-        const uint32_t t0 = 2u * q, t1 = t0 + 1u;  // NT is even: both tiles are in the same generation of the ring
-        const uint32_t *c0 = P.tile_count + (t0 % P.NT), *c1 = P.tile_count + (t1 % P.NT);
-        const uint32_t want = AS_TILE * (t0 / P.NT + 1u);
-        const uint32_t row_lo = t0 * AS_TILE, row_hi = row_lo + 2u * AS_TILE;
-        unsigned long long t_partial = 0;
-        bool flushed = false;
-        for (uint32_t spins = 0;; ++spins) {
-            if (as_ld_volatile(c0) >= want && as_ld_volatile(c1) >= want) break;
-            if (as_ld_volatile(&st->abort)) {
-                q = AS_NONE;
-                break;
-            }
-            const bool all_done = as_ld_volatile(&st->done_trees) >= L.B;
-            const uint32_t tail = as_ld_volatile(&st->row_tail);
-            if (all_done && tail <= row_lo) {  // every tree has finished and no row has reached this double tile
-                q = AS_NONE;
-                break;
-            }
-            if (!flushed && tail > row_lo && tail < row_hi) {
-                const unsigned long long now = as_now();
-                if (t_partial == 0) t_partial = now;
-                if (all_done || now - t_partial > P.flush_ns) {  // top the stale double tile up with dummy rows
-                    const uint32_t k = row_hi - tail;
-                    const uint32_t old = atomicAdd(&st->row_tail, k);
-                    for (uint32_t i = 0; i < k; ++i) P.slot_tree[(old + i) % (P.NT * AS_TILE)] = AS_NONE;
-                    __threadfence();
-                    for (uint32_t r = old; r < old + k;) {  // one add per ring tile the dummies fall into
-                        const uint32_t t = r / AS_TILE, n = min(old + k, (t + 1u) * AS_TILE) - r;
-                        atomicAdd(P.tile_count + (t % P.NT), n);
-                        r += n;
-                    }
-                    atomicAdd(&st->rows_dummy, k);
-                    flushed = true;
-                }
-            }
-            __nanosleep(100);
-            if ((spins & 255u) == 255u && as_now() - t_start > P.timeout_ns) {
-                atomicExch(&st->abort, 1u);
-                q = AS_NONE;
-                break;
-            }
-        }
-#if AS_ACQUIRE
-        if (q != AS_NONE) {  // the tiles' rows and owners are read after this
-            (void)as_ld_acquire(c0);
-            (void)as_ld_acquire(c1);
-        }
-#endif
-        box.tile = q;
-        __threadfence();
-        atomicAdd(&box.seq, 1u);
-    } else {
-        for (uint32_t spins = 0; as_ld_volatile(&box.seq) <= seq; ++spins) {
-            if ((spins & 4095u) == 4095u && as_now() - t_start > P.timeout_ns) atomicExch(&st->abort, 1u);
-            if (as_ld_volatile(&st->abort)) break;
-        }
-#if AS_ACQUIRE
-        (void)as_ld_acquire(&box.seq);
-#endif
-        q = as_ld_volatile(&st->abort) ? AS_NONE : as_ld_volatile(&box.tile);
-    }
-    return q;
-}
-
-// ---- warp 0 of each CTA of a pair: feeds its own activation tile and its half of the weight tile
-__device__ __forceinline__ void pair_worker_producer(const AzbLayout &L, const AzbAsyncParams &P, const AzbAsyncMaps &M, const uint32_t worker,
-                                                     const uint32_t rank, uint8_t *smem, AsWorkerShared &S) {
-    const uint32_t lane = threadIdx.x & 31;
-    if (lane == 0) {
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&M.ring) : "memory");
-        for (int l = 0; l < 4; ++l) asm volatile("prefetch.tensormap [%0];" ::"l"(&M.w[l]) : "memory");
-        for (int l = 0; l < 3; ++l) asm volatile("prefetch.tensormap [%0];" ::"l"(&M.act[l]) : "memory");
-    }
-    __syncwarp();
-    AS_MARK(worker, 0, 2);
-    as_named_bar(1, AS_MLP_THREADS);
-    AS_MARK(worker, 0, 3);
-    const unsigned long long t_start = as_now();
-    uint32_t kbc = 0, seq = 0, lbc = 0, seen = 0;  // lbc: stored passes before the current layer's input
-    long long d_acq = 0, d_w0 = 0, d_w1 = 0, d_busy = 0, d_tiles = 0;
-    for (;;) {
-        if (lane == 0) {
-            const long long tq0 = AS_CLK();
-            const uint32_t q = as_pair_next_ticket(L, P, worker, rank, seq, t_start);
-            S.tile = q == AS_NONE ? AS_NONE : 2u * q + rank;  // this CTA's own 128-row ring tile
-            d_acq += AS_CLK() - tq0;
-        }
-        __syncwarp();
-        AS_MARK(worker, 0, 4u | (S.tile << 8));
-        as_named_bar(1, AS_MLP_THREADS);
-        const uint32_t q = S.tile;
-        if (q == AS_NONE) break;
-        const uint32_t ring_row0 = (q % P.NT) * AS_TILE;
-        if (tc_elect_one()) {
-            const long long tt0 = AS_CLK();
-            d_tiles += 1;
-            const uint64_t w_policy = as_policy_evict_last(), a_policy = as_policy_evict_first();
-            as_fence_proxy_async();  // the tile's rows were written by tree warps through the generic proxy
-            const uint32_t nseg = P.wide == 2u ? 3u : 1u;
-            for (uint32_t l = 0; l < 4; ++l) {
-                const uint32_t k_blocks = P.kpad[l] / TC_BK, kb_all = nseg * k_blocks;
-                const uint32_t n_tiles = (P.npad[l] + 127u) / 128u;
-                // a k-block of layer l > 0 reads 64 columns of the previous layer's output: it goes out once this CTA's own
-                // epilogue has stored the pass those columns belong to (AS_ACC * 128 columns per pass, AS_EPI_WARPS counts each)
-                const uint32_t in_passes = l > 0 ? ((P.npad[l - 1] + 127u) / 128u + AS_ACC - 1u) / AS_ACC : 0u;
-                const CUtensorMap *ma = l == 0 ? &M.ring : &M.act[l - 1];
-                const int arow = (int)(l == 0 ? ring_row0 : worker * AS_TILE);
-                for (uint32_t p0 = 0; p0 < n_tiles; p0 += AS_ACC) {
-                    // the pass's columns [128 p0, 128 p0 + w): this CTA holds the w / 2 weight rows 128 p0 + rank w / 2 ..
-                    // (the box is always 128 rows; with w = 128 its upper half is not read)
-                    const uint32_t w = min((uint32_t)AS_ACC, n_tiles - p0) * 128u;
-                    const int brow = (int)(p0 * 128u + rank * (w >> 1));
-                    for (uint32_t kb = 0; kb < kb_all; ++kb, ++kbc) {
-                        const uint32_t s = kbc % AS_PAIR_STAGES, ph = (kbc / AS_PAIR_STAGES) & 1u;
-                        const uint32_t seg = kb / k_blocks, kj = kb - seg * k_blocks;
-                        const int a_col = (int)(((seg == 2u ? k_blocks : 0u) + kj) * TC_BK);
-                        const int w_col = (int)(((seg == 1u ? k_blocks : 0u) + kj) * TC_BK);
-                        uint8_t *a_dst = smem + (size_t)s * AS_PAIR_STAGE_BYTES;
-                        if (l > 0) {
-                            const uint32_t need = AS_EPI_WARPS * (lbc + min(in_passes, kj / (AS_ACC * 128u / TC_BK) + 1u));
-                            if (seen < need) {
-                                const long long tw1 = AS_CLK();
-                                for (uint32_t spins = 0; (seen = *reinterpret_cast<volatile uint32_t *>(&S.stored)) < need;)
-                                    if ((++spins & 0xffffu) == 0u && (as_ld_volatile(&P.st->abort) || spins >= (1u << 26))) {
-                                        if (spins >= (1u << 26)) as_mbar_stuck(P.st, 1u);
-                                        break;
-                                    }
-                                d_w1 += AS_CLK() - tw1;
-                                asm volatile("fence.acq_rel.cta;" ::: "memory");
-                                as_fence_proxy_async();
-                            }
-                        }
-                        const long long tw = AS_CLK();
-                        as_mbar_spin_wd(&S.empty_bar[s], ph ^ 1u, P.st, 2u);
-                        d_w0 += AS_CLK() - tw;
-                        // the full barrier of the stage is the first CTA's: it expects the bytes of both CTAs
-                        if (rank == 0) tc_mbar_expect_tx(&S.full_bar[s], 2u * AS_PAIR_STAGE_BYTES);
-                        as_tma_load_2d_pair(a_dst, ma, &S.full_bar[s], a_col, arow, a_policy);
-                        as_tma_load_2d_pair(a_dst + AS_TILE_BYTES, &M.w[l], &S.full_bar[s], w_col, brow, w_policy);
-                    }
-                }
-                lbc += in_passes;  // passes of hidden layers this CTA's epilogue has stored once layer l's input is complete
-            }
-            d_busy += AS_CLK() - tt0;
-        }
-        __syncwarp();
-        seq += 1u;
-        AS_MARK(worker, 0, 5u | (seq << 8));
-        as_named_bar(1, AS_MLP_THREADS);
-        AS_MARK(worker, 0, 6u | (seq << 8));
-    }
-#ifdef AZB_PROFILE
-    if (P.dbg && lane == 0) {
-        atomicAdd(P.dbg + 0, (unsigned long long)d_acq);
-        atomicAdd(P.dbg + 1, (unsigned long long)d_w0);
-        atomicAdd(P.dbg + 2, (unsigned long long)d_w1);
-        atomicAdd(P.dbg + 3, (unsigned long long)d_busy);
-        atomicAdd(P.dbg + 4, (unsigned long long)d_tiles);
-    }
-#endif
-    (void)d_acq; (void)d_w0; (void)d_w1; (void)d_busy; (void)d_tiles;
-    as_named_bar(1, AS_MLP_THREADS);
-}
-
-// ---- warp 1: TMEM of the pair (allocated by both CTAs together); the first CTA's warp issues the MMAs of both
-__device__ __forceinline__ void pair_worker_mma(const AzbAsyncParams &P, const uint32_t worker, const uint32_t rank, uint8_t *smem,
-                                                AsWorkerShared &S) {
-    AS_MARK(worker, 1, 2);
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tc_smem_u32(&S.tmem_slot)), "r"(512u)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    AS_MARK(worker, 1, 3);
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    as_named_bar(1, AS_MLP_THREADS);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem_base = S.tmem_slot;
-    uint32_t kbc = 0, ntc = 0;
-    long long d_w0 = 0, d_w1 = 0;
-    const uint32_t nseg = P.wide == 2u ? 3u : 1u;
-    for (;;) {
-        as_named_bar(1, AS_MLP_THREADS);
-        const uint32_t q = S.tile;
-        AS_MARK(worker, 1, 4u | (q << 8));
-        if (q == AS_NONE) break;
-        if (rank == 0)
-            for (uint32_t l = 0; l < 4; ++l) {
-                const uint32_t k_blocks = nseg * (P.kpad[l] / TC_BK);
-                const uint32_t n_tiles = (P.npad[l] + 127u) / 128u;
-                for (uint32_t p0 = 0; p0 < n_tiles; p0 += AS_ACC, ++ntc) {
-                    const uint32_t w = min((uint32_t)AS_ACC, n_tiles - p0) * 128u;
-                    long long tw = AS_CLK();
-                    const uint32_t slot = ntc & 1u, acc_ph = (ntc >> 1) & 1u;
-                    as_mbar_spin_wd(&S.acc_empty[slot], acc_ph ^ 1u, P.st, 3u);  // both CTAs' epilogues have drained the pass before last
-                    d_w1 += AS_CLK() - tw;
-                    const uint32_t tmem_acc = tmem_base + slot * (AS_ACC * 128u);
-                    // D[256 x w] (rows 128 r .. in CTA r), A[256 x 64] (one tile per CTA), B[w x 64] (w / 2 rows per CTA)
-                    const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((w >> 3) << 17) | ((256u >> 4) << 24);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                    for (uint32_t kb = 0; kb < k_blocks; ++kb, ++kbc) {
-                        const uint32_t s = kbc % AS_PAIR_STAGES, ph = (kbc / AS_PAIR_STAGES) & 1u;
-                        tw = AS_CLK();
-                        as_mbar_spin_wd(&S.full_bar[s], ph, P.st, 4u);
-                        d_w0 += AS_CLK() - tw;
-                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                        if (tc_elect_one()) {
-                            const uint32_t a_addr = tc_smem_u32(smem + (size_t)s * AS_PAIR_STAGE_BYTES), b_addr = a_addr + AS_TILE_BYTES;
-#pragma unroll
-                            for (uint32_t k = 0; k < TC_BK / 16; ++k)
-                                as_umma_f16_pair(tmem_acc, tc_smem_desc(a_addr + k * 32u), tc_smem_desc(b_addr + k * 32u), idesc,
-                                                 (kb | k) != 0u ? 1u : 0u);
-                            as_umma_commit_pair(&S.empty_bar[s]);
-                            if (kb + 1 == k_blocks) as_umma_commit_pair(&S.acc_full[slot]);
-                        }
-                        __syncwarp();
-                    }
-                }
-            }
-        as_named_bar(1, AS_MLP_THREADS);
-    }
-#ifdef AZB_PROFILE
-    if (P.dbg && (threadIdx.x & 31) == 0 && rank == 0) {
-        atomicAdd(P.dbg + 5 + 1, (unsigned long long)d_w0);
-        atomicAdd(P.dbg + 5 + 2, (unsigned long long)d_w1);
-    }
-#endif
-    (void)d_w0; (void)d_w1;
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    as_named_bar(1, AS_MLP_THREADS);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    AS_MARK(worker, 1, 7);
-    // Neither CTA may leave while the other can still reach into it (the peer's epilogue warps arrive on the first CTA's
-    // accumulator barriers, tcgen05.commit signals the second CTA's): the two MMA warps shake hands through their exit
-    // barriers.  (A cluster barrier here — with the CTA's other warps exiting instead of arriving — never completed.)
-    if ((threadIdx.x & 31) == 0) as_mbar_arrive_peer(&S.exit_bar);
-    as_mbar_spin_wd(&S.exit_bar, 0u, P.st, 6u);
-    __syncwarp();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    AS_MARK(worker, 1, 9);
-}
-
 // ---- warps 4-11: TMEM -> registers -> bias + activation -> scratch / prior rows
-template <bool PAIR>
 __device__ __forceinline__ void async_worker_epilogue(const AzbLayout &L, const AzbAsyncParams &P, const AsWorkerId id, uint8_t *smem,
                                       AsWorkerShared &S) {
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -903,20 +537,6 @@ __device__ __forceinline__ void async_worker_epilogue(const AzbLayout &L, const 
         if (q == AS_NONE) break;
         const uint32_t ring_row0 = (q % P.NT) * AS_TILE;
         const uint32_t arrive_target = G * (seq + 1u);
-        if (AS_DBG(16u)) {  // timing experiment: answer the tile at once with whatever the prior rows hold
-            if (mem == 0 && et < AS_TILE) {
-                const uint32_t t = __ldcg(P.slot_tree + ring_row0 + et);
-                if (t != AS_NONE) atomicAdd(P.h_flag + t, 1u);
-            }
-            if (et == 0u) {
-                if (mem == 0) atomicAdd(P.tile_retired + (q % P.NT), 1u);
-                atomicAdd(&st->grp[grp].done, 1u);
-            }
-            seq += 1u;
-            as_named_bar(1, AS_MLP_THREADS);
-            continue;
-        }
-        if (warp == AS_EPI_WARP0) AS_MARK(id.grp, 2, 4u | (q << 8));
         if (et < AS_TILE) S.rowtree[et] = __ldcg(P.slot_tree + ring_row0 + et);
         as_named_bar(2, AS_EPI_WARPS * 32);
         const uint32_t my_tree = S.rowtree[row];
@@ -927,8 +547,7 @@ __device__ __forceinline__ void async_worker_epilogue(const AzbLayout &L, const 
                 const uint32_t np = min((uint32_t)AS_ACC, mine - p0);
                 const long long tw = AS_CLK();
                 const uint32_t slot = ntc & 1u, acc_ph = (ntc >> 1) & 1u;
-                if (PAIR) as_mbar_spin_wd(&S.acc_full[slot], acc_ph, st, 5u);
-                else as_mbar_spin(&S.acc_full[slot], acc_ph);
+                as_mbar_spin(&S.acc_full[slot], acc_ph);
                 const uint32_t tmem_acc = tmem_base + slot * (AS_ACC * 128u);
                 const long long tb = AS_CLK();
                 d_w0 += tb - tw;
@@ -993,7 +612,7 @@ __device__ __forceinline__ void async_worker_epilogue(const AzbLayout &L, const 
                                     const uint32_t rw = it * (32u / AS_EPI_CHUNKS) + rr;
                                     const uint32_t sw2 = AS_EPI_CHUNKS == 8 ? (rw & 7u) : ((rw >> 1) & 3u);
                                     const uint4 v = as_lds128(tc_smem_u32(stg) + rw * (AS_EPI_COLS * 2u) + ((cc ^ sw2) << 4));
-                                    if (!AS_DBG(1u)) *reinterpret_cast<uint4 *>(dst0 + (size_t)rw * act_ld) = v;
+                                    *reinterpret_cast<uint4 *>(dst0 + (size_t)rw * act_ld) = v;
                                 }
                                 __syncwarp();
                             }
@@ -1041,25 +660,10 @@ __device__ __forceinline__ void async_worker_epilogue(const AzbLayout &L, const 
                 }
                 asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
                 __syncwarp();
-                if (lane == 0) {
-                    if (PAIR) as_mbar_arrive_leader(&S.acc_empty[slot]);  // the MMA issuer sits in the pair's first CTA
-                    else as_mbar_arrive(&S.acc_empty[slot]);
-                }
-                if (PAIR && l < 3u) {
-                    // pair form: the next layer starts on the columns this pass has stored (its k-blocks wait for S.stored,
-                    // not for the whole layer): this warp's rows of the pass are visible to TMA, count them
-                    // (writer and reader sit in one CTA: the cross-proxy fence plus a CTA-scope release is what the memory
-                    // model asks for; a GPU-scope fence here waits for every store's acknowledgement, once per pass)
-                    as_fence_proxy_async();
-                    asm volatile("fence.acq_rel.cta;" ::: "memory");
-                    __syncwarp();
-                    if (lane == 0) atomicAdd(&S.stored, 1u);
-                }
+                if (lane == 0) as_mbar_arrive(&S.acc_empty[slot]);
                 d_busy += AS_CLK() - tb;
             }
-            if (PAIR && l < 3u) continue;  // (no layer barrier in the pair form)
             // ---- layer boundary: this member's share of the layer is stored; tell the group
-            if (warp == AS_EPI_WARP0) AS_MARK(id.grp, 2, 5u | (l << 4) | (q << 8));
             const long long tf0 = AS_CLK();
             if (l < 3) as_fence_proxy_async();  // the next layer reads these stores through TMA
             // a single worker hands its hidden activations to its OWN producer warp: the cross-proxy fence, the CTA barrier
@@ -1108,7 +712,6 @@ __device__ __forceinline__ void async_worker_epilogue(const AzbLayout &L, const 
 }
 
 // Role dispatch of a model CTA (all 1024 threads enter): re-divide the registers, then run the role
-template <bool PAIR>
 __device__ __forceinline__ void async_model_cta(const AzbLayout &L, const AzbAsyncParams &P, const AzbAsyncMaps &M,
                                                 const uint32_t worker, uint8_t *smem, AsWorkerShared &S) {
     const uint32_t warp = threadIdx.x >> 5, wg = warp >> 2;
@@ -1116,45 +719,18 @@ __device__ __forceinline__ void async_model_cta(const AzbLayout &L, const AzbAsy
     id.G = P.group;
     id.grp = worker / P.group;
     id.mem = worker % P.group;
-    const uint32_t rank = worker & 1u;  // pair form: this CTA's rank in its cluster of two (workers 2c and 2c + 1)
-    if constexpr (PAIR) {
-        // the pair's barriers: the full and accumulator-empty barriers that count are the first CTA's (both CTAs initialise
-        // theirs the same way); nobody may arrive on a peer's barrier before it exists, hence the cluster barrier
-        if (threadIdx.x == 0) {
-            for (int s = 0; s < AS_PAIR_STAGES; ++s) {
-                tc_mbar_init(&S.full_bar[s], 1);   // the first CTA's producer (arrive.expect_tx for the bytes of both CTAs)
-                tc_mbar_init(&S.empty_bar[s], 1);  // tcgen05.commit, multicast to both CTAs
-            }
-            for (int a = 0; a < 2; ++a) {
-                tc_mbar_init(&S.acc_full[a], 1);                  // tcgen05.commit, multicast
-                tc_mbar_init(&S.acc_empty[a], 2 * AS_EPI_WARPS);  // the epilogue warps of both CTAs
-            }
-            tc_mbar_init(&S.layer_bar, 1);
-            S.stored = 0u;
-            tc_mbar_init(&S.exit_bar, 1);  // the peer's MMA warp, once nothing of the peer touches this CTA any more
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-        if (warp == 2u) AS_MARK(worker, 7, 1);
-        as_cluster_sync();
-        if (warp == 2u) AS_MARK(worker, 7, 2);
-    }
     if (wg >= 3u) {
         asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(AS_REGS_IDLE));
         return;
     }
     if (wg == 0u) {
         asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(AS_REGS_FRONT));
-        if constexpr (PAIR) {
-            if (warp == 0u) pair_worker_producer(L, P, M, worker, rank, smem, S);
-            else if (warp == 1u) pair_worker_mma(P, worker, rank, smem, S);
-        } else {
-            if (warp == 0u) async_worker_producer(L, P, M, id, smem, S);
-            else if (warp == 1u) async_worker_mma(P, id, smem, S);
-        }
+        if (warp == 0u) async_worker_producer(L, P, M, id, smem, S);
+        else if (warp == 1u) async_worker_mma(P, id, smem, S);
         return;
     }
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(AS_REGS_EPI));
-    async_worker_epilogue<PAIR>(L, P, id, smem, S);
+    async_worker_epilogue(L, P, id, smem, S);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1251,11 +827,7 @@ __device__ void shared_model_warpgroup(const AzbLayout &L, const AzbAsyncParams 
     id.grp = member / P.group;
     id.mem = member % P.group;
     const uint32_t G = id.G, grp = id.grp, mem = id.mem;
-#ifdef SH_CONST_STAGES
-    const uint32_t stage_bytes = sh_stage_bytes(P), n_stages = SH_CONST_STAGES;
-#else
     const uint32_t stage_bytes = sh_stage_bytes(P), n_stages = P.sh_stages;
-#endif
     // this member's bias slices behind the operand ring, then one staging tile per warp
     float *s_bias = reinterpret_cast<float *>(smem + (size_t)n_stages * stage_bytes);
     uint32_t bias_end = 0;
@@ -1339,9 +911,7 @@ __device__ void shared_model_warpgroup(const AzbLayout &L, const AzbAsyncParams 
                         const long long tw = AS_CLK();
                         const uint32_t *lp = &st->grp[grp].layer[l - 1];
                         while (as_ld_volatile(lp) < arrive_target && !as_ld_volatile(&st->abort)) {}
-#if AS_ACQUIRE
                         (void)as_ld_acquire(lp);
-#endif
                         d_w1 += AS_CLK() - tw;
                         as_fence_proxy_async();
                     }
@@ -1629,7 +1199,7 @@ __device__ void async_tree_worker(const AzbLayout &L, const AzbAsyncParams &P, c
             if (runnable == 0u) {
                 // every tree of this warp waits for its priors.  The round trip is tens of microseconds, so the first sleeps
                 // after a walk are long and only then does the warp poll every microsecond
-                __nanosleep(naps < P.nap_count ? P.nap_long_ns : P.nap_short_ns);
+                __nanosleep(naps < AS_NAP_COUNT ? AS_NAP_LONG_NS : AS_NAP_SHORT_NS);
                 ++naps;
                 if ((++idle & 31u) == 0u) {
                     if (as_ld_volatile(&st->abort)) break;
@@ -1643,10 +1213,8 @@ __device__ void async_tree_worker(const AzbLayout &L, const AzbAsyncParams &P, c
             const int k = __ffs(__ballot_sync(FULL, my_state == 0u && my_steps == behind)) - 1;
             pick = warp + k * (int)P.tree_warps;
             naps = 0;
-#if AS_ACQUIRE
             // the relaxed poll saw this tree's flag: one acquire load of it orders the prior row (read in add_actions) behind it
             if (__shfl_sync(FULL, my_sub, k) != 0u) (void)as_ld_acquire(P.h_flag + tree0 + (uint32_t)pick);
-#endif
         } else {
             // ---- a runnable slot: first among this warp's HOME slots (i = warp mod tree_warps: disjoint between warps, so
             // a loaded CTA behaves like static ownership and nobody fights over a slot), the one that is furthest behind —
@@ -1677,9 +1245,9 @@ __device__ void async_tree_worker(const AzbLayout &L, const AzbAsyncParams &P, c
                 // ---- nothing runnable: look at the answer flags of waiting slots
                 uint32_t found = 0;
                 // more trees than warps: ONE warp at a time sweeps ALL waiting slots of the CTA (32 flags per ld.volatile
-                // round trip), at most once per sweep_gap cycles; the others nap and rescan shared memory only
+                // round trip), at most once per AS_SWEEP_GAP cycles; the others nap and rescan shared memory only
                 uint32_t got = 0;
-                if (lane == 0 && (uint32_t)clock64() - as_lds_volatile(T.ctl + 3) >= P.sweep_gap)
+                if (lane == 0 && (uint32_t)clock64() - as_lds_volatile(T.ctl + 3) >= AS_SWEEP_GAP)
                     got = atomicCAS(T.ctl + 1, 0u, 1u) == 0u ? 1u : 0u;
                 got = __shfl_sync(FULL, got, 0);
                 if (got) {
@@ -1713,7 +1281,7 @@ __device__ void async_tree_worker(const AzbLayout &L, const AzbAsyncParams &P, c
                 // Every wake-up costs issue slots next to the walking warps, and an answer is tens of microseconds away.  With
                 // take-overs the CTA's idle warps wake at different times, so long naps still bring a sweep round every
                 // microsecond or so; a warp that polls for itself sleeps long at first and then polls every microsecond.
-                __nanosleep(P.nap_long_ns);
+                __nanosleep(AS_NAP_LONG_NS);
                 if ((++idle & 7u) == 0u) {
                     if (as_ld_volatile(&st->abort)) break;
                     if ((idle & 511u) == 0u && as_now() - *reinterpret_cast<const unsigned long long *>(cx.ct + 28) > P.timeout_ns)
@@ -1768,9 +1336,7 @@ __device__ void async_tree_worker(const AzbLayout &L, const AzbAsyncParams &P, c
             // never lap a tile the workers have not retired yet (the ring is sized so that this does not spin)
             const uint32_t q = slot / AS_TILE;
             while (as_ld_volatile(P.tile_retired + (q % P.NT)) < q / P.NT && !as_ld_volatile(&st->abort)) __nanosleep(100);
-#if AS_ACQUIRE
             if (q >= P.NT) (void)as_ld_acquire(P.tile_retired + (q % P.NT));  // the row is overwritten after this
-#endif
             const uint32_t pos = slot % ring_rows;
             tree_pack<true>(L, c, tree, P.ring + (size_t)pos * P.ring_ld);
             // the row of the launch's last step is answered in here like every other (the tree does not wait for it: its
@@ -1789,9 +1355,9 @@ __device__ void async_tree_worker(const AzbLayout &L, const AzbAsyncParams &P, c
         };
         if (cx.err == 0 && cx.wk[WK_STEP] < P.target_step && !(cx.wk[WK_FLAGS] & 1u)) {
             // Early hand-over pays where a tree's own chain (walk -> model -> walk) is the bound, i.e. while there is a
-            // warp for every tree; with several trees per warp it only lengthens the hot loop (32 768 roots: -11 %), so
-            // those launches take the instantiation that submits after the walk.
-            if (P.early)
+            // warp for every tree; with several trees per warp (P.steal) it only lengthens the hot loop (32 768 roots:
+            // -11 %), so those launches take the instantiation that submits after the walk.
+            if (!P.steal)
                 tree_rollout<DEPTH, PUCT>(L, cx, tree, 0u, submit);
             else
                 tree_rollout<DEPTH, PUCT>(L, cx, tree, 0u);
@@ -1900,10 +1466,7 @@ __device__ void async_tree_worker(const AzbLayout &L, const AzbAsyncParams &P, c
     if (lane == 0 && my_rows) atomicAdd(&st->rows_real, my_rows);
 }
 
-// PAIR: the CTA-pair form of the model CTAs (its own instantiation: a kernel that contains cta_group::2 code can only be
-// launched in clusters — the driver refuses anything else as a "cluster misconfiguration" — and a cooperative launch in
-// clusters fails under ncu, so the default form stays free of it and keeps its plain cooperative launch)
-template <int DEPTH, bool COUNT, bool PAIR, bool PUCT = false>  // PUCT: azb_config.selection == AZB_SELECT_PUCT
+template <int DEPTH, bool COUNT, bool PUCT = false>  // PUCT: azb_config.selection == AZB_SELECT_PUCT
 __global__ void __launch_bounds__(AS_THREADS, 1)
     azb_async_kernel(const AzbLayout L, const AzbAsyncParams P, const __grid_constant__ AzbAsyncMaps M) {
     extern __shared__ __align__(1024) uint8_t as_smem[];
@@ -1911,12 +1474,7 @@ __global__ void __launch_bounds__(AS_THREADS, 1)
     __shared__ uint32_t s_role, s_idx;
     // the first CTA to arrive on each of n_workers SMs becomes that SM's model CTA; every other CTA walks trees.  The
     // launch is cooperative with one CTA per SM, so every role is resident from the start.
-    if (threadIdx.x == 0 && PAIR) {
-        // CTA pairs: the launch is clustered (CTAs 2c and 2c + 1 share a TPC), so roles go by cluster — the first
-        // n_workers / 2 clusters serve the model
-        s_role = blockIdx.x < P.n_workers ? 1u : 0u;
-        s_idx = blockIdx.x < P.n_workers ? blockIdx.x : blockIdx.x - P.n_workers;
-    } else if (threadIdx.x == 0 && !P.shared_sm) {
+    if (threadIdx.x == 0 && !P.shared_sm) {
         uint32_t smid;
         asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
         uint32_t role = 0, idx = 0;
@@ -1952,7 +1510,7 @@ __global__ void __launch_bounds__(AS_THREADS, 1)
         }
     } else if (s_role) {
         uint8_t *smem = (uint8_t *)(((uintptr_t)as_smem + 1023) & ~(uintptr_t)1023);
-        async_model_cta<PAIR>(L, P, M, s_idx, smem, s_worker);
+        async_model_cta(L, P, M, s_idx, smem, s_worker);
         return;
     } else {
         if constexpr (DEPTH == 5) {

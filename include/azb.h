@@ -122,8 +122,7 @@ typedef struct azb_config {
                                    pairs per tile below 4096 —, 36 beyond; 16 for N >= 47), or the lock step where the
                                    asynchronous kernel does not apply (no tensor-core model, fewer than 1024 roots,
                                    max_episodes or n_groups set); azb_get_config shows the choice.  Environment, read when the
-                                   handle first runs this way: AZB_ASYNC_GROUP=g (worker SMs per tile), AZB_ASYNC_PAIR=1 (model
-                                   CTAs as CTA pairs of one cluster: tcgen05.mma.cta_group::2, even async_workers),
+                                   handle first runs this way: AZB_ASYNC_GROUP=g (worker SMs per tile),
                                    AZB_ASYNC_STEAL=0/1 (tree scheduling inside a CTA), AZB_ASYNC_FLUSH_NS,
                                    AZB_ASYNC_TIMEOUT_MS (watchdog floor, default 2000). */
     uint32_t selection;         /* AZB_SELECT_*; 0 = the reference's next_action */

@@ -27,11 +27,12 @@ def _same(ha, hb, b):
     assert ha.counters() == hb.counters()
 
 
-@pytest.mark.parametrize("n,b,workers", [(19, 300, 4), (19, 1024, 8), (12, 77, 4), (33, 160, 4), (64, 96, 4)])
-def test_async_equals_lock_step(capi, n, b, workers):
+@pytest.mark.parametrize("n,b,workers,mlp", [(19, 300, 4, "tc"), (19, 1024, 8, "tc"), (12, 77, 4, "tc"), (33, 160, 4, "tc"),
+                                             (64, 96, 4, "tc"), (19, 200, 4, "tc3")])
+def test_async_equals_lock_step(capi, n, b, workers, mlp):
     steps = 36
     parents, masks = capi.generate_roots(5, 0, b, n)
-    kw = dict(prior_mode=capi.PRIOR_MLP, mlp_mode=capi.MLP_TC, max_steps=2 * steps + 2)
+    kw = dict(prior_mode=capi.PRIOR_MLP, mlp_mode=capi.MLP_TC3 if mlp == "tc3" else capi.MLP_TC, max_steps=2 * steps + 2)
     with _mk(capi, n, b, **kw) as lock, _mk(capi, n, b, async_workers=workers, **kw) as asy:
         for h in (lock, asy):
             h.mlp_init(3)
@@ -65,44 +66,6 @@ def test_async_variants_equal_lock_step(capi, monkeypatch, env, n, b, workers):
             h.step(steps)
             h.step(steps)
         _same(lock, asy, b)
-
-
-@pytest.mark.parametrize("n,b,workers,mlp", [(19, 300, 4, "tc"), (19, 129, 2, "tc"), (19, 1, 2, "tc"), (12, 77, 4, "tc"), (19, 1024, 8, "tc"),
-                                             (19, 200, 4, "tc3"), (33, 160, 4, "tc"), (64, 96, 4, "tc")])
-def test_cta_pair_form_equals_lock_step(capi, monkeypatch, n, b, workers, mlp):
-    """AZB_ASYNC_PAIR=1: the model CTAs work as CTA pairs of one cluster — two 128-row tiles per tcgen05.mma.cta_group::2
-    (M = 256), every weight tile fetched once per pair, barriers across the pair, per-pass hand-over of the hidden
-    activations.  A row's dot products run over K in the same order, so the trees are the lock step's, bit for bit."""
-    steps = 36
-    monkeypatch.setenv("AZB_ASYNC_PAIR", "1")
-    parents, masks = capi.generate_roots(5, 0, b, n)
-    kw = dict(prior_mode=capi.PRIOR_MLP, mlp_mode=capi.MLP_TC3 if mlp == "tc3" else capi.MLP_TC, max_steps=2 * steps + 2)
-    with _mk(capi, n, b, **kw) as lock, _mk(capi, n, b, async_workers=workers, **kw) as asy:
-        for h in (lock, asy):
-            h.mlp_init(3)
-            h.set_roots(parents, masks)
-            h.init_trees()
-        n1, log1 = lock.step(steps, cap=256)
-        n2, log2 = asy.step(steps, cap=256)
-        assert n1 == n2 and [tuple(x) for x in log1] == [tuple(x) for x in log2]
-        _same(lock, asy, b)
-        for h in (lock, asy):
-            h.step(1)
-            h.step(steps)
-        _same(lock, asy, b)
-
-
-def test_cta_pair_form_needs_an_even_worker_count(capi, monkeypatch):
-    monkeypatch.setenv("AZB_ASYNC_PAIR", "1")
-    n, b = 19, 64
-    parents, masks = capi.generate_roots(3, 0, b, n)
-    with _mk(capi, n, b, prior_mode=capi.PRIOR_MLP, mlp_mode=capi.MLP_TC, async_workers=3, max_steps=20) as h:
-        h.mlp_init(1)
-        h.set_roots(parents, masks)
-        h.init_trees()
-        with pytest.raises(capi.AzbError) as e:
-            h.step(10)
-        assert e.value.code == capi.ERR_INVALID
 
 
 @pytest.mark.parametrize("steal", ["0", "1"])

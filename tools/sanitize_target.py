@@ -5,17 +5,16 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from azdopt_b200 import capi
 
 CASES = ((19, 24, 30, "tc"), (19, 9, 25, "hash"), (33, 6, 12, "fp32"), (19, 130, 6, "groups"), (19, 200, 10, "async"),
-         (19, 300, 8, "steal"), (19, 300, 8, "pair"), (33, 96, 6, "steal"), (64, 40, 4, "steal"))
+         (19, 300, 8, "steal"), (33, 96, 6, "steal"), (64, 40, 4, "steal"))
 if len(sys.argv) > 1:  # e.g. `sanitize_target.py async`
     CASES = tuple(c for c in CASES if c[3] in sys.argv[1:])
 for n, b, steps, mode in CASES:
     kw = dict(max_steps=steps + 4)
     if mode == "hash":
         kw.update(prior_mode=capi.PRIOR_HASH, max_episodes=2)
-    elif mode in ("async", "steal", "pair"):
+    elif mode in ("async", "steal"):
         kw.update(prior_mode=capi.PRIOR_MLP, mlp_mode=capi.MLP_TC, async_workers=2)
         os.environ["AZB_ASYNC_STEAL"] = "1" if mode == "steal" else "0"  # the table form / the register form of a tree CTA
-        os.environ["AZB_ASYNC_PAIR"] = "1" if mode == "pair" else "0"    # model CTAs as a cluster of two
     elif mode == "groups":
         kw.update(prior_mode=capi.PRIOR_MLP, mlp_mode=capi.MLP_TC, n_groups=2)
     else:
