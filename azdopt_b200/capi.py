@@ -97,6 +97,7 @@ SIGNATURES = {
     "azb_get_priors": (C.c_int, [C.c_void_p, f32p]),
     "azb_eval_costs": (C.c_int, [C.c_void_p, u8p, C.c_uint32, f64p, u32p, f32p, f32p]),
     "azb_eval_graph_costs": (C.c_int, [C.c_void_p, u32p, C.c_uint32, C.c_uint32, f64p, u32p, u32p, f32p]),
+    "azb_eval_graph_costs64": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64), C.c_uint32, C.c_uint32, f64p, u32p, u32p, f32p]),
     "azb_write_observations": (C.c_int, [C.c_void_p, C.c_uint32, f32p, f32p, f32p]),
     "azb_adam_config": (C.c_int, [C.c_void_p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float]),
     "azb_model_update": (C.c_int, [C.c_void_p, f32p, f32p, f32p, C.c_uint32, f32p]),
@@ -396,6 +397,18 @@ class Handle:
         ms = C.c_float()
         self._ck(self._L.azb_eval_graph_costs(self._h, _p(g, C.c_uint32), m, n, _p(lam, C.c_double), _p(mu, C.c_uint32),
                                               _p(kinds, C.c_uint32), C.byref(ms)))
+        return lam, mu, kinds, float(ms.value)
+
+    def eval_graph_costs64(self, nbr):
+        """eval_graph_costs for neighbourhood masks u64[M, n], 2 <= n <= 64 (ConnectedBitsetGraph<N, B64>)."""
+        g = np.ascontiguousarray(nbr, dtype=np.uint64)
+        m, n = g.shape
+        lam = np.zeros(m, dtype=np.float64)
+        mu = np.zeros(m, dtype=np.uint32)
+        kinds = np.zeros((m, (n * (n - 1) + 31) // 32), dtype=np.uint32)
+        ms = C.c_float()
+        self._ck(self._L.azb_eval_graph_costs64(self._h, _p(g, C.c_uint64), m, n, _p(lam, C.c_double), _p(mu, C.c_uint32),
+                                                _p(kinds, C.c_uint32), C.byref(ms)))
         return lam, mu, kinds, float(ms.value)
 
     def write_observations(self, n_obs_tol):

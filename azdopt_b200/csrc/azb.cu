@@ -1432,16 +1432,18 @@ int azb_eval_costs(azb_handle *h, const uint8_t *parents, uint32_t m, double *la
 }
 
 // ---- stand-alone cost + action kinds of connected bitset graphs (SURVEY 8(f) row 3) ----
-int azb_eval_graph_costs(azb_handle *h, const uint32_t *nbr, uint32_t m, uint32_t n, double *lambda1, uint32_t *mu,
-                         uint32_t *kinds, float *ms) {
-    if (!h || !nbr || m == 0) return AZB_ERR_INVALID;
-    if (n < 2 || n > 32) return fail(h, AZB_ERR_INVALID, "graphs have 2..32 vertices (B32 neighbourhoods), got %u", n);
+}  // extern "C"
+
+// shared by the B32 and B64 entries: the slab, the copies, the timing and the error words; `launch` enqueues the kernel
+template <typename W, typename Launch>
+static int eval_graph_costs_dev(azb_handle *h, const char *fn, const W *nbr, uint32_t m, uint32_t n, double *lambda1,
+                                uint32_t *mu, uint32_t *kinds, float *ms, Launch launch) {
     // loops, asymmetric neighbourhoods, neighbours >= N and disconnected inputs are found by the kernel itself
     CK(cudaSetDevice(h->cfg.device));
     const uint32_t kw = (n * (n - 1) + 31) / 32;
     // one slab on the handle, grown when a larger batch arrives (a cudaMalloc per call costs more than the kernel)
     auto up = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    const size_t o_l1 = 0, o_nbr = o_l1 + up((size_t)m * 8), o_mu = o_nbr + up((size_t)m * n * 4), o_kinds = o_mu + up((size_t)m * 4),
+    const size_t o_l1 = 0, o_nbr = o_l1 + up((size_t)m * 8), o_mu = o_nbr + up((size_t)m * n * sizeof(W)), o_kinds = o_mu + up((size_t)m * 4),
                  o_err = o_kinds + up((size_t)m * kw * 4), total = o_err + 256;
     if (total > h->graph_cap) {
         if (h->graph_buf) cudaFree(h->graph_buf);
@@ -1451,19 +1453,17 @@ int azb_eval_graph_costs(azb_handle *h, const uint32_t *nbr, uint32_t m, uint32_
         h->graph_cap = total;
     }
     double *d_l1 = reinterpret_cast<double *>(h->graph_buf + o_l1);
-    uint32_t *d_nbr = reinterpret_cast<uint32_t *>(h->graph_buf + o_nbr), *d_mu = reinterpret_cast<uint32_t *>(h->graph_buf + o_mu),
-             *d_kinds = reinterpret_cast<uint32_t *>(h->graph_buf + o_kinds), *d_err = reinterpret_cast<uint32_t *>(h->graph_buf + o_err);
-    auto release = []() {};
-    cudaError_t ce = cudaMemcpyAsync(d_nbr, nbr, (size_t)m * n * 4, cudaMemcpyHostToDevice, h->stream);
+    W *d_nbr = reinterpret_cast<W *>(h->graph_buf + o_nbr);
+    uint32_t *d_mu = reinterpret_cast<uint32_t *>(h->graph_buf + o_mu), *d_kinds = reinterpret_cast<uint32_t *>(h->graph_buf + o_kinds),
+             *d_err = reinterpret_cast<uint32_t *>(h->graph_buf + o_err);
+    cudaError_t ce = cudaMemcpyAsync(d_nbr, nbr, (size_t)m * n * sizeof(W), cudaMemcpyHostToDevice, h->stream);
     const uint32_t err0[2] = {0u, 0xffffffffu};  // [0] bit AZB_ERR_* per kind of failure, [1] first rejected graph
     if (ce == cudaSuccess) ce = cudaMemcpyAsync(d_err, err0, 8, cudaMemcpyHostToDevice, h->stream);
     if (ce == cudaSuccess) ce = cudaEventRecord(h->ev0, h->stream);
     if (ce == cudaSuccess) {
-        const uint32_t blocks = (m + AZG_WARPS - 1) / AZG_WARPS, smem = AZG_WARPS * azg_warp_bytes(n);
-        if (azg_packed(n)) azb_graph_cost_kernel<true><<<blocks, AZG_WARPS * 32, smem, h->stream>>>(d_nbr, m, n, kw, d_l1, d_mu, d_kinds, d_err);
-        else azb_graph_cost_kernel<false><<<blocks, AZG_WARPS * 32, smem, h->stream>>>(d_nbr, m, n, kw, d_l1, d_mu, d_kinds, d_err);
+        ce = launch(d_nbr, kw, d_l1, d_mu, d_kinds, d_err);
         h->launches += 1;
-        ce = cudaGetLastError();
+        if (ce == cudaSuccess) ce = cudaGetLastError();
     }
     if (ce == cudaSuccess) ce = cudaEventRecord(h->ev1, h->stream);
     uint32_t err[2] = {0u, 0u};
@@ -1473,12 +1473,66 @@ int azb_eval_graph_costs(azb_handle *h, const uint32_t *nbr, uint32_t m, uint32_
     if (ce == cudaSuccess) ce = cudaMemcpyAsync(err, d_err, 8, cudaMemcpyDeviceToHost, h->stream);
     if (ce == cudaSuccess) ce = cudaStreamSynchronize(h->stream);
     if (ce == cudaSuccess && ms) ce = cudaEventElapsedTime(ms, h->ev0, h->ev1);
-    release();
-    if (ce != cudaSuccess) return fail(h, AZB_ERR_CUDA, "azb_eval_graph_costs: %s", cudaGetErrorString(ce));
+    if (ce != cudaSuccess) return fail(h, AZB_ERR_CUDA, "%s: %s", fn, cudaGetErrorString(ce));
     if (err[0] & (1u << AZB_ERR_INVALID))
         return fail(h, AZB_ERR_INVALID, "graph %u is not a connected simple graph (a loop, a neighbour >= N, asymmetric neighbourhoods, or disconnected)", err[1]);
     if (err[0] & (1u << AZB_ERR_LAMBDA)) return fail(h, AZB_ERR_LAMBDA, "%s", azb_strerror(AZB_ERR_LAMBDA));
     return AZB_OK;
+}
+
+extern "C" {
+
+int azb_eval_graph_costs(azb_handle *h, const uint32_t *nbr, uint32_t m, uint32_t n, double *lambda1, uint32_t *mu,
+                         uint32_t *kinds, float *ms) {
+    if (!h || !nbr || m == 0) return AZB_ERR_INVALID;
+    if (n < 2 || n > 32) return fail(h, AZB_ERR_INVALID, "graphs have 2..32 vertices (B32 neighbourhoods), got %u", n);
+    return eval_graph_costs_dev(h, "azb_eval_graph_costs", nbr, m, n, lambda1, mu, kinds, ms,
+                                [&](const uint32_t *d_nbr, uint32_t kw, double *d_l1, uint32_t *d_mu, uint32_t *d_kinds, uint32_t *d_err) {
+        const uint32_t blocks = (m + AZG_WARPS - 1) / AZG_WARPS, smem = AZG_WARPS * azg_warp_bytes(n);
+        if (azg_packed(n)) azb_graph_cost_kernel<true><<<blocks, AZG_WARPS * 32, smem, h->stream>>>(d_nbr, m, n, kw, d_l1, d_mu, d_kinds, d_err);
+        else azb_graph_cost_kernel<false><<<blocks, AZG_WARPS * 32, smem, h->stream>>>(d_nbr, m, n, kw, d_l1, d_mu, d_kinds, d_err);
+        return cudaSuccess;
+    });
+}
+
+}  // extern "C"
+
+// warps per CTA of the B64 kernel: the count among 1, 2, 4 with the most resident warps per SM for this N's
+// shared-memory footprint (19.5 KB per warp at N = 64, 7.6 KB at N = 33); ties go to the larger CTA
+template <bool PACKED>
+static cudaError_t launch_graph_cost64(azb_handle *h, const uint64_t *d_nbr, uint32_t m, uint32_t n, uint32_t kw, double *d_l1,
+                                       uint32_t *d_mu, uint32_t *d_kinds, uint32_t *d_err) {
+    const uint32_t bytes = azg64_warp_bytes(n);
+    uint32_t warps = 1;
+    int best = 0;
+    for (uint32_t wc = 1; wc <= AZG64_MAX_WARPS; wc *= 2) {
+        cudaError_t ce = cudaFuncSetAttribute(azb_graph_cost64_kernel<PACKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(wc * bytes));
+        int blocks = 0;
+        if (ce == cudaSuccess) ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, azb_graph_cost64_kernel<PACKED>, (int)wc * 32, wc * bytes);
+        if (ce != cudaSuccess) return ce;
+        if (blocks * (int)wc >= best) {
+            best = blocks * (int)wc;
+            warps = wc;
+        }
+    }
+    cudaError_t ce = cudaFuncSetAttribute(azb_graph_cost64_kernel<PACKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(warps * bytes));
+    if (ce != cudaSuccess) return ce;
+    azb_graph_cost64_kernel<PACKED><<<(m + warps - 1) / warps, warps * 32, warps * bytes, h->stream>>>(d_nbr, m, n, kw, d_l1, d_mu, d_kinds, d_err);
+    return cudaSuccess;
+}
+
+extern "C" {
+
+int azb_eval_graph_costs64(azb_handle *h, const uint64_t *nbr, uint32_t m, uint32_t n, double *lambda1, uint32_t *mu,
+                           uint32_t *kinds, float *ms) {
+    if (!h || !nbr || m == 0) return AZB_ERR_INVALID;
+    if (n < 2 || n > 64) return fail(h, AZB_ERR_INVALID, "graphs have 2..64 vertices (B64 neighbourhoods), got %u", n);
+    // every n runs the B64 kernel, n <= 32 included: one code path, and bits 32..63 are validated like any other
+    return eval_graph_costs_dev(h, "azb_eval_graph_costs64", nbr, m, n, lambda1, mu, kinds, ms,
+                                [&](const uint64_t *d_nbr, uint32_t kw, double *d_l1, uint32_t *d_mu, uint32_t *d_kinds, uint32_t *d_err) {
+        return azg_packed(n) ? launch_graph_cost64<true>(h, d_nbr, m, n, kw, d_l1, d_mu, d_kinds, d_err)
+                             : launch_graph_cost64<false>(h, d_nbr, m, n, kw, d_l1, d_mu, d_kinds, d_err);
+    });
 }
 
 // ---- results ----

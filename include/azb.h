@@ -247,6 +247,11 @@ int azb_eval_costs(azb_handle *h, const uint8_t *parents /*[M*N]*/, uint32_t m, 
  *      reject); AZB_ERR_LAMBDA where the reference asserts lambda_1 > 1.4.  Any output pointer may be NULL. ---- */
 int azb_eval_graph_costs(azb_handle *h, const uint32_t *nbr /*[M*n]*/, uint32_t m, uint32_t n, double *lambda1,
                          uint32_t *mu, uint32_t *kinds, float *ms);
+/* ---- the same row for ConnectedBitsetGraph<N, B64>: nbr[g*n + v] = u64 neighbourhood of v, 2 <= n <= 64.  Outputs,
+ *      kinds layout (ceil(n(n-1)/32) words per graph, 126 at n = 64) and errors as above; AZB_ERR_INVALID also for
+ *      n outside 2..64 and for any bit >= n (bits 32..63 included when n <= 32). ---- */
+int azb_eval_graph_costs64(azb_handle *h, const uint64_t *nbr /*[M*n]*/, uint32_t m, uint32_t n, double *lambda1,
+                           uint32_t *mu, uint32_t *kinds, float *ms);
 
 /* ---- epoch boundary ("next" rows): par_update_model's observation pass (tree/mod.rs:242-264,
  *      optimizer/mod.rs:262-278) ---- */

@@ -196,10 +196,13 @@ class NablaOptimizer {
     std::vector<float> state_vecs_, h_theta_;
 };
 
-// ---- SURVEY 8(f) row 3: ConnectedBitsetGraph<N, B32> (simple_graph/connected_bitset_graph/mod.rs:18-21) ----
-template <uint32_t N>
+// ---- SURVEY 8(f) row 3: ConnectedBitsetGraph<N, B> (simple_graph/connected_bitset_graph/mod.rs:18-21) over the
+// reference's two bitset words (bitset/primitive.rs): B32 (N <= 32, the default) and B64 (N <= 64) ----
+using B32 = uint32_t;
+using B64 = uint64_t;
+template <uint32_t N, typename B = B32>
 struct ConnectedBitsetGraph {
-    uint32_t neighborhoods[N];  // bit u of neighborhoods[v] <=> uv is an edge
+    B neighborhoods[N];  // bit u of neighborhoods[v] <=> uv is an edge
 };
 struct Conjecture2Dot1Cost {  // mod.rs:340-344; only matching.len() is read anywhere, so the size is what is kept
     double lambda_1;
@@ -217,6 +220,23 @@ std::vector<Conjecture2Dot1Cost> conjecture_2_1_costs(NablaOptimizer &on, const 
     if (action_kinds) action_kinds->assign((size_t)m * kw, 0u);
     const int rc = m ? azb_eval_graph_costs(on.handle(), &graphs[0].neighborhoods[0], m, N, l1.data(), mu.data(),
                                             action_kinds ? action_kinds->data() : nullptr, nullptr)
+                     : AZB_OK;
+    if (rc != AZB_OK) throw Error(rc, std::string(azb_strerror(rc)) + ": " + azb_last_error(on.handle()));
+    std::vector<Conjecture2Dot1Cost> out(m);
+    for (uint32_t i = 0; i < m; ++i) out[i] = {l1[i], mu[i]};
+    return out;
+}
+// the same for ConnectedBitsetGraph<N, B64>
+template <uint32_t N>
+std::vector<Conjecture2Dot1Cost> conjecture_2_1_costs(NablaOptimizer &on, const std::vector<ConnectedBitsetGraph<N, B64>> &graphs,
+                                                      std::vector<uint32_t> *action_kinds = nullptr) {
+    static_assert(N >= 2 && N <= 64, "B64 neighbourhoods");
+    const uint32_t m = (uint32_t)graphs.size(), kw = (N * (N - 1) + 31) / 32;
+    std::vector<double> l1(m);
+    std::vector<uint32_t> mu(m);
+    if (action_kinds) action_kinds->assign((size_t)m * kw, 0u);
+    const int rc = m ? azb_eval_graph_costs64(on.handle(), &graphs[0].neighborhoods[0], m, N, l1.data(), mu.data(),
+                                              action_kinds ? action_kinds->data() : nullptr, nullptr)
                      : AZB_OK;
     if (rc != AZB_OK) throw Error(rc, std::string(azb_strerror(rc)) + ": " + azb_last_error(on.handle()));
     std::vector<Conjecture2Dot1Cost> out(m);

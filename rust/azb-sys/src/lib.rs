@@ -130,6 +130,7 @@ extern "C" {
     pub fn azb_get_priors(h: *mut azb_handle, priors: *mut f32) -> c_int;
     pub fn azb_eval_costs(h: *mut azb_handle, parents: *const u8, m: u32, lambda1: *mut f64, mu: *mut u32, c: *mut f32, ms: *mut f32) -> c_int;
     pub fn azb_eval_graph_costs(h: *mut azb_handle, nbr: *const u32, m: u32, n: u32, lambda1: *mut f64, mu: *mut u32, kinds: *mut u32, ms: *mut f32) -> c_int;
+    pub fn azb_eval_graph_costs64(h: *mut azb_handle, nbr: *const u64, m: u32, n: u32, lambda1: *mut f64, mu: *mut u32, kinds: *mut u32, ms: *mut f32) -> c_int;
     pub fn azb_write_observations(h: *mut azb_handle, n_obs_tol: u32, state_vecs: *mut f32, observations: *mut f32, weights: *mut f32) -> c_int;
     pub fn azb_adam_config(h: *mut azb_handle, lr: f32, beta1: f32, beta2: f32, eps: f32, l2: f32) -> c_int;
     pub fn azb_model_update(h: *mut azb_handle, states: *const f32, observations: *const f32, action_weights: *const f32, rows: u32, loss: *mut f32) -> c_int;
