@@ -41,6 +41,7 @@ struct azb_handle {
     float *params;      // dfdx order, f32
     float *act[3];      // hidden activations of the fp32 path
     float *mlp_x, *mlp_y;
+    uint16_t *sv16_save;  // azb_model_write_predictions: the walkers' bf16 state rows while their buffer serves the call
     uint32_t mlp_rows;  // rows the staging buffers hold
     AzbMlpTc tc;        // tensor-core path state (bf16 weights, activations)
     // stand-alone cost kernel scratch
@@ -207,7 +208,7 @@ int azb_destroy(azb_handle *h) {
         if (p) cudaFree(p);
     void *ptrs[] = {h->grad, h->adam_m, h->adam_v, h->tr_p, h->tr_dz[0], h->tr_dz[1], h->tr_x, h->tr_scal, h->tr_part, h->comm_buf,
                     h->L.walker, h->L.node, h->L.blk, h->L.inl, h->L.key, h->L.hash, h->L.casc, h->L.cand, h->L.stepmin, (void *)h->L.lut, h->L.sv,
-                    h->L.h, h->L.g, h->L.log, h->params, h->act[0], h->act[1], h->act[2], h->mlp_x, h->mlp_y,
+                    h->L.h, h->L.g, h->L.log, h->params, h->act[0], h->act[1], h->act[2], h->mlp_x, h->mlp_y, h->sv16_save,
                     h->cost_par, h->cost_l1, h->cost_mu, h->cost_c, h->cost_err, h->obs, h->obs_w, h->flush_buf, h->graph_buf};
     for (void *p : ptrs)
         if (p) cudaFree(p);
@@ -635,9 +636,18 @@ int azb_model_write_predictions(azb_handle *h, const float *states, float *predi
         CK(dmalloc(h, &h->mlp_x, (size_t)h->L.B * h->S));
         CK(dmalloc(h, &h->mlp_y, (size_t)h->L.B * h->A));
     }
+    // with AZB_PRIOR_MLP on the tensor cores the layer-0 input rows ARE the walkers' state vectors (L.sv16): they are
+    // set aside while the caller's rows pass through and put back afterwards (bf16x3: both halves, so the lo half the
+    // search kernels never write is zero again)
+    const size_t sv16_bytes = h->L.sv16 ? (size_t)rows * h->L.sv16_ld * 2 : 0;
+    if (sv16_bytes) {
+        if (!h->sv16_save) CK(dmalloc(h, &h->sv16_save, (size_t)h->L.B * h->L.sv16_ld));
+        CK(cudaMemcpyAsync(h->sv16_save, h->L.sv16, sv16_bytes, cudaMemcpyDeviceToDevice, h->stream));
+    }
     CK(cudaMemcpyAsync(h->mlp_x, states, (size_t)rows * h->S * 4, cudaMemcpyHostToDevice, h->stream));
     int rc = mlp_forward(h, h->mlp_x, h->S, h->mlp_y, h->A, 0, rows, h->stream);
     if (rc) return rc;
+    if (sv16_bytes) CK(cudaMemcpyAsync(h->L.sv16, h->sv16_save, sv16_bytes, cudaMemcpyDeviceToDevice, h->stream));
     CK(cudaMemcpyAsync(predictions, h->mlp_y, (size_t)rows * h->A * 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return AZB_OK;

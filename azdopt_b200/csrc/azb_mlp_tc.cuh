@@ -342,12 +342,16 @@ static inline const char *azb_mlp_tc_create(AzbMlpTc &t, uint32_t rows, const ui
         // weight rows are padded (zeros) to a multiple of 128 so that a 128-row TMA box never leaves the tensor
         const uint32_t kw = (t.split ? 2u : 1u) * t.kpad[l];  // row width in elements: [hi | lo] when split
         const size_t abytes = (size_t)t.rows_pad * kw * 2, wbytes = (size_t)((t.npad[l] + 127u) / 128u * 128u) * kw * 2;
+        // the epilogue reads the bias 32 columns at a time and a head's npad is only a multiple of 16: the biases are
+        // allocated to the next multiple of 32 floats, the tail zero (azb_params_to_bf16_kernel writes npad of them)
+        const size_t bbytes = (size_t)((t.npad[l] + 31u) & ~31u) * 4;
         if (cudaMalloc((void **)&t.act[l], abytes) != cudaSuccess) return "cudaMalloc (activations) failed";
         if (cudaMalloc((void **)&t.w[l], wbytes) != cudaSuccess) return "cudaMalloc (weights) failed";
-        if (cudaMalloc((void **)&t.bias[l], (size_t)t.npad[l] * 4) != cudaSuccess) return "cudaMalloc (bias) failed";
+        if (cudaMalloc((void **)&t.bias[l], bbytes) != cudaSuccess) return "cudaMalloc (bias) failed";
         cudaMemset(t.act[l], 0, abytes);
         cudaMemset(t.w[l], 0, wbytes);
-        if (dev_bytes) *dev_bytes += abytes + wbytes + (size_t)t.npad[l] * 4;
+        cudaMemset(t.bias[l], 0, bbytes);
+        if (dev_bytes) *dev_bytes += abytes + wbytes + bbytes;
         const char *why = azb_tc_make_map(enc, &t.map_x[l], t.act[l], t.rows_pad, kw, TC_BM);
         if (why) return why;
         why = azb_tc_make_map(enc, &t.map_w[l], t.w[l], t.npad[l], kw, t.bn[l]);
@@ -394,12 +398,6 @@ static inline const char *azb_mlp_tc_forward(AzbMlpTc &t, const float *x, uint32
             head ? ldy : wide * t.kpad[l + 1], row0, row0 + rows, t.dims[l + 1], t.kpad[l] / TC_BK, t.bn[l], t.split ? 3u : 1u,
             head ? 0u : t.kpad[l + 1]);
         if (launches) *launches += 1;
-    }
-    if (x && t.split) {
-        // the search kernels' write_vec only ever writes the hi half of a layer-0 row (its entries are exactly 0 or 1):
-        // leave the lo half of the rows just used as zero as it found them
-        cudaMemset2DAsync(t.act[0] + (size_t)row0 * 2u * t.kpad[0] + t.kpad[0], (size_t)2u * t.kpad[0] * 2, 0, (size_t)t.kpad[0] * 2,
-                          rows, stream);
     }
     return cudaGetLastError() == cudaSuccess ? nullptr : "tensor-core forward launch failed";
 }
