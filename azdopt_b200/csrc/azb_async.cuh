@@ -18,8 +18,8 @@
 //     warpgroups 3-7 shrink to 24 and leave.  A worker takes the next full tile and runs the four Linear layers on
 //     the tensor cores in passes of two 128-column blocks (per 64-deep k-block one activation tile and two weight
 //     tiles, issued as ONE N = 256 MMA per k-step; the 512 TMEM columns hold two passes, so the epilogue of one pass
-//     overlaps the MMAs of the next), hidden activations
-//     round-trip through an L2-resident scratch, the Sigmoid head scatters f32 rows to the owning trees' prior rows
+//     overlaps the MMAs of the next), hidden activations of width <= 512 stay in tensor memory as the next layer's A
+//     operand (single worker, bf16) and the others round-trip through an L2-resident scratch, the Sigmoid head scatters f32 rows to the owning trees' prior rows
 //     and the last writer raises their flags.  A tile that stays partial for `flush_ns` is topped up with dummy rows
 //     and run anyway (tail of the run, tiny batches).
 // Results are identical to the lock-step path: a tree's walk depends only on its own priors, and a row's forward
@@ -208,13 +208,75 @@ __device__ __forceinline__ void as_sts128(uint32_t saddr, uint32_t a, uint32_t b
     asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(saddr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
 __device__ __forceinline__ void as_fence_proxy_async() { asm volatile("fence.proxy.async;" ::: "memory"); }
+__device__ __forceinline__ void as_tmem_st32(uint32_t taddr, const uint32_t (&r)[32]) {
+    asm volatile(
+        "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
+        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
+        "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};" ::"r"(taddr),
+        "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
+        "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]), "r"(r[18]),
+        "r"(r[19]), "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]), "r"(r[27]),
+        "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
+        : "memory");
+}
+// D (+)= A B^T with the A operand [128 x 16] in tensor memory (row = lane, two bf16 per column) and B in shared memory
+__device__ __forceinline__ void as_umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "setp.ne.b32 p, %4, 0;\n"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n"
+        "}\n" ::"r"(tmem_d),
+        "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
+// bias + ReLU of one 16-column TMEM slice, as eight bf16 pairs (half 1, bf16x3 only: what bf16 lost, itself rounded to bf16)
+__device__ __forceinline__ void as_relu_pack(const uint32_t (&r)[16], uint32_t bias_s, uint32_t half, uint32_t *pk) {
+#pragma unroll
+    for (int t = 0; t < 8; t += 2) {
+        const uint4 b4 = as_lds128(bias_s + 2u * t * 4u);
+        float v0 = __uint_as_float(r[2 * t]) + __uint_as_float(b4.x);
+        float v1 = __uint_as_float(r[2 * t + 1]) + __uint_as_float(b4.y);
+        float v2 = __uint_as_float(r[2 * t + 2]) + __uint_as_float(b4.z);
+        float v3 = __uint_as_float(r[2 * t + 3]) + __uint_as_float(b4.w);
+        v0 = fmaxf(v0, 0.f);
+        v1 = fmaxf(v1, 0.f);
+        v2 = fmaxf(v2, 0.f);
+        v3 = fmaxf(v3, 0.f);
+        __nv_bfloat162 h01 = __floats2bfloat162_rn(v0, v1), h23 = __floats2bfloat162_rn(v2, v3);
+        if (half) {
+            h01 = __floats2bfloat162_rn(v0 - __low2float(h01), v1 - __high2float(h01));
+            h23 = __floats2bfloat162_rn(v2 - __low2float(h23), v3 - __high2float(h23));
+        }
+        pk[t] = *reinterpret_cast<uint32_t *>(&h01);
+        pk[t + 1] = *reinterpret_cast<uint32_t *>(&h23);
+    }
+}
 
 // ---------------------------------------------------------------------------------------------------------------
 // Model CTA.  Roles: warp 0 TMA producer and tile taker, warp 1 MMA issuer and TMEM owner (warpgroup 0, 56 registers),
 // warps 4-11 epilogue (warpgroups 1-2, 168 registers).  Each role is its own function with its own copy of the loop
 // over tiles, so that no code is shared between register budgets; they meet at named barrier 1 (AS_MLP_THREADS).
+//
+// Hidden layers in tensor memory.  A single worker (G = 1) with bf16 operands keeps a hidden layer of width <= 512 on
+// chip: the epilogue packs it to bf16 pairs into TMEM columns [0, width / 2) (row = lane), and the next layer's MMAs read
+// their A operand from there (tcgen05.mma with A in TMEM) while only weight tiles stream through the operand ring.  That
+// saves the activation tile the layer would reload once per pass and the L2 round trip with its fences.  TMEM plan of a
+// tile (as_a_in_tmem, as_acc_col):
+//   * a layer whose input comes through shared memory runs passes of AS_ACC blocks, pass p in [256 (p & 1), + 256);
+//     when it produces a TMEM hidden layer (npad <= 512, so at most two passes), pass p's epilogue writes its packed
+//     columns to [128 p, 128 p + 128): in place for p = 0, over pass 0's accumulator for p = 1.  The two epilogue warps
+//     of a TMEM lane quadrant meet at a pair barrier before every packed store, so neither overwrites columns the other
+//     has not read yet;
+//   * a layer whose input is in TMEM keeps its accumulators in [256, 512): one pass of up to AS_ACC blocks, or
+//     128-column passes double-buffered in [256, 384) / [384, 512).  Its MMAs start behind h_bar, which the epilogue
+//     arrives at once the whole hidden layer is stored (tcgen05.wait::st, fence, arrive) — and so once every pass of the
+//     previous layer is drained.  Its own output cannot go to TMEM (it would overwrite the input its later passes read),
+//     so layers alternate and a layer after a TMEM-input layer takes its input from the L2 scratch, behind layer_bar:
+//     that chain also orders the MMAs that read a hidden layer before the MMAs that reuse its columns.
+// G > 1 (a layer is split over SMs) and bf16x3 (hi and lo halves do not fit) keep every hand-over in L2.
 struct AsWorkerShared {
-    uint64_t full_bar[AS_STAGES], empty_bar[AS_STAGES], acc_full[2], acc_empty[2], layer_bar;
+    uint64_t full_bar[AS_STAGES], empty_bar[AS_STAGES], acc_full[2], acc_empty[2], layer_bar, h_bar;
     uint32_t tmem_slot, tile, epi_last;
     uint32_t bias_off[4];  // first entry of layer l's biases in the shared-memory copy
     uint32_t rowtree[AS_TILE];
@@ -232,7 +294,19 @@ __device__ __forceinline__ uint32_t as_blocks_of_member(uint32_t npad, const AsW
     return n_tiles > id.mem ? (n_tiles - id.mem + id.G - 1u) / id.G : 0u;
 }
 #define AS_TILE_BYTES (AS_TILE * TC_BK * 2u)              // one 128 x 64 bf16 operand tile, 16 KB
-#define AS_STAGE_BYTES ((1u + AS_ACC) * AS_TILE_BYTES)    // [A | B0 | B1]
+#define AS_STAGE_BYTES ((1u + AS_ACC) * AS_TILE_BYTES)    // [A | B0 | B1]; weight-only stages (A in TMEM): up to three B tiles
+
+// Layer l reads its A operand from TMEM (see "Hidden layers in tensor memory" above): a single worker, bf16 operands, an
+// input of at most 512 columns (256 packed), and layer l - 1 did not itself read from TMEM
+__device__ __forceinline__ bool as_a_in_tmem(const AzbAsyncParams &P, const uint32_t l) {
+    bool in = false;  // layer 0 reads the ring
+    for (uint32_t j = 1; j <= l; ++j) in = P.group == 1u && P.wide == 1u && P.kpad[j] <= 512u && !in;
+    return in;
+}
+// 128-column blocks per pass: 128-column passes when the input is in TMEM and the layer does not fit one pass
+__device__ __forceinline__ uint32_t as_pass_blocks(const bool a_tmem, const uint32_t mine) { return a_tmem && mine > AS_ACC ? 1u : AS_ACC; }
+// first TMEM column of pass p's accumulator
+__device__ __forceinline__ uint32_t as_acc_col(const bool a_tmem, const uint32_t p) { return a_tmem ? 256u + (p & 1u) * 128u : (p & 1u) * 256u; }
 
 // Lane 0 of a group's first warp: the tile the group answers next (AS_NONE: leave).  The leader (member 0) waits until
 // every member has finished the previous tile (its scratch is reused), takes the next ticket, waits until that tile is
@@ -318,6 +392,7 @@ __device__ __forceinline__ void async_worker_producer(const AzbLayout &L, const 
             tc_mbar_init(&S.acc_empty[a], AS_EPI_WARPS);
         }
         tc_mbar_init(&S.layer_bar, 1);
+        tc_mbar_init(&S.h_bar, AS_EPI_WARPS);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("prefetch.tensormap [%0];" ::"l"(&M.ring) : "memory");
         for (int l = 0; l < 4; ++l) asm volatile("prefetch.tensormap [%0];" ::"l"(&M.w[l]) : "memory");
@@ -355,6 +430,27 @@ __device__ __forceinline__ void async_worker_producer(const AzbLayout &L, const 
                 // this member's blocks nt = mem, mem + G, ... in passes of up to AS_ACC: per k-block ONE A tile and the
                 // pass's B tiles, so a tile's activations are read once per pass instead of once per block
                 const uint32_t mine = as_blocks_of_member(P.npad[l], id);
+                if (as_a_in_tmem(P, l)) {
+                    // A is in TMEM: weight tiles only, up to three per stage (all k-blocks of a pass in order), and no
+                    // layer barrier — the MMA warp waits for the hidden layer itself
+                    const uint32_t pb = as_pass_blocks(true, mine);
+                    for (uint32_t p0 = 0; p0 < mine; p0 += pb) {
+                        const uint32_t np = min(pb, mine - p0), kps = (1u + AS_ACC) / np;
+                        for (uint32_t kb = 0; kb < k_blocks; kb += kps, ++kbc) {
+                            const uint32_t s = kbc % AS_STAGES, ph = (kbc / AS_STAGES) & 1u, nk = min(kps, k_blocks - kb);
+                            uint8_t *dst = smem + (size_t)s * AS_STAGE_BYTES;
+                            const long long tw = AS_CLK();
+                            as_mbar_spin(&S.empty_bar[s], ph ^ 1u);
+                            d_w0 += AS_CLK() - tw;
+                            tc_mbar_expect_tx(&S.full_bar[s], nk * np * AS_TILE_BYTES);
+                            for (uint32_t i = 0; i < nk; ++i)
+                                for (uint32_t j = 0; j < np; ++j)
+                                    as_tma_load_2d_hint(dst + (i * np + j) * AS_TILE_BYTES, &M.w[l], &S.full_bar[s], (int)((kb + i) * TC_BK),
+                                                        (int)((p0 + j) * 128u), w_policy);
+                        }
+                    }
+                    continue;
+                }
                 uint32_t pre = 0;  // k-blocks of the first pass whose weight tiles were requested ahead of the layer barrier
                 if (l > 0) {  // this layer's input is the previous layer's output, written by all members
                     // the weights do not depend on it: while the epilogue warps still drain the previous layer, the
@@ -435,7 +531,7 @@ __device__ __forceinline__ void async_worker_mma(const AzbAsyncParams &P, const 
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = S.tmem_slot;
     const uint32_t G = id.G, mem = id.mem;
-    uint32_t kbc = 0, ntc = 0;
+    uint32_t kbc = 0, ntc = 0, hbc = 0;  // ring stages, passes, hidden layers read from TMEM (phase of h_bar)
     long long d_w0 = 0, d_w1 = 0;
     for (;;) {
         as_named_bar(1, AS_MLP_THREADS);
@@ -444,14 +540,47 @@ __device__ __forceinline__ void async_worker_mma(const AzbAsyncParams &P, const 
         for (uint32_t l = 0; l < 4; ++l) {
             const uint32_t k_blocks = (P.wide == 2u ? 3u : 1u) * (P.kpad[l] / TC_BK);  // all k-segments
             const uint32_t mine = as_blocks_of_member(P.npad[l], id);
-            for (uint32_t p0 = 0; p0 < mine; p0 += AS_ACC, ++ntc) {
-                const uint32_t np = min((uint32_t)AS_ACC, mine - p0);
+            const bool a_tmem = as_a_in_tmem(P, l);
+            const uint32_t pb = as_pass_blocks(a_tmem, mine);
+            for (uint32_t p0 = 0, p = 0; p0 < mine; p0 += pb, ++p, ++ntc) {
+                const uint32_t np = min(pb, mine - p0);
                 long long tw = AS_CLK();
-                const uint32_t slot = ntc & 1u, acc_ph = (ntc >> 1) & 1u;  // TMEM half of this pass, phase of its barriers
+                const uint32_t slot = ntc & 1u, acc_ph = (ntc >> 1) & 1u;  // barriers of this pass and their phase
                 as_mbar_spin(&S.acc_empty[slot], acc_ph ^ 1u);  // the epilogue has drained the pass before last
                 d_w1 += AS_CLK() - tw;
-                const uint32_t tmem_acc = tmem_base + slot * (AS_ACC * 128u);
+                if (a_tmem && p0 == 0u) {  // the hidden layer is in TMEM (and every pass of the previous layer drained)
+                    tw = AS_CLK();
+                    as_mbar_spin(&S.h_bar, hbc & 1u);
+                    ++hbc;
+                    d_w0 += AS_CLK() - tw;
+                }
+                const uint32_t tmem_acc = tmem_base + as_acc_col(a_tmem, p);
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                if (a_tmem) {
+                    // weight-only stages of kps k-blocks; per k-step 16 deep the A operand is 8 packed TMEM columns
+                    const uint32_t kps = (1u + AS_ACC) / np, bn = min(np * 128u, P.npad[l] - p0 * 128u);
+                    const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((bn >> 3) << 17) | ((AS_TILE >> 4) << 24);
+                    for (uint32_t kb = 0; kb < k_blocks; kb += kps, ++kbc) {
+                        const uint32_t s = kbc % AS_STAGES, ph = (kbc / AS_STAGES) & 1u, nk = min(kps, k_blocks - kb);
+                        tw = AS_CLK();
+                        as_mbar_spin(&S.full_bar[s], ph);
+                        d_w0 += AS_CLK() - tw;
+                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                        if (tc_elect_one()) {
+                            const uint32_t st_addr = tc_smem_u32(smem + (size_t)s * AS_STAGE_BYTES);
+                            for (uint32_t i = 0; i < nk; ++i) {
+                                const uint32_t b_addr = st_addr + i * np * AS_TILE_BYTES, ka = tmem_base + (kb + i) * (TC_BK / 2u);
+#pragma unroll
+                                for (uint32_t k = 0; k < TC_BK / 16; ++k)
+                                    as_umma_f16_ts(tmem_acc, ka + k * 8u, tc_smem_desc(b_addr + k * 32u), idesc, ((kb + i) | k) != 0u ? 1u : 0u);
+                            }
+                            tc_umma_commit(&S.empty_bar[s]);
+                            if (kb + nk == k_blocks) tc_umma_commit(&S.acc_full[slot]);
+                        }
+                        __syncwarp();
+                    }
+                    continue;
+                }
                 for (uint32_t kb = 0; kb < k_blocks; ++kb, ++kbc) {
                     const uint32_t s = kbc % AS_STAGES, ph = (kbc / AS_STAGES) & 1u;
                     tw = AS_CLK();
@@ -543,19 +672,42 @@ __device__ __forceinline__ void async_worker_epilogue(const AzbLayout &L, const 
         for (uint32_t l = 0; l < 4; ++l) {
             const float *bias = s_bias + S.bias_off[l];
             const uint32_t mine = as_blocks_of_member(P.npad[l], id);
-            for (uint32_t p0 = 0; p0 < mine; p0 += AS_ACC, ++ntc) {
-                const uint32_t np = min((uint32_t)AS_ACC, mine - p0);
+            const bool a_tmem = as_a_in_tmem(P, l), out_tmem = l < 3u && as_a_in_tmem(P, l + 1u);
+            const uint32_t pb = as_pass_blocks(a_tmem, mine);
+            for (uint32_t p0 = 0, p = 0; p0 < mine; p0 += pb, ++p, ++ntc) {
+                const uint32_t np = min(pb, mine - p0);
                 const long long tw = AS_CLK();
                 const uint32_t slot = ntc & 1u, acc_ph = (ntc >> 1) & 1u;
                 as_mbar_spin(&S.acc_full[slot], acc_ph);
-                const uint32_t tmem_acc = tmem_base + slot * (AS_ACC * 128u);
+                const uint32_t tmem_acc = tmem_base + as_acc_col(a_tmem, p);
                 const long long tb = AS_CLK();
                 d_w0 += tb - tw;
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 for (uint32_t ja = 0; ja < np; ++ja) {
                     const uint32_t nt = mem + (p0 + ja) * G;
                     const uint32_t bn = min(128u, P.npad[l] - nt * 128u);
-                    if (l < 3) {
+                    if (out_tmem) {
+                        // the next layer's A operand: this warp's 64 columns of the block, bias + ReLU, bf16 pairs into TMEM
+                        // column (nt * 128 + col0) / 2 + i of its own lanes.  Those columns belong to pass 0's accumulator;
+                        // the quadrant's other warp has read its part of them once it reaches the pair barrier
+                        uint32_t pk[AS_EPI_COLS / 2];
+                        if (col0 < bn) {
+                            uint32_t r[AS_EPI_SLICES][16];
+                            const long long tl0 = AS_CLK();
+#pragma unroll
+                            for (uint32_t sl = 0; sl < AS_EPI_SLICES; ++sl)
+                                as_tmem_ld16_issue(tmem_acc + ((q4 * 32u) << 16) + ja * 128u + col0 + sl * 16u, r[sl]);
+                            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                            d_acq += AS_CLK() - tl0;
+                            const uint32_t bias_s = tc_smem_u32(bias + nt * 128u + col0);
+#pragma unroll
+                            for (uint32_t sl = 0; sl < AS_EPI_SLICES; ++sl) as_relu_pack(r[sl], bias_s + sl * 64u, 0u, pk + sl * 8u);
+                        }
+                        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                        as_named_bar(4u + q4, 64u);
+                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                        if (col0 < bn) as_tmem_st32(tmem_base + ((q4 * 32u) << 16) + (nt * 128u + col0) / 2u, pk);
+                    } else if (l < 3) {
                         // this warp's 64 columns of the block: four 16-column TMEM slices in flight at once, bias + ReLU,
                         // bf16 pairs into the warp's staging tile [32 rows x 128 B]; 16-byte chunks XOR-swizzled by row,
                         // so these stores and the row-wise reads below are both bank-conflict free
@@ -577,25 +729,7 @@ __device__ __forceinline__ void async_worker_epilogue(const AzbLayout &L, const 
 #pragma unroll
                                 for (uint32_t sl = 0; sl < AS_EPI_SLICES; ++sl) {
                                     uint32_t pk[8];
-#pragma unroll
-                                    for (int t = 0; t < 8; t += 2) {
-                                        const uint4 b4 = as_lds128(bias_s + (sl * 16u + 2u * t) * 4u);
-                                        float v0 = __uint_as_float(r[sl][2 * t]) + __uint_as_float(b4.x);
-                                        float v1 = __uint_as_float(r[sl][2 * t + 1]) + __uint_as_float(b4.y);
-                                        float v2 = __uint_as_float(r[sl][2 * t + 2]) + __uint_as_float(b4.z);
-                                        float v3 = __uint_as_float(r[sl][2 * t + 3]) + __uint_as_float(b4.w);
-                                        v0 = fmaxf(v0, 0.f);
-                                        v1 = fmaxf(v1, 0.f);
-                                        v2 = fmaxf(v2, 0.f);
-                                        v3 = fmaxf(v3, 0.f);
-                                        __nv_bfloat162 h01 = __floats2bfloat162_rn(v0, v1), h23 = __floats2bfloat162_rn(v2, v3);
-                                        if (half) {
-                                            h01 = __floats2bfloat162_rn(v0 - __low2float(h01), v1 - __high2float(h01));
-                                            h23 = __floats2bfloat162_rn(v2 - __low2float(h23), v3 - __high2float(h23));
-                                        }
-                                        pk[t] = *reinterpret_cast<uint32_t *>(&h01);
-                                        pk[t + 1] = *reinterpret_cast<uint32_t *>(&h23);
-                                    }
+                                    as_relu_pack(r[sl], bias_s + sl * 64u, half, pk);
                                     const uint32_t ch = 2u * sl;  // this slice's two 16-byte chunks in the staged row
                                     as_sts128(srow + ((ch ^ sw) << 4), pk[0], pk[1], pk[2], pk[3]);
                                     as_sts128(srow + (((ch + 1u) ^ sw) << 4), pk[4], pk[5], pk[6], pk[7]);
@@ -663,8 +797,16 @@ __device__ __forceinline__ void async_worker_epilogue(const AzbLayout &L, const 
                 if (lane == 0) as_mbar_arrive(&S.acc_empty[slot]);
                 d_busy += AS_CLK() - tb;
             }
-            // ---- layer boundary: this member's share of the layer is stored; tell the group
             const long long tf0 = AS_CLK();
+            if (out_tmem) {  // the hidden layer is in TMEM: the MMA warp reads it behind h_bar
+                asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                __syncwarp();
+                if (lane == 0) as_mbar_arrive(&S.h_bar);
+                d_w1 += AS_CLK() - tf0;
+                continue;
+            }
+            // ---- layer boundary: this member's share of the layer is stored; tell the group
             if (l < 3) as_fence_proxy_async();  // the next layer reads these stores through TMA
             // a single worker hands its hidden activations to its OWN producer warp: the cross-proxy fence, the CTA barrier
             // and the mbarrier's release/acquire are what the memory model asks for.  A GPU-scope fence is needed where
@@ -795,25 +937,7 @@ __device__ __forceinline__ void sh_tmem_ld16_issue(uint32_t taddr, uint32_t (&r)
 // bias + ReLU + bf16 of one 16-column TMEM slice into two 16-byte chunks of the warp's staged row
 __device__ __forceinline__ void sh_relu_pack_store(const uint32_t (&r)[16], uint32_t bias_s, uint32_t half, uint32_t srow, uint32_t ch, uint32_t sw) {
     uint32_t pk[8];
-#pragma unroll
-    for (int t = 0; t < 8; t += 2) {
-        const uint4 b4 = as_lds128(bias_s + 2u * t * 4u);
-        float v0 = __uint_as_float(r[2 * t]) + __uint_as_float(b4.x);
-        float v1 = __uint_as_float(r[2 * t + 1]) + __uint_as_float(b4.y);
-        float v2 = __uint_as_float(r[2 * t + 2]) + __uint_as_float(b4.z);
-        float v3 = __uint_as_float(r[2 * t + 3]) + __uint_as_float(b4.w);
-        v0 = fmaxf(v0, 0.f);
-        v1 = fmaxf(v1, 0.f);
-        v2 = fmaxf(v2, 0.f);
-        v3 = fmaxf(v3, 0.f);
-        __nv_bfloat162 h01 = __floats2bfloat162_rn(v0, v1), h23 = __floats2bfloat162_rn(v2, v3);
-        if (half) {  // bf16x3: what bf16 lost, itself rounded to bf16
-            h01 = __floats2bfloat162_rn(v0 - __low2float(h01), v1 - __high2float(h01));
-            h23 = __floats2bfloat162_rn(v2 - __low2float(h23), v3 - __high2float(h23));
-        }
-        pk[t] = *reinterpret_cast<uint32_t *>(&h01);
-        pk[t + 1] = *reinterpret_cast<uint32_t *>(&h23);
-    }
+    as_relu_pack(r, bias_s, half, pk);
     as_sts128(srow + ((ch ^ sw) << 4), pk[0], pk[1], pk[2], pk[3]);
     as_sts128(srow + (((ch + 1u) ^ sw) << 4), pk[4], pk[5], pk[6], pk[7]);
 }
