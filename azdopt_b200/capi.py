@@ -87,6 +87,8 @@ SIGNATURES = {
     "azb_add_actions_host": (C.c_int, [C.c_void_p, f32p, C.POINTER(C.c_int)]),
     "azb_get_argmin": (C.c_int, [C.c_void_p, u8p, u32p, f64p, u32p, f32p]),
     "azb_get_node_state": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, u8p, u32p]),
+    "azb_tree_codes": (C.c_int, [C.c_void_p, u8p, C.c_uint32, C.POINTER(C.c_uint64), f32p]),
+    "azb_best_trees": (C.c_int, [C.c_void_p, C.c_uint32, u32p, f32p, C.POINTER(C.c_uint64), u32p, u32p, u8p, u32p, f64p, u32p]),
     "azb_get_walkers": (C.c_int, [C.c_void_p, u8p, u32p, u32p, u32p, u32p]),
     "azb_tree_sizes": (C.c_int, [C.c_void_p, C.c_uint32, u32p, u32p, u32p]),
     "azb_dump_tree": (C.c_int, [C.c_void_p, C.c_uint32, u32p, u32p, u32p, u32p]),
@@ -475,6 +477,31 @@ class Handle:
         permitted = np.zeros(self.w, dtype=np.uint32)
         self._ck(self._L.azb_get_node_state(self._h, tree, node, _p(parents, C.c_uint8), _p(permitted, C.c_uint32)))
         return parents, permitted
+
+    def tree_codes(self, parents):
+        """Canonical codes u64[M, 2] of M trees given as parent arrays u8[M, N] (include/azb.h): equal rows <=> isomorphic."""
+        p = np.ascontiguousarray(parents, dtype=np.uint8)
+        m = p.shape[0]
+        if p.shape != (m, self.n):
+            raise ValueError("parent rows")
+        codes = np.zeros((m, 2), dtype=np.uint64)
+        self._ck(self._L.azb_tree_codes(self._h, _p(p, C.c_uint8), m, _p(codes, C.c_uint64), None))
+        return codes
+
+    def best_trees(self, k: int):
+        """The k best isomorphism classes among all nodes of all trees (azb_best_trees), ascending by (eval, code):
+        dict of arrays eval f32, code u64[., 2], tree, node, parents u8[., N], permitted u32[., W], lambda1 f64, mu."""
+        kk = max(int(k), 1)
+        out = dict(eval=np.zeros(kk, dtype=np.float32), code=np.zeros((kk, 2), dtype=np.uint64),
+                   tree=np.zeros(kk, dtype=np.uint32), node=np.zeros(kk, dtype=np.uint32),
+                   parents=np.zeros((kk, self.n), dtype=np.uint8), permitted=np.zeros((kk, self.w), dtype=np.uint32),
+                   lambda1=np.zeros(kk, dtype=np.float64), mu=np.zeros(kk, dtype=np.uint32))
+        n = C.c_uint32()
+        self._ck(self._L.azb_best_trees(self._h, k, C.byref(n), _p(out["eval"], C.c_float), _p(out["code"], C.c_uint64),
+                                        _p(out["tree"], C.c_uint32), _p(out["node"], C.c_uint32),
+                                        _p(out["parents"], C.c_uint8), _p(out["permitted"], C.c_uint32),
+                                        _p(out["lambda1"], C.c_double), _p(out["mu"], C.c_uint32)))
+        return {name: a[:n.value] for name, a in out.items()}
 
     def comm_allreduce_bench(self, reps: int = 20) -> float:
         ms = C.c_float()

@@ -25,6 +25,7 @@
 #include "azb_tree.cuh"
 #include "azb_train.cuh"
 #include "azb_async.cuh"
+#include "azb_best.cuh"
 
 #include <dlfcn.h>
 
@@ -53,6 +54,12 @@ struct azb_handle {
     uint32_t cost_cap;
     uint8_t *graph_buf;  // azb_eval_graph_costs: one grow-only slab [l1 | nbr | mu | kinds | err]
     size_t graph_cap;
+    // azb_tree_codes / azb_best_trees (azb_best.cuh): one grow-only slab, the selection round's state, and the cap on the
+    // first round's M that tests set through AZB_TEST_BEST_CAP (0 = none)
+    uint8_t *best_buf;
+    size_t best_cap;
+    AzbBestState *best_st;
+    uint32_t best_m_cap;
     // observations scratch
     float *obs, *obs_w;
     // training step (azb_train.cuh): gradient (parameter order), Adam moments, predictions, two dZ buffers, scalars
@@ -209,7 +216,8 @@ int azb_destroy(azb_handle *h) {
     void *ptrs[] = {h->grad, h->adam_m, h->adam_v, h->tr_p, h->tr_dz[0], h->tr_dz[1], h->tr_x, h->tr_scal, h->tr_part, h->comm_buf,
                     h->L.walker, h->L.node, h->L.blk, h->L.inl, h->L.key, h->L.hash, h->L.casc, h->L.cand, h->L.stepmin, (void *)h->L.lut, h->L.sv,
                     h->L.h, h->L.g, h->L.log, h->params, h->act[0], h->act[1], h->act[2], h->mlp_x, h->mlp_y, h->sv16_save,
-                    h->cost_par, h->cost_l1, h->cost_mu, h->cost_c, h->cost_err, h->obs, h->obs_w, h->flush_buf, h->graph_buf};
+                    h->cost_par, h->cost_l1, h->cost_mu, h->cost_c, h->cost_err, h->obs, h->obs_w, h->flush_buf, h->graph_buf,
+                    h->best_buf, h->best_st};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     azb_mlp_tc_destroy(h->tc);
@@ -358,6 +366,8 @@ int azb_create(const azb_config *cfg_in, azb_handle **out) {
     L.frontier_cap = AZB_FRONTIER_CAP;
     if (const char *e = getenv("AZB_TEST_FRONTIER_CAP"))  // tests: push ordinary cascades through the global continuation
         L.frontier_cap = std::min<uint32_t>(AZB_FRONTIER_CAP, std::max(1, atoi(e)));
+    if (const char *e = getenv("AZB_TEST_BEST_CAP"))  // tests: force azb_best_trees through several widening rounds
+        h->best_m_cap = (uint32_t)std::max(1, atoi(e));
     L.first_root = cfg.first_root;
     L.prior_seed = cfg.prior_seed;
     CK(dmalloc(h, &L.walker, (size_t)B * L.WS));
@@ -1777,6 +1787,164 @@ extern "C" int azb_get_node_state(azb_handle *h, uint32_t tree, uint32_t node, u
         parents[child] = (uint8_t)(a - first);
         for (uint32_t q = first; q < first + child; ++q) permitted[q >> 5] &= ~(1u << (q & 31));
     }
+    return AZB_OK;
+}
+
+// ---- the k best isomorphism classes (azb_best.cuh) ----
+static size_t best_up(size_t x) { return (x + 255) & ~(size_t)255; }
+
+// the grow-only slab of azb_tree_codes / azb_best_trees (counted in azb_device_bytes)
+static int best_slab(azb_handle *h, size_t bytes) {
+    if (bytes <= h->best_cap) return AZB_OK;
+    if (h->best_buf) {
+        CK(cudaStreamSynchronize(h->stream));
+        CK(cudaFree(h->best_buf));
+        h->dev_bytes -= h->best_cap;
+    }
+    h->best_buf = nullptr;
+    h->best_cap = 0;
+    CK(dmalloc(h, &h->best_buf, bytes));
+    h->best_cap = bytes;
+    return AZB_OK;
+}
+
+static void launch_code_kernel(azb_handle *h, const uint8_t *dev_parents, uint32_t m, unsigned long long *codes, uint32_t stride,
+                               uint32_t *bad) {
+    azb_tree_code_kernel<<<(m + AZB_CODE_WARPS - 1) / AZB_CODE_WARPS, AZB_CODE_WARPS * 32, 0, h->stream>>>(dev_parents, m, h->N, codes,
+                                                                                                        stride, bad);
+    h->launches += 1;
+}
+
+extern "C" int azb_tree_codes(azb_handle *h, const uint8_t *parents, uint32_t m, uint64_t *codes, float *ms) {
+    if (!h || !parents || m == 0) return AZB_ERR_INVALID;
+    CK(cudaSetDevice(h->cfg.device));
+    const size_t o_codes = best_up((size_t)m * h->N), o_bad = o_codes + best_up((size_t)m * 16);
+    int rc = best_slab(h, o_bad + 256);
+    if (rc) return rc;
+    uint8_t *d_par = h->best_buf;
+    unsigned long long *d_codes = reinterpret_cast<unsigned long long *>(h->best_buf + o_codes);
+    uint32_t *d_bad = reinterpret_cast<uint32_t *>(h->best_buf + o_bad);
+    CK(cudaMemcpyAsync(d_par, parents, (size_t)m * h->N, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemsetAsync(d_bad, 0xff, 4, h->stream));
+    CK(cudaEventRecord(h->ev0, h->stream));
+    launch_code_kernel(h, d_par, m, d_codes, 2, d_bad);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(h->ev1, h->stream));
+    uint32_t bad = 0;
+    if (codes) CK(cudaMemcpyAsync(codes, d_codes, (size_t)m * 16, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (ms) CK(cudaEventElapsedTime(ms, h->ev0, h->ev1));
+    if (bad != AZB_NONE) {
+        for (uint32_t v = 1; v < h->N; ++v)
+            if (parents[(size_t)bad * h->N + v] >= v) return fail(h, AZB_ERR_INVALID, "tree %u: parents[%u] is not < %u", bad, v, v);
+    }
+    return AZB_OK;
+}
+
+// One selection round per pass of the loop: the M-th smallest ord(c) over all node records is T, every node with
+// ord(c) <= T is a candidate, and the distinct codes among the candidates are classes whose value (<= T) and
+// representative are exact; every class not found has a value above T.  While fewer than k classes came out and some
+// node was left out, the next round asks for twice the candidates.
+extern "C" int azb_best_trees(azb_handle *h, uint32_t k, uint32_t *n_out, float *eval, uint64_t *codes, uint32_t *tree,
+                              uint32_t *node, uint8_t *parents, uint32_t *permitted, double *lambda1, uint32_t *mu) {
+    if (!h) return AZB_ERR_INVALID;
+    if (!h->trees_init) return fail(h, AZB_ERR_STATE, "azb_init_trees has not been called");
+    if (k == 0 || k > AZB_BEST_MAX_K) return fail(h, AZB_ERR_INVALID, "k must be in 1..%u, got %u", AZB_BEST_MAX_K, k);
+    CK(cudaSetDevice(h->cfg.device));
+    // behind any enqueued steps, and their errors first (the trees may be incomplete after one)
+    int rc = check_device_error(h);
+    if (rc) return rc;
+    if (!h->best_st) CK(dmalloc(h, &h->best_st, 1));
+    const AzbLayout &L = h->L;
+    const uint32_t N = h->N, W = h->W;
+    const int grid = (int)std::min<uint32_t>(L.B, 1184u);
+    uint32_t M = 4u * k;
+    if (h->best_m_cap) M = std::min(M, h->best_m_cap);
+    AzbBestState st;
+    size_t o_b = 0, o_par = 0, o_perm = 0, o_tmp = 0, tmp_bytes = 0;
+    AzbCand *d_a = nullptr, *d_b = nullptr;
+    for (;;) {
+        CK(cudaMemsetAsync(h->best_st, 0, sizeof(AzbBestState), h->stream));
+        CK(cudaMemsetAsync(&h->best_st->bad, 0xff, 4, h->stream));
+        for (int shift = 24; shift >= 0; shift -= 8) {
+            azb_best_hist_kernel<<<grid, 256, 0, h->stream>>>(L, h->best_st, (uint32_t)shift);
+            azb_best_pick_kernel<<<1, 1, 0, h->stream>>>(h->best_st, (uint32_t)shift, M);
+            h->launches += 2;
+        }
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(&st, h->best_st, sizeof(st), cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        const uint32_t C = st.count;
+        if (C == 0) return fail(h, AZB_ERR_STATE, "the trees hold no node");
+        size_t t1 = 0, t2 = 0;
+        CK(cub::DeviceRadixSort::SortKeys(nullptr, t1, (const AzbCand *)nullptr, (AzbCand *)nullptr, C, AzbByCode{}, h->stream));
+        CK(cub::DeviceRadixSort::SortKeys(nullptr, t2, (const AzbCand *)nullptr, (AzbCand *)nullptr, C, AzbByValue{}, h->stream));
+        tmp_bytes = std::max(t1, t2);
+        o_b = best_up((size_t)C * sizeof(AzbCand));
+        o_par = 2 * o_b;
+        o_perm = o_par + best_up((size_t)C * N);
+        o_tmp = o_perm + best_up((size_t)C * W * 4);
+        rc = best_slab(h, o_tmp + tmp_bytes);
+        if (rc) return rc;
+        d_a = reinterpret_cast<AzbCand *>(h->best_buf);
+        d_b = reinterpret_cast<AzbCand *>(h->best_buf + o_b);
+        uint8_t *d_par = h->best_buf + o_par;
+        const uint32_t blocks = (C + 255) / 256;
+        azb_best_compact_kernel<<<grid, 256, 0, h->stream>>>(L, h->best_st, d_a);
+        azb_best_replay_kernel<<<blocks, 256, 0, h->stream>>>(L, d_a, C, d_par, nullptr);
+        launch_code_kernel(h, d_par, C, reinterpret_cast<unsigned long long *>(d_a), sizeof(AzbCand) / 8, &h->best_st->bad);
+        h->launches += 2;
+        CK(cudaGetLastError());
+        CK(cub::DeviceRadixSort::SortKeys(h->best_buf + o_tmp, tmp_bytes, d_a, d_b, C, AzbByCode{}, h->stream));
+        azb_best_heads_kernel<<<blocks, 256, 0, h->stream>>>(d_b, C, d_a, h->best_st);
+        h->launches += 1;
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(&st, h->best_st, sizeof(st), cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        if (st.bad != 0xffffffffu) {
+            // a rejected candidate keeps the all-zero code of the compaction (a code starts with 1), so it sorted first
+            AzbCand c0;
+            CK(cudaMemcpyAsync(&c0, d_b, sizeof(c0), cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+            return fail(h, AZB_ERR_INVALID, "tree %u node %u: the replayed parent array has parents[v] >= v", (uint32_t)(c0.id >> 20),
+                        (uint32_t)(c0.id & 0xfffffu));
+        }
+        if (st.n_class >= k || C >= st.total) break;
+        M = 2u * C > C ? 2u * C : 0xffffffffu;
+    }
+    const uint32_t n_cls = st.n_class, n = std::min(k, n_cls);
+    CK(cub::DeviceRadixSort::SortKeys(h->best_buf + o_tmp, tmp_bytes, d_a, d_b, n_cls, AzbByValue{}, h->stream));
+    uint8_t *d_par = h->best_buf + o_par;
+    uint32_t *d_perm = reinterpret_cast<uint32_t *>(h->best_buf + o_perm);
+    azb_best_replay_kernel<<<(n + 255) / 256, 256, 0, h->stream>>>(L, d_b, n, d_par, d_perm);
+    h->launches += 1;
+    CK(cudaGetLastError());
+    rc = cost_buffers(h, n);
+    if (rc) return rc;
+    CK(cudaMemsetAsync(h->cost_err, 0, 4, h->stream));
+    launch_cost_kernel(h, d_par, n);
+    CK(cudaGetLastError());
+    std::vector<AzbCand> cls(n);
+    uint32_t cerr = 0;
+    CK(cudaMemcpyAsync(cls.data(), d_b, (size_t)n * sizeof(AzbCand), cudaMemcpyDeviceToHost, h->stream));
+    if (parents) CK(cudaMemcpyAsync(parents, d_par, (size_t)n * N, cudaMemcpyDeviceToHost, h->stream));
+    if (permitted) CK(cudaMemcpyAsync(permitted, d_perm, (size_t)n * W * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (lambda1) CK(cudaMemcpyAsync(lambda1, h->cost_l1, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (mu) CK(cudaMemcpyAsync(mu, h->cost_mu, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(&cerr, h->cost_err, 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (cerr) return fail(h, (int)cerr, "%s", azb_strerror((int)cerr));
+    for (uint32_t i = 0; i < n; ++i) {
+        if (eval) eval[i] = azb_ord2f(cls[i].c);
+        if (codes) {
+            codes[2 * i] = cls[i].hi;
+            codes[2 * i + 1] = cls[i].lo;
+        }
+        if (tree) tree[i] = (uint32_t)(cls[i].id >> 20);
+        if (node) node[i] = (uint32_t)(cls[i].id & 0xfffffu);
+    }
+    if (n_out) *n_out = n;
     return AZB_OK;
 }
 

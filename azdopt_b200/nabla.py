@@ -71,6 +71,45 @@ class ArgminData:  # log.rs:1-11
     eval: np.float32
 
 
+@dataclasses.dataclass
+class BestTree:
+    """One isomorphism class of azb_best_trees: its value, its representative node's state and cost, the canonical
+    code (two 64-bit words, include/azb.h) and where the representative lives (global root index, node)."""
+    eval: np.float32
+    lambda_1: float
+    mu: int
+    parents: np.ndarray
+    permitted: np.ndarray
+    code: tuple
+    root: int
+    node: int
+
+
+class BestTrees:
+    """The k best isomorphism classes over many best_trees lists (epochs, shards), ascending by (eval, code).  A class
+    seen again keeps its existing entry unless the new one has a lower eval, so lists added in epoch or rank order keep
+    the earliest representative.  Trimming to k after every merge is exact: a class in the top k of the union is in the
+    top k of the list that holds its minimum, because every class ahead of it there is ahead of it in the union."""
+
+    def __init__(self, k: int):
+        if k < 1:
+            raise ValueError("k >= 1")
+        self.k = k
+        self._by_code = {}
+
+    def add(self, trees) -> "BestTrees":
+        for t in trees:
+            cur = self._by_code.get(t.code)
+            if cur is None or np.float32(t.eval) < np.float32(cur.eval):
+                self._by_code[t.code] = t
+        keep = self.result()
+        self._by_code = {t.code: t for t in keep}
+        return self
+
+    def result(self) -> list:
+        return sorted(self._by_code.values(), key=lambda t: (np.float32(t.eval), t.code))[:self.k]
+
+
 class NablaOptimizer:
     def __init__(self):
         raise TypeError("use NablaOptimizer.par_new")
@@ -179,6 +218,16 @@ class NablaOptimizer:
     def argmin_data(self) -> ArgminData:  # optimizer/mod.rs:361-363
         a = self.h.argmin()
         return ArgminData(a["parents"], a["permitted"], a["lambda1"], a["mu"], a["eval"])
+
+    def best_trees(self, k: int) -> list:
+        """The k best isomorphism classes among every node the search has evaluated since the last reset
+        (azb_best_trees), as BestTree records ascending by (eval, code).  Call it before par_reset_trees, which
+        discards the trees; a BestTrees accumulator merges the lists of several epochs."""
+        r = self.h.best_trees(k)
+        first = int(self.h.cfg.first_root)
+        return [BestTree(r["eval"][i], float(r["lambda1"][i]), int(r["mu"][i]), r["parents"][i].copy(),
+                         r["permitted"][i].copy(), (int(r["code"][i, 0]), int(r["code"][i, 1])), first + int(r["tree"][i]),
+                         int(r["node"][i])) for i in range(len(r["eval"]))]
 
     def par_update_model_observations(self, n_obs_tol: int):
         """The data par_update_model hands to NablaModel::update_model (optimizer/mod.rs:253-280):

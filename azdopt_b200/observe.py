@@ -47,6 +47,31 @@ def graph6_of_state(parents: Sequence[int]) -> bytes:
     return graph6_from_edges(len(parents), tree_edges(parents))
 
 
+# ---- canonical code of a tree (include/azb.h: azb_tree_codes) -------------------------------------------------------
+def tree_code(parents: Sequence[int]) -> Tuple[int, int]:
+    """The canonical code of the tree with edges {v, parents[v]} (parents[v] < v), as two 64-bit words: the maximum over
+    the centres r of enc(r) = 1 . enc(c_1) ... enc(c_d) . 0 with the children's codes in descending order, string bit i
+    at bit 63 - i % 64 of word i // 64.  Equal codes <=> isomorphic trees.  The plain statement azb_tree_codes is
+    checked against."""
+    n = len(parents)
+    adj = [[] for _ in range(n)]
+    for v in range(1, n):
+        p = int(parents[v])
+        if not 0 <= p < v:
+            raise ValueError(f"parents[{v}] = {p} is not < {v}")
+        adj[v].append(p)
+        adj[p].append(v)
+    alive = set(range(n))
+    while len(alive) > 2:  # the centres: strip every leaf at once
+        alive -= {v for v in alive if sum(u in alive for u in adj[v]) <= 1}
+
+    def enc(v, up):
+        return "1" + "".join(sorted((enc(u, v) for u in adj[v] if u != up), reverse=True)) + "0"
+
+    bits = int(max(enc(r, -1) for r in alive).ljust(128, "0"), 2)
+    return bits >> 64, bits & ((1 << 64) - 1)
+
+
 # ---- Graphviz ------------------------------------------------------------------------------------------------------
 def search_tree_dot(dump: dict) -> str:
     """DOT text of one SearchTree from its canonical dump (capi.Handle.dump_tree / the oracle's dump): node label

@@ -43,3 +43,19 @@ def sum_counters(counters: dict, dist=None, device="cpu") -> dict:
     t = torch.tensor([counters[k] for k in keys], dtype=torch.int64, device=device)
     dist.all_reduce(t)
     return {k: int(v) for k, v in zip(keys, t.cpu().tolist())}
+
+
+def global_best_trees(local: list, k: int, dist=None) -> list:
+    """The k best isomorphism classes over all ranks: every rank's best_trees list (nabla.BestTree records) gathered
+    and merged in rank order, so a class found on several ranks at one value keeps the lowest rank's representative —
+    the lowest global root, as one unsharded handle would pick."""
+    from .nabla import BestTrees
+
+    if dist is None or not dist.is_initialized() or dist.get_world_size() == 1:
+        return BestTrees(k).add(local).result()
+    lists = [None] * dist.get_world_size()
+    dist.all_gather_object(lists, list(local))
+    acc = BestTrees(k)
+    for lst in lists:
+        acc.add(lst)
+    return acc.result()

@@ -31,6 +31,8 @@ def main():
     ap.add_argument("--n-obs-tol", type=int, default=200)   # :135
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--out", default="c21_out")
+    ap.add_argument("--best", type=int, default=0, metavar="K",
+                    help="also keep the K best non-isomorphic trees over all epochs in best_trees.g6")
     args = ap.parse_args()
     os.makedirs(args.out, exist_ok=True)
     space = nabla.ROTModifyParentsOnce(n=N)
@@ -38,6 +40,7 @@ def main():
     roots = capi.generate_roots(args.seed, 0, args.batch, N)  # ROTWithActionPermissions::generate, k ~ U{5..A/2} (:85,108-112)
     opt = nabla.NablaOptimizer.par_new(space, roots, model, args.batch, max_steps=args.episodes)
     goal = squish(5.2)                                         # :117
+    best = nabla.BestTrees(args.best) if args.best else None
     with open(os.path.join(args.out, "tfevents-losses"), "wb") as f:
         writer = observe.TensorboardWriter(f)
         writer.write_file_version()
@@ -52,6 +55,8 @@ def main():
         for epoch in range(1, args.epochs + 1):
             print(f"==== EPOCH: {epoch} ====")
             improved = opt.roll_out(args.episodes)             # the inner loop :141-150, fused on the device
+            if best:                                           # every node of this epoch's trees, before the reset
+                best.add(opt.best_trees(args.best))
             for (step, tree, node, ev) in improved:
                 print(f"  step {args.episodes * (epoch - 1) + step + 1}: tree {tree} node {node} eval {ev:.6f}")
             if improved and process_argmin(opt.argmin_data(), args.episodes * epoch):
@@ -68,6 +73,10 @@ def main():
     with open(os.path.join(args.out, "best.g6"), "wb") as g:
         g.write(opt.argmin_graph6() + b"\n")
     print("best tree (graph6):", opt.argmin_graph6().decode())
+    if best:
+        with open(os.path.join(args.out, "best_trees.g6"), "wb") as g:
+            for t in best.result():
+                g.write(observe.graph6_of_state(t.parents) + f" {t.eval:.9g}\n".encode())
     opt.close()
     return 0
 

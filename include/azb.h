@@ -215,6 +215,33 @@ int azb_get_argmin(azb_handle *h, uint8_t *parents /*[N]*/, uint32_t *permitted 
  * par_update_argmmim_data does for the winning node (optimizer/mod.rs:224-239).  Does not wait for enqueued steps, so
  * an azb_step_poll record (tree, node) can be turned into ArgminData while later steps still run. */
 int azb_get_node_state(azb_handle *h, uint32_t tree, uint32_t node, uint8_t *parents /*[N]*/, uint32_t *permitted /*[W]*/);
+/* ---- extension (no reference item): canonical codes of trees and the k best isomorphism classes the search has
+ *      evaluated.
+ * The code of a tree T on N vertices (a parent array: edges {v, parents[v]} for v = 1..N-1, parents[v] < v) ignores the
+ * root and the labels.  The centres are the vertices of minimum eccentricity (one or two).  For the tree rooted at r,
+ * enc(v) = 1 . enc(c_1) . ... . enc(c_d) . 0 with the children ordered so that enc(c_1) >= ... >= enc(c_d)
+ * lexicographically (1 > 0); every enc is a prime Dyck word, so none is a proper prefix of another and the first
+ * differing bit decides.  code(T) = the maximum over the centres r of enc(r), exactly 2N bits, stored in two uint64_t
+ * words: string bit i is bit 63 - i % 64 of word i / 64, unused bits 0, so comparing (word0, word1) as unsigned integers
+ * compares the strings.  Two trees on N vertices have equal codes <=> they are isomorphic.
+ * azb_tree_codes: the codes of M trees of the handle's N (parents[v] < v, as azb_eval_costs checks; AZB_ERR_INVALID
+ * names the first tree that breaks it).  ms (may be NULL) = device time of the kernel alone; codes may be NULL. */
+int azb_tree_codes(azb_handle *h, const uint8_t *parents /*[M*N]*/, uint32_t m, uint64_t *codes /*[M*2]*/, float *ms);
+/* azb_best_trees: the k best isomorphism classes among ALL nodes (0..n_nodes-1) of ALL trees of the handle, at call time.
+ * A class is one isomorphism class (one code) among the states of all nodes of all trees.  The value of a class is the
+ * minimum c over its member nodes (at N >= 23 the cost is a labelling-dependent sectioning program, so isomorphic trees
+ * may differ in the last bit of c: equal codes do not mean equal c).  The representative is, among the members whose c
+ * equals the class value, the one with the smallest (first_root + tree, node), so a sharded run picks what one unsharded
+ * handle would.  Classes are sorted ascending by (value, code) and the first min(k, #classes) are returned; *n_out is
+ * that count.  Per class: eval = the class value; tree, node = the representative's local indices; parents, permitted =
+ * exactly what azb_get_node_state(tree, node) returns; lambda1, mu = the cost kernel on the representative's parents, as
+ * azb_get_argmin does (eval equals that node's stored c bits).  Any output pointer may be NULL.  The call is enqueued on
+ * the library stream behind any enqueued steps and reports their errors.  AZB_ERR_STATE before azb_init_trees;
+ * AZB_ERR_INVALID for k == 0 or k > 65536, and for parent arrays azb_eval_costs would reject, naming the first bad tree.
+ * The call changes nothing: no tree, walker, counter, argmin or RNG state. */
+int azb_best_trees(azb_handle *h, uint32_t k, uint32_t *n_out, float *eval /*[k]*/, uint64_t *codes /*[k*2]*/,
+                   uint32_t *tree /*[k]*/, uint32_t *node /*[k]*/, uint8_t *parents /*[k*N]*/,
+                   uint32_t *permitted /*[k*W]*/, double *lambda1 /*[k]*/, uint32_t *mu /*[k]*/);
 /* persistent walker state: states, paths, last_positions (optimizer/mod.rs:10-14) */
 int azb_get_walkers(azb_handle *h, uint8_t *parents, uint32_t *permitted, uint32_t *path, uint32_t *pos,
                     uint32_t *path_len);

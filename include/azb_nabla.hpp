@@ -30,6 +30,13 @@ struct ArgminData {  // log.rs:1-11
     float eval = 0;
 };
 
+// one isomorphism class of best_trees: the representative's ArgminData, the canonical code (azb.h), its tree and node
+struct BestTree {
+    ArgminData data;
+    uint64_t code[2] = {0, 0};
+    uint32_t tree = 0, node = 0;
+};
+
 // NablaModel (nabla/model/mod.rs:4-8) for models that live on the host
 struct NablaModel {
     virtual ~NablaModel() = default;
@@ -132,6 +139,33 @@ class NablaOptimizer {
         d.permitted.resize(w_);
         ck(azb_get_argmin(h_, d.parents.data(), d.permitted.data(), &d.lambda_1, &d.mu, &d.eval));
         return d;
+    }
+    // the k best isomorphism classes among every node of the trees (azb_best_trees), ascending by (eval, code); call it
+    // before par_reset_trees, which discards the trees
+    std::vector<BestTree> best_trees(uint32_t k) {
+        const size_t kk = k ? k : 1, n_v = cfg_.n_vertices;
+        std::vector<float> eval(kk);
+        std::vector<uint64_t> codes(2 * kk);
+        std::vector<uint32_t> tree(kk), node(kk), mask(kk * w_), mu(kk);
+        std::vector<uint8_t> parents(kk * n_v);
+        std::vector<double> l1(kk);
+        uint32_t n = 0;
+        ck(azb_best_trees(h_, k, &n, eval.data(), codes.data(), tree.data(), node.data(), parents.data(), mask.data(), l1.data(),
+                          mu.data()));
+        std::vector<BestTree> out(n);
+        for (uint32_t i = 0; i < n; ++i) {
+            BestTree &b = out[i];
+            b.data.parents.assign(parents.begin() + i * n_v, parents.begin() + (i + 1) * n_v);
+            b.data.permitted.assign(mask.begin() + (size_t)i * w_, mask.begin() + (size_t)(i + 1) * w_);
+            b.data.lambda_1 = l1[i];
+            b.data.mu = mu[i];
+            b.data.eval = eval[i];
+            b.code[0] = codes[2 * i];
+            b.code[1] = codes[2 * i + 1];
+            b.tree = tree[i];
+            b.node = node[i];
+        }
+        return out;
     }
     // the inputs par_update_model hands to NablaModel::update_model (optimizer/mod.rs:253-280)
     void observations(uint32_t n_obs_tol, std::vector<float> &state_vecs, std::vector<float> &obs, std::vector<float> &w) {

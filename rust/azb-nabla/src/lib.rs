@@ -117,6 +117,18 @@ fn ck(h: *const sys::azb_handle, rc: c_int) {
 /// `pub(crate)`, so the parents of children 2..N-2 are read back from the public edge-index iterator
 /// (rooted_tree/mod.rs:60-72); parents[1] and parents[N-1] are 0 for every state this space generates
 /// (rooted_tree/mod.rs:14-20), and act() never touches them (actions are edges of children 2..N-2).
+/// One isomorphism class of `best_trees`: its value, the representative node's state and cost, the canonical code
+/// (include/azb.h) and where the representative lives (local tree, node).
+pub struct BestTree<const N: usize> {
+    pub eval: f32,
+    pub lambda_1: f64,
+    pub mu: u32,
+    pub state: State<N>,
+    pub code: [u64; 2],
+    pub tree: u32,
+    pub node: u32,
+}
+
 pub fn flatten<const N: usize>(s: &State<N>, parents: &mut [u8], permitted: &mut [u32]) {
     assert!(parents.len() == N && permitted.len() == mask_words(N));
     parents.fill(0);
@@ -394,6 +406,33 @@ impl<const N: usize, M: NablaModel> B200Optimizer<N, M> {
 
     pub fn argmin_data(&self) -> &ArgminData<State<N>, Cost> {
         &self.argmin_data
+    }
+
+    /// The `k` best isomorphism classes among every node the trees hold (azb_best_trees, an extension with no
+    /// reference item), ascending by (eval, canonical code).  Call it before `par_reset_trees`, which discards the trees.
+    pub fn best_trees(&mut self, k: u32) -> Vec<BestTree<N>> {
+        if self.enqueued > 0 {
+            self.finish_batch();
+        }
+        let kk = k.max(1) as usize;
+        let (mut eval, mut codes, mut tree, mut node) = (vec![0f32; kk], vec![0u64; 2 * kk], vec![0u32; kk], vec![0u32; kk]);
+        let (mut parents, mut mask, mut l1, mut mu) = (vec![0u8; kk * N], vec![0u32; kk * Self::W], vec![0f64; kk], vec![0u32; kk]);
+        let mut n: u32 = 0;
+        ck(self.h, unsafe {
+            sys::azb_best_trees(self.h, k, &mut n, eval.as_mut_ptr(), codes.as_mut_ptr(), tree.as_mut_ptr(), node.as_mut_ptr(),
+                                parents.as_mut_ptr(), mask.as_mut_ptr(), l1.as_mut_ptr(), mu.as_mut_ptr())
+        });
+        (0..n as usize)
+            .map(|i| BestTree {
+                eval: eval[i],
+                lambda_1: l1[i],
+                mu: mu[i],
+                state: unflatten::<N>(&parents[i * N..(i + 1) * N], &mask[i * Self::W..(i + 1) * Self::W]),
+                code: [codes[2 * i], codes[2 * i + 1]],
+                tree: tree[i],
+                node: node[i],
+            })
+            .collect()
     }
 
     /// `par_update_model` (optimizer/mod.rs:249-281).  Device model: observations, f32 forward/backward and the Adam

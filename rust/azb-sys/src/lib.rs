@@ -120,6 +120,8 @@ extern "C" {
     pub fn azb_add_actions_host(h: *mut azb_handle, h_theta: *const f32, improved: *mut c_int) -> c_int;
     pub fn azb_get_argmin(h: *mut azb_handle, parents: *mut u8, permitted: *mut u32, lambda1: *mut f64, mu: *mut u32, eval: *mut f32) -> c_int;
     pub fn azb_get_node_state(h: *mut azb_handle, tree: u32, node: u32, parents: *mut u8, permitted: *mut u32) -> c_int;
+    pub fn azb_tree_codes(h: *mut azb_handle, parents: *const u8, m: u32, codes: *mut u64, ms: *mut f32) -> c_int;
+    pub fn azb_best_trees(h: *mut azb_handle, k: u32, n_out: *mut u32, eval: *mut f32, codes: *mut u64, tree: *mut u32, node: *mut u32, parents: *mut u8, permitted: *mut u32, lambda1: *mut f64, mu: *mut u32) -> c_int;
     pub fn azb_get_walkers(h: *mut azb_handle, parents: *mut u8, permitted: *mut u32, path: *mut u32, pos: *mut u32, path_len: *mut u32) -> c_int;
     pub fn azb_tree_sizes(h: *mut azb_handle, tree: u32, n_nodes: *mut u32, n_arcs: *mut u32, n_preds: *mut u32) -> c_int;
     pub fn azb_dump_tree(h: *mut azb_handle, tree: u32, nodes: *mut u32, keys: *mut u32, preds: *mut u32, arcs: *mut u32) -> c_int;
