@@ -89,6 +89,9 @@ SIGNATURES = {
     "azb_get_node_state": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, u8p, u32p]),
     "azb_tree_codes": (C.c_int, [C.c_void_p, u8p, C.c_uint32, C.POINTER(C.c_uint64), f32p]),
     "azb_best_trees": (C.c_int, [C.c_void_p, C.c_uint32, u32p, f32p, C.POINTER(C.c_uint64), u32p, u32p, u8p, u32p, f64p, u32p]),
+    "azb_checkpoint_size": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
+    "azb_checkpoint_save": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]),
+    "azb_checkpoint_load": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64), C.c_uint32]),
     "azb_get_walkers": (C.c_int, [C.c_void_p, u8p, u32p, u32p, u32p, u32p]),
     "azb_tree_sizes": (C.c_int, [C.c_void_p, C.c_uint32, u32p, u32p, u32p]),
     "azb_dump_tree": (C.c_int, [C.c_void_p, C.c_uint32, u32p, u32p, u32p, u32p]),
@@ -330,6 +333,34 @@ class Handle:
         lam, mu, ev = C.c_double(), C.c_uint32(), C.c_float()
         self._ck(self._L.azb_get_argmin(self._h, _p(p, C.c_uint8), _p(m, C.c_uint32), C.byref(lam), C.byref(mu), C.byref(ev)))
         return dict(parents=p, permitted=m, lambda1=lam.value, mu=mu.value, eval=np.float32(ev.value))
+
+    # ---- checkpoints (format in include/azb.h; azdopt_b200/checkpoint.py reads it) ----
+    def checkpoint_size(self) -> int:
+        n = C.c_uint64()
+        self._ck(self._L.azb_checkpoint_size(self._h, C.byref(n)))
+        return int(n.value)
+
+    def checkpoint_save(self, out=None) -> np.ndarray:
+        """The handle's search and training state as a uint8 array (written into ``out`` when given: a writable
+        uint8 array or np.memmap of at least checkpoint_size() bytes; the returned array is its used prefix)."""
+        size = self.checkpoint_size()
+        buf = np.empty(size, dtype=np.uint8) if out is None else out
+        if buf.dtype != np.uint8 or buf.ndim != 1 or not buf.flags.c_contiguous or not buf.flags.writeable:
+            raise ValueError("out must be a writable contiguous uint8 array")
+        written = C.c_uint64()
+        self._ck(self._L.azb_checkpoint_save(self._h, buf.ctypes.data_as(C.c_void_p), buf.size, C.byref(written)))
+        return buf[:written.value]
+
+    def checkpoint_load(self, blobs):
+        """Rebuild the state from one blob or a list of blobs (bytes, uint8 numpy arrays or np.memmap) whose root
+        ranges cover this handle's exactly once."""
+        if isinstance(blobs, (bytes, bytearray, memoryview, np.ndarray)):
+            blobs = [blobs]
+        arrs = [np.frombuffer(b, dtype=np.uint8) if not isinstance(b, np.ndarray) else np.ascontiguousarray(b).view(np.uint8).reshape(-1)
+                for b in blobs]
+        ptrs = (C.c_void_p * len(arrs))(*[a.ctypes.data for a in arrs])
+        sizes = (C.c_uint64 * len(arrs))(*[a.size for a in arrs])
+        self._ck(self._L.azb_checkpoint_load(self._h, ptrs, sizes, len(arrs)))
 
     def walkers(self):
         p = np.zeros((self.b, self.n), dtype=np.uint8)

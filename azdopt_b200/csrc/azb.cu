@@ -14,6 +14,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <tuple>
 #include <vector>
 
 #include "../../include/azb.h"
@@ -26,6 +27,7 @@
 #include "azb_train.cuh"
 #include "azb_async.cuh"
 #include "azb_best.cuh"
+#include "azb_ckpt.cuh"
 
 #include <dlfcn.h>
 
@@ -60,6 +62,16 @@ struct azb_handle {
     size_t best_cap;
     AzbBestState *best_st;
     uint32_t best_m_cap;
+    // azb_checkpoint_* (azb_ckpt.cuh): one grow-only staging slab, a copy stream and its events, the chunk size tests set
+    // through AZB_TEST_CKPT_CHUNK (0 = the default), and the running best's global position when a load took it from a
+    // root outside this handle's range (AzbGlobals::argmin_tree is AZB_NONE then)
+    uint8_t *ckpt_buf;
+    size_t ckpt_cap;
+    cudaStream_t ckpt_stream;
+    cudaEvent_t ckpt_ev[4];
+    uint64_t ckpt_chunk;
+    uint64_t ckpt_best_root;
+    uint32_t ckpt_best_node;
     // observations scratch
     float *obs, *obs_w;
     // training step (azb_train.cuh): gradient (parameter order), Adam moments, predictions, two dZ buffers, scalars
@@ -91,6 +103,7 @@ struct azb_handle {
     size_t flush_bytes;
     uint64_t launches, dev_bytes;
     bool roots_set, trees_init, pending_add, first_init_done, params_set, count_full;
+    bool host_add_pending;  // azb_rollout_host has run, its azb_add_actions_host has not
     int improved_last_rollout;
     uint32_t steps_done;   // steps every tree has completed since init_trees
     uint32_t argmin_from;  // first candidate slot the argmin pass has not consumed yet
@@ -217,7 +230,7 @@ int azb_destroy(azb_handle *h) {
                     h->L.walker, h->L.node, h->L.blk, h->L.inl, h->L.key, h->L.hash, h->L.casc, h->L.cand, h->L.stepmin, (void *)h->L.lut, h->L.sv,
                     h->L.h, h->L.g, h->L.log, h->params, h->act[0], h->act[1], h->act[2], h->mlp_x, h->mlp_y, h->sv16_save,
                     h->cost_par, h->cost_l1, h->cost_mu, h->cost_c, h->cost_err, h->obs, h->obs_w, h->flush_buf, h->graph_buf,
-                    h->best_buf, h->best_st};
+                    h->best_buf, h->best_st, h->ckpt_buf};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     azb_mlp_tc_destroy(h->tc);
@@ -226,6 +239,9 @@ int azb_destroy(azb_handle *h) {
         if (h->gevent[g]) cudaEventDestroy(h->gevent[g]);
     }
     if (h->fork_event) cudaEventDestroy(h->fork_event);
+    for (cudaEvent_t e : h->ckpt_ev)
+        if (e) cudaEventDestroy(e);
+    if (h->ckpt_stream) cudaStreamDestroy(h->ckpt_stream);
     if (h->pin_g) cudaFreeHost(h->pin_g);
     if (h->poll_pin) cudaFreeHost(h->poll_pin);
     if (h->roots_pin) cudaFreeHost(h->roots_pin);
@@ -368,6 +384,8 @@ int azb_create(const azb_config *cfg_in, azb_handle **out) {
         L.frontier_cap = std::min<uint32_t>(AZB_FRONTIER_CAP, std::max(1, atoi(e)));
     if (const char *e = getenv("AZB_TEST_BEST_CAP"))  // tests: force azb_best_trees through several widening rounds
         h->best_m_cap = (uint32_t)std::max(1, atoi(e));
+    if (const char *e = getenv("AZB_TEST_CKPT_CHUNK"))  // tests: push checkpoints through many staging chunks
+        h->ckpt_chunk = std::max<uint64_t>(8, strtoull(e, nullptr, 10));
     L.first_root = cfg.first_root;
     L.prior_seed = cfg.prior_seed;
     CK(dmalloc(h, &L.walker, (size_t)B * L.WS));
@@ -791,6 +809,7 @@ int azb_init_trees(azb_handle *h) {
     rc = launch_tree(h, AZB_F_ADD, 0);
     if (rc) return rc;
     h->pending_add = false;
+    h->host_add_pending = false;
     h->steps_done = 0;
     h->argmin_from = first ? 0u : 1u;
     h->poll_next = 1u;
@@ -1365,6 +1384,7 @@ int azb_rollout_host(azb_handle *h, float *state_vecs) {
     if (rc) return rc;
     rc = run_argmin(h, h->steps_done + 1);
     if (rc) return rc;
+    h->host_add_pending = true;
     rc = copy_state_vecs(h, state_vecs);
     if (rc) return rc;
     AzbGlobals g;
@@ -1383,6 +1403,7 @@ int azb_add_actions_host(azb_handle *h, const float *h_theta, int *improved) {
     int rc = launch_tree(h, AZB_F_ADD, h->steps_done, AZB_PRIOR_INJECTED);
     if (rc) return rc;
     h->pending_add = false;
+    h->host_add_pending = false;
     rc = check_device_error(h);
     if (rc) return rc;
     if (improved) *improved = h->improved_last_rollout;
@@ -2397,3 +2418,476 @@ int azb_flush_l2(azb_handle *h) {
 }
 
 }  // extern "C"
+
+// ---- checkpoints (azb_ckpt.cuh; format in include/azb.h) ------------------------------------------------------------
+enum {
+    CK_MAGIC = 0, CK_FORMAT, CK_VERSION, CK_BYTES, CK_N, CK_CLO, CK_CUP, CK_TOL, CK_TOL_LEN = CK_TOL + AZB_MAX_TOL, CK_TOL_DEF,
+    CK_HIDDEN, CK_MLP_MODE = CK_HIDDEN + 3, CK_PRIOR_MODE, CK_PRIOR_SEED, CK_SELECTION, CK_PUCT_C, CK_FIRST, CK_NROOTS,
+    CK_STEPS, CK_EPOCH, CK_ADAM_T, CK_ADAM, CK_FLAGS = CK_ADAM + 5, CK_BEST_C, CK_BEST_ROOT, CK_BEST_NODE, CK_BEST_STATE,
+    CK_NPARAMS = CK_BEST_STATE + 39, CK_MODEL_OFF, CK_MODEL_BYTES, CK_TABLE_OFF, CK_TABLE_BYTES, CK_TREES_OFF, CK_TREES_BYTES,
+    CK_MODEL_DIGEST, CK_TABLE_DIGEST, CK_HDR_DIGEST = AZB_CKPT_HEADER_WORDS - 1
+};
+static_assert(CK_TABLE_DIGEST < CK_HDR_DIGEST, "checkpoint header layout");
+static const uint64_t k_ckpt_hdr_bytes = AZB_CKPT_HEADER_WORDS * 8ull;
+static const uint64_t k_ckpt_half_max = 128ull << 20;  // each of the staging slab's two halves: 256 MB in all
+
+static uint64_t ckpt_digest(const void *p, uint64_t n) {  // include/azb.h; the buffer need not be 8-byte aligned
+    const uint8_t *b = static_cast<const uint8_t *>(p);
+    uint64_t s = 0;
+    for (uint64_t i = 0; i < n; ++i) {
+        uint64_t w;
+        memcpy(&w, b + 8 * i, 8);
+        s += azb_ckpt_term(w, i);
+    }
+    return azb_mix64(s ^ n);
+}
+static uint32_t f2u(float f) {
+    uint32_t u;
+    memcpy(&u, &f, 4);
+    return u;
+}
+static uint64_t model_bytes(const azb_handle *h) { return (h->n_params * 12 + 7) & ~7ull; }
+
+// the staging slab: [len | offsets (B + 1 each) | CUB scratch | bad words | half 0 | half 1]
+struct CkptSlab {
+    unsigned long long *len, *off, *bad;
+    void *tmp;
+    size_t tmp_bytes;
+    uint8_t *half[2];
+};
+static int ckpt_slab(azb_handle *h, uint64_t half_bytes, CkptSlab &s) {
+    const size_t n = (size_t)h->L.B + 1;
+    s.tmp_bytes = 0;
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, s.tmp_bytes, (const unsigned long long *)nullptr, (unsigned long long *)nullptr, (int)n,
+                                     h->stream));
+    const size_t o_off = best_up(n * 8), o_tmp = o_off + best_up(n * 8), o_bad = o_tmp + best_up(s.tmp_bytes), o_h0 = o_bad + 256,
+                 o_h1 = o_h0 + best_up(half_bytes), total = o_h1 + best_up(half_bytes);
+    if (total > h->ckpt_cap) {
+        if (h->ckpt_buf) {
+            CK(cudaStreamSynchronize(h->stream));
+            CK(cudaFree(h->ckpt_buf));
+            h->dev_bytes -= h->ckpt_cap;
+        }
+        h->ckpt_buf = nullptr;
+        h->ckpt_cap = 0;
+        CK(dmalloc(h, &h->ckpt_buf, total));
+        h->ckpt_cap = total;
+    }
+    if (!h->ckpt_stream) {
+        CK(cudaStreamCreateWithFlags(&h->ckpt_stream, cudaStreamNonBlocking));
+        for (cudaEvent_t &e : h->ckpt_ev) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    }
+    uint8_t *b = h->ckpt_buf;
+    s.len = reinterpret_cast<unsigned long long *>(b);
+    s.off = reinterpret_cast<unsigned long long *>(b + o_off);
+    s.tmp = b + o_tmp;
+    s.bad = reinterpret_cast<unsigned long long *>(b + o_bad);
+    s.half[0] = b + o_h0;
+    s.half[1] = b + o_h1;
+    return AZB_OK;
+}
+
+// chunks of whole records [t0, t1) with at most `half` bytes each (a record larger than that gets a chunk of its own,
+// and the halves are sized for the largest record)
+static uint64_t ckpt_half_bytes(const azb_handle *h, const uint64_t *off, uint32_t n) {
+    uint64_t max_rec = 0;
+    for (uint32_t i = 0; i < n; ++i) max_rec = std::max<uint64_t>(max_rec, off[i + 1] - off[i]);
+    uint64_t half = h->ckpt_chunk ? h->ckpt_chunk : std::min<uint64_t>(k_ckpt_half_max, (off[n] - off[0] + 1) / 2);
+    return std::max(half, max_rec);
+}
+// CTAs per record for the records [t0, t1): enough slices of AZB_CKPT_SLICE_BYTES for the largest, at most 64
+static uint32_t ckpt_slices(const uint64_t *off, uint32_t t0, uint32_t t1) {
+    uint64_t m = 0;
+    for (uint32_t t = t0; t < t1; ++t) m = std::max<uint64_t>(m, off[t + 1] - off[t]);
+    return (uint32_t)std::min<uint64_t>(64, std::max<uint64_t>(1, (m + AZB_CKPT_SLICE_BYTES - 1) / AZB_CKPT_SLICE_BYTES));
+}
+static std::vector<std::pair<uint32_t, uint32_t>> ckpt_chunks(const uint64_t *off, uint32_t n, uint64_t half) {
+    std::vector<std::pair<uint32_t, uint32_t>> out;
+    for (uint32_t t0 = 0; t0 < n;) {
+        uint32_t t1 = t0 + 1;
+        while (t1 < n && off[t1 + 1] - off[t0] <= half) ++t1;
+        out.emplace_back(t0, t1);
+        t0 = t1;
+    }
+    return out;
+}
+
+// the state checks of save / size, the deferred add_actions, and the offset table (host copy; device copy in s.off)
+static int ckpt_prepare(azb_handle *h, std::vector<uint64_t> &off, CkptSlab &s, uint64_t half_bytes) {
+    if (!h->trees_init) return fail(h, AZB_ERR_STATE, "azb_init_trees has not been called");
+    if (h->host_add_pending) return fail(h, AZB_ERR_STATE, "azb_add_actions_host must follow azb_rollout_host first");
+    if (h->argmin_from != h->steps_done + 1)
+        return fail(h, AZB_ERR_STATE, "enqueued steps are not complete (azb_step(h, 0, ...) first)");
+    CK(cudaSetDevice(h->cfg.device));
+    int rc = flush_pending(h);
+    if (rc) return rc;
+    rc = check_device_error(h);
+    if (rc) return rc;
+    rc = ckpt_slab(h, half_bytes, s);
+    if (rc) return rc;
+    const uint32_t B = h->L.B;
+    azb_ckpt_size_kernel<<<(B + 256) / 256, 256, 0, h->stream>>>(h->L, s.len);
+    h->launches += 1;
+    CK(cudaGetLastError());
+    CK(cub::DeviceScan::ExclusiveSum(s.tmp, s.tmp_bytes, s.len, s.off, (int)B + 1, h->stream));
+    h->launches += 1;
+    off.resize((size_t)B + 1);
+    CK(cudaMemcpyAsync(off.data(), s.off, off.size() * 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return AZB_OK;
+}
+
+static uint64_t ckpt_total(const azb_handle *h, uint64_t trees_bytes) {
+    return k_ckpt_hdr_bytes + model_bytes(h) + ((uint64_t)h->L.B + 1) * 8 + trees_bytes;
+}
+
+extern "C" int azb_checkpoint_size(azb_handle *h, uint64_t *bytes) {
+    if (!h || !bytes) return AZB_ERR_INVALID;
+    std::vector<uint64_t> off;
+    CkptSlab s;
+    int rc = ckpt_prepare(h, off, s, 0);
+    if (rc) return rc;
+    *bytes = ckpt_total(h, off.back());
+    return AZB_OK;
+}
+
+extern "C" int azb_checkpoint_save(azb_handle *h, void *buf, uint64_t size, uint64_t *written) {
+    if (!h || !buf) return AZB_ERR_INVALID;
+    std::vector<uint64_t> off;
+    CkptSlab s;
+    int rc = ckpt_prepare(h, off, s, 0);
+    if (rc) return rc;
+    const uint32_t B = h->L.B;
+    const uint64_t total = ckpt_total(h, off.back());
+    if (size < total) return fail(h, AZB_ERR_INVALID, "the buffer holds %llu bytes, the checkpoint needs %llu", (unsigned long long)size,
+                                  (unsigned long long)total);
+    const uint64_t half = ckpt_half_bytes(h, off.data(), B);
+    rc = ckpt_slab(h, half, s);  // the offsets stay where ckpt_prepare left them (a grown slab is re-filled below)
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(s.off, off.data(), off.size() * 8, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemsetAsync(s.len, 0, ((size_t)B + 1) * 8, h->stream));  // the digest sums
+    uint8_t *out = static_cast<uint8_t *>(buf);
+    const uint64_t o_model = k_ckpt_hdr_bytes, o_table = o_model + model_bytes(h), o_trees = o_table + ((uint64_t)B + 1) * 8;
+    // trees: chunk c is packed into half c & 1 while chunk c - 1 goes to the host on the copy stream
+    const auto chunks = ckpt_chunks(off.data(), B, half);
+    cudaEvent_t *packed = h->ckpt_ev, *copied = h->ckpt_ev + 2;
+    auto pack = [&](size_t c) -> int {
+        if (c >= 2) CK(cudaStreamWaitEvent(h->stream, copied[c & 1], 0));
+        const uint32_t t0 = chunks[c].first, t1 = chunks[c].second;
+        uint32_t *stage = reinterpret_cast<uint32_t *>(s.half[c & 1]);
+        azb_ckpt_pack_kernel<<<dim3(t1 - t0, ckpt_slices(off.data(), t0, t1)), AZB_CKPT_THREADS, 0, h->stream>>>(h->L, s.off, t0, off[t0],
+                                                                                                           stage, s.len);
+        azb_ckpt_pack_finish_kernel<<<(t1 - t0 + 255) / 256, 256, 0, h->stream>>>(h->L, s.off, t0, t1, off[t0], stage, s.len);
+        h->launches += 2;
+        CK(cudaGetLastError());
+        CK(cudaEventRecord(packed[c & 1], h->stream));
+        return AZB_OK;
+    };
+    if (!chunks.empty()) {
+        rc = pack(0);
+        if (rc) return rc;
+    }
+    for (size_t c = 0; c < chunks.size(); ++c) {
+        if (c + 1 < chunks.size()) {
+            rc = pack(c + 1);
+            if (rc) return rc;
+        }
+        const uint32_t t0 = chunks[c].first, t1 = chunks[c].second;
+        CK(cudaStreamWaitEvent(h->ckpt_stream, packed[c & 1], 0));
+        CK(cudaMemcpyAsync(out + o_trees + off[t0], s.half[c & 1], off[t1] - off[t0], cudaMemcpyDeviceToHost, h->ckpt_stream));
+        CK(cudaEventRecord(copied[c & 1], h->ckpt_stream));
+    }
+    // model, running best
+    const size_t n = h->n_params;
+    memset(out + o_model, 0, model_bytes(h));
+    if (h->params_set) CK(cudaMemcpyAsync(out + o_model, h->params, n * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (h->adam_m) {
+        CK(cudaMemcpyAsync(out + o_model + n * 4, h->adam_m, n * 4, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaMemcpyAsync(out + o_model + n * 8, h->adam_v, n * 4, cudaMemcpyDeviceToHost, h->stream));
+    }
+    AzbGlobals g;
+    CK(cudaMemcpyAsync(&g, h->L.g, sizeof(g), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaStreamSynchronize(h->ckpt_stream));
+    memcpy(out + o_table, off.data(), off.size() * 8);
+    uint64_t hw[AZB_CKPT_HEADER_WORDS];
+    memset(hw, 0, sizeof(hw));
+    const azb_config &cf = h->cfg;
+    hw[CK_MAGIC] = AZB_CKPT_MAGIC;
+    hw[CK_FORMAT] = AZB_CKPT_FORMAT;
+    hw[CK_VERSION] = AZB_VERSION;
+    hw[CK_BYTES] = total;
+    hw[CK_N] = cf.n_vertices;
+    hw[CK_CLO] = f2u(cf.c_lower);
+    hw[CK_CUP] = f2u(cf.c_upper);
+    for (int i = 0; i < AZB_MAX_TOL; ++i) hw[CK_TOL + i] = cf.n_as_tol[i];
+    hw[CK_TOL_LEN] = cf.n_as_tol_len;
+    hw[CK_TOL_DEF] = cf.n_as_tol_default;
+    for (int i = 0; i < 3; ++i) hw[CK_HIDDEN + i] = cf.mlp_hidden[i];
+    hw[CK_MLP_MODE] = cf.mlp_mode;
+    hw[CK_PRIOR_MODE] = cf.prior_mode;
+    hw[CK_PRIOR_SEED] = cf.prior_seed;
+    hw[CK_SELECTION] = cf.selection;
+    hw[CK_PUCT_C] = f2u(cf.puct_c);
+    hw[CK_FIRST] = cf.first_root;
+    hw[CK_NROOTS] = B;
+    hw[CK_STEPS] = h->steps_done;
+    hw[CK_EPOCH] = h->epoch;
+    hw[CK_ADAM_T] = h->adam_t;
+    const float adam[5] = {h->adam.lr, h->adam.beta1, h->adam.beta2, h->adam.eps, h->adam.l2};
+    for (int i = 0; i < 5; ++i) hw[CK_ADAM + i] = f2u(adam[i]);
+    hw[CK_FLAGS] = h->params_set ? 1u : 0u;
+    hw[CK_BEST_C] = g.best_c;
+    hw[CK_BEST_ROOT] = g.argmin_tree == AZB_NONE ? h->ckpt_best_root : cf.first_root + g.argmin_tree;
+    hw[CK_BEST_NODE] = g.argmin_tree == AZB_NONE ? h->ckpt_best_node : g.argmin_node;
+    memcpy(hw + CK_BEST_STATE, g.argmin_state, sizeof(g.argmin_state));
+    hw[CK_NPARAMS] = n;
+    hw[CK_MODEL_OFF] = o_model;
+    hw[CK_MODEL_BYTES] = model_bytes(h);
+    hw[CK_TABLE_OFF] = o_table;
+    hw[CK_TABLE_BYTES] = ((uint64_t)B + 1) * 8;
+    hw[CK_TREES_OFF] = o_trees;
+    hw[CK_TREES_BYTES] = off.back();
+    hw[CK_MODEL_DIGEST] = ckpt_digest(out + o_model, model_bytes(h) / 8);
+    hw[CK_TABLE_DIGEST] = ckpt_digest(out + o_table, (uint64_t)B + 1);
+    hw[CK_HDR_DIGEST] = ckpt_digest(hw, CK_HDR_DIGEST);
+    memcpy(out, hw, sizeof(hw));
+    if (written) *written = total;
+    return AZB_OK;
+}
+
+// one blob's header, checked against itself and the handle
+struct CkptBlob {
+    const uint8_t *p;
+    uint64_t size, first, n;
+    uint64_t hw[AZB_CKPT_HEADER_WORDS];
+};
+
+static int ckpt_check_header(azb_handle *h, uint32_t i, CkptBlob &b) {
+    if (b.size < k_ckpt_hdr_bytes) return fail(h, AZB_ERR_INVALID, "blob %u: %llu bytes, shorter than a header", i, (unsigned long long)b.size);
+    memcpy(b.hw, b.p, k_ckpt_hdr_bytes);
+    const uint64_t *w = b.hw;
+    if (w[CK_MAGIC] != AZB_CKPT_MAGIC) return fail(h, AZB_ERR_INVALID, "blob %u: bad magic", i);
+    if (w[CK_FORMAT] != AZB_CKPT_FORMAT) return fail(h, AZB_ERR_INVALID, "blob %u: format %llu, expected %d", i, (unsigned long long)w[CK_FORMAT], AZB_CKPT_FORMAT);
+    if (w[CK_VERSION] != AZB_VERSION) return fail(h, AZB_ERR_INVALID, "blob %u: version %llu, expected %d", i, (unsigned long long)w[CK_VERSION], AZB_VERSION);
+    if (ckpt_digest(w, CK_HDR_DIGEST) != w[CK_HDR_DIGEST]) return fail(h, AZB_ERR_INVALID, "blob %u: header digest", i);
+    if (w[CK_BYTES] != b.size)
+        return fail(h, AZB_ERR_INVALID, "blob %u: %llu bytes, its header says %llu (truncated?)", i, (unsigned long long)b.size,
+                    (unsigned long long)w[CK_BYTES]);
+    const azb_config &cf = h->cfg;
+    struct { const char *name; uint64_t have, want; } fields[] = {
+        {"n_vertices", w[CK_N], cf.n_vertices}, {"c_lower", w[CK_CLO], f2u(cf.c_lower)}, {"c_upper", w[CK_CUP], f2u(cf.c_upper)},
+        {"n_as_tol_len", w[CK_TOL_LEN], cf.n_as_tol_len}, {"n_as_tol_default", w[CK_TOL_DEF], cf.n_as_tol_default},
+        {"mlp_hidden[0]", w[CK_HIDDEN], cf.mlp_hidden[0]}, {"mlp_hidden[1]", w[CK_HIDDEN + 1], cf.mlp_hidden[1]},
+        {"mlp_hidden[2]", w[CK_HIDDEN + 2], cf.mlp_hidden[2]}, {"mlp_mode", w[CK_MLP_MODE], cf.mlp_mode},
+        {"prior_mode", w[CK_PRIOR_MODE], cf.prior_mode}, {"prior_seed", w[CK_PRIOR_SEED], cf.prior_seed},
+        {"selection", w[CK_SELECTION], cf.selection}, {"puct_c", w[CK_PUCT_C], f2u(cf.puct_c)}, {"n_params", w[CK_NPARAMS], h->n_params}};
+    for (const auto &f : fields)
+        if (f.have != f.want) return fail(h, AZB_ERR_INVALID, "blob %u: config field %s differs from the handle's", i, f.name);
+    for (uint32_t k = 0; k < cf.n_as_tol_len; ++k)
+        if (w[CK_TOL + k] != cf.n_as_tol[k]) return fail(h, AZB_ERR_INVALID, "blob %u: config field n_as_tol[%u] differs from the handle's", i, k);
+    b.first = w[CK_FIRST];
+    b.n = w[CK_NROOTS];
+    const uint64_t o_model = k_ckpt_hdr_bytes, o_table = o_model + model_bytes(h), o_trees = o_table + (b.n + 1) * 8;
+    if (b.n == 0 || w[CK_MODEL_OFF] != o_model || w[CK_MODEL_BYTES] != model_bytes(h) || w[CK_TABLE_OFF] != o_table ||
+        w[CK_TABLE_BYTES] != (b.n + 1) * 8 || w[CK_TREES_OFF] != o_trees || o_trees + w[CK_TREES_BYTES] != b.size)
+        return fail(h, AZB_ERR_INVALID, "blob %u: section table", i);
+    if (w[CK_STEPS] > 0xffffffffull || w[CK_ADAM_T] > 0xffffffffull) return fail(h, AZB_ERR_INVALID, "blob %u: step counts", i);
+    return AZB_OK;
+}
+
+// everything a failed load leaves: the trees are invalid until a load succeeds or set_roots + init_trees run
+static void ckpt_invalidate(azb_handle *h) {
+    h->trees_init = false;
+    h->first_init_done = false;
+    h->pending_add = false;
+    h->host_add_pending = false;
+}
+
+extern "C" int azb_checkpoint_load(azb_handle *h, const void *const *blobs, const uint64_t *sizes, uint32_t n_blobs) {
+    if (!h || !blobs || !sizes || n_blobs == 0) return AZB_ERR_INVALID;
+    std::vector<CkptBlob> bl(n_blobs);
+    for (uint32_t i = 0; i < n_blobs; ++i) {
+        if (!blobs[i]) return fail(h, AZB_ERR_INVALID, "blob %u is NULL", i);
+        bl[i].p = static_cast<const uint8_t *>(blobs[i]);
+        bl[i].size = sizes[i];
+        int rc = ckpt_check_header(h, i, bl[i]);
+        if (rc) return rc;
+    }
+    // one run: every blob agrees on the counters, the Adam state and the model
+    const CkptBlob &b0 = bl[0];
+    const uint64_t mb = model_bytes(h);
+    if (ckpt_digest(b0.p + k_ckpt_hdr_bytes, mb / 8) != b0.hw[CK_MODEL_DIGEST]) return fail(h, AZB_ERR_INVALID, "blob 0: model digest");
+    for (uint32_t i = 1; i < n_blobs; ++i) {
+        static const struct { int w, n; const char *name; } same[] = {
+            {CK_STEPS, 1, "steps_done"}, {CK_EPOCH, 1, "reset count"}, {CK_ADAM_T, 1, "Adam step"}, {CK_ADAM, 5, "Adam config"},
+            {CK_FLAGS, 1, "flags"}, {CK_MODEL_DIGEST, 1, "model section"}};
+        for (const auto &f : same)
+            if (memcmp(bl[i].hw + f.w, b0.hw + f.w, 8 * f.n)) return fail(h, AZB_ERR_INVALID, "blob %u: %s differs from blob 0's", i, f.name);
+        if (memcmp(bl[i].p + k_ckpt_hdr_bytes, b0.p + k_ckpt_hdr_bytes, mb)) return fail(h, AZB_ERR_INVALID, "blob %u: model section differs from blob 0's", i);
+    }
+    // ranges: pairwise disjoint, covering [F, F + B) exactly
+    const uint64_t F = h->cfg.first_root, B = h->L.B;
+    std::vector<uint32_t> ord(n_blobs);
+    for (uint32_t i = 0; i < n_blobs; ++i) ord[i] = i;
+    std::sort(ord.begin(), ord.end(), [&](uint32_t a, uint32_t b) { return bl[a].first < bl[b].first; });
+    for (uint32_t k = 0; k + 1 < n_blobs; ++k)
+        if (bl[ord[k]].first + bl[ord[k]].n > bl[ord[k + 1]].first)
+            return fail(h, AZB_ERR_INVALID, "blobs %u and %u overlap", ord[k], ord[k + 1]);
+    uint64_t covered = F;
+    for (uint32_t k = 0; k < n_blobs; ++k) {
+        const CkptBlob &b = bl[ord[k]];
+        if (b.first + b.n <= F || b.first >= F + B) continue;
+        if (b.first > covered) break;
+        covered = b.first + b.n;
+    }
+    if (covered < F + B) return fail(h, AZB_ERR_INVALID, "no blob holds global root %llu of the handle's range", (unsigned long long)covered);
+    if (b0.hw[CK_STEPS] > h->cfg.max_steps)
+        return fail(h, AZB_ERR_CAPACITY, "the checkpoint is %llu steps into its epoch, max_steps is %u", (unsigned long long)b0.hw[CK_STEPS],
+                    h->cfg.max_steps);
+    // the offset tables of the blobs that hold some of the handle's roots
+    std::vector<std::vector<uint64_t>> tables(n_blobs);
+    for (uint32_t i = 0; i < n_blobs; ++i) {
+        const CkptBlob &b = bl[i];
+        if (b.first + b.n <= F || b.first >= F + B) continue;
+        auto &t = tables[i];
+        t.resize(b.n + 1);
+        memcpy(t.data(), b.p + b.hw[CK_TABLE_OFF], t.size() * 8);
+        if (ckpt_digest(t.data(), t.size()) != b.hw[CK_TABLE_DIGEST]) return fail(h, AZB_ERR_INVALID, "blob %u: tree offset table digest", i);
+        bool ok = t[0] == 0 && t[b.n] == b.hw[CK_TREES_BYTES];
+        for (uint64_t r = 0; r < b.n && ok; ++r) ok = t[r + 1] > t[r] && (t[r + 1] - t[r]) % 8 == 0;
+        if (!ok) return fail(h, AZB_ERR_INVALID, "blob %u: tree offset table", i);
+    }
+    // the running best: first minimum by (eval, global root, node) over every blob
+    uint32_t best = 0;
+    for (uint32_t i = 1; i < n_blobs; ++i) {
+        const uint64_t *a = bl[i].hw, *c = bl[best].hw;
+        if (std::make_tuple(a[CK_BEST_C], a[CK_BEST_ROOT], a[CK_BEST_NODE]) < std::make_tuple(c[CK_BEST_C], c[CK_BEST_ROOT], c[CK_BEST_NODE])) best = i;
+    }
+
+    // ---- device: from here on a failure leaves the trees invalid
+    CK(cudaSetDevice(h->cfg.device));
+    CK(cudaStreamSynchronize(h->stream));
+    ckpt_invalidate(h);
+    uint64_t half = 0;
+    for (uint32_t i = 0; i < n_blobs; ++i)
+        if (!tables[i].empty()) {
+            const uint64_t lo = std::max(F, bl[i].first) - bl[i].first, hi = std::min(F + B, bl[i].first + bl[i].n) - bl[i].first;
+            half = std::max(half, ckpt_half_bytes(h, tables[i].data() + lo, (uint32_t)(hi - lo)));
+        }
+    CkptSlab s;
+    int rc = ckpt_slab(h, half, s);
+    if (rc) return rc;
+    static const unsigned long long none2[2] = {~0ull, ~0ull};
+    CK(cudaMemcpyAsync(s.bad, none2, 16, cudaMemcpyHostToDevice, h->stream));
+    cudaEvent_t *copied = h->ckpt_ev, *used = h->ckpt_ev + 2;
+    for (uint32_t i = 0; i < n_blobs; ++i) {
+        if (tables[i].empty()) continue;
+        const CkptBlob &b = bl[i];
+        const uint64_t lo = std::max(F, b.first) - b.first, hi = std::min(F + B, b.first + b.n) - b.first;
+        const uint32_t cnt = (uint32_t)(hi - lo), local0 = (uint32_t)(b.first + lo - F);
+        const uint64_t *t = tables[i].data() + lo;
+        CK(cudaMemcpyAsync(s.off, t, ((size_t)cnt + 1) * 8, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemsetAsync(s.len, 0, ((size_t)cnt + 1) * 8, h->stream));  // the digest sums
+        const uint8_t *src = b.p + b.hw[CK_TREES_OFF];
+        const auto chunks = ckpt_chunks(t, cnt, half);
+        // chunk c goes to half c & 1 on the copy stream while chunk c - 1 is unpacked
+        auto copy = [&](size_t c) -> int {
+            if (c >= 2) CK(cudaStreamWaitEvent(h->ckpt_stream, used[c & 1], 0));
+            const uint32_t c0 = chunks[c].first, c1 = chunks[c].second;
+            CK(cudaMemcpyAsync(s.half[c & 1], src + t[c0], t[c1] - t[c0], cudaMemcpyHostToDevice, h->ckpt_stream));
+            CK(cudaEventRecord(copied[c & 1], h->ckpt_stream));
+            return AZB_OK;
+        };
+        rc = copy(0);
+        if (rc) return rc;
+        for (size_t c = 0; c < chunks.size(); ++c) {
+            const uint32_t c0 = chunks[c].first, c1 = chunks[c].second;
+            CK(cudaStreamWaitEvent(h->stream, copied[c & 1], 0));
+            const uint32_t *stage = reinterpret_cast<const uint32_t *>(s.half[c & 1]);
+            azb_ckpt_unpack_kernel<<<dim3(c1 - c0, ckpt_slices(t, c0, c1)), AZB_CKPT_THREADS, 0, h->stream>>>(h->L, s.off, c0, t[c0], stage, local0,
+                                                                                                       b.first + lo, s.len, s.bad);
+            azb_ckpt_unpack_finish_kernel<<<(c1 - c0 + 255) / 256, 256, 0, h->stream>>>(h->L, s.off, c0, c1, t[c0], stage, b.first + lo, s.len,
+                                                                                        s.bad);
+            h->launches += 2;
+            CK(cudaGetLastError());
+            CK(cudaEventRecord(used[c & 1], h->stream));
+            if (c + 1 < chunks.size()) {
+                rc = copy(c + 1);
+                if (rc) return rc;
+            }
+        }
+        CK(cudaStreamSynchronize(h->ckpt_stream));
+        CK(cudaStreamSynchronize(h->stream));
+    }
+    unsigned long long bad[2];
+    auto read_bad = [&]() -> int {
+        CK(cudaMemcpyAsync(bad, s.bad, 16, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        if (bad[0] == ~0ull && bad[1] == ~0ull) return AZB_OK;
+        if (bad[0] <= bad[1]) return fail(h, AZB_ERR_INVALID, "the record of global root %llu is corrupt (digest or length)", bad[0]);
+        return fail(h, AZB_ERR_CAPACITY, "the record of global root %llu does not fit the handle's capacities (cap_nodes, cap_preds, cap_parents)",
+                    bad[1]);
+    };
+    rc = read_bad();
+    if (rc) return rc;
+    if (azb_stack_depth(h->N) == 5)
+        azb_ckpt_hash_kernel<true><<<(h->L.B + AZB_CKPT_WARPS - 1) / AZB_CKPT_WARPS, AZB_CKPT_WARPS * 32, 0, h->stream>>>(h->L, s.bad);
+    else
+        azb_ckpt_hash_kernel<false><<<(h->L.B + AZB_CKPT_WARPS - 1) / AZB_CKPT_WARPS, AZB_CKPT_WARPS * 32, 0, h->stream>>>(h->L, s.bad);
+    h->launches += 1;
+    CK(cudaGetLastError());
+    rc = read_bad();
+    if (rc) return rc;
+
+    // model and Adam state
+    const uint64_t *w = b0.hw;
+    const size_t n = h->n_params;
+    const uint8_t *model = b0.p + k_ckpt_hdr_bytes;
+    if (w[CK_FLAGS] & 1u) {
+        CK(cudaMemcpyAsync(h->params, model, n * 4, cudaMemcpyHostToDevice, h->stream));
+        if (h->tc.ready) {
+            const char *why = azb_mlp_tc_load(h->tc, h->params, h->stream, &h->launches);
+            if (why) return fail(h, AZB_ERR_CUDA, "tensor-core MLP: %s", why);
+        }
+    }
+    if (w[CK_ADAM_T] || h->adam_m) {
+        rc = train_alloc(h);
+        if (rc) return rc;
+        CK(cudaMemcpyAsync(h->adam_m, model + n * 4, n * 4, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemcpyAsync(h->adam_v, model + n * 8, n * 4, cudaMemcpyHostToDevice, h->stream));
+    }
+    // globals: the running best, the next candidate slot, no error, counters from zero
+    AzbGlobals g;
+    CK(cudaMemcpyAsync(&g, h->L.g, sizeof(g), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    const uint64_t *bw = bl[best].hw;
+    const uint32_t steps = (uint32_t)w[CK_STEPS];
+    g.best_c = (uint32_t)bw[CK_BEST_C];
+    const bool mine = bw[CK_BEST_ROOT] >= F && bw[CK_BEST_ROOT] < F + B;
+    g.argmin_tree = mine ? (uint32_t)(bw[CK_BEST_ROOT] - F) : AZB_NONE;
+    g.argmin_node = mine ? (uint32_t)bw[CK_BEST_NODE] : AZB_NONE;
+    h->ckpt_best_root = bw[CK_BEST_ROOT];
+    h->ckpt_best_node = (uint32_t)bw[CK_BEST_NODE];
+    memcpy(g.argmin_state, bw + CK_BEST_STATE, sizeof(g.argmin_state));
+    g.n_improved = 0;
+    g.err = g.err_tree = g.err_step = 0;
+    g.improved_last = 0;
+    g.behind_accum = g.n_behind = g.blocks_done = 0;
+    g.next_slot = steps + 1;
+    memset(&g.counters, 0, sizeof(g.counters));
+    CK(cudaMemcpyAsync(h->L.g, &g, sizeof(g), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (w[CK_FLAGS] & 1u) h->params_set = true;
+    h->adam_t = (uint32_t)w[CK_ADAM_T];
+    float adam[5];
+    for (int i = 0; i < 5; ++i) memcpy(adam + i, w + CK_ADAM + i, 4);
+    h->adam = AzbAdam{adam[0], adam[1], adam[2], adam[3], adam[4], 1.f, 1.f};
+    h->epoch = w[CK_EPOCH];
+    h->steps_done = steps;
+    h->argmin_from = h->poll_next = steps + 1;
+    h->poll_best_valid = false;
+    h->roots_set = true;
+    h->first_init_done = h->trees_init = true;
+    return AZB_OK;
+}

@@ -132,6 +132,34 @@ __device__ __forceinline__ uint32_t key_hash(uint32_t k0, uint32_t k1, int lane,
     return hv;
 }
 
+// transposition-table probe of a tree's table for the key (k0, k1) with hash hv (key_hash): the index of the node with
+// that key, or -1 with `slot` = the empty slot where the key goes.  The search kernels and the checkpoint load's rebuild
+// (azb_ckpt.cuh) share it, so a table rebuilt by inserting nodes 0..n-1 in index order is the one the search built.
+template <bool WIDE>  // W > 32 (N >= 47): the key's second word per lane
+__device__ __forceinline__ int hash_probe(const AzbLayout &L, const uint32_t *hash, const uint32_t *key, uint32_t k0, uint32_t k1,
+                                          int lane, uint32_t hv, uint32_t &slot) {
+    const uint32_t fp = hv >> 21;
+    slot = hv & (L.cap_hash - 1);
+    for (uint32_t probes = 0; probes < L.cap_hash; ++probes) {
+        const uint32_t e = hash[slot];
+        if (e == 0u) break;
+        if ((e >> 21) == fp) {
+            const uint32_t idx = (e & 0x1fffffu) - 1u;
+            bool eq = true;
+            if ((uint32_t)lane < L.W) eq = key[(size_t)idx * L.W + lane] == k0;
+            if constexpr (WIDE)
+                if ((uint32_t)lane + 32 < L.W) eq = eq && (key[(size_t)idx * L.W + lane + 32] == k1);
+            if (__all_sync(0xffffffffu, eq)) return (int)idx;
+        }
+        slot = (slot + 1) & (L.cap_hash - 1);
+    }
+    return -1;
+}
+// entry of node `node` (hash hv) in the empty slot hash_probe returned
+__device__ __forceinline__ void hash_insert(uint32_t *hash, uint32_t slot, uint32_t node, uint32_t hv) {
+    hash[slot] = (node + 1u) | ((hv >> 21) << 21);
+}
+
 // current-edge mask of the walker state into cx.cur (rooted_tree/mod.rs:60-72)
 __device__ __forceinline__ void build_cur_mask(const AzbLayout &L, WarpCtx &cx) {
 #pragma unroll 1
@@ -754,25 +782,8 @@ __device__ void tree_rollout(const AzbLayout &L, WarpCtx &cx, uint32_t tree, uin
         if constexpr (DEPTH == 5)  // W > 32 only for N >= 47
             k1 = (uint32_t)lane + 32 < L.W ? (cx.keym[lane + 32] | (((a >> 5) == (uint32_t)lane + 32) ? 1u << (a & 31) : 0u)) : 0u;
         const uint32_t hv = key_hash(k0, k1, lane, L.W);
-        const uint32_t fp = hv >> 21;
-        uint32_t slot = hv & (L.cap_hash - 1);
-        int hit = -1;
-        for (uint32_t probes = 0; probes < L.cap_hash; ++probes) {
-            const uint32_t e = cx.hash[slot];
-            if (e == 0u) break;
-            if ((e >> 21) == fp) {
-                const uint32_t idx = (e & 0x1fffffu) - 1u;
-                bool eq = true;
-                if ((uint32_t)lane < L.W) eq = cx.key[(size_t)idx * L.W + lane] == k0;
-                if constexpr (DEPTH == 5)
-                    if ((uint32_t)lane + 32 < L.W) eq = eq && (cx.key[(size_t)idx * L.W + lane + 32] == k1);
-                if (__all_sync(FULL, eq)) {
-                    hit = (int)idx;
-                    break;
-                }
-            }
-            slot = (slot + 1) & (L.cap_hash - 1);
-        }
+        uint32_t slot;
+        const int hit = hash_probe<DEPTH == 5>(L, cx.hash, cx.key, k0, k1, lane, hv, slot);
         PROF_ADD(cx, PH_PROBE);
         const uint32_t kidx = lo2 + 1u + n_out;  // this arc's kid entry (16-byte index)
         const uint32_t narcs = cx.wk[WK_NARCS];
@@ -854,7 +865,7 @@ __device__ void tree_rollout(const AzbLayout &L, WarpCtx &cx, uint32_t tree, uin
             if constexpr (DEPTH == 5)
                 if ((uint32_t)lane + 32 < L.W) cx.key[(size_t)nn * L.W + lane + 32] = k1;
             if (lane == 0) {
-                cx.hash[slot] = (nn + 1u) | (fp << 21);
+                hash_insert(cx.hash, slot, nn, hv);
                 cx.wk[WK_NNODES] = nn + 1;
                 cx.wk[WK_INTOP] = in_off + in_need;
                 // add_arc: the child is inactive until its own add_actions (actions = 0..0)
@@ -1015,7 +1026,7 @@ __global__ void __launch_bounds__(AZB_WARPS_PER_BLOCK * 32, AZB_TREE_MIN_BLOCKS)
                 if ((uint32_t)lane + 32 < L.W) cx.key[lane + 32] = 0u;
             const uint32_t hv = key_hash(0u, 0u, lane, L.W);  // the empty path hashes like every other key
             if (lane == 0) {
-                cx.hash[hv & (L.cap_hash - 1)] = 1u | ((hv >> 21) << 21);
+                hash_insert(cx.hash, hv & (L.cap_hash - 1), 0u, hv);
                 cx.wk[WK_POS] = 0;
                 cx.wk[WK_DEPTH] = 0;
                 cx.wk[WK_NNODES] = 1;

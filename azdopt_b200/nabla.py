@@ -9,6 +9,7 @@ device MLP), :class:`TrivialModel`, or any object with ``write_predictions(state
 from __future__ import annotations
 
 import dataclasses
+import os
 from typing import Callable, Optional, Sequence
 
 import numpy as np
@@ -108,6 +109,27 @@ class BestTrees:
 
     def result(self) -> list:
         return sorted(self._by_code.values(), key=lambda t: (np.float32(t.eval), t.code))[:self.k]
+
+    def state(self) -> dict:
+        """The accumulator as a dict of numpy arrays (np.savez can store it beside a checkpoint blob)."""
+        r = self.result()
+        n = r[0].parents.size if r else 0
+        w = r[0].permitted.size if r else 0
+        return dict(k=np.int64(self.k), eval=np.array([t.eval for t in r], dtype=np.float32),
+                    lambda_1=np.array([t.lambda_1 for t in r], dtype=np.float64), mu=np.array([t.mu for t in r], dtype=np.uint32),
+                    parents=np.array([t.parents for t in r], dtype=np.uint8).reshape(len(r), n),
+                    permitted=np.array([t.permitted for t in r], dtype=np.uint32).reshape(len(r), w),
+                    code=np.array([t.code for t in r], dtype=np.uint64).reshape(len(r), 2),
+                    root=np.array([t.root for t in r], dtype=np.uint64), node=np.array([t.node for t in r], dtype=np.uint32))
+
+    @classmethod
+    def from_state(cls, st) -> "BestTrees":
+        """The accumulator state() described (a dict or an np.load result)."""
+        acc = cls(int(st["k"]))
+        acc.add(BestTree(np.float32(st["eval"][i]), float(st["lambda_1"][i]), int(st["mu"][i]), np.array(st["parents"][i]),
+                         np.array(st["permitted"][i]), (int(st["code"][i][0]), int(st["code"][i][1])), int(st["root"][i]),
+                         int(st["node"][i])) for i in range(len(st["eval"])))
+        return acc
 
 
 class NablaOptimizer:
@@ -214,6 +236,47 @@ class NablaOptimizer:
             improved, rec = self.h.step_poll()
             yield rec[0], improved, rec
         self.h.step(0)
+
+    # ---- checkpoints (azb_checkpoint_save / _load; format in include/azb.h)
+    def save(self, path: str) -> int:
+        """Write the search and training state to ``path`` (through a temporary file and os.replace, so the file is
+        either the old or the new checkpoint); returns its size.  ActionModel only: a host model keeps its own state."""
+        if not isinstance(self.model, ActionModel):
+            raise TypeError("checkpoints hold the device model's state; a host model saves its own")
+        blob = self.h.checkpoint_save()
+        tmp = f"{path}.tmp{os.getpid()}"
+        with open(tmp, "wb") as f:
+            f.write(memoryview(blob))
+            f.flush()
+            os.fsync(f.fileno())
+        os.replace(tmp, path)
+        return int(blob.size)
+
+    @classmethod
+    def resume(cls, paths, space: ROTModifyParentsOnce, model: ActionModel, batch: int, *, first_root: int = 0,
+               device: int = 0, max_steps: int = 800, async_workers: Optional[int] = None) -> "NablaOptimizer":
+        """A new optimizer over the global roots [first_root, first_root + batch) continuing from checkpoint files
+        (one path or several, e.g. every rank's file of a run with another number of shards): exactly where the saved
+        run stopped.  The search settings (n_as_tol, selection, model widths) come from the checkpoint; a different
+        space or model arithmetic is refused by the load."""
+        from . import checkpoint
+
+        paths = [paths] if isinstance(paths, (str, os.PathLike)) else list(paths)
+        blobs = [np.memmap(p, dtype=np.uint8, mode="r") for p in paths]
+        hdr = checkpoint.read_header(blobs[0])
+        self = object.__new__(cls)
+        self.space, self.model, self.batch = space, model, batch
+        self._tol = (tuple(hdr.n_as_tol), hdr.n_as_tol_default)
+        mlp = capi.MLP_TC if model.arithmetic == "tc" else capi.MLP_FP32
+        cfg = capi.default_config(space.n, batch, device=device, first_root=first_root, c_lower=space.c_lower,
+                                  c_upper=space.c_upper, n_as_tol=hdr.n_as_tol, n_as_tol_default=hdr.n_as_tol_default,
+                                  prior_mode=capi.PRIOR_MLP, mlp_mode=mlp, mlp_hidden=hdr.mlp_hidden, max_steps=max_steps,
+                                  async_workers=capi.ASYNC_AUTO if async_workers is None else async_workers,
+                                  selection=hdr.selection, puct_c=hdr.puct_c)
+        self.h = capi.Handle(cfg)
+        self._host_vecs = self._host_h = None
+        self.h.checkpoint_load(blobs)
+        return self
 
     def argmin_data(self) -> ArgminData:  # optimizer/mod.rs:361-363
         a = self.h.argmin()

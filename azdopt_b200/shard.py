@@ -2,6 +2,9 @@
 inside a step; epoch-boundary collectives over torch.distributed (NCCL on GPUs, gloo in CPU tests)."""
 from __future__ import annotations
 
+import glob
+import os
+
 import numpy as np
 
 
@@ -59,3 +62,26 @@ def global_best_trees(local: list, k: int, dist=None) -> list:
     for lst in lists:
         acc.add(lst)
     return acc.result()
+
+
+def checkpoint_path(directory: str, rank: int) -> str:
+    """Where rank `rank` keeps its checkpoint blob inside a run's checkpoint directory."""
+    return os.path.join(directory, f"rank{rank:05d}.azbckpt")
+
+
+def checkpoint_paths(directory: str) -> list:
+    """Every rank's checkpoint blob in `directory`, in rank order (temporary files of an interrupted save excluded)."""
+    return sorted(p for p in glob.glob(os.path.join(directory, "rank*.azbckpt")) if os.path.isfile(p))
+
+
+def resume_sharded(directory: str, space, model, total: int, rank: int, world: int, **kw):
+    """This rank's NablaOptimizer over its shard_range of `total` roots, loaded from EVERY rank's file in `directory`
+    (written by a run with any number of ranks): each file is memory-mapped, so only the headers and the records of this
+    rank's roots are read."""
+    from .nabla import NablaOptimizer
+
+    lo, hi = shard_range(total, rank, world)
+    paths = checkpoint_paths(directory)
+    if not paths:
+        raise FileNotFoundError(f"no checkpoint in {directory}")
+    return NablaOptimizer.resume(paths, space, model, hi - lo, first_root=lo, **kw)

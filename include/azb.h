@@ -242,6 +242,70 @@ int azb_tree_codes(azb_handle *h, const uint8_t *parents /*[M*N]*/, uint32_t m, 
 int azb_best_trees(azb_handle *h, uint32_t k, uint32_t *n_out, float *eval /*[k]*/, uint64_t *codes /*[k*2]*/,
                    uint32_t *tree /*[k]*/, uint32_t *node /*[k]*/, uint8_t *parents /*[k*N]*/,
                    uint32_t *permitted /*[k*W]*/, double *lambda1 /*[k]*/, uint32_t *mu /*[k]*/);
+/* ---- extension (no reference item; the reference has no checkpointing): save a handle's search and training state
+ *      and resume it bit for bit in a new process, on the same or another split of the roots.
+ * azb_checkpoint_save works whenever the handle is at rest after azb_init_trees / azb_reset_trees (after any completed
+ * azb_step, after azb_update_model, around azb_best_trees).  Like every reading call it first runs the deferred
+ * add_actions of the last step; apart from that it changes nothing (no tree, walker, counter, argmin or RNG state), so
+ * two saves in a row give identical bytes.  AZB_ERR_STATE before the first azb_init_trees (or after azb_set_roots),
+ * while steps enqueued with azb_step_enqueue have not been completed by azb_step(h, 0, ...), and between
+ * azb_rollout_host and azb_add_actions_host.  azb_checkpoint_size gives the exact number of bytes save writes;
+ * AZB_ERR_INVALID when `size` is smaller.  The buffer may be pageable.
+ *
+ * Blob format AZB_CKPT_FORMAT, little-endian, every section a multiple of 8 bytes:
+ *   header  AZB_CKPT_HEADER_WORDS uint64 words; 32-bit values sit in the low half of their word, floats as their bits:
+ *     0 AZB_CKPT_MAGIC   1 AZB_CKPT_FORMAT   2 AZB_VERSION   3 blob bytes
+ *     4 n_vertices  5 c_lower  6 c_upper (derived)  7..14 n_as_tol[0..7]  15 n_as_tol_len  16 n_as_tol_default
+ *     17..19 mlp_hidden  20 mlp_mode  21 prior_mode  22 prior_seed  23 selection  24 puct_c
+ *     25 first_root  26 n_roots (the blob's global roots are [first_root, first_root + n_roots))
+ *     27 steps_done (steps since the last init/reset)  28 resets so far (keys azb_reset_trees' draws)  29 Adam step count
+ *     30..34 Adam lr, beta1, beta2, eps, l2   35 flags (bit 0: model parameters set)
+ *     36 running best: orderable bits of its eval (float bits u -> u | 0x80000000 if the sign bit is clear, else ~u)
+ *     37 its global root  38 its node  39..77 its state: 77 uint32 words (parents packed 4 per word in 16 words, then
+ *        61 permitted-mask words) two per uint64, low half first
+ *     78 n_params  79/80 model section offset/bytes  81/82 tree offset table offset/bytes  83/84 tree section offset/bytes
+ *     85 model section digest  86 tree offset table digest  87..94 zero  95 digest of words 0..94
+ *   model   params, Adam m, Adam v: n_params float32 each (m and v are zero before the first training step), zero-padded
+ *   table   uint64[n_roots + 1]: byte offset of every tree record inside the tree section; entry n_roots = its size
+ *   trees   one record per root in root order, uint32 words: the walker block (WS = 80 + 2 ceil(N/4) + 3W words: state,
+ *           path, bump pointers, step clock, root parents and permitted mask) | n_nodes node records of 16 words |
+ *           n_nodes keys of W words | the block arena units [64, nblk) of 2 words | the overflow in-arcs [0, intop) of 2
+ *           words | a zero word if the count is odd | the record's uint64 digest.  n_nodes, nblk and intop are walker
+ *           words 2, 3 and 5.  Not saved: the transposition table (rebuilt on load), cascade scratch, the consumed
+ *           per-step candidates, state vectors and priors (consumed by the add_actions that ran before the save), the
+ *           asynchronous kernel's ring and the workload counters.
+ * Digest of n uint64 words w_0..w_{n-1} (w_i = bytes 8i..8i+7 of the section, little-endian), with
+ *   mix64(z): z += 0x9E3779B97F4A7C15; z = (z ^ z >> 30) * 0xBF58476D1CE4E5B9; z = (z ^ z >> 27) * 0x94D049BB133111EB;
+ *             return z ^ z >> 31                                                              (all mod 2^64)
+ *   digest = mix64(S ^ n),  S = sum over i of mix64(w_i ^ (i * 0x9E3779B97F4A7C15)) mod 2^64.
+ * The sum makes it independent of the order in which its terms are added; it detects corruption and truncation and is
+ * not a security check.  Blocks and the overflow in-arc arena keep slots reserved for arcs not added yet; their
+ * bytes are whatever the arena held, so two handles holding the same trees may write different blobs, while two saves
+ * of one handle write the same bytes.
+ *
+ * azb_checkpoint_load rebuilds the handle's whole search and training state from one or more blobs whose ranges must
+ * cover the handle's [first_root, first_root + n_roots) exactly once; a blob may reach past it (its other roots are
+ * ignored) or lie outside it (only its header is read).  AZB_ERR_INVALID (azb_last_error names the field), before
+ * anything is written to the device: bad magic, format, version or header digest, a blob size that differs from its
+ * header's, a config field that differs from the handle's (N, c_lower, c_upper, n_as_tol, mlp_hidden, mlp_mode,
+ * prior_mode, prior_seed, selection, puct_c), blobs that disagree on steps_done, resets, Adam step or config, or model
+ * section, overlapping ranges, a gap in the handle's range, a bad model or table digest.  AZB_ERR_CAPACITY when the
+ * handle's max_steps is below steps_done.  Everything else may differ: n_roots and first_root (resharding), device,
+ * async_workers, n_groups, max_episodes, max_steps and the cap_* capacities.  A tree record that fails its digest is
+ * AZB_ERR_INVALID, one that does not fit the handle's capacities AZB_ERR_CAPACITY; the message names the lowest global
+ * root at fault, and the handle then behaves as before its first azb_init_trees until a load succeeds or azb_set_roots +
+ * azb_init_trees run.  After a successful load: the saved roots, walkers and trees; parameters, Adam m, v, step count
+ * and config; the reset count; steps_done; the running best = the first minimum by (eval, global root, node) over the
+ * running bests of ALL given blobs (with one blob of the same split, exactly the saved one; resharded, every shard starts
+ * from the global best, so the continued run's global best equals the uninterrupted run's, while azb_comm_argmin's owner
+ * and each shard's improvement log may differ).  Workload counters restart at zero: saved + continued counters equal the
+ * uninterrupted run's.  A communicator is not part of the state: attach it again with azb_comm_init. */
+#define AZB_CKPT_MAGIC 0x3154504B43425A41ull /* "AZBCKPT1" */
+#define AZB_CKPT_FORMAT 1
+#define AZB_CKPT_HEADER_WORDS 96
+int azb_checkpoint_size(azb_handle *h, uint64_t *bytes);
+int azb_checkpoint_save(azb_handle *h, void *buf, uint64_t size, uint64_t *written);
+int azb_checkpoint_load(azb_handle *h, const void *const *blobs, const uint64_t *sizes, uint32_t n_blobs);
 /* persistent walker state: states, paths, last_positions (optimizer/mod.rs:10-14) */
 int azb_get_walkers(azb_handle *h, uint8_t *parents, uint32_t *permitted, uint32_t *path, uint32_t *pos,
                     uint32_t *path_len);

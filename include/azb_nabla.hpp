@@ -78,6 +78,35 @@ class NablaOptimizer {
         o.reseed(root_parents, root_permitted);
         return o;
     }
+    // a new optimizer over cfg's roots continuing from checkpoint blobs (azb_checkpoint_load: one per rank of the saving
+    // run, any number of ranks); the built-in device model only
+    static NablaOptimizer resume(const azb_config &cfg, const std::vector<std::vector<uint8_t>> &blobs) {
+        NablaOptimizer o;
+        o.cfg_ = cfg;
+        o.cfg_.prior_mode = AZB_PRIOR_MLP;
+        o.ck(azb_create(&o.cfg_, &o.h_));
+        o.ck(azb_get_config(o.h_, &o.cfg_));
+        const uint32_t n = o.cfg_.n_vertices;
+        o.a_ = (n - 1) * (n - 2) / 2 - 1;
+        o.w_ = (o.a_ + 31) / 32;
+        std::vector<const void *> ptrs;
+        std::vector<uint64_t> sizes;
+        for (const auto &b : blobs) {
+            ptrs.push_back(b.data());
+            sizes.push_back(b.size());
+        }
+        o.ck(azb_checkpoint_load(o.h_, ptrs.data(), sizes.data(), (uint32_t)blobs.size()));
+        return o;
+    }
+    // the search and training state as a blob (azb_checkpoint_save; format in azb.h)
+    std::vector<uint8_t> save_checkpoint() {
+        uint64_t size = 0, written = 0;
+        ck(azb_checkpoint_size(h_, &size));
+        std::vector<uint8_t> blob(size);
+        ck(azb_checkpoint_save(h_, blob.data(), size, &written));
+        blob.resize(written);
+        return blob;
+    }
     NablaOptimizer(NablaOptimizer &&o) noexcept { *this = std::move(o); }
     NablaOptimizer &operator=(NablaOptimizer &&o) noexcept {
         std::swap(h_, o.h_);

@@ -15,7 +15,7 @@
 //! Not compiled in the build image (no Rust toolchain): see rust/README.md for what is checked instead.
 #![feature(isqrt)]
 
-use std::{collections::BTreeSet, ffi::CStr, os::raw::c_int};
+use std::{collections::BTreeSet, ffi::CStr, os::raw::{c_int, c_void}};
 
 use az_discrete_opt::{
     log::ArgminData,
@@ -202,6 +202,75 @@ impl<const N: usize, M: NablaModel> B200Optimizer<N, M> {
         max_steps_per_epoch: u32,
         selection: Selection,
     ) -> Self {
+        let roots: Vec<State<N>> = (0..batch).map(|_| init_states()).collect();
+        let mut me = Self::with_handle(space, model, roots, n_as_tol, max_steps_per_epoch, selection, 0);
+        me.assert_space_is_c21();
+        me.upload_roots_and_init();
+        me.refresh_argmin(true);
+        me
+    }
+
+    /// Continue a saved run (azb_checkpoint_load): a handle over `batch` roots from global root `first_root`, loaded
+    /// from the blobs of every rank of the saving run (any number of ranks).  Roots, trees, walkers, the device model
+    /// and its Adam state, the running best and the reset count are the saved ones; a host model keeps its own state.
+    /// The space, `n_as_tol` and `selection` must be the saving run's (the load refuses a different configuration).
+    pub fn resume(
+        space: Space<N>,
+        model: Model<M>,
+        batch: usize,
+        first_root: u64,
+        n_as_tol: impl Fn(usize) -> u32,
+        max_steps_per_epoch: u32,
+        selection: Selection,
+        blobs: &[&[u8]],
+    ) -> Self {
+        assert!(!blobs.is_empty() && blobs[0].len() >= 8 * sys::AZB_CKPT_HEADER_WORDS as usize, "checkpoint blobs");
+        let roots: Vec<State<N>> = (0..batch).map(|_| unflatten::<N>(&[0u8; N], &vec![0u32; Self::W])).collect();
+        let mut me = Self::with_handle(space, model, roots, n_as_tol, max_steps_per_epoch, selection, first_root);
+        let ptrs: Vec<*const c_void> = blobs.iter().map(|b| b.as_ptr() as *const c_void).collect();
+        let sizes: Vec<u64> = blobs.iter().map(|b| b.len() as u64).collect();
+        ck(me.h, unsafe { sys::azb_checkpoint_load(me.h, ptrs.as_ptr(), sizes.as_ptr(), blobs.len() as u32) });
+        // the device reset seeds continue from the saved reset count (header word 28, include/azb.h)
+        let resets = u64::from_le_bytes(blobs[0][8 * 28..8 * 29].try_into().unwrap());
+        for _ in 0..resets {
+            me.reset_seed = me.reset_seed.wrapping_mul(0x9E37_79B9_7F4A_7C15).wrapping_add(1);
+        }
+        let mut parents = vec![0u8; batch * N];
+        let mut masks = vec![0u32; batch * Self::W];
+        ck(me.h, unsafe { sys::azb_get_roots(me.h, parents.as_mut_ptr(), masks.as_mut_ptr()) });
+        for (i, r) in me.roots.iter_mut().enumerate() {
+            *r = unflatten::<N>(&parents[i * N..(i + 1) * N], &masks[i * Self::W..(i + 1) * Self::W]);
+        }
+        me.assert_space_is_c21();
+        me.refresh_argmin(true);
+        me
+    }
+
+    /// The search and training state as a checkpoint blob (azb_checkpoint_save; format in include/azb.h), after the
+    /// steps `roll_out_ahead` enqueued have completed.
+    pub fn save_checkpoint(&mut self) -> Vec<u8> {
+        if self.enqueued > 0 {
+            self.finish_batch();
+        }
+        let mut size = 0u64;
+        ck(self.h, unsafe { sys::azb_checkpoint_size(self.h, &mut size) });
+        let mut blob = vec![0u8; size as usize];
+        let mut written = 0u64;
+        ck(self.h, unsafe { sys::azb_checkpoint_save(self.h, blob.as_mut_ptr() as *mut c_void, size, &mut written) });
+        blob.truncate(written as usize);
+        blob
+    }
+
+    fn with_handle(
+        space: Space<N>,
+        model: Model<M>,
+        roots: Vec<State<N>>,
+        n_as_tol: impl Fn(usize) -> u32,
+        max_steps_per_epoch: u32,
+        selection: Selection,
+        first_root: u64,
+    ) -> Self {
+        let batch = roots.len();
         assert!(N >= 5 && N <= sys::AZB_MAX_VERTICES as usize && batch > 0);
         let mut cfg: sys::azb_config = unsafe { std::mem::zeroed() };
         ck(std::ptr::null(), unsafe { sys::azb_config_default(&mut cfg, N as u32, batch as u32) });
@@ -214,6 +283,7 @@ impl<const N: usize, M: NablaModel> B200Optimizer<N, M> {
         cfg.n_as_tol_len = 8;
         cfg.n_as_tol_default = table[8];
         cfg.max_steps = max_steps_per_epoch;
+        cfg.first_root = first_root;
         if let Selection::Puct { c_puct } = selection {
             cfg.selection = sys::AZB_SELECT_PUCT;
             cfg.puct_c = c_puct;
@@ -243,8 +313,7 @@ impl<const N: usize, M: NablaModel> B200Optimizer<N, M> {
             ck(h, unsafe { sys::azb_mlp_set_params(h, p.as_ptr()) });
         }
 
-        let roots: Vec<State<N>> = (0..batch).map(|_| init_states()).collect();
-        let mut me = Self {
+        Self {
             h,
             space,
             model: host_model,
@@ -257,11 +326,7 @@ impl<const N: usize, M: NablaModel> B200Optimizer<N, M> {
             n_as_tol: table,
             enqueued: 0,
             reset_seed: 0x5EED,
-        };
-        me.assert_space_is_c21();
-        me.upload_roots_and_init();
-        me.refresh_argmin(true);
-        me
+        }
     }
 
     /// The kernels hard-wire the c21 closures; refuse any other space (two probe states, bit-exact f32).

@@ -1,12 +1,15 @@
 //! Raw bindings, one to one with `include/azb.h` (same order, same names).  `tests/test_rust_binding.py` checks the
 //! struct layouts, the function list and the constants against the header and the ctypes binding.
 #![allow(non_camel_case_types)]
-use std::os::raw::{c_char, c_int};
+use std::os::raw::{c_char, c_int, c_void};
 
 pub const AZB_VERSION: c_int = 100;
 pub const AZB_NONE: u32 = 0xFFFF_FFFF;
 pub const AZB_MAX_VERTICES: u32 = 64;
 pub const AZB_MAX_TOL: usize = 8;
+pub const AZB_CKPT_MAGIC: u64 = 0x3154_504B_4342_5A41; // "AZBCKPT1"
+pub const AZB_CKPT_FORMAT: u32 = 1;
+pub const AZB_CKPT_HEADER_WORDS: u32 = 96;
 pub const AZB_ASYNC_AUTO: u32 = 0xFFFF_FFFF;
 
 pub const AZB_OK: c_int = 0;
@@ -122,6 +125,9 @@ extern "C" {
     pub fn azb_get_node_state(h: *mut azb_handle, tree: u32, node: u32, parents: *mut u8, permitted: *mut u32) -> c_int;
     pub fn azb_tree_codes(h: *mut azb_handle, parents: *const u8, m: u32, codes: *mut u64, ms: *mut f32) -> c_int;
     pub fn azb_best_trees(h: *mut azb_handle, k: u32, n_out: *mut u32, eval: *mut f32, codes: *mut u64, tree: *mut u32, node: *mut u32, parents: *mut u8, permitted: *mut u32, lambda1: *mut f64, mu: *mut u32) -> c_int;
+    pub fn azb_checkpoint_size(h: *mut azb_handle, bytes: *mut u64) -> c_int;
+    pub fn azb_checkpoint_save(h: *mut azb_handle, buf: *mut c_void, size: u64, written: *mut u64) -> c_int;
+    pub fn azb_checkpoint_load(h: *mut azb_handle, blobs: *const *const c_void, sizes: *const u64, n_blobs: u32) -> c_int;
     pub fn azb_get_walkers(h: *mut azb_handle, parents: *mut u8, permitted: *mut u32, path: *mut u32, pos: *mut u32, path_len: *mut u32) -> c_int;
     pub fn azb_tree_sizes(h: *mut azb_handle, tree: u32, n_nodes: *mut u32, n_arcs: *mut u32, n_preds: *mut u32) -> c_int;
     pub fn azb_dump_tree(h: *mut azb_handle, tree: u32, nodes: *mut u32, keys: *mut u32, preds: *mut u32, arcs: *mut u32) -> c_int;
