@@ -89,6 +89,10 @@ SIGNATURES = {
     "azb_get_node_state": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, u8p, u32p]),
     "azb_tree_codes": (C.c_int, [C.c_void_p, u8p, C.c_uint32, C.POINTER(C.c_uint64), f32p]),
     "azb_best_trees": (C.c_int, [C.c_void_p, C.c_uint32, u32p, f32p, C.POINTER(C.c_uint64), u32p, u32p, u8p, u32p, f64p, u32p]),
+    "azb_free_tree_count": (C.c_int, [C.c_uint32, C.POINTER(C.c_uint64)]),
+    "azb_free_trees": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint32, u8p]),
+    "azb_exhaustive_best": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_double, u32p, C.POINTER(C.c_uint64),
+                                      C.POINTER(C.c_uint64), u8p, f64p, u32p, f32p, f32p]),
     "azb_checkpoint_size": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     "azb_checkpoint_save": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]),
     "azb_checkpoint_load": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64), C.c_uint32]),
@@ -190,6 +194,15 @@ def generate_roots(seed, first_root, count, n, k_min=5, k_max=0):
     if rc:
         raise AzbError(rc, lib().azb_strerror(rc).decode())
     return parents, masks
+
+
+def free_tree_count(n: int) -> int:
+    """A000055(n): the number of free trees on n vertices, 5 <= n <= 32 (host only)."""
+    out = C.c_uint64()
+    rc = lib().azb_free_tree_count(n, C.byref(out))
+    if rc:
+        raise AzbError(rc, f"{lib().azb_strerror(rc).decode()}: n must be in 5..32, got {n}")
+    return int(out.value)
 
 
 class Handle:
@@ -533,6 +546,32 @@ class Handle:
                                         _p(out["parents"], C.c_uint8), _p(out["permitted"], C.c_uint32),
                                         _p(out["lambda1"], C.c_double), _p(out["mu"], C.c_uint32)))
         return {name: a[:n.value] for name, a in out.items()}
+
+    def free_trees(self, start: int, m: int):
+        """Parent arrays u8[m, N] of the free trees with indices [start, start + m) of the enumeration in include/azb.h."""
+        out = np.zeros((max(int(m), 1), self.n), dtype=np.uint8)
+        self._ck(self._L.azb_free_trees(self._h, start, m, _p(out, C.c_uint8)))
+        return out[:m]
+
+    def exhaustive_best(self, start: int = 0, count=None, k: int = 100, bound=None):
+        """The exact k best free trees of indices [start, start + count) (default: to the end) by key = mu + lambda1, ties
+        by index (azb_exhaustive_best): dict of arrays index u64, parents u8[., N], lambda1 f64, mu u32, eval f32, plus
+        n_below (trees with key < bound; default sqrt(N - 1) + 1, the star's key) and ms (device time)."""
+        if count is None:
+            count = free_tree_count(self.n) - start if self.n <= 32 else 1  # N > 32: the library refuses the handle
+        if bound is None:
+            bound = float(np.sqrt(self.n - 1)) + 1.0
+        kk = max(min(int(k), int(count)), 1)
+        out = dict(index=np.zeros(kk, dtype=np.uint64), parents=np.zeros((kk, self.n), dtype=np.uint8),
+                   lambda1=np.zeros(kk, dtype=np.float64), mu=np.zeros(kk, dtype=np.uint32), eval=np.zeros(kk, dtype=np.float32))
+        n, below, ms = C.c_uint32(), C.c_uint64(), C.c_float()
+        self._ck(self._L.azb_exhaustive_best(self._h, start, count, k, bound, C.byref(n), C.byref(below),
+                                             _p(out["index"], C.c_uint64), _p(out["parents"], C.c_uint8),
+                                             _p(out["lambda1"], C.c_double), _p(out["mu"], C.c_uint32),
+                                             _p(out["eval"], C.c_float), C.byref(ms)))
+        res = {name: a[:n.value] for name, a in out.items()}
+        res.update(n_below=int(below.value), ms=float(ms.value))
+        return res
 
     def comm_allreduce_bench(self, reps: int = 20) -> float:
         ms = C.c_float()

@@ -28,6 +28,7 @@
 #include "azb_async.cuh"
 #include "azb_best.cuh"
 #include "azb_ckpt.cuh"
+#include "azb_enum.cuh"
 
 #include <dlfcn.h>
 
@@ -72,6 +73,12 @@ struct azb_handle {
     uint64_t ckpt_chunk;
     uint64_t ckpt_best_root;
     uint32_t ckpt_best_node;
+    // azb_free_trees / azb_exhaustive_best (azb_enum.cuh): the enumeration tables (built on first use) and the chunk size
+    // tests set through AZB_TEST_ENUM_CHUNK (0 = AZB_ENUM_CHUNK); their scratch is best_buf
+    AzbEnum en;
+    unsigned long long *en_P;
+    uint8_t *en_rp;
+    uint32_t en_chunk;
     // observations scratch
     float *obs, *obs_w;
     // training step (azb_train.cuh): gradient (parameter order), Adam moments, predictions, two dZ buffers, scalars
@@ -230,7 +237,7 @@ int azb_destroy(azb_handle *h) {
                     h->L.walker, h->L.node, h->L.blk, h->L.inl, h->L.key, h->L.hash, h->L.casc, h->L.cand, h->L.stepmin, (void *)h->L.lut, h->L.sv,
                     h->L.h, h->L.g, h->L.log, h->params, h->act[0], h->act[1], h->act[2], h->mlp_x, h->mlp_y, h->sv16_save,
                     h->cost_par, h->cost_l1, h->cost_mu, h->cost_c, h->cost_err, h->obs, h->obs_w, h->flush_buf, h->graph_buf,
-                    h->best_buf, h->best_st, h->ckpt_buf};
+                    h->best_buf, h->best_st, h->ckpt_buf, h->en_P, h->en_rp};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     azb_mlp_tc_destroy(h->tc);
@@ -386,6 +393,8 @@ int azb_create(const azb_config *cfg_in, azb_handle **out) {
         h->best_m_cap = (uint32_t)std::max(1, atoi(e));
     if (const char *e = getenv("AZB_TEST_CKPT_CHUNK"))  // tests: push checkpoints through many staging chunks
         h->ckpt_chunk = std::max<uint64_t>(8, strtoull(e, nullptr, 10));
+    if (const char *e = getenv("AZB_TEST_ENUM_CHUNK"))  // tests: push azb_exhaustive_best through many threshold updates
+        h->en_chunk = (uint32_t)std::max(1, atoi(e));
     L.first_root = cfg.first_root;
     L.prior_seed = cfg.prior_seed;
     CK(dmalloc(h, &L.walker, (size_t)B * L.WS));
@@ -1814,7 +1823,7 @@ extern "C" int azb_get_node_state(azb_handle *h, uint32_t tree, uint32_t node, u
 // ---- the k best isomorphism classes (azb_best.cuh) ----
 static size_t best_up(size_t x) { return (x + 255) & ~(size_t)255; }
 
-// the grow-only slab of azb_tree_codes / azb_best_trees (counted in azb_device_bytes)
+// the grow-only slab of azb_tree_codes, azb_best_trees, azb_free_trees and azb_exhaustive_best (counted in azb_device_bytes)
 static int best_slab(azb_handle *h, size_t bytes) {
     if (bytes <= h->best_cap) return AZB_OK;
     if (h->best_buf) {
@@ -1966,6 +1975,176 @@ extern "C" int azb_best_trees(azb_handle *h, uint32_t k, uint32_t *n_out, float 
         if (node) node[i] = (uint32_t)(cls[i].id & 0xfffffu);
     }
     if (n_out) *n_out = n;
+    return AZB_OK;
+}
+
+// ---- every free tree on N <= 32 vertices by index, and the exact k best of an index range (azb_enum.cuh) ----
+extern "C" int azb_free_tree_count(uint32_t n, uint64_t *count) {
+    if (!count || n < 5 || n > AZB_ENUM_MAX_N) return AZB_ERR_INVALID;
+    uint64_t U = 0;
+    azb_enum_counts(n, &U, count);
+    return AZB_OK;
+}
+
+static uint64_t enum_total(const azb_handle *h) {
+    const AzbEnum &E = h->en;
+    const uint64_t t = E.n % 2 == 0 ? E.off[E.smax + 1] - E.off[E.smax] : 0;  // rooted trees of size N / 2
+    return E.U + t * (t + 1) / 2;
+}
+
+// the tables of the handle's N, built on the host and uploaded on first use (counted in azb_device_bytes)
+static int enum_tables(azb_handle *h, const char *fn) {
+    if (h->N > AZB_ENUM_MAX_N)
+        return fail(h, AZB_ERR_INVALID, "%s: the enumeration covers N <= %u, the handle has N = %u", fn, AZB_ENUM_MAX_N, h->N);
+    if (h->en.P) return AZB_OK;
+    std::vector<unsigned long long> P;
+    std::vector<uint8_t> rp;
+    AzbEnum E;
+    azb_enum_build(h->N, E, P, rp);
+    if (!h->en_P) CK(dmalloc(h, &h->en_P, P.size()));
+    if (!h->en_rp) CK(dmalloc(h, &h->en_rp, rp.size()));
+    CK(cudaMemcpyAsync(h->en_P, P.data(), P.size() * 8, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->en_rp, rp.data(), rp.size(), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    E.P = h->en_P;
+    E.rp = h->en_rp;
+    h->en = E;
+    return AZB_OK;
+}
+
+static int enum_range(azb_handle *h, const char *fn, uint64_t start, uint64_t count) {
+    const uint64_t total = enum_total(h);
+    if (count == 0 || start > total || count > total - start)
+        return fail(h, AZB_ERR_INVALID, "%s: %llu trees from index %llu are not all in [0, %llu)", fn, (unsigned long long)count,
+                    (unsigned long long)start, (unsigned long long)total);
+    return AZB_OK;
+}
+
+static int enum_sms(azb_handle *h, int *sms) {
+    CK(cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, h->cfg.device));
+    return AZB_OK;
+}
+
+extern "C" int azb_free_trees(azb_handle *h, uint64_t start, uint32_t m, uint8_t *parents) {
+    if (!h) return AZB_ERR_INVALID;
+    CK(cudaSetDevice(h->cfg.device));
+    int rc = enum_tables(h, "azb_free_trees");
+    if (rc) return rc;
+    if (!parents) return fail(h, AZB_ERR_INVALID, "azb_free_trees: parents is NULL");
+    rc = enum_range(h, "azb_free_trees", start, m);
+    if (rc) return rc;
+    int sms = 0;
+    rc = enum_sms(h, &sms);
+    if (rc) return rc;
+    const uint32_t N = h->N, chunk = h->en_chunk ? h->en_chunk : AZB_ENUM_CHUNK;
+    rc = best_slab(h, (size_t)std::min(m, chunk) * N);
+    if (rc) return rc;
+    for (uint32_t done = 0; done < m;) {
+        const uint32_t c = std::min(chunk, m - done);
+        azb_enum_trees_kernel<<<std::min<uint32_t>((c + 7) / 8, (uint32_t)sms * 16u), 256, 0, h->stream>>>(h->en, start + done, nullptr, c,
+                                                                                                          h->best_buf);
+        h->launches += 1;
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(parents + (size_t)done * N, h->best_buf, (size_t)c * N, cudaMemcpyDeviceToHost, h->stream));
+        done += c;
+    }
+    CK(cudaStreamSynchronize(h->stream));
+    return AZB_OK;
+}
+
+struct AzbEnumScalars {
+    unsigned long long thr;    // the k-th best key bits so far (all ones until k trees are in)
+    unsigned long long below;  // trees with key < bound
+    uint32_t n_cand, err;
+};
+
+// Chunks in ascending index order.  The running top k sits at the front of buffer A; a chunk's candidates (key bits <= the
+// k-th best so far) land behind it, the whole is radix-sorted by (key bits, index) into B and the first k go back to A.  A
+// later tree whose key equals the threshold has a larger index than all k kept ones and would lose the tie, so the
+// result is the exact top k of the range.
+extern "C" int azb_exhaustive_best(azb_handle *h, uint64_t start, uint64_t count, uint32_t k, double bound, uint32_t *n_out,
+                                   uint64_t *n_below, uint64_t *index, uint8_t *parents, double *lambda1, uint32_t *mu, float *eval,
+                                   float *ms) {
+    if (!h) return AZB_ERR_INVALID;
+    CK(cudaSetDevice(h->cfg.device));
+    int rc = enum_tables(h, "azb_exhaustive_best");
+    if (rc) return rc;
+    if (k == 0 || k > AZB_BEST_MAX_K) return fail(h, AZB_ERR_INVALID, "k must be in 1..%u, got %u", AZB_BEST_MAX_K, k);
+    rc = enum_range(h, "azb_exhaustive_best", start, count);
+    if (rc) return rc;
+    int sms = 0;
+    rc = enum_sms(h, &sms);
+    if (rc) return rc;
+    const uint32_t N = h->N, chunk = h->en_chunk ? h->en_chunk : AZB_ENUM_CHUNK, cap = k + chunk;
+    const uint32_t n_res = (uint32_t)std::min<uint64_t>(k, count);
+    int bps = 0;
+    if (N <= 22) CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, azb_enum_best_kernel<3>, 256, 0));
+    else CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, azb_enum_best_kernel<4>, 256, 0));
+    const uint32_t grid = (uint32_t)std::max(1, sms * bps);
+    size_t tmp_bytes = 0;
+    CK(cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, (const AzbEnumCand *)nullptr, (AzbEnumCand *)nullptr, cap, AzbEnumByKey{},
+                                      h->stream));
+    const size_t o_b = best_up((size_t)cap * sizeof(AzbEnumCand)), o_par = 2 * o_b, o_sc = o_par + best_up((size_t)k * N),
+                 o_tmp = o_sc + 256;
+    rc = best_slab(h, o_tmp + tmp_bytes);
+    if (rc) return rc;
+    rc = cost_buffers(h, n_res);
+    if (rc) return rc;
+    AzbEnumCand *d_a = reinterpret_cast<AzbEnumCand *>(h->best_buf), *d_b = reinterpret_cast<AzbEnumCand *>(h->best_buf + o_b);
+    uint8_t *d_par = h->best_buf + o_par;
+    AzbEnumScalars *d_sc = reinterpret_cast<AzbEnumScalars *>(h->best_buf + o_sc);
+    CK(cudaEventRecord(h->ev0, h->stream));
+    CK(cudaMemsetAsync(d_sc, 0, sizeof(AzbEnumScalars), h->stream));
+    CK(cudaMemsetAsync(&d_sc->thr, 0xff, 8, h->stream));
+    uint32_t nb = 0;  // entries of the running top k at the front of A
+    for (uint64_t done = 0; done < count;) {
+        const uint32_t c = (uint32_t)std::min<uint64_t>(chunk, count - done);
+        const uint32_t blocks = std::min(grid, (c + 7) / 8);
+        CK(cudaMemsetAsync(&d_sc->n_cand, 0, 4, h->stream));
+        if (N <= 22)
+            azb_enum_best_kernel<3><<<blocks, 256, 0, h->stream>>>(h->en, start + done, c, &d_sc->thr, bound, d_a + nb, &d_sc->n_cand,
+                                                                   &d_sc->below, &d_sc->err);
+        else
+            azb_enum_best_kernel<4><<<blocks, 256, 0, h->stream>>>(h->en, start + done, c, &d_sc->thr, bound, d_a + nb, &d_sc->n_cand,
+                                                                   &d_sc->below, &d_sc->err);
+        h->launches += 1;
+        CK(cudaGetLastError());
+        uint32_t nc = 0;
+        CK(cudaMemcpyAsync(&nc, &d_sc->n_cand, 4, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        done += c;
+        if (nc == 0) continue;
+        const uint32_t tot = nb + nc;
+        CK(cub::DeviceRadixSort::SortKeys(h->best_buf + o_tmp, tmp_bytes, d_a, d_b, tot, AzbEnumByKey{}, h->stream));
+        nb = std::min(k, tot);
+        CK(cudaMemcpyAsync(d_a, d_b, (size_t)nb * sizeof(AzbEnumCand), cudaMemcpyDeviceToDevice, h->stream));
+        if (nb == k) CK(cudaMemcpyAsync(&d_sc->thr, &d_b[k - 1].key, 8, cudaMemcpyDeviceToDevice, h->stream));
+    }
+    // the result's parent arrays, and lambda_1, mu and eval from the stand-alone cost kernel (what azb_eval_costs gives)
+    azb_enum_trees_kernel<<<std::min<uint32_t>((nb + 7) / 8, (uint32_t)sms * 16u), 256, 0, h->stream>>>(h->en, 0ull, d_a, nb, d_par);
+    h->launches += 1;
+    CK(cudaGetLastError());
+    CK(cudaMemsetAsync(h->cost_err, 0, 4, h->stream));
+    launch_cost_kernel(h, d_par, nb);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(h->ev1, h->stream));
+    std::vector<AzbEnumCand> res(nb);
+    AzbEnumScalars sc;
+    uint32_t cerr = 0;
+    CK(cudaMemcpyAsync(res.data(), d_a, (size_t)nb * sizeof(AzbEnumCand), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(&sc, d_sc, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
+    if (parents) CK(cudaMemcpyAsync(parents, d_par, (size_t)nb * N, cudaMemcpyDeviceToHost, h->stream));
+    if (lambda1) CK(cudaMemcpyAsync(lambda1, h->cost_l1, (size_t)nb * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (mu) CK(cudaMemcpyAsync(mu, h->cost_mu, (size_t)nb * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (eval) CK(cudaMemcpyAsync(eval, h->cost_c, (size_t)nb * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(&cerr, h->cost_err, 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (ms) CK(cudaEventElapsedTime(ms, h->ev0, h->ev1));
+    if (sc.err || cerr) return fail(h, AZB_ERR_LAMBDA, "%s", azb_strerror(AZB_ERR_LAMBDA));
+    if (index)
+        for (uint32_t i = 0; i < nb; ++i) index[i] = res[i].idx;
+    if (n_below) *n_below = sc.below;
+    if (n_out) *n_out = nb;
     return AZB_OK;
 }
 

@@ -64,6 +64,28 @@ def global_best_trees(local: list, k: int, dist=None) -> list:
     return acc.result()
 
 
+def merge_exhaustive_best(results: list, k: int) -> dict:
+    """The k best of several Handle.exhaustive_best results over disjoint index ranges, by (key, index) with key =
+    mu + lambda1 in f64 as the library computes it, so the merge equals one call over the union; n_below is summed."""
+    cat = {name: np.concatenate([r[name] for r in results]) for name in ("index", "parents", "lambda1", "mu", "eval")}
+    key = cat["mu"].astype(np.float64) + cat["lambda1"]
+    order = np.lexsort((cat["index"], key))[:k]
+    out = {name: a[order] for name, a in cat.items()}
+    out["n_below"] = sum(int(r["n_below"]) for r in results)
+    return out
+
+
+def global_exhaustive_best(local: dict, k: int, dist=None) -> dict:
+    """The k best free trees over all ranks, each rank having ranked its shard_range(A000055(N), rank, world) of the
+    enumeration with Handle.exhaustive_best: gathered and merged by (key, index), equal to one call over the whole range;
+    n_below is summed."""
+    if dist is None or not dist.is_initialized() or dist.get_world_size() == 1:
+        return merge_exhaustive_best([local], k)
+    lists = [None] * dist.get_world_size()
+    dist.all_gather_object(lists, {name: local[name] for name in ("index", "parents", "lambda1", "mu", "eval", "n_below")})
+    return merge_exhaustive_best(lists, k)
+
+
 def checkpoint_path(directory: str, rank: int) -> str:
     """Where rank `rank` keeps its checkpoint blob inside a run's checkpoint directory."""
     return os.path.join(directory, f"rank{rank:05d}.azbckpt")

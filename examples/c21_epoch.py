@@ -3,12 +3,15 @@
 mirror of NablaOptimizer (azdopt_b200/nabla.py) — same constants, same outputs:
 
     python examples/c21_epoch.py [--batch 512] [--epochs 3] [--episodes 800] [--out out_dir] [--checkpoint DIR [--resume]]
+                                 [--exhaustive]
 
 Per epoch: `episodes` search steps fused on the device (improvements are printed with their step like the example's
 process_argmin), par_update_model (loss), par_reset_trees with the example's modify_root policy.  Writes a TensorBoard
 event file with the example's scalar tags, the best tree as graph6 and the first search DAG as Graphviz DOT.
 With --checkpoint DIR the run is saved after every epoch (search and training state, the BestTrees accumulator and the
 epoch count); --resume continues from the last save exactly where the interrupted run would have gone on.
+With --exhaustive every tree on N vertices is ranked on the device before the first epoch (each rank its share of the
+enumeration, like the roots) and every epoch logs the gap between the run's best and that exact optimum.
 """
 import argparse
 import os
@@ -39,6 +42,8 @@ def main():
                     help="also keep the K best non-isomorphic trees over all epochs in best_trees.g6")
     ap.add_argument("--checkpoint", metavar="DIR", help="save the run here after every epoch")
     ap.add_argument("--resume", action="store_true", help="continue from the last checkpoint in --checkpoint DIR")
+    ap.add_argument("--exhaustive", action="store_true",
+                    help="rank every tree on N vertices first and log each epoch's gap to the exact optimum")
     args = ap.parse_args()
     if args.resume and not args.checkpoint:
         ap.error("--resume needs --checkpoint DIR")
@@ -57,6 +62,15 @@ def main():
         roots = capi.generate_roots(args.seed, 0, args.batch, N)  # ROTWithActionPermissions::generate, k ~ U{5..A/2} (:85,108-112)
         opt = nabla.NablaOptimizer.par_new(space, roots, model, args.batch, max_steps=args.episodes)
     goal = squish(5.2)                                         # :117
+    optimum = None
+    if args.exhaustive:
+        rank, world = 0, 1                                     # one process here; each rank of a sharded run takes its range
+        total = capi.free_tree_count(N)
+        lo, hi = shard.shard_range(total, rank, world)
+        ex = shard.global_exhaustive_best(opt.h.exhaustive_best(lo, hi - lo, k=1), 1)
+        optimum = float(ex["eval"][0])
+        print(f"exact optimum over all {total} trees: eval {optimum:.6f} lambda_1={ex['lambda1'][0]:.6f} mu={ex['mu'][0]} "
+              f"(index {ex['index'][0]}); {ex['n_below']} trees below the star's sqrt(N - 1) + 1")
 
     def save_checkpoint(epoch):
         os.makedirs(args.checkpoint, exist_ok=True)
@@ -87,6 +101,8 @@ def main():
                 best.add(opt.best_trees(args.best))
             for (step, tree, node, ev) in improved:
                 print(f"  step {args.episodes * (epoch - 1) + step + 1}: tree {tree} node {node} eval {ev:.6f}")
+            if optimum is not None:
+                print(f"  gap to the exact optimum: {opt.argmin_data().eval - optimum:.6f}")
             if improved and process_argmin(opt.argmin_data(), args.episodes * epoch):
                 print("state is optimal:", opt.argmin_data().parents.tolist())
                 break

@@ -306,6 +306,40 @@ int azb_best_trees(azb_handle *h, uint32_t k, uint32_t *n_out, float *eval /*[k]
 int azb_checkpoint_size(azb_handle *h, uint64_t *bytes);
 int azb_checkpoint_save(azb_handle *h, void *buf, uint64_t size, uint64_t *written);
 int azb_checkpoint_load(azb_handle *h, const void *const *blobs, const uint64_t *sizes, uint32_t n_blobs);
+/* ---- extension (no reference item): every free tree on N <= 32 vertices by index, and the exact k best of any index
+ *      range by the c21 cost.
+ * The enumeration.  Rooted trees carry global ids, ordered by size first (the single vertex is id 0), then by rank
+ * within their size s: a rooted tree of size s is its root plus the multiset of its child subtrees, written as the
+ * NON-INCREASING sequence of the children's global ids (their sizes sum to s - 1), and rank orders these sequences
+ * lexicographically ascending (none is a proper prefix of another: all have the same size sum).  Size s has A000081(s)
+ * ids.  A free tree on N vertices is rooted at its centroid:
+ *   - unicentroidal trees take the indices [0, U): a non-increasing sequence of global ids whose sizes sum to N - 1, every
+ *     size <= floor((N - 1) / 2), in lexicographically ascending order; U is the number of such sequences;
+ *   - for even N the bicentroidal trees follow: the unordered pair of rooted trees of size N / 2 with in-size ranks
+ *     i >= j has index U + i (i + 1) / 2 + j.
+ * Labels are preorder with children visited in sequence order: the root is vertex 0, then the subtree of each element of
+ * the sequence in turn, each laid out the same way (its root first, with parent the vertex it hangs from).  A bicentroidal
+ * tree has the root of tree i at vertex 0, tree j at vertices 1 .. N/2 (its root at 1, parent 0), then tree i's child
+ * subtrees.  So parents[v] < v, vertex 0 is a centroid, and A000055(N) indices cover every isomorphism class once.
+ * Unranking: with P[r][g] = the number of non-increasing sequences of ids <= g whose sizes sum to r, the sequences of sum
+ * r with first element < g number P[r][g - 1]; an index is decoded one element at a time (the smallest g with P[r][g] > x,
+ * then x -= P[r][g - 1], r -= size(g)).  The handle builds P (rows r = 0..N-1, 32 x 141 083 words at N = 32) and the
+ * preorder arrays of all rooted trees of size <= N/2 on first use; both count in azb_device_bytes.
+ * azb_free_tree_count: A000055(n) for 5 <= n <= 32, host only.
+ * azb_free_trees: the parent arrays of indices [start, start + m) of the handle's N.
+ * azb_exhaustive_best: every tree of [start, start + count) through the cost kernel of azb_eval_costs; the first
+ * min(k, count) sorted ascending by key = (double)mu + lambda1 (one IEEE add), ties by index.  Per entry: the index, its
+ * parent array (exactly azb_free_trees'), lambda1, mu and eval = the f32 c azb_eval_costs gives for it.  *n_out = the
+ * number of entries, *n_below = the number of trees of the range with key < bound (bound = sqrt(N - 1) + 1, the star's
+ * key, counts the counterexamples of the conjecture).  ms = device time of the whole call.  Any output pointer may be NULL.
+ * Both calls: AZB_ERR_INVALID for a handle with N > 32 and for a range that is empty (count or m = 0) or reaches past
+ * A000055(N); azb_exhaustive_best also for k == 0 or k > 65536 and AZB_ERR_LAMBDA as azb_eval_costs.  They work before
+ * azb_init_trees, run on the library stream and change no tree, walker, counter, argmin, model or RNG state. */
+int azb_free_tree_count(uint32_t n, uint64_t *count);
+int azb_free_trees(azb_handle *h, uint64_t start, uint32_t m, uint8_t *parents /*[m*N]*/);
+int azb_exhaustive_best(azb_handle *h, uint64_t start, uint64_t count, uint32_t k, double bound, uint32_t *n_out,
+                        uint64_t *n_below, uint64_t *index /*[k]*/, uint8_t *parents /*[k*N]*/, double *lambda1 /*[k]*/,
+                        uint32_t *mu /*[k]*/, float *eval /*[k]*/, float *ms);
 /* persistent walker state: states, paths, last_positions (optimizer/mod.rs:10-14) */
 int azb_get_walkers(azb_handle *h, uint8_t *parents, uint32_t *permitted, uint32_t *path, uint32_t *pos,
                     uint32_t *path_len);

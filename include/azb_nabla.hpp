@@ -6,6 +6,7 @@
 // (nabla/model/mod.rs:4-8), ArgminData (log.rs:1-11), ArgminImprovement (optimizer/mod.rs:24-27).
 // Error behaviour: the reference panics (process abort); here every violation throws azb::Error.
 #pragma once
+#include <cmath>
 #include <cstdint>
 #include <functional>
 #include <optional>
@@ -35,6 +36,15 @@ struct BestTree {
     ArgminData data;
     uint64_t code[2] = {0, 0};
     uint32_t tree = 0, node = 0;
+};
+
+// one entry of exhaustive_best: a free tree of the enumeration in azb.h, by its index
+struct ExhaustiveTree {
+    uint64_t index = 0;
+    std::vector<uint8_t> parents;
+    double lambda_1 = 0.0;
+    uint32_t mu = 0;
+    float eval = 0.0f;
 };
 
 // NablaModel (nabla/model/mod.rs:4-8) for models that live on the host
@@ -193,6 +203,35 @@ class NablaOptimizer {
             b.code[1] = codes[2 * i + 1];
             b.tree = tree[i];
             b.node = node[i];
+        }
+        return out;
+    }
+    // the exact k best free trees of enumeration indices [start, start + count) by mu + lambda_1, ties by index
+    // (azb_exhaustive_best, N <= 32; count 0 = to the end of the enumeration); bound as in azb.h (< 0: sqrt(N - 1) + 1)
+    std::vector<ExhaustiveTree> exhaustive_best(uint64_t start = 0, uint64_t count = 0, uint32_t k = 100, double bound = -1.0,
+                                                uint64_t *n_below = nullptr) {
+        const size_t n_v = cfg_.n_vertices;
+        if (count == 0) {
+            uint64_t total = 0;
+            if (azb_free_tree_count(cfg_.n_vertices, &total) == AZB_OK && total > start) count = total - start;
+        }
+        if (bound < 0.0) bound = std::sqrt((double)(n_v - 1)) + 1.0;
+        const size_t kk = k ? k : 1;
+        std::vector<uint64_t> index(kk);
+        std::vector<uint8_t> parents(kk * n_v);
+        std::vector<double> l1(kk);
+        std::vector<uint32_t> mu(kk);
+        std::vector<float> eval(kk);
+        uint32_t n = 0;
+        ck(azb_exhaustive_best(h_, start, count, k, bound, &n, n_below, index.data(), parents.data(), l1.data(), mu.data(),
+                               eval.data(), nullptr));
+        std::vector<ExhaustiveTree> out(n);
+        for (uint32_t i = 0; i < n; ++i) {
+            out[i].index = index[i];
+            out[i].parents.assign(parents.begin() + i * n_v, parents.begin() + (i + 1) * n_v);
+            out[i].lambda_1 = l1[i];
+            out[i].mu = mu[i];
+            out[i].eval = eval[i];
         }
         return out;
     }
