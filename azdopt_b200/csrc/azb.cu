@@ -9,6 +9,7 @@
 #include <time.h>
 
 #include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -29,6 +30,7 @@
 #include "azb_best.cuh"
 #include "azb_ckpt.cuh"
 #include "azb_enum.cuh"
+#include "azb_grow.cuh"
 
 #include <dlfcn.h>
 
@@ -79,6 +81,9 @@ struct azb_handle {
     unsigned long long *en_P;
     uint8_t *en_rp;
     uint32_t en_chunk;
+    // azb_trees_within (azb_grow.cuh): children per chunk, set by tests through AZB_TEST_GROW_CHUNK (0 = AZB_GROW_CHUNK);
+    // its scratch is best_buf
+    uint32_t grow_chunk;
     // observations scratch
     float *obs, *obs_w;
     // training step (azb_train.cuh): gradient (parameter order), Adam moments, predictions, two dZ buffers, scalars
@@ -395,6 +400,8 @@ int azb_create(const azb_config *cfg_in, azb_handle **out) {
         h->ckpt_chunk = std::max<uint64_t>(8, strtoull(e, nullptr, 10));
     if (const char *e = getenv("AZB_TEST_ENUM_CHUNK"))  // tests: push azb_exhaustive_best through many threshold updates
         h->en_chunk = (uint32_t)std::max(1, atoi(e));
+    if (const char *e = getenv("AZB_TEST_GROW_CHUNK"))  // tests: push azb_trees_within through many chunks and merges
+        h->grow_chunk = (uint32_t)std::max(1, atoi(e));
     L.first_root = cfg.first_root;
     L.prior_seed = cfg.prior_seed;
     CK(dmalloc(h, &L.walker, (size_t)B * L.WS));
@@ -1439,14 +1446,20 @@ static int cost_buffers(azb_handle *h, uint32_t m) {
     return AZB_OK;
 }
 
-static void launch_cost_kernel(azb_handle *h, const uint8_t *dev_parents, uint32_t m) {
+// the cost kernel on m trees of n vertices (azb_trees_within evaluates every level below N with it)
+static void launch_cost_n(azb_handle *h, const uint8_t *dev_parents, uint32_t m, uint32_t n, double *l1, uint32_t *mu, float *c,
+                          uint32_t *err) {
     const uint32_t threads = 256, blocks = (m + 7) / 8;
-    switch (azb_stack_depth(h->N)) {
-        case 3: azb_cost_kernel<3><<<blocks, threads, 0, h->stream>>>(dev_parents, m, h->N, h->L.c_lower, h->L.slope, h->cost_l1, h->cost_mu, h->cost_c, h->cost_err); break;
-        case 4: azb_cost_kernel<4><<<blocks, threads, 0, h->stream>>>(dev_parents, m, h->N, h->L.c_lower, h->L.slope, h->cost_l1, h->cost_mu, h->cost_c, h->cost_err); break;
-        default: azb_cost_kernel<5><<<blocks, threads, 0, h->stream>>>(dev_parents, m, h->N, h->L.c_lower, h->L.slope, h->cost_l1, h->cost_mu, h->cost_c, h->cost_err); break;
+    switch (azb_stack_depth(n)) {
+        case 3: azb_cost_kernel<3><<<blocks, threads, 0, h->stream>>>(dev_parents, m, n, h->L.c_lower, h->L.slope, l1, mu, c, err); break;
+        case 4: azb_cost_kernel<4><<<blocks, threads, 0, h->stream>>>(dev_parents, m, n, h->L.c_lower, h->L.slope, l1, mu, c, err); break;
+        default: azb_cost_kernel<5><<<blocks, threads, 0, h->stream>>>(dev_parents, m, n, h->L.c_lower, h->L.slope, l1, mu, c, err); break;
     }
     h->launches += 1;
+}
+
+static void launch_cost_kernel(azb_handle *h, const uint8_t *dev_parents, uint32_t m) {
+    launch_cost_n(h, dev_parents, m, h->N, h->cost_l1, h->cost_mu, h->cost_c, h->cost_err);
 }
 
 static int eval_costs_dev(azb_handle *h, const uint8_t *parents, uint32_t m, double *lambda1, uint32_t *mu, float *c,
@@ -1823,7 +1836,8 @@ extern "C" int azb_get_node_state(azb_handle *h, uint32_t tree, uint32_t node, u
 // ---- the k best isomorphism classes (azb_best.cuh) ----
 static size_t best_up(size_t x) { return (x + 255) & ~(size_t)255; }
 
-// the grow-only slab of azb_tree_codes, azb_best_trees, azb_free_trees and azb_exhaustive_best (counted in azb_device_bytes)
+// the grow-only slab of azb_tree_codes, azb_best_trees, azb_free_trees, azb_exhaustive_best and azb_trees_within (counted
+// in azb_device_bytes)
 static int best_slab(azb_handle *h, size_t bytes) {
     if (bytes <= h->best_cap) return AZB_OK;
     if (h->best_buf) {
@@ -2145,6 +2159,192 @@ extern "C" int azb_exhaustive_best(azb_handle *h, uint64_t start, uint64_t count
         for (uint32_t i = 0; i < nb; ++i) index[i] = res[i].idx;
     if (n_below) *n_below = sc.below;
     if (n_out) *n_out = nb;
+    return AZB_OK;
+}
+
+// ---- every tree on N <= 64 vertices with key <= a bound, grown leaf by leaf (azb_grow.cuh) ----
+// Level n (the classes on n vertices) is built from level n - 1 in chunks of parents; azb_grow.cuh lists the passes of
+// one chunk.  The host keeps each finished level as its list of codes and lays the slab out anew for the next one: the
+// level's parents decoded (LP), the chunk's buffers, and the list of kept classes (A) with the other half of its sorts (B).
+extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out, uint64_t *n_within,
+                                uint64_t *n_below, uint64_t *codes, uint8_t *parents, double *lambda1, uint32_t *mu, float *eval,
+                                float *ms) {
+    if (!h) return AZB_ERR_INVALID;
+    if (k == 0 || k > AZB_BEST_MAX_K) return fail(h, AZB_ERR_INVALID, "k must be in 1..%u, got %u", AZB_BEST_MAX_K, k);
+    if (std::isnan(bound)) return fail(h, AZB_ERR_INVALID, "azb_trees_within: the bound is NaN");
+    CK(cudaSetDevice(h->cfg.device));
+    const uint32_t N = h->N, chunk = h->grow_chunk ? h->grow_chunk : AZB_GROW_CHUNK;
+    const bool trace = getenv("AZB_TRACE_WITHIN") != nullptr;  // one line per level on stderr (tools/within_probe.py)
+    const size_t E = sizeof(AzbGrowEnt);
+    CK(cudaEventRecord(h->ev0, h->stream));
+    int rc = AZB_OK;
+    if (bound < 0.0) {  // the star's key on its canonical labelling: every vertex under vertex 0
+        const size_t o_par = 256, o_l1 = o_par + best_up(N), o_mu = o_l1 + 256, o_c = o_mu + 256;
+        rc = best_slab(h, o_c + 256);
+        if (rc) return rc;
+        AzbGrowScalars *d_sc = reinterpret_cast<AzbGrowScalars *>(h->best_buf);
+        CK(cudaMemsetAsync(h->best_buf, 0, o_c + 256, h->stream));
+        launch_cost_n(h, h->best_buf + o_par, 1, N, reinterpret_cast<double *>(h->best_buf + o_l1),
+                      reinterpret_cast<uint32_t *>(h->best_buf + o_mu), reinterpret_cast<float *>(h->best_buf + o_c), &d_sc->err);
+        CK(cudaGetLastError());
+        double l1 = 0.0;
+        uint32_t m1 = 0;
+        CK(cudaMemcpyAsync(&l1, h->best_buf + o_l1, 8, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaMemcpyAsync(&m1, h->best_buf + o_mu, 4, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        bound = (double)m1 + l1;
+    }
+    // the classes one level may hold: max_level, what the device has room for (per class: the list and the other half
+    // of its sort, CUB's scratch, the codes and parents of the next level; the chunk's buffers set aside), and what one
+    // CUB pass takes
+    const uint64_t kc_max = (uint64_t)std::max(chunk, 64u) + 64u;
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    const uint64_t avail = (uint64_t)free_b + h->best_cap, set_aside = kc_max * (64 + 4 * E + 16) + (256ull << 20);
+    const uint64_t fit = avail > set_aside ? (avail - set_aside) / (5 * E + 64) : 0;
+    const uint64_t cap_level = std::min<uint64_t>({max_level ? max_level : fit, fit, (1ull << 31) - 1 - kc_max});
+    // L_4: the path (code 11100100) and the star (11010100); every tree on 5 or more vertices grows from one of them
+    std::vector<AzbGrowEnt> lvl = {AzbGrowEnt{0xE4ull << 56, 0ull, 0ull}, AzbGrowEnt{0xD4ull << 56, 0ull, 0ull}};
+    AzbGrowEnt *d_a = nullptr, *d_b = nullptr;
+    AzbGrowScalars *d_sc = nullptr;
+    uint8_t *d_res = nullptr;
+    size_t tmp_bytes = 0;
+    uint8_t *d_tmp = nullptr;
+    uint64_t nacc = 0;
+    for (uint32_t s = 4; s < N; ++s) {
+        const auto t0 = std::chrono::steady_clock::now();
+        const uint32_t n = s + 1, lo_bit = 128 - 2 * n;  // a code of n vertices occupies the top 2n of the 128 bits
+        const bool last = n == N;
+        const uint64_t ns = lvl.size();
+        const uint32_t pc = std::max(1u, chunk / s), kc = pc * s;  // parents and children of a full chunk
+        const uint64_t acap = std::min<uint64_t>(ns * s, cap_level) + kc;
+        size_t t[5] = {0, 0, 0, 0, 0};
+        CK(cub::DeviceRadixSort::SortKeys(nullptr, t[0], (const AzbGrowEnt *)nullptr, (AzbGrowEnt *)nullptr, kc, AzbGrowByCode{},
+                                          lo_bit, 128, h->stream));
+        CK(cub::DeviceRadixSort::SortKeys(nullptr, t[1], (const AzbGrowEnt *)nullptr, (AzbGrowEnt *)nullptr, (uint32_t)acap, AzbGrowByCode{},
+                                          lo_bit, 128, h->stream));
+        CK(cub::DeviceSelect::Unique(nullptr, t[2], (const AzbGrowEnt *)nullptr, (AzbGrowEnt *)nullptr, (uint32_t *)nullptr, (uint32_t)acap,
+                                     h->stream));
+        if (last)
+            CK(cub::DeviceRadixSort::SortKeys(nullptr, t[3], (const AzbGrowEnt *)nullptr, (AzbGrowEnt *)nullptr, (uint32_t)acap, AzbGrowByKey{},
+                                              h->stream));
+        tmp_bytes = *std::max_element(t, t + 5);
+        const size_t o_lp = best_up(ns * E), o_k = o_lp + best_up(ns * s), o_e1 = o_k + best_up((size_t)kc * n),
+                     o_e2 = o_e1 + best_up((size_t)kc * E), o_l1 = o_e2 + best_up((size_t)kc * E), o_mu = o_l1 + best_up((size_t)kc * 8),
+                     o_c = o_mu + best_up((size_t)kc * 4), o_a = o_c + best_up((size_t)kc * 4), o_b = o_a + best_up(acap * E),
+                     o_sc = o_b + best_up(acap * E), o_res = o_sc + 256, o_tmp = o_res + best_up((size_t)k * N);
+        rc = best_slab(h, o_tmp + tmp_bytes);
+        if (rc) return rc;
+        uint8_t *base = h->best_buf, *d_lp = base + o_lp, *d_k = base + o_k;
+        AzbGrowEnt *d_lv = reinterpret_cast<AzbGrowEnt *>(base), *d_e1 = reinterpret_cast<AzbGrowEnt *>(base + o_e1),
+                   *d_e2 = reinterpret_cast<AzbGrowEnt *>(base + o_e2);
+        double *d_l1 = reinterpret_cast<double *>(base + o_l1);
+        uint32_t *d_mu = reinterpret_cast<uint32_t *>(base + o_mu);
+        float *d_c = reinterpret_cast<float *>(base + o_c);
+        d_a = reinterpret_cast<AzbGrowEnt *>(base + o_a);
+        d_b = reinterpret_cast<AzbGrowEnt *>(base + o_b);
+        d_sc = reinterpret_cast<AzbGrowScalars *>(base + o_sc);
+        d_res = base + o_res;
+        d_tmp = base + o_tmp;
+        CK(cudaMemcpyAsync(d_lv, lvl.data(), ns * E, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemsetAsync(d_sc, 0, sizeof(AzbGrowScalars), h->stream));
+        azb_grow_decode_kernel<<<(uint32_t)((ns + 255) / 256), 256, 0, h->stream>>>(d_lv, (uint32_t)ns, s, d_lp);
+        h->launches += 1;
+        CK(cudaGetLastError());
+        const double thr = last ? bound : bound + AZB_GROW_EPS;
+        uint64_t children = 0, evaluated = 0;
+        nacc = 0;
+        for (uint64_t done = 0; done < ns;) {
+            const uint32_t p = (uint32_t)std::min<uint64_t>(pc, ns - done), m = p * s;
+            azb_grow_expand_kernel<<<(uint32_t)std::min<size_t>(((size_t)m * n + 255) / 256, 8192), 256, 0, h->stream>>>(d_lp + done * s, p,
+                                                                                                                     s, d_k);
+            azb_tree_code_kernel<<<(m + AZB_CODE_WARPS - 1) / AZB_CODE_WARPS, AZB_CODE_WARPS * 32, 0, h->stream>>>(
+                d_k, m, n, reinterpret_cast<unsigned long long *>(d_e1), (uint32_t)(E / 8), &d_sc->bad);
+            h->launches += 2;
+            CK(cudaGetLastError());
+            CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_e1, d_e2, m, AzbGrowByCode{}, lo_bit, 128, h->stream));
+            CK(cub::DeviceSelect::Unique(d_tmp, tmp_bytes, d_e2, d_e1, &d_sc->n_sel, m, h->stream));
+            uint32_t u = 0, kept = 0;
+            CK(cudaMemcpyAsync(&u, &d_sc->n_sel, 4, cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+            azb_grow_decode_kernel<<<(u + 255) / 256, 256, 0, h->stream>>>(d_e1, u, n, d_k);
+            launch_cost_n(h, d_k, u, n, d_l1, d_mu, d_c, &d_sc->err);
+            CK(cudaMemsetAsync(&d_sc->n_keep, 0, 4, h->stream));
+            azb_grow_keep_kernel<<<(u + 255) / 256, 256, 0, h->stream>>>(d_e1, d_l1, d_mu, u, thr, d_a + nacc, &d_sc->n_keep);
+            h->launches += 2;
+            CK(cudaGetLastError());
+            CK(cudaMemcpyAsync(&kept, &d_sc->n_keep, 4, cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+            nacc += kept;
+            children += m;
+            evaluated += u;
+            done += p;
+            if (nacc && (nacc + kc > acap || done == ns)) {  // one entry per class, sorted by code
+                uint32_t nu = 0;
+                CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_a, d_b, (uint32_t)nacc, AzbGrowByCode{}, lo_bit, 128, h->stream));
+                CK(cub::DeviceSelect::Unique(d_tmp, tmp_bytes, d_b, d_a, &d_sc->n_sel, (uint32_t)nacc, h->stream));
+                CK(cudaMemcpyAsync(&nu, &d_sc->n_sel, 4, cudaMemcpyDeviceToHost, h->stream));
+                CK(cudaStreamSynchronize(h->stream));
+                nacc = nu;
+                if (nacc > cap_level)
+                    return fail(h, AZB_ERR_CAPACITY,
+                                "azb_trees_within: level %u (trees on %u vertices) holds more than %llu classes (at least %llu found; "
+                                "max_level %llu, room on the device for %llu)",
+                                n, n, (unsigned long long)cap_level, (unsigned long long)nacc, (unsigned long long)max_level,
+                                (unsigned long long)fit);
+            }
+        }
+        uint32_t err = 0;
+        CK(cudaMemcpyAsync(&err, &d_sc->err, 4, cudaMemcpyDeviceToHost, h->stream));
+        lvl.resize(last ? 0 : nacc);
+        if (!last && nacc) CK(cudaMemcpyAsync(lvl.data(), d_a, nacc * E, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        if (err) return fail(h, AZB_ERR_LAMBDA, "%s", azb_strerror(AZB_ERR_LAMBDA));
+        if (trace)
+            fprintf(stderr, "azb_trees_within: N %u level %u: %llu classes, %llu children, %llu evaluated, %.3f ms\n", N, n,
+                    (unsigned long long)nacc, (unsigned long long)children, (unsigned long long)evaluated,
+                    std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
+        if (nacc == 0) break;  // no tree on more vertices is within the bound either
+    }
+    // the last level, by (key bits, code): count the keys below the bound, and the first k through the cost kernel of
+    // azb_eval_costs on their canonical parent arrays
+    const uint32_t nres = (uint32_t)std::min<uint64_t>(k, nacc);
+    if (nacc) {
+        CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_a, d_b, (uint32_t)nacc, AzbGrowByKey{}, h->stream));
+        azb_grow_below_kernel<<<(uint32_t)((nacc + 255) / 256), 256, 0, h->stream>>>(d_b, (uint32_t)nacc, bound, &d_sc->below);
+        azb_grow_decode_kernel<<<(nres + 255) / 256, 256, 0, h->stream>>>(d_b, nres, N, d_res);
+        h->launches += 2;
+        CK(cudaGetLastError());
+        rc = cost_buffers(h, nres);
+        if (rc) return rc;
+        CK(cudaMemsetAsync(h->cost_err, 0, 4, h->stream));
+        launch_cost_kernel(h, d_res, nres);
+        CK(cudaGetLastError());
+    }
+    CK(cudaEventRecord(h->ev1, h->stream));
+    std::vector<AzbGrowEnt> res(nres);
+    unsigned long long below = 0;
+    uint32_t cerr = 0;
+    if (nres) {
+        CK(cudaMemcpyAsync(res.data(), d_b, (size_t)nres * E, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaMemcpyAsync(&below, &d_sc->below, 8, cudaMemcpyDeviceToHost, h->stream));
+        if (parents) CK(cudaMemcpyAsync(parents, d_res, (size_t)nres * N, cudaMemcpyDeviceToHost, h->stream));
+        if (lambda1) CK(cudaMemcpyAsync(lambda1, h->cost_l1, (size_t)nres * 8, cudaMemcpyDeviceToHost, h->stream));
+        if (mu) CK(cudaMemcpyAsync(mu, h->cost_mu, (size_t)nres * 4, cudaMemcpyDeviceToHost, h->stream));
+        if (eval) CK(cudaMemcpyAsync(eval, h->cost_c, (size_t)nres * 4, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaMemcpyAsync(&cerr, h->cost_err, 4, cudaMemcpyDeviceToHost, h->stream));
+    }
+    CK(cudaStreamSynchronize(h->stream));
+    if (ms) CK(cudaEventElapsedTime(ms, h->ev0, h->ev1));
+    if (cerr) return fail(h, AZB_ERR_LAMBDA, "%s", azb_strerror(AZB_ERR_LAMBDA));
+    if (codes)
+        for (uint32_t i = 0; i < nres; ++i) {
+            codes[2 * i] = res[i].hi;
+            codes[2 * i + 1] = res[i].lo;
+        }
+    if (n_out) *n_out = nres;
+    if (n_within) *n_within = nacc;
+    if (n_below) *n_below = below;
     return AZB_OK;
 }
 

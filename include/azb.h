@@ -340,6 +340,33 @@ int azb_free_trees(azb_handle *h, uint64_t start, uint32_t m, uint8_t *parents /
 int azb_exhaustive_best(azb_handle *h, uint64_t start, uint64_t count, uint32_t k, double bound, uint32_t *n_out,
                         uint64_t *n_below, uint64_t *index /*[k]*/, uint8_t *parents /*[k*N]*/, double *lambda1 /*[k]*/,
                         uint32_t *mu /*[k]*/, float *eval /*[k]*/, float *ms);
+/* ---- extension (no reference item): every tree on the handle's N (5 <= N <= 64) vertices whose c21 key is at most a
+ *      bound, found without enumerating all trees.
+ * The canonical labelling of an isomorphism class is the decoding of its code (azb_tree_codes): read the 2N bits from
+ * the left; the first 1 is vertex 0 (the centre the code is taken at) and becomes the current vertex; each later 1 is
+ * the next unused vertex, whose parent is the current vertex, and becomes the current vertex; each 0 makes the current
+ * vertex's parent current (the last 0 closes vertex 0).  So vertices are numbered in preorder, children in code order,
+ * and parents[v] < v.  The key of a class is (double)mu + lambda1 (one IEEE add) with lambda1 and mu what azb_eval_costs
+ * gives for the canonical labelling: from N = 23 on lambda1 depends on the labelling in its last bits, and this makes it
+ * a function of the class.
+ * azb_trees_within: the classes on N vertices with key <= bound (bound < 0: the key of the star K1,N-1, so the star is
+ * in the set and the set is the star and every tree at least as good).  *n_within = their number, *n_below = the number
+ * with key < bound, and the first min(k, n_within) sorted ascending by (key, code) are returned: per entry the code (two
+ * words as azb_tree_codes), the canonical parent array, and lambda1, mu, eval exactly as azb_eval_costs gives for it;
+ * *n_out = the number of entries.  ms = device time of the whole call.  Any output pointer may be NULL.
+ * Method (exact): a subtree's key is below its tree's (Perron-Frobenius for lambda1, and mu cannot grow), and every tree
+ * on s + 1 vertices is one on s vertices plus a leaf.  The classes on s = 5 .. N - 1 vertices with key <= bound + 1e-9
+ * are grown level by level from the trees on 4 vertices, one leaf at a time, and the children of the last of them with
+ * key <= bound are the result; the slack covers the rounding of lambda1 (DESIGN.md §4.11).  A level's size, not
+ * A000055(N), sets the cost.
+ * AZB_ERR_INVALID for k == 0, k > 65536 or a NaN bound.  AZB_ERR_CAPACITY when a level would hold more than max_level
+ * classes (0: as many as fit in the device's free memory, which also bounds a larger max_level); azb_last_error names the
+ * level and the classes found so far, and no output is written.  AZB_ERR_LAMBDA as azb_eval_costs.  The call works
+ * before azb_init_trees, runs on the library stream, changes no tree, walker, counter, argmin, model or RNG state, and
+ * its scratch is the slab of azb_best_trees (counted in azb_device_bytes). */
+int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out, uint64_t *n_within,
+                     uint64_t *n_below, uint64_t *codes /*[k*2]*/, uint8_t *parents /*[k*N]*/, double *lambda1 /*[k]*/,
+                     uint32_t *mu /*[k]*/, float *eval /*[k]*/, float *ms);
 /* persistent walker state: states, paths, last_positions (optimizer/mod.rs:10-14) */
 int azb_get_walkers(azb_handle *h, uint8_t *parents, uint32_t *permitted, uint32_t *path, uint32_t *pos,
                     uint32_t *path_len);

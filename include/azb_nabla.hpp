@@ -47,6 +47,15 @@ struct ExhaustiveTree {
     float eval = 0.0f;
 };
 
+// one entry of trees_within: an isomorphism class by its code, in its canonical labelling (azb.h)
+struct TreeWithin {
+    uint64_t code[2] = {0, 0};
+    std::vector<uint8_t> parents;
+    double lambda_1 = 0.0;
+    uint32_t mu = 0;
+    float eval = 0.0f;
+};
+
 // NablaModel (nabla/model/mod.rs:4-8) for models that live on the host
 struct NablaModel {
     virtual ~NablaModel() = default;
@@ -228,6 +237,30 @@ class NablaOptimizer {
         std::vector<ExhaustiveTree> out(n);
         for (uint32_t i = 0; i < n; ++i) {
             out[i].index = index[i];
+            out[i].parents.assign(parents.begin() + i * n_v, parents.begin() + (i + 1) * n_v);
+            out[i].lambda_1 = l1[i];
+            out[i].mu = mu[i];
+            out[i].eval = eval[i];
+        }
+        return out;
+    }
+    // every class on N vertices with mu + lambda_1 <= bound (< 0: the star's key), the first k by (key, code)
+    // (azb_trees_within); max_level caps the classes of a level (0: what fits in device memory)
+    std::vector<TreeWithin> trees_within(double bound = -1.0, uint32_t k = 100, uint64_t max_level = 0, uint64_t *n_within = nullptr,
+                                         uint64_t *n_below = nullptr) {
+        const size_t n_v = cfg_.n_vertices, kk = k ? k : 1;
+        std::vector<uint64_t> codes(kk * 2);
+        std::vector<uint8_t> parents(kk * n_v);
+        std::vector<double> l1(kk);
+        std::vector<uint32_t> mu(kk);
+        std::vector<float> eval(kk);
+        uint32_t n = 0;
+        ck(azb_trees_within(h_, bound, k, max_level, &n, n_within, n_below, codes.data(), parents.data(), l1.data(), mu.data(),
+                            eval.data(), nullptr));
+        std::vector<TreeWithin> out(n);
+        for (uint32_t i = 0; i < n; ++i) {
+            out[i].code[0] = codes[2 * i];
+            out[i].code[1] = codes[2 * i + 1];
             out[i].parents.assign(parents.begin() + i * n_v, parents.begin() + (i + 1) * n_v);
             out[i].lambda_1 = l1[i];
             out[i].mu = mu[i];
