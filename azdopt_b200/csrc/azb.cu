@@ -50,39 +50,28 @@ struct azb_handle {
     uint16_t *sv16_save;  // azb_model_write_predictions: the walkers' bf16 state rows while their buffer serves the call
     uint32_t mlp_rows;  // rows the staging buffers hold
     AzbMlpTc tc;        // tensor-core path state (bf16 weights, activations)
-    // stand-alone cost kernel scratch
-    uint8_t *cost_par;
-    double *cost_l1;
-    uint32_t *cost_mu;
-    float *cost_c;
-    uint32_t *cost_err;
-    uint32_t cost_cap;
-    uint8_t *graph_buf;  // azb_eval_graph_costs: one grow-only slab [l1 | nbr | mu | kinds | err]
-    size_t graph_cap;
-    // azb_tree_codes / azb_best_trees (azb_best.cuh): one grow-only slab, the selection round's state, and the cap on the
-    // first round's M that tests set through AZB_TEST_BEST_CAP (0 = none)
-    uint8_t *best_buf;
-    size_t best_cap;
+    // the device scratch of every call outside the search step: one grow-only slab (scratch_grow, Carve)
+    uint8_t *scratch;
+    size_t scratch_cap;
+    // azb_best_trees (azb_best.cuh): the selection round's state, and the cap on the first round's M that tests set
+    // through AZB_TEST_BEST_CAP (0 = none)
     AzbBestState *best_st;
     uint32_t best_m_cap;
-    // azb_checkpoint_* (azb_ckpt.cuh): one grow-only staging slab, a copy stream and its events, the chunk size tests set
-    // through AZB_TEST_CKPT_CHUNK (0 = the default), and the running best's global position when a load took it from a
-    // root outside this handle's range (AzbGlobals::argmin_tree is AZB_NONE then)
-    uint8_t *ckpt_buf;
-    size_t ckpt_cap;
+    // azb_checkpoint_* (azb_ckpt.cuh): a copy stream and its events, the chunk size tests set through AZB_TEST_CKPT_CHUNK
+    // (0 = the default), and the running best's global position when a load took it from a root outside this handle's
+    // range (AzbGlobals::argmin_tree is AZB_NONE then)
     cudaStream_t ckpt_stream;
     cudaEvent_t ckpt_ev[4];
     uint64_t ckpt_chunk;
     uint64_t ckpt_best_root;
     uint32_t ckpt_best_node;
     // azb_free_trees / azb_exhaustive_best (azb_enum.cuh): the enumeration tables (built on first use) and the chunk size
-    // tests set through AZB_TEST_ENUM_CHUNK (0 = AZB_ENUM_CHUNK); their scratch is best_buf
+    // tests set through AZB_TEST_ENUM_CHUNK (0 = AZB_ENUM_CHUNK)
     AzbEnum en;
     unsigned long long *en_P;
     uint8_t *en_rp;
     uint32_t en_chunk;
-    // azb_trees_within (azb_grow.cuh): children per chunk, set by tests through AZB_TEST_GROW_CHUNK (0 = AZB_GROW_CHUNK);
-    // its scratch is best_buf
+    // azb_trees_within (azb_grow.cuh): children per chunk, set by tests through AZB_TEST_GROW_CHUNK (0 = AZB_GROW_CHUNK)
     uint32_t grow_chunk;
     // observations scratch
     float *obs, *obs_w;
@@ -166,6 +155,47 @@ static cudaError_t dmalloc(azb_handle *h, T **p, size_t count) {
     return e;
 }
 
+// Every call outside the search step takes its device buffers from one grow-only slab on the handle (a cudaMalloc per
+// call would cost more than most of these calls' kernels).  A call writes its layout once, as a function of a Carve, and
+// scratch() runs it twice: without a base to size the slab, then on the slab for the pointers.  A grow frees the old
+// slab, so every region a call reads after its last scratch() must come from that same layout.
+struct Carve {
+    uint8_t *base;
+    size_t off;
+    template <class T>
+    T *take(size_t count) {  // the next `count` T's, 256-byte aligned
+        T *p = base ? reinterpret_cast<T *>(base + off) : nullptr;
+        off += (count * sizeof(T) + 255) & ~(size_t)255;
+        return p;
+    }
+};
+
+static int scratch_grow(azb_handle *h, size_t bytes) {
+    if (bytes <= h->scratch_cap) return AZB_OK;
+    if (h->scratch) {  // the library stream and the checkpoint copy stream are the only ones that use the slab
+        CK(cudaStreamSynchronize(h->stream));
+        if (h->ckpt_stream) CK(cudaStreamSynchronize(h->ckpt_stream));
+        CK(cudaFree(h->scratch));
+        h->dev_bytes -= h->scratch_cap;
+    }
+    h->scratch = nullptr;
+    h->scratch_cap = 0;
+    CK(dmalloc(h, &h->scratch, bytes));
+    h->scratch_cap = bytes;
+    return AZB_OK;
+}
+
+template <class Layout>
+static int scratch(azb_handle *h, Layout layout) {
+    Carve size{nullptr, 0};
+    layout(size);
+    int rc = scratch_grow(h, size.off);
+    if (rc) return rc;
+    Carve c{h->scratch, 0};
+    layout(c);
+    return AZB_OK;
+}
+
 static uint32_t isqrt_ceil(uint32_t x) {
     uint32_t s = 0;
     while ((s + 1) * (s + 1) <= x) ++s;
@@ -241,8 +271,7 @@ int azb_destroy(azb_handle *h) {
     void *ptrs[] = {h->grad, h->adam_m, h->adam_v, h->tr_p, h->tr_dz[0], h->tr_dz[1], h->tr_x, h->tr_scal, h->tr_part, h->comm_buf,
                     h->L.walker, h->L.node, h->L.blk, h->L.inl, h->L.key, h->L.hash, h->L.casc, h->L.cand, h->L.stepmin, (void *)h->L.lut, h->L.sv,
                     h->L.h, h->L.g, h->L.log, h->params, h->act[0], h->act[1], h->act[2], h->mlp_x, h->mlp_y, h->sv16_save,
-                    h->cost_par, h->cost_l1, h->cost_mu, h->cost_c, h->cost_err, h->obs, h->obs_w, h->flush_buf, h->graph_buf,
-                    h->best_buf, h->best_st, h->ckpt_buf, h->en_P, h->en_rp};
+                    h->scratch, h->obs, h->obs_w, h->flush_buf, h->best_st, h->en_P, h->en_rp};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     azb_mlp_tc_destroy(h->tc);
@@ -1427,25 +1456,6 @@ int azb_add_actions_host(azb_handle *h, const float *h_theta, int *improved) {
 }
 
 // ---- stand-alone cost kernel ----
-static int cost_buffers(azb_handle *h, uint32_t m) {
-    if (m > h->cost_cap) {
-        void *old[] = {h->cost_par, h->cost_l1, h->cost_mu, h->cost_c};
-        for (void *p : old)
-            if (p) cudaFree(p);
-        h->cost_par = nullptr;
-        h->cost_l1 = nullptr;
-        h->cost_mu = nullptr;
-        h->cost_c = nullptr;
-        CK(dmalloc(h, &h->cost_par, (size_t)m * h->N));
-        CK(dmalloc(h, &h->cost_l1, m));
-        CK(dmalloc(h, &h->cost_mu, m));
-        CK(dmalloc(h, &h->cost_c, m));
-        h->cost_cap = m;
-    }
-    if (!h->cost_err) CK(dmalloc(h, &h->cost_err, 1));
-    return AZB_OK;
-}
-
 // the cost kernel on m trees of n vertices (azb_trees_within evaluates every level below N with it)
 static void launch_cost_n(azb_handle *h, const uint8_t *dev_parents, uint32_t m, uint32_t n, double *l1, uint32_t *mu, float *c,
                           uint32_t *err) {
@@ -1458,25 +1468,51 @@ static void launch_cost_n(azb_handle *h, const uint8_t *dev_parents, uint32_t m,
     h->launches += 1;
 }
 
-static void launch_cost_kernel(azb_handle *h, const uint8_t *dev_parents, uint32_t m) {
-    launch_cost_n(h, dev_parents, m, h->N, h->cost_l1, h->cost_mu, h->cost_c, h->cost_err);
+// the cost kernel's outputs for m trees, carved from a call's scratch
+struct CostOut {
+    double *l1;
+    uint32_t *mu;
+    float *c;
+    uint32_t *err;
+    void take(Carve &cv, size_t m) {
+        l1 = cv.take<double>(m);
+        mu = cv.take<uint32_t>(m);
+        c = cv.take<float>(m);
+        err = cv.take<uint32_t>(1);
+    }
+};
+
+// The cost kernel of azb_eval_costs on m device parent arrays of n vertices into d, then the copies of whichever of the
+// parent arrays, lambda_1, mu and eval the caller asks for (the non-null destinations) and of the error word, all on the
+// library stream; t0 and t1, when given, are recorded around the kernel.  The caller synchronises and maps *err.
+static int cost_tail(azb_handle *h, const uint8_t *d_par, uint32_t m, uint32_t n, const CostOut &d, cudaEvent_t t0, cudaEvent_t t1,
+                     uint8_t *parents, double *lambda1, uint32_t *mu, float *eval, uint32_t *err) {
+    CK(cudaMemsetAsync(d.err, 0, 4, h->stream));
+    if (t0) CK(cudaEventRecord(t0, h->stream));
+    launch_cost_n(h, d_par, m, n, d.l1, d.mu, d.c, d.err);
+    CK(cudaGetLastError());
+    if (t1) CK(cudaEventRecord(t1, h->stream));
+    if (parents) CK(cudaMemcpyAsync(parents, d_par, (size_t)m * n, cudaMemcpyDeviceToHost, h->stream));
+    if (lambda1) CK(cudaMemcpyAsync(lambda1, d.l1, (size_t)m * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (mu) CK(cudaMemcpyAsync(mu, d.mu, (size_t)m * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (eval) CK(cudaMemcpyAsync(eval, d.c, (size_t)m * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(err, d.err, 4, cudaMemcpyDeviceToHost, h->stream));
+    return AZB_OK;
 }
 
 static int eval_costs_dev(azb_handle *h, const uint8_t *parents, uint32_t m, double *lambda1, uint32_t *mu, float *c,
                           float *ms) {
-    int rc0 = cost_buffers(h, m);
-    if (rc0) return rc0;
-    CK(cudaMemcpyAsync(h->cost_par, parents, (size_t)m * h->N, cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemsetAsync(h->cost_err, 0, 4, h->stream));
-    CK(cudaEventRecord(h->ev0, h->stream));
-    launch_cost_kernel(h, h->cost_par, m);
-    CK(cudaGetLastError());
-    CK(cudaEventRecord(h->ev1, h->stream));
+    uint8_t *d_par = nullptr;
+    CostOut d;
+    int rc = scratch(h, [&](Carve &cv) {
+        d_par = cv.take<uint8_t>((size_t)m * h->N);
+        d.take(cv, m);
+    });
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(d_par, parents, (size_t)m * h->N, cudaMemcpyHostToDevice, h->stream));
     uint32_t err = 0;
-    if (lambda1) CK(cudaMemcpyAsync(lambda1, h->cost_l1, (size_t)m * 8, cudaMemcpyDeviceToHost, h->stream));
-    if (mu) CK(cudaMemcpyAsync(mu, h->cost_mu, (size_t)m * 4, cudaMemcpyDeviceToHost, h->stream));
-    if (c) CK(cudaMemcpyAsync(c, h->cost_c, (size_t)m * 4, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(&err, h->cost_err, 4, cudaMemcpyDeviceToHost, h->stream));
+    rc = cost_tail(h, d_par, m, h->N, d, h->ev0, h->ev1, nullptr, lambda1, mu, c, &err);
+    if (rc) return rc;
     CK(cudaStreamSynchronize(h->stream));
     if (ms) CK(cudaEventElapsedTime(ms, h->ev0, h->ev1));
     if (err) return fail(h, (int)err, "%s", azb_strerror((int)err));
@@ -1497,28 +1533,24 @@ int azb_eval_costs(azb_handle *h, const uint8_t *parents, uint32_t m, double *la
 // ---- stand-alone cost + action kinds of connected bitset graphs (SURVEY 8(f) row 3) ----
 }  // extern "C"
 
-// shared by the B32 and B64 entries: the slab, the copies, the timing and the error words; `launch` enqueues the kernel
+// shared by the B32 and B64 entries: the scratch, the copies, the timing and the error words; `launch` enqueues the kernel
 template <typename W, typename Launch>
 static int eval_graph_costs_dev(azb_handle *h, const char *fn, const W *nbr, uint32_t m, uint32_t n, double *lambda1,
                                 uint32_t *mu, uint32_t *kinds, float *ms, Launch launch) {
     // loops, asymmetric neighbourhoods, neighbours >= N and disconnected inputs are found by the kernel itself
     CK(cudaSetDevice(h->cfg.device));
     const uint32_t kw = (n * (n - 1) + 31) / 32;
-    // one slab on the handle, grown when a larger batch arrives (a cudaMalloc per call costs more than the kernel)
-    auto up = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    const size_t o_l1 = 0, o_nbr = o_l1 + up((size_t)m * 8), o_mu = o_nbr + up((size_t)m * n * sizeof(W)), o_kinds = o_mu + up((size_t)m * 4),
-                 o_err = o_kinds + up((size_t)m * kw * 4), total = o_err + 256;
-    if (total > h->graph_cap) {
-        if (h->graph_buf) cudaFree(h->graph_buf);
-        h->graph_buf = nullptr;
-        h->graph_cap = 0;
-        CK(cudaMalloc((void **)&h->graph_buf, total));
-        h->graph_cap = total;
-    }
-    double *d_l1 = reinterpret_cast<double *>(h->graph_buf + o_l1);
-    W *d_nbr = reinterpret_cast<W *>(h->graph_buf + o_nbr);
-    uint32_t *d_mu = reinterpret_cast<uint32_t *>(h->graph_buf + o_mu), *d_kinds = reinterpret_cast<uint32_t *>(h->graph_buf + o_kinds),
-             *d_err = reinterpret_cast<uint32_t *>(h->graph_buf + o_err);
+    double *d_l1 = nullptr;
+    W *d_nbr = nullptr;
+    uint32_t *d_mu = nullptr, *d_kinds = nullptr, *d_err = nullptr;
+    int rc = scratch(h, [&](Carve &cv) {
+        d_l1 = cv.take<double>(m);
+        d_nbr = cv.take<W>((size_t)m * n);
+        d_mu = cv.take<uint32_t>(m);
+        d_kinds = cv.take<uint32_t>((size_t)m * kw);
+        d_err = cv.take<uint32_t>(2);
+    });
+    if (rc) return rc;
     cudaError_t ce = cudaMemcpyAsync(d_nbr, nbr, (size_t)m * n * sizeof(W), cudaMemcpyHostToDevice, h->stream);
     const uint32_t err0[2] = {0u, 0xffffffffu};  // [0] bit AZB_ERR_* per kind of failure, [1] first rejected graph
     if (ce == cudaSuccess) ce = cudaMemcpyAsync(d_err, err0, 8, cudaMemcpyHostToDevice, h->stream);
@@ -1603,23 +1635,21 @@ int azb_get_argmin(azb_handle *h, uint8_t *parents, uint32_t *permitted, double 
     if (!h) return AZB_ERR_INVALID;
     if (!h->trees_init) return fail(h, AZB_ERR_STATE, "azb_init_trees has not been called");
     CK(cudaSetDevice(h->cfg.device));
-    int rc = cost_buffers(h, 1);
+    CostOut d;
+    int rc = scratch(h, [&](Carve &cv) { d.take(cv, 1); });
     if (rc) return rc;
     if (!h->pin_rg) {
         CK(cudaMallocHost((void **)&h->pin_rg, sizeof(AzbGlobals)));
         CK(cudaMallocHost((void **)&h->pin_abort, 16));
     }
+    if (!h->pin_cost) CK(cudaMallocHost((void **)&h->pin_cost, 32));
     // *cost = space.cost(state); *eval = space.evaluate(cost)  (optimizer/mod.rs:240-241): the cost kernel reads the argmin
     // state where the argmin pass left it, and everything comes back behind ONE synchronisation into pinned memory
-    CK(cudaMemsetAsync(h->cost_err, 0, 4, h->stream));
-    launch_cost_kernel(h, reinterpret_cast<const uint8_t *>(h->L.g->argmin_state), 1);
-    CK(cudaGetLastError());
-    if (!h->pin_cost) CK(cudaMallocHost((void **)&h->pin_cost, 32));
+    uint32_t *pc = h->pin_cost;
+    rc = cost_tail(h, reinterpret_cast<const uint8_t *>(h->L.g->argmin_state), 1, h->N, d, nullptr, nullptr, nullptr,
+                   reinterpret_cast<double *>(pc), pc + 2, reinterpret_cast<float *>(pc + 3), pc + 4);
+    if (rc) return rc;
     CK(cudaMemcpyAsync(h->pin_rg, h->L.g, sizeof(AzbGlobals), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(h->pin_cost, h->cost_l1, 8, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(h->pin_cost + 2, h->cost_mu, 4, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(h->pin_cost + 3, h->cost_c, 4, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(h->pin_cost + 4, h->cost_err, 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     const AzbGlobals &g = *h->pin_rg;
     if (parents) memcpy(parents, g.argmin_state, h->N);
@@ -1834,27 +1864,10 @@ extern "C" int azb_get_node_state(azb_handle *h, uint32_t tree, uint32_t node, u
 }
 
 // ---- the k best isomorphism classes (azb_best.cuh) ----
-static size_t best_up(size_t x) { return (x + 255) & ~(size_t)255; }
-
-// the grow-only slab of azb_tree_codes, azb_best_trees, azb_free_trees, azb_exhaustive_best and azb_trees_within (counted
-// in azb_device_bytes)
-static int best_slab(azb_handle *h, size_t bytes) {
-    if (bytes <= h->best_cap) return AZB_OK;
-    if (h->best_buf) {
-        CK(cudaStreamSynchronize(h->stream));
-        CK(cudaFree(h->best_buf));
-        h->dev_bytes -= h->best_cap;
-    }
-    h->best_buf = nullptr;
-    h->best_cap = 0;
-    CK(dmalloc(h, &h->best_buf, bytes));
-    h->best_cap = bytes;
-    return AZB_OK;
-}
-
-static void launch_code_kernel(azb_handle *h, const uint8_t *dev_parents, uint32_t m, unsigned long long *codes, uint32_t stride,
-                               uint32_t *bad) {
-    azb_tree_code_kernel<<<(m + AZB_CODE_WARPS - 1) / AZB_CODE_WARPS, AZB_CODE_WARPS * 32, 0, h->stream>>>(dev_parents, m, h->N, codes,
+// the code kernel on m trees of n vertices (azb_trees_within codes every level below N with it)
+static void launch_code_kernel(azb_handle *h, const uint8_t *dev_parents, uint32_t m, uint32_t n, unsigned long long *codes,
+                               uint32_t stride, uint32_t *bad) {
+    azb_tree_code_kernel<<<(m + AZB_CODE_WARPS - 1) / AZB_CODE_WARPS, AZB_CODE_WARPS * 32, 0, h->stream>>>(dev_parents, m, n, codes,
                                                                                                         stride, bad);
     h->launches += 1;
 }
@@ -1862,16 +1875,19 @@ static void launch_code_kernel(azb_handle *h, const uint8_t *dev_parents, uint32
 extern "C" int azb_tree_codes(azb_handle *h, const uint8_t *parents, uint32_t m, uint64_t *codes, float *ms) {
     if (!h || !parents || m == 0) return AZB_ERR_INVALID;
     CK(cudaSetDevice(h->cfg.device));
-    const size_t o_codes = best_up((size_t)m * h->N), o_bad = o_codes + best_up((size_t)m * 16);
-    int rc = best_slab(h, o_bad + 256);
+    uint8_t *d_par = nullptr;
+    unsigned long long *d_codes = nullptr;
+    uint32_t *d_bad = nullptr;
+    int rc = scratch(h, [&](Carve &cv) {
+        d_par = cv.take<uint8_t>((size_t)m * h->N);
+        d_codes = cv.take<unsigned long long>((size_t)m * 2);
+        d_bad = cv.take<uint32_t>(1);
+    });
     if (rc) return rc;
-    uint8_t *d_par = h->best_buf;
-    unsigned long long *d_codes = reinterpret_cast<unsigned long long *>(h->best_buf + o_codes);
-    uint32_t *d_bad = reinterpret_cast<uint32_t *>(h->best_buf + o_bad);
     CK(cudaMemcpyAsync(d_par, parents, (size_t)m * h->N, cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemsetAsync(d_bad, 0xff, 4, h->stream));
     CK(cudaEventRecord(h->ev0, h->stream));
-    launch_code_kernel(h, d_par, m, d_codes, 2, d_bad);
+    launch_code_kernel(h, d_par, m, h->N, d_codes, 2, d_bad);
     CK(cudaGetLastError());
     CK(cudaEventRecord(h->ev1, h->stream));
     uint32_t bad = 0;
@@ -1906,8 +1922,11 @@ extern "C" int azb_best_trees(azb_handle *h, uint32_t k, uint32_t *n_out, float 
     uint32_t M = 4u * k;
     if (h->best_m_cap) M = std::min(M, h->best_m_cap);
     AzbBestState st;
-    size_t o_b = 0, o_par = 0, o_perm = 0, o_tmp = 0, tmp_bytes = 0;
+    size_t tmp_bytes = 0;
     AzbCand *d_a = nullptr, *d_b = nullptr;
+    uint8_t *d_par = nullptr, *d_tmp = nullptr;
+    uint32_t *d_perm = nullptr;
+    CostOut d_cost;
     for (;;) {
         CK(cudaMemsetAsync(h->best_st, 0, sizeof(AzbBestState), h->stream));
         CK(cudaMemsetAsync(&h->best_st->bad, 0xff, 4, h->stream));
@@ -1925,22 +1944,22 @@ extern "C" int azb_best_trees(azb_handle *h, uint32_t k, uint32_t *n_out, float 
         CK(cub::DeviceRadixSort::SortKeys(nullptr, t1, (const AzbCand *)nullptr, (AzbCand *)nullptr, C, AzbByCode{}, h->stream));
         CK(cub::DeviceRadixSort::SortKeys(nullptr, t2, (const AzbCand *)nullptr, (AzbCand *)nullptr, C, AzbByValue{}, h->stream));
         tmp_bytes = std::max(t1, t2);
-        o_b = best_up((size_t)C * sizeof(AzbCand));
-        o_par = 2 * o_b;
-        o_perm = o_par + best_up((size_t)C * N);
-        o_tmp = o_perm + best_up((size_t)C * W * 4);
-        rc = best_slab(h, o_tmp + tmp_bytes);
+        rc = scratch(h, [&](Carve &cv) {
+            d_a = cv.take<AzbCand>(C);
+            d_b = cv.take<AzbCand>(C);
+            d_par = cv.take<uint8_t>((size_t)C * N);
+            d_perm = cv.take<uint32_t>((size_t)C * W);
+            d_tmp = cv.take<uint8_t>(tmp_bytes);
+            d_cost.take(cv, std::min(k, C));  // the result's costs (at most k classes of at most C candidates)
+        });
         if (rc) return rc;
-        d_a = reinterpret_cast<AzbCand *>(h->best_buf);
-        d_b = reinterpret_cast<AzbCand *>(h->best_buf + o_b);
-        uint8_t *d_par = h->best_buf + o_par;
         const uint32_t blocks = (C + 255) / 256;
         azb_best_compact_kernel<<<grid, 256, 0, h->stream>>>(L, h->best_st, d_a);
         azb_best_replay_kernel<<<blocks, 256, 0, h->stream>>>(L, d_a, C, d_par, nullptr);
-        launch_code_kernel(h, d_par, C, reinterpret_cast<unsigned long long *>(d_a), sizeof(AzbCand) / 8, &h->best_st->bad);
+        launch_code_kernel(h, d_par, C, N, reinterpret_cast<unsigned long long *>(d_a), sizeof(AzbCand) / 8, &h->best_st->bad);
         h->launches += 2;
         CK(cudaGetLastError());
-        CK(cub::DeviceRadixSort::SortKeys(h->best_buf + o_tmp, tmp_bytes, d_a, d_b, C, AzbByCode{}, h->stream));
+        CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_a, d_b, C, AzbByCode{}, h->stream));
         azb_best_heads_kernel<<<blocks, 256, 0, h->stream>>>(d_b, C, d_a, h->best_st);
         h->launches += 1;
         CK(cudaGetLastError());
@@ -1958,25 +1977,16 @@ extern "C" int azb_best_trees(azb_handle *h, uint32_t k, uint32_t *n_out, float 
         M = 2u * C > C ? 2u * C : 0xffffffffu;
     }
     const uint32_t n_cls = st.n_class, n = std::min(k, n_cls);
-    CK(cub::DeviceRadixSort::SortKeys(h->best_buf + o_tmp, tmp_bytes, d_a, d_b, n_cls, AzbByValue{}, h->stream));
-    uint8_t *d_par = h->best_buf + o_par;
-    uint32_t *d_perm = reinterpret_cast<uint32_t *>(h->best_buf + o_perm);
+    CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_a, d_b, n_cls, AzbByValue{}, h->stream));
     azb_best_replay_kernel<<<(n + 255) / 256, 256, 0, h->stream>>>(L, d_b, n, d_par, d_perm);
     h->launches += 1;
     CK(cudaGetLastError());
-    rc = cost_buffers(h, n);
-    if (rc) return rc;
-    CK(cudaMemsetAsync(h->cost_err, 0, 4, h->stream));
-    launch_cost_kernel(h, d_par, n);
-    CK(cudaGetLastError());
     std::vector<AzbCand> cls(n);
     uint32_t cerr = 0;
+    rc = cost_tail(h, d_par, n, N, d_cost, nullptr, nullptr, parents, lambda1, mu, nullptr, &cerr);
+    if (rc) return rc;
     CK(cudaMemcpyAsync(cls.data(), d_b, (size_t)n * sizeof(AzbCand), cudaMemcpyDeviceToHost, h->stream));
-    if (parents) CK(cudaMemcpyAsync(parents, d_par, (size_t)n * N, cudaMemcpyDeviceToHost, h->stream));
     if (permitted) CK(cudaMemcpyAsync(permitted, d_perm, (size_t)n * W * 4, cudaMemcpyDeviceToHost, h->stream));
-    if (lambda1) CK(cudaMemcpyAsync(lambda1, h->cost_l1, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
-    if (mu) CK(cudaMemcpyAsync(mu, h->cost_mu, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(&cerr, h->cost_err, 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     if (cerr) return fail(h, (int)cerr, "%s", azb_strerror((int)cerr));
     for (uint32_t i = 0; i < n; ++i) {
@@ -2051,15 +2061,16 @@ extern "C" int azb_free_trees(azb_handle *h, uint64_t start, uint32_t m, uint8_t
     rc = enum_sms(h, &sms);
     if (rc) return rc;
     const uint32_t N = h->N, chunk = h->en_chunk ? h->en_chunk : AZB_ENUM_CHUNK;
-    rc = best_slab(h, (size_t)std::min(m, chunk) * N);
+    uint8_t *d_par = nullptr;
+    rc = scratch(h, [&](Carve &cv) { d_par = cv.take<uint8_t>((size_t)std::min(m, chunk) * N); });
     if (rc) return rc;
     for (uint32_t done = 0; done < m;) {
         const uint32_t c = std::min(chunk, m - done);
         azb_enum_trees_kernel<<<std::min<uint32_t>((c + 7) / 8, (uint32_t)sms * 16u), 256, 0, h->stream>>>(h->en, start + done, nullptr, c,
-                                                                                                          h->best_buf);
+                                                                                                          d_par);
         h->launches += 1;
         CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(parents + (size_t)done * N, h->best_buf, (size_t)c * N, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaMemcpyAsync(parents + (size_t)done * N, d_par, (size_t)c * N, cudaMemcpyDeviceToHost, h->stream));
         done += c;
     }
     CK(cudaStreamSynchronize(h->stream));
@@ -2098,15 +2109,19 @@ extern "C" int azb_exhaustive_best(azb_handle *h, uint64_t start, uint64_t count
     size_t tmp_bytes = 0;
     CK(cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, (const AzbEnumCand *)nullptr, (AzbEnumCand *)nullptr, cap, AzbEnumByKey{},
                                       h->stream));
-    const size_t o_b = best_up((size_t)cap * sizeof(AzbEnumCand)), o_par = 2 * o_b, o_sc = o_par + best_up((size_t)k * N),
-                 o_tmp = o_sc + 256;
-    rc = best_slab(h, o_tmp + tmp_bytes);
+    AzbEnumCand *d_a = nullptr, *d_b = nullptr;
+    uint8_t *d_par = nullptr, *d_tmp = nullptr;
+    AzbEnumScalars *d_sc = nullptr;
+    CostOut d_cost;
+    rc = scratch(h, [&](Carve &cv) {
+        d_a = cv.take<AzbEnumCand>(cap);
+        d_b = cv.take<AzbEnumCand>(cap);
+        d_par = cv.take<uint8_t>((size_t)k * N);
+        d_sc = cv.take<AzbEnumScalars>(1);
+        d_tmp = cv.take<uint8_t>(tmp_bytes);
+        d_cost.take(cv, n_res);
+    });
     if (rc) return rc;
-    rc = cost_buffers(h, n_res);
-    if (rc) return rc;
-    AzbEnumCand *d_a = reinterpret_cast<AzbEnumCand *>(h->best_buf), *d_b = reinterpret_cast<AzbEnumCand *>(h->best_buf + o_b);
-    uint8_t *d_par = h->best_buf + o_par;
-    AzbEnumScalars *d_sc = reinterpret_cast<AzbEnumScalars *>(h->best_buf + o_sc);
     CK(cudaEventRecord(h->ev0, h->stream));
     CK(cudaMemsetAsync(d_sc, 0, sizeof(AzbEnumScalars), h->stream));
     CK(cudaMemsetAsync(&d_sc->thr, 0xff, 8, h->stream));
@@ -2129,7 +2144,7 @@ extern "C" int azb_exhaustive_best(azb_handle *h, uint64_t start, uint64_t count
         done += c;
         if (nc == 0) continue;
         const uint32_t tot = nb + nc;
-        CK(cub::DeviceRadixSort::SortKeys(h->best_buf + o_tmp, tmp_bytes, d_a, d_b, tot, AzbEnumByKey{}, h->stream));
+        CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_a, d_b, tot, AzbEnumByKey{}, h->stream));
         nb = std::min(k, tot);
         CK(cudaMemcpyAsync(d_a, d_b, (size_t)nb * sizeof(AzbEnumCand), cudaMemcpyDeviceToDevice, h->stream));
         if (nb == k) CK(cudaMemcpyAsync(&d_sc->thr, &d_b[k - 1].key, 8, cudaMemcpyDeviceToDevice, h->stream));
@@ -2138,20 +2153,13 @@ extern "C" int azb_exhaustive_best(azb_handle *h, uint64_t start, uint64_t count
     azb_enum_trees_kernel<<<std::min<uint32_t>((nb + 7) / 8, (uint32_t)sms * 16u), 256, 0, h->stream>>>(h->en, 0ull, d_a, nb, d_par);
     h->launches += 1;
     CK(cudaGetLastError());
-    CK(cudaMemsetAsync(h->cost_err, 0, 4, h->stream));
-    launch_cost_kernel(h, d_par, nb);
-    CK(cudaGetLastError());
-    CK(cudaEventRecord(h->ev1, h->stream));
     std::vector<AzbEnumCand> res(nb);
     AzbEnumScalars sc;
     uint32_t cerr = 0;
+    rc = cost_tail(h, d_par, nb, N, d_cost, nullptr, h->ev1, parents, lambda1, mu, eval, &cerr);
+    if (rc) return rc;
     CK(cudaMemcpyAsync(res.data(), d_a, (size_t)nb * sizeof(AzbEnumCand), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaMemcpyAsync(&sc, d_sc, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
-    if (parents) CK(cudaMemcpyAsync(parents, d_par, (size_t)nb * N, cudaMemcpyDeviceToHost, h->stream));
-    if (lambda1) CK(cudaMemcpyAsync(lambda1, h->cost_l1, (size_t)nb * 8, cudaMemcpyDeviceToHost, h->stream));
-    if (mu) CK(cudaMemcpyAsync(mu, h->cost_mu, (size_t)nb * 4, cudaMemcpyDeviceToHost, h->stream));
-    if (eval) CK(cudaMemcpyAsync(eval, h->cost_c, (size_t)nb * 4, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(&cerr, h->cost_err, 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     if (ms) CK(cudaEventElapsedTime(ms, h->ev0, h->ev1));
     if (sc.err || cerr) return fail(h, AZB_ERR_LAMBDA, "%s", azb_strerror(AZB_ERR_LAMBDA));
@@ -2179,19 +2187,20 @@ extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_
     CK(cudaEventRecord(h->ev0, h->stream));
     int rc = AZB_OK;
     if (bound < 0.0) {  // the star's key on its canonical labelling: every vertex under vertex 0
-        const size_t o_par = 256, o_l1 = o_par + best_up(N), o_mu = o_l1 + 256, o_c = o_mu + 256;
-        rc = best_slab(h, o_c + 256);
+        uint8_t *d_star = nullptr;
+        CostOut d_cost;
+        rc = scratch(h, [&](Carve &cv) {
+            d_star = cv.take<uint8_t>(N);
+            d_cost.take(cv, 1);
+        });
         if (rc) return rc;
-        AzbGrowScalars *d_sc = reinterpret_cast<AzbGrowScalars *>(h->best_buf);
-        CK(cudaMemsetAsync(h->best_buf, 0, o_c + 256, h->stream));
-        launch_cost_n(h, h->best_buf + o_par, 1, N, reinterpret_cast<double *>(h->best_buf + o_l1),
-                      reinterpret_cast<uint32_t *>(h->best_buf + o_mu), reinterpret_cast<float *>(h->best_buf + o_c), &d_sc->err);
-        CK(cudaGetLastError());
+        CK(cudaMemsetAsync(d_star, 0, N, h->stream));
         double l1 = 0.0;
-        uint32_t m1 = 0;
-        CK(cudaMemcpyAsync(&l1, h->best_buf + o_l1, 8, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaMemcpyAsync(&m1, h->best_buf + o_mu, 4, cudaMemcpyDeviceToHost, h->stream));
+        uint32_t m1 = 0, err = 0;
+        rc = cost_tail(h, d_star, 1, N, d_cost, nullptr, nullptr, nullptr, &l1, &m1, nullptr, &err);
+        if (rc) return rc;
         CK(cudaStreamSynchronize(h->stream));
+        if (err) return fail(h, AZB_ERR_LAMBDA, "%s", azb_strerror(AZB_ERR_LAMBDA));
         bound = (double)m1 + l1;
     }
     // the classes one level may hold: max_level, what the device has room for (per class: the list and the other half
@@ -2200,7 +2209,7 @@ extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_
     const uint64_t kc_max = (uint64_t)std::max(chunk, 64u) + 64u;
     size_t free_b = 0, total_b = 0;
     CK(cudaMemGetInfo(&free_b, &total_b));
-    const uint64_t avail = (uint64_t)free_b + h->best_cap, set_aside = kc_max * (64 + 4 * E + 16) + (256ull << 20);
+    const uint64_t avail = (uint64_t)free_b + h->scratch_cap, set_aside = kc_max * (64 + 4 * E + 16) + (256ull << 20);
     const uint64_t fit = avail > set_aside ? (avail - set_aside) / (5 * E + 64) : 0;
     const uint64_t cap_level = std::min<uint64_t>({max_level ? max_level : fit, fit, (1ull << 31) - 1 - kc_max});
     // L_4: the path (code 11100100) and the star (11010100); every tree on 5 or more vertices grows from one of them
@@ -2208,6 +2217,7 @@ extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_
     AzbGrowEnt *d_a = nullptr, *d_b = nullptr;
     AzbGrowScalars *d_sc = nullptr;
     uint8_t *d_res = nullptr;
+    CostOut d_res_cost;
     size_t tmp_bytes = 0;
     uint8_t *d_tmp = nullptr;
     uint64_t nacc = 0;
@@ -2229,23 +2239,28 @@ extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_
             CK(cub::DeviceRadixSort::SortKeys(nullptr, t[3], (const AzbGrowEnt *)nullptr, (AzbGrowEnt *)nullptr, (uint32_t)acap, AzbGrowByKey{},
                                               h->stream));
         tmp_bytes = *std::max_element(t, t + 5);
-        const size_t o_lp = best_up(ns * E), o_k = o_lp + best_up(ns * s), o_e1 = o_k + best_up((size_t)kc * n),
-                     o_e2 = o_e1 + best_up((size_t)kc * E), o_l1 = o_e2 + best_up((size_t)kc * E), o_mu = o_l1 + best_up((size_t)kc * 8),
-                     o_c = o_mu + best_up((size_t)kc * 4), o_a = o_c + best_up((size_t)kc * 4), o_b = o_a + best_up(acap * E),
-                     o_sc = o_b + best_up(acap * E), o_res = o_sc + 256, o_tmp = o_res + best_up((size_t)k * N);
-        rc = best_slab(h, o_tmp + tmp_bytes);
+        AzbGrowEnt *d_lv = nullptr, *d_e1 = nullptr, *d_e2 = nullptr;
+        uint8_t *d_lp = nullptr, *d_k = nullptr;
+        double *d_l1 = nullptr;
+        uint32_t *d_mu = nullptr;
+        float *d_c = nullptr;
+        rc = scratch(h, [&](Carve &cv) {
+            d_lv = cv.take<AzbGrowEnt>(ns);
+            d_lp = cv.take<uint8_t>(ns * s);
+            d_k = cv.take<uint8_t>((size_t)kc * n);
+            d_e1 = cv.take<AzbGrowEnt>(kc);
+            d_e2 = cv.take<AzbGrowEnt>(kc);
+            d_l1 = cv.take<double>(kc);
+            d_mu = cv.take<uint32_t>(kc);
+            d_c = cv.take<float>(kc);
+            d_a = cv.take<AzbGrowEnt>(acap);
+            d_b = cv.take<AzbGrowEnt>(acap);
+            d_sc = cv.take<AzbGrowScalars>(1);
+            d_res = cv.take<uint8_t>((size_t)k * N);
+            d_res_cost.take(cv, k);
+            d_tmp = cv.take<uint8_t>(tmp_bytes);
+        });
         if (rc) return rc;
-        uint8_t *base = h->best_buf, *d_lp = base + o_lp, *d_k = base + o_k;
-        AzbGrowEnt *d_lv = reinterpret_cast<AzbGrowEnt *>(base), *d_e1 = reinterpret_cast<AzbGrowEnt *>(base + o_e1),
-                   *d_e2 = reinterpret_cast<AzbGrowEnt *>(base + o_e2);
-        double *d_l1 = reinterpret_cast<double *>(base + o_l1);
-        uint32_t *d_mu = reinterpret_cast<uint32_t *>(base + o_mu);
-        float *d_c = reinterpret_cast<float *>(base + o_c);
-        d_a = reinterpret_cast<AzbGrowEnt *>(base + o_a);
-        d_b = reinterpret_cast<AzbGrowEnt *>(base + o_b);
-        d_sc = reinterpret_cast<AzbGrowScalars *>(base + o_sc);
-        d_res = base + o_res;
-        d_tmp = base + o_tmp;
         CK(cudaMemcpyAsync(d_lv, lvl.data(), ns * E, cudaMemcpyHostToDevice, h->stream));
         CK(cudaMemsetAsync(d_sc, 0, sizeof(AzbGrowScalars), h->stream));
         azb_grow_decode_kernel<<<(uint32_t)((ns + 255) / 256), 256, 0, h->stream>>>(d_lv, (uint32_t)ns, s, d_lp);
@@ -2258,9 +2273,8 @@ extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_
             const uint32_t p = (uint32_t)std::min<uint64_t>(pc, ns - done), m = p * s;
             azb_grow_expand_kernel<<<(uint32_t)std::min<size_t>(((size_t)m * n + 255) / 256, 8192), 256, 0, h->stream>>>(d_lp + done * s, p,
                                                                                                                      s, d_k);
-            azb_tree_code_kernel<<<(m + AZB_CODE_WARPS - 1) / AZB_CODE_WARPS, AZB_CODE_WARPS * 32, 0, h->stream>>>(
-                d_k, m, n, reinterpret_cast<unsigned long long *>(d_e1), (uint32_t)(E / 8), &d_sc->bad);
-            h->launches += 2;
+            launch_code_kernel(h, d_k, m, n, reinterpret_cast<unsigned long long *>(d_e1), (uint32_t)(E / 8), &d_sc->bad);
+            h->launches += 1;
             CK(cudaGetLastError());
             CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_e1, d_e2, m, AzbGrowByCode{}, lo_bit, 128, h->stream));
             CK(cub::DeviceSelect::Unique(d_tmp, tmp_bytes, d_e2, d_e1, &d_sc->n_sel, m, h->stream));
@@ -2309,30 +2323,21 @@ extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_
     // the last level, by (key bits, code): count the keys below the bound, and the first k through the cost kernel of
     // azb_eval_costs on their canonical parent arrays
     const uint32_t nres = (uint32_t)std::min<uint64_t>(k, nacc);
-    if (nacc) {
+    std::vector<AzbGrowEnt> res(nres);
+    unsigned long long below = 0;
+    uint32_t cerr = 0;
+    if (nres) {
         CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_a, d_b, (uint32_t)nacc, AzbGrowByKey{}, h->stream));
         azb_grow_below_kernel<<<(uint32_t)((nacc + 255) / 256), 256, 0, h->stream>>>(d_b, (uint32_t)nacc, bound, &d_sc->below);
         azb_grow_decode_kernel<<<(nres + 255) / 256, 256, 0, h->stream>>>(d_b, nres, N, d_res);
         h->launches += 2;
         CK(cudaGetLastError());
-        rc = cost_buffers(h, nres);
+        rc = cost_tail(h, d_res, nres, N, d_res_cost, nullptr, h->ev1, parents, lambda1, mu, eval, &cerr);
         if (rc) return rc;
-        CK(cudaMemsetAsync(h->cost_err, 0, 4, h->stream));
-        launch_cost_kernel(h, d_res, nres);
-        CK(cudaGetLastError());
-    }
-    CK(cudaEventRecord(h->ev1, h->stream));
-    std::vector<AzbGrowEnt> res(nres);
-    unsigned long long below = 0;
-    uint32_t cerr = 0;
-    if (nres) {
         CK(cudaMemcpyAsync(res.data(), d_b, (size_t)nres * E, cudaMemcpyDeviceToHost, h->stream));
         CK(cudaMemcpyAsync(&below, &d_sc->below, 8, cudaMemcpyDeviceToHost, h->stream));
-        if (parents) CK(cudaMemcpyAsync(parents, d_res, (size_t)nres * N, cudaMemcpyDeviceToHost, h->stream));
-        if (lambda1) CK(cudaMemcpyAsync(lambda1, h->cost_l1, (size_t)nres * 8, cudaMemcpyDeviceToHost, h->stream));
-        if (mu) CK(cudaMemcpyAsync(mu, h->cost_mu, (size_t)nres * 4, cudaMemcpyDeviceToHost, h->stream));
-        if (eval) CK(cudaMemcpyAsync(eval, h->cost_c, (size_t)nres * 4, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaMemcpyAsync(&cerr, h->cost_err, 4, cudaMemcpyDeviceToHost, h->stream));
+    } else {
+        CK(cudaEventRecord(h->ev1, h->stream));
     }
     CK(cudaStreamSynchronize(h->stream));
     if (ms) CK(cudaEventElapsedTime(ms, h->ev0, h->ev1));
@@ -2808,7 +2813,7 @@ enum {
 };
 static_assert(CK_TABLE_DIGEST < CK_HDR_DIGEST, "checkpoint header layout");
 static const uint64_t k_ckpt_hdr_bytes = AZB_CKPT_HEADER_WORDS * 8ull;
-static const uint64_t k_ckpt_half_max = 128ull << 20;  // each of the staging slab's two halves: 256 MB in all
+static const uint64_t k_ckpt_half_max = 128ull << 20;  // each of the staging area's two halves: 256 MB in all
 
 static uint64_t ckpt_digest(const void *p, uint64_t n) {  // include/azb.h; the buffer need not be 8-byte aligned
     const uint8_t *b = static_cast<const uint8_t *>(p);
@@ -2827,7 +2832,8 @@ static uint32_t f2u(float f) {
 }
 static uint64_t model_bytes(const azb_handle *h) { return (h->n_params * 12 + 7) & ~7ull; }
 
-// the staging slab: [len | offsets (B + 1 each) | CUB scratch | bad words | half 0 | half 1]
+// the staging buffers: [len | offsets (B + 1 each) | CUB scratch | bad words | half 0 | half 1]; the layout up to the
+// halves does not depend on their size
 struct CkptSlab {
     unsigned long long *len, *off, *bad;
     void *tmp;
@@ -2839,30 +2845,19 @@ static int ckpt_slab(azb_handle *h, uint64_t half_bytes, CkptSlab &s) {
     s.tmp_bytes = 0;
     CK(cub::DeviceScan::ExclusiveSum(nullptr, s.tmp_bytes, (const unsigned long long *)nullptr, (unsigned long long *)nullptr, (int)n,
                                      h->stream));
-    const size_t o_off = best_up(n * 8), o_tmp = o_off + best_up(n * 8), o_bad = o_tmp + best_up(s.tmp_bytes), o_h0 = o_bad + 256,
-                 o_h1 = o_h0 + best_up(half_bytes), total = o_h1 + best_up(half_bytes);
-    if (total > h->ckpt_cap) {
-        if (h->ckpt_buf) {
-            CK(cudaStreamSynchronize(h->stream));
-            CK(cudaFree(h->ckpt_buf));
-            h->dev_bytes -= h->ckpt_cap;
-        }
-        h->ckpt_buf = nullptr;
-        h->ckpt_cap = 0;
-        CK(dmalloc(h, &h->ckpt_buf, total));
-        h->ckpt_cap = total;
-    }
+    int rc = scratch(h, [&](Carve &cv) {
+        s.len = cv.take<unsigned long long>(n);
+        s.off = cv.take<unsigned long long>(n);
+        s.tmp = cv.take<uint8_t>(s.tmp_bytes);
+        s.bad = cv.take<unsigned long long>(2);
+        s.half[0] = cv.take<uint8_t>(half_bytes);
+        s.half[1] = cv.take<uint8_t>(half_bytes);
+    });
+    if (rc) return rc;
     if (!h->ckpt_stream) {
         CK(cudaStreamCreateWithFlags(&h->ckpt_stream, cudaStreamNonBlocking));
         for (cudaEvent_t &e : h->ckpt_ev) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     }
-    uint8_t *b = h->ckpt_buf;
-    s.len = reinterpret_cast<unsigned long long *>(b);
-    s.off = reinterpret_cast<unsigned long long *>(b + o_off);
-    s.tmp = b + o_tmp;
-    s.bad = reinterpret_cast<unsigned long long *>(b + o_bad);
-    s.half[0] = b + o_h0;
-    s.half[1] = b + o_h1;
     return AZB_OK;
 }
 

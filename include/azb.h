@@ -324,7 +324,7 @@ int azb_checkpoint_load(azb_handle *h, const void *const *blobs, const uint64_t 
  * Unranking: with P[r][g] = the number of non-increasing sequences of ids <= g whose sizes sum to r, the sequences of sum
  * r with first element < g number P[r][g - 1]; an index is decoded one element at a time (the smallest g with P[r][g] > x,
  * then x -= P[r][g - 1], r -= size(g)).  The handle builds P (rows r = 0..N-1, 32 x 141 083 words at N = 32) and the
- * preorder arrays of all rooted trees of size <= N/2 on first use; both count in azb_device_bytes.
+ * preorder arrays of all rooted trees of size <= N/2 on first use; they and the calls' scratch count in azb_device_bytes.
  * azb_free_tree_count: A000055(n) for 5 <= n <= 32, host only.
  * azb_free_trees: the parent arrays of indices [start, start + m) of the handle's N.
  * azb_exhaustive_best: every tree of [start, start + count) through the cost kernel of azb_eval_costs; the first
@@ -363,7 +363,7 @@ int azb_exhaustive_best(azb_handle *h, uint64_t start, uint64_t count, uint32_t 
  * classes (0: as many as fit in the device's free memory, which also bounds a larger max_level); azb_last_error names the
  * level and the classes found so far, and no output is written.  AZB_ERR_LAMBDA as azb_eval_costs.  The call works
  * before azb_init_trees, runs on the library stream, changes no tree, walker, counter, argmin, model or RNG state, and
- * its scratch is the slab of azb_best_trees (counted in azb_device_bytes). */
+ * its scratch counts in azb_device_bytes. */
 int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out, uint64_t *n_within,
                      uint64_t *n_below, uint64_t *codes /*[k*2]*/, uint8_t *parents /*[k*N]*/, double *lambda1 /*[k]*/,
                      uint32_t *mu /*[k]*/, float *eval /*[k]*/, float *ms);
@@ -451,7 +451,10 @@ int azb_comm_allreduce_bench(azb_handle *h, uint32_t reps, float *ms);
 
 /* ---- measurement helpers ---- */
 int azb_kernel_launches(const azb_handle *h, uint64_t *n);   /* kernels launched by this handle so far */
-int azb_device_bytes(const azb_handle *h, uint64_t *bytes);  /* HBM held by this handle */
+/* HBM held by this handle.  Every call outside the search step (the stand-alone costs, azb_get_argmin's cost, codes, best
+ * trees, enumeration, azb_trees_within, checkpoints) takes its device buffers from one grow-only scratch slab, so this
+ * counts the largest scratch any of them has needed so far. */
+int azb_device_bytes(const azb_handle *h, uint64_t *bytes);
 int azb_flush_l2(azb_handle *h);                             /* overwrite a >L2 scratch buffer */
 /* cascades (cascade_new_terminal / cascade_old_node, nabla/tree/empty_transitions.rs:50-127) whose ancestor wave
  * outgrew the on-chip work list and continued in the tree's HBM scratch, since azb_create.  The reference's BTreeMap
