@@ -95,6 +95,8 @@ SIGNATURES = {
                                       C.POINTER(C.c_uint64), u8p, f64p, u32p, f32p, f32p]),
     "azb_trees_within": (C.c_int, [C.c_void_p, C.c_double, C.c_uint32, C.c_uint64, u32p, C.POINTER(C.c_uint64),
                                    C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), u8p, f64p, u32p, f32p, f32p]),
+    "azb_comm_trees_within": (C.c_int, [C.c_void_p, C.c_double, C.c_uint32, C.c_uint64, u32p, C.POINTER(C.c_uint64),
+                                        C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), u8p, f64p, u32p, f32p, f32p]),
     "azb_checkpoint_size": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     "azb_checkpoint_save": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]),
     "azb_checkpoint_load": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64), C.c_uint32]),
@@ -580,14 +582,21 @@ class Handle:
         key), the first k ascending by (key, code): dict of arrays code u64[., 2], parents u8[., N] (canonical labelling),
         lambda1 f64, mu u32, eval f32, plus n_within, n_below (key < bound) and ms (device time).  max_level caps the
         classes of any level (0: what fits in device memory); beyond it AzbError with ERR_CAPACITY."""
+        return self._trees_within(self._L.azb_trees_within, bound, k, max_level)
+
+    def comm_trees_within(self, bound=None, k: int = 100, max_level: int = 0):
+        """trees_within split over the ranks of the attached communicator (azb_comm_trees_within): collective, every rank
+        calls it with the same arguments and gets the same dict, bit for bit what trees_within gives on one handle."""
+        return self._trees_within(self._L.azb_comm_trees_within, bound, k, max_level)
+
+    def _trees_within(self, fn, bound, k, max_level):
         kk = max(int(k), 1)
         out = dict(code=np.zeros((kk, 2), dtype=np.uint64), parents=np.zeros((kk, self.n), dtype=np.uint8),
                    lambda1=np.zeros(kk, dtype=np.float64), mu=np.zeros(kk, dtype=np.uint32), eval=np.zeros(kk, dtype=np.float32))
         n, within, below, ms = C.c_uint32(), C.c_uint64(), C.c_uint64(), C.c_float()
-        self._ck(self._L.azb_trees_within(self._h, -1.0 if bound is None else float(bound), k, max_level, C.byref(n),
-                                          C.byref(within), C.byref(below), _p(out["code"], C.c_uint64),
-                                          _p(out["parents"], C.c_uint8), _p(out["lambda1"], C.c_double),
-                                          _p(out["mu"], C.c_uint32), _p(out["eval"], C.c_float), C.byref(ms)))
+        self._ck(fn(self._h, -1.0 if bound is None else float(bound), k, max_level, C.byref(n), C.byref(within), C.byref(below),
+                    _p(out["code"], C.c_uint64), _p(out["parents"], C.c_uint8), _p(out["lambda1"], C.c_double),
+                    _p(out["mu"], C.c_uint32), _p(out["eval"], C.c_float), C.byref(ms)))
         res = {name: a[:n.value] for name, a in out.items()}
         res.update(n_within=int(within.value), n_below=int(below.value), ms=float(ms.value))
         return res

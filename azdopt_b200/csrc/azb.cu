@@ -2174,18 +2174,92 @@ extern "C" int azb_exhaustive_best(azb_handle *h, uint64_t start, uint64_t count
 // Level n (the classes on n vertices) is built from level n - 1 in chunks of parents; azb_grow.cuh lists the passes of
 // one chunk.  The host keeps each finished level as its list of codes and lays the slab out anew for the next one: the
 // level's parents decoded (LP), the chunk's buffers, and the list of kept classes (A) with the other half of its sorts (B).
-extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out, uint64_t *n_within,
-                                uint64_t *n_below, uint64_t *codes, uint8_t *parents, double *lambda1, uint32_t *mu, float *eval,
-                                float *ms) {
-    if (!h) return AZB_ERR_INVALID;
-    if (k == 0 || k > AZB_BEST_MAX_K) return fail(h, AZB_ERR_INVALID, "k must be in 1..%u, got %u", AZB_BEST_MAX_K, k);
-    if (std::isnan(bound)) return fail(h, AZB_ERR_INVALID, "azb_trees_within: the bound is NaN");
+//
+// Sharded (azb_comm_trees_within; include/azb.h has the algorithm): a rank holds the classes of each level it owns, and
+// the level runs in rounds that every rank takes part in, one chunk of its own parents each (possibly none).  A round
+// routes the chunk's distinct classes to their owners, all-gathers one record per rank (WR_* below) and exchanges
+// the runs; the received codes are then sorted, made unique and costed in pieces of at most one chunk.  One more record
+// closes each level.  Every stop is decided from the records, so all ranks return it from the same collective.
+static int comm_allgather(azb_handle *h, const unsigned long long *send, unsigned long long *recv, size_t count);
+static int comm_exchange(azb_handle *h, const ulonglong2 *send, const unsigned long long *rec, ulonglong2 *recv);
+
+// a rank's record of one round, all-gathered: send counts to every rank, then these
+enum { WR_SHARE = 0, WR_CAP, WR_ERR, WR_WORDS };  // kept list at its last merge, the rank's cap on it, cost error word
+
+// the first collective of azb_comm_trees_within: every rank's arguments and chunk; refuses on every rank what one
+// rank's arguments make invalid.  chunks = every rank's children per chunk.
+static int within_agree_args(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t chunk,
+                             std::vector<uint32_t> &chunks) {
+    const uint32_t world = (uint32_t)h->comm_world;
+    enum { A_N, A_BOUND, A_K, A_MAX, A_CHUNK, A_WORDS };
+    unsigned long long *d_args = nullptr;
+    int rc = scratch(h, [&](Carve &cv) { d_args = cv.take<unsigned long long>((size_t)A_WORDS * (world + 1)); });
+    if (rc) return rc;
+    unsigned long long mine[A_WORDS] = {h->N, 0, k, max_level, chunk};
+    memcpy(&mine[A_BOUND], &bound, 8);
+    std::vector<unsigned long long> a((size_t)A_WORDS * world);
+    CK(cudaMemcpyAsync(d_args + (size_t)A_WORDS * world, mine, sizeof(mine), cudaMemcpyHostToDevice, h->stream));
+    rc = comm_allgather(h, d_args + (size_t)A_WORDS * world, d_args, A_WORDS);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(a.data(), d_args, a.size() * 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    const char *name[A_WORDS] = {"N", "bound", "k", "max_level", "chunk"};
+    for (uint32_t r = 0; r < world; ++r) {
+        const unsigned long long *ar = a.data() + (size_t)A_WORDS * r;
+        double b;
+        memcpy(&b, &ar[A_BOUND], 8);
+        if (ar[A_K] == 0 || ar[A_K] > AZB_BEST_MAX_K)
+            return fail(h, AZB_ERR_INVALID, "azb_comm_trees_within: rank %u passes k = %llu; k must be in 1..%u", r, ar[A_K],
+                        AZB_BEST_MAX_K);
+        if (std::isnan(b)) return fail(h, AZB_ERR_INVALID, "azb_comm_trees_within: rank %u passes a NaN bound", r);
+        for (int f = A_N; f < A_CHUNK; ++f)
+            if (ar[f] != a[f])
+                return fail(h, AZB_ERR_INVALID, "azb_comm_trees_within: rank %u's %s (%s 0x%llx) differs from rank 0's (0x%llx)", r,
+                            name[f], f == A_BOUND ? "bits" : "value", ar[f], a[f]);
+        chunks[r] = (uint32_t)ar[A_CHUNK];
+    }
+    return AZB_OK;
+}
+
+// The stop every rank returns after an all-gather of records (world x (world + WR_WORDS) words): a level over max_level
+// (the sum of the shares), a rank's share over its cap, a cost error on any rank.
+static int within_agreed_stop(azb_handle *h, const std::vector<unsigned long long> &rec, uint32_t world, uint32_t n,
+                              uint64_t max_level) {
+    const size_t R = world + WR_WORDS;
+    unsigned long long total = 0;
+    for (uint32_t r = 0; r < world; ++r) total += rec[R * r + world + WR_SHARE];
+    if (max_level && total > max_level)
+        return fail(h, AZB_ERR_CAPACITY,
+                    "azb_comm_trees_within: level %u (trees on %u vertices) holds more than %llu classes (at least %llu found on "
+                    "%u ranks; max_level %llu)",
+                    n, n, (unsigned long long)max_level, total, world, (unsigned long long)max_level);
+    for (uint32_t r = 0; r < world; ++r)
+        if (rec[R * r + world + WR_SHARE] > rec[R * r + world + WR_CAP])
+            return fail(h, AZB_ERR_CAPACITY,
+                        "azb_comm_trees_within: level %u (trees on %u vertices): rank %u's share holds more than %llu classes, "
+                        "the room on its device (at least %llu found; max_level %llu)",
+                        n, n, r, rec[R * r + world + WR_CAP], rec[R * r + world + WR_SHARE], (unsigned long long)max_level);
+    for (uint32_t r = 0; r < world; ++r)
+        if (rec[R * r + world + WR_ERR]) return fail(h, AZB_ERR_LAMBDA, "%s", azb_strerror(AZB_ERR_LAMBDA));
+    return AZB_OK;
+}
+
+// azb_trees_within (sharded = false: this handle alone, no collective) and azb_comm_trees_within (sharded = true)
+static int trees_within(azb_handle *h, bool sharded, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out,
+                        uint64_t *n_within, uint64_t *n_below, uint64_t *codes, uint8_t *parents, double *lambda1, uint32_t *mu,
+                        float *eval, float *ms) {
     CK(cudaSetDevice(h->cfg.device));
     const uint32_t N = h->N, chunk = h->grow_chunk ? h->grow_chunk : AZB_GROW_CHUNK;
-    const bool trace = getenv("AZB_TRACE_WITHIN") != nullptr;  // one line per level on stderr (tools/within_probe.py)
-    const size_t E = sizeof(AzbGrowEnt);
-    CK(cudaEventRecord(h->ev0, h->stream));
+    const uint32_t world = sharded ? (uint32_t)h->comm_world : 1u, me = sharded ? (uint32_t)h->comm_rank : 0u;
+    const bool trace = getenv("AZB_TRACE_WITHIN") != nullptr;  // one line per level (and rank) on stderr (tools/within_probe.py)
+    const size_t E = sizeof(AzbGrowEnt), R = world + WR_WORDS, tw = 2 + 3 * (size_t)k;  // tw: words of a rank's first k
     int rc = AZB_OK;
+    std::vector<uint32_t> chunks(world, chunk);  // every rank's children per chunk (tests give the ranks different ones)
+    if (sharded) {
+        rc = within_agree_args(h, bound, k, max_level, chunk, chunks);
+        if (rc) return rc;
+    }
+    CK(cudaEventRecord(h->ev0, h->stream));
     if (bound < 0.0) {  // the star's key on its canonical labelling: every vertex under vertex 0
         uint8_t *d_star = nullptr;
         CostOut d_cost;
@@ -2204,31 +2278,53 @@ extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_
         bound = (double)m1 + l1;
     }
     // the classes one level may hold: max_level, what the device has room for (per class: the list and the other half
-    // of its sort, CUB's scratch, the codes and parents of the next level; the chunk's buffers set aside), and what one
-    // CUB pass takes
+    // of its sort, CUB's scratch, the codes and parents of the next level; the chunk's buffers set aside, and when
+    // sharded the codes one round can bring with the other half of their sort and its CUB scratch), and what one CUB
+    // pass takes
     const uint64_t kc_max = (uint64_t)std::max(chunk, 64u) + 64u;
+    uint64_t recv_max = 0;
+    if (sharded)
+        for (uint32_t c : chunks) recv_max += (uint64_t)std::max(c, 64u) + 64u;
     size_t free_b = 0, total_b = 0;
     CK(cudaMemGetInfo(&free_b, &total_b));
-    const uint64_t avail = (uint64_t)free_b + h->scratch_cap, set_aside = kc_max * (64 + 4 * E + 16) + (256ull << 20);
+    const uint64_t avail = (uint64_t)free_b + h->scratch_cap;
+    const uint64_t set_aside = kc_max * (64 + 4 * E + 16) + recv_max * 3 * E + (256ull << 20);
     const uint64_t fit = avail > set_aside ? (avail - set_aside) / (5 * E + 64) : 0;
     const uint64_t cap_level = std::min<uint64_t>({max_level ? max_level : fit, fit, (1ull << 31) - 1 - kc_max});
-    // L_4: the path (code 11100100) and the star (11010100); every tree on 5 or more vertices grows from one of them
-    std::vector<AzbGrowEnt> lvl = {AzbGrowEnt{0xE4ull << 56, 0ull, 0ull}, AzbGrowEnt{0xD4ull << 56, 0ull, 0ull}};
+    // L_4: the path (code 11100100) and the star (11010100); every tree on 5 or more vertices grows from one of them.
+    // share[r] = the classes of the current level rank r holds.
+    std::vector<AzbGrowEnt> lvl;
+    std::vector<uint64_t> share(world, 0);
+    for (const AzbGrowEnt &e : {AzbGrowEnt{0xE4ull << 56, 0ull, 0ull}, AzbGrowEnt{0xD4ull << 56, 0ull, 0ull}}) {
+        const uint32_t o = azb_grow_owner(e.hi, e.lo, world);
+        share[o] += 1;
+        if (o == me) lvl.push_back(e);
+    }
+    std::vector<unsigned long long> rec(R * world);
     AzbGrowEnt *d_a = nullptr, *d_b = nullptr;
     AzbGrowScalars *d_sc = nullptr;
     uint8_t *d_res = nullptr;
+    unsigned long long *d_top = nullptr;
     CostOut d_res_cost;
     size_t tmp_bytes = 0;
     uint8_t *d_tmp = nullptr;
-    uint64_t nacc = 0;
+    uint64_t nacc = 0, total = 2;
     for (uint32_t s = 4; s < N; ++s) {
         const auto t0 = std::chrono::steady_clock::now();
         const uint32_t n = s + 1, lo_bit = 128 - 2 * n;  // a code of n vertices occupies the top 2n of the 128 bits
         const bool last = n == N;
         const uint64_t ns = lvl.size();
         const uint32_t pc = std::max(1u, chunk / s), kc = pc * s;  // parents and children of a full chunk
-        const uint64_t acap = std::min<uint64_t>(ns * s, cap_level) + kc;
-        size_t t[5] = {0, 0, 0, 0, 0};
+        const uint64_t acap = std::min<uint64_t>(total * s, cap_level) + kc;
+        uint32_t rounds = 0;  // the most chunks any rank has at this level
+        uint64_t rmax = 0;    // sharded: the most codes one round can bring, a full chunk from every rank
+        for (uint32_t r = 0; r < world; ++r) {
+            const uint32_t pr = std::max(1u, chunks[r] / s);
+            rounds = std::max<uint32_t>(rounds, (uint32_t)((share[r] + pr - 1) / pr));
+            rmax += (uint64_t)pr * s;
+        }
+        if (!sharded) rmax = 0;
+        size_t t[6] = {0, 0, 0, 0, 0, 0};
         CK(cub::DeviceRadixSort::SortKeys(nullptr, t[0], (const AzbGrowEnt *)nullptr, (AzbGrowEnt *)nullptr, kc, AzbGrowByCode{},
                                           lo_bit, 128, h->stream));
         CK(cub::DeviceRadixSort::SortKeys(nullptr, t[1], (const AzbGrowEnt *)nullptr, (AzbGrowEnt *)nullptr, (uint32_t)acap, AzbGrowByCode{},
@@ -2238,12 +2334,20 @@ extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_
         if (last)
             CK(cub::DeviceRadixSort::SortKeys(nullptr, t[3], (const AzbGrowEnt *)nullptr, (AzbGrowEnt *)nullptr, (uint32_t)acap, AzbGrowByKey{},
                                               h->stream));
-        tmp_bytes = *std::max_element(t, t + 5);
-        AzbGrowEnt *d_lv = nullptr, *d_e1 = nullptr, *d_e2 = nullptr;
+        if (sharded) {
+            CK(cub::DeviceRadixSort::SortKeys(nullptr, t[4], (const AzbGrowEnt *)nullptr, (AzbGrowEnt *)nullptr, (uint32_t)rmax,
+                                              AzbGrowByCode{}, lo_bit, 128, h->stream));
+            CK(cub::DeviceSelect::Unique(nullptr, t[5], (const AzbGrowEnt *)nullptr, (AzbGrowEnt *)nullptr, (uint32_t *)nullptr,
+                                         (uint32_t)rmax, h->stream));
+        }
+        tmp_bytes = *std::max_element(t, t + 6);
+        AzbGrowEnt *d_lv = nullptr, *d_e1 = nullptr, *d_e2 = nullptr, *d_r1 = nullptr, *d_r2 = nullptr;
         uint8_t *d_lp = nullptr, *d_k = nullptr;
         double *d_l1 = nullptr;
         uint32_t *d_mu = nullptr;
         float *d_c = nullptr;
+        ulonglong2 *d_send = nullptr;
+        unsigned long long *d_rec = nullptr, *d_cursor = nullptr;
         rc = scratch(h, [&](Carve &cv) {
             d_lv = cv.take<AzbGrowEnt>(ns);
             d_lp = cv.take<uint8_t>(ns * s);
@@ -2254,88 +2358,206 @@ extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_
             d_mu = cv.take<uint32_t>(kc);
             d_c = cv.take<float>(kc);
             d_a = cv.take<AzbGrowEnt>(acap);
-            d_b = cv.take<AzbGrowEnt>(acap);
+            d_b = cv.take<AzbGrowEnt>(sharded && last ? std::max<uint64_t>(acap, k) : acap);  // sharded: the merged first k
             d_sc = cv.take<AzbGrowScalars>(1);
             d_res = cv.take<uint8_t>((size_t)k * N);
             d_res_cost.take(cv, k);
             d_tmp = cv.take<uint8_t>(tmp_bytes);
+            // sharded only (all empty otherwise); the received runs land in d_r2's bytes, copied out before its sort
+            d_send = cv.take<ulonglong2>(sharded ? kc : 0);
+            d_r1 = cv.take<AzbGrowEnt>(rmax);
+            d_r2 = cv.take<AzbGrowEnt>(rmax);
+            d_rec = cv.take<unsigned long long>(sharded ? R * (world + 1) : 0);
+            d_cursor = cv.take<unsigned long long>(sharded ? world : 0);
+            d_top = cv.take<unsigned long long>(sharded && last ? tw * (world + 1) : 0);  // count, below, first k entries
         });
         if (rc) return rc;
         CK(cudaMemcpyAsync(d_lv, lvl.data(), ns * E, cudaMemcpyHostToDevice, h->stream));
         CK(cudaMemsetAsync(d_sc, 0, sizeof(AzbGrowScalars), h->stream));
-        azb_grow_decode_kernel<<<(uint32_t)((ns + 255) / 256), 256, 0, h->stream>>>(d_lv, (uint32_t)ns, s, d_lp);
-        h->launches += 1;
-        CK(cudaGetLastError());
-        const double thr = last ? bound : bound + AZB_GROW_EPS;
-        uint64_t children = 0, evaluated = 0;
-        nacc = 0;
-        for (uint64_t done = 0; done < ns;) {
-            const uint32_t p = (uint32_t)std::min<uint64_t>(pc, ns - done), m = p * s;
-            azb_grow_expand_kernel<<<(uint32_t)std::min<size_t>(((size_t)m * n + 255) / 256, 8192), 256, 0, h->stream>>>(d_lp + done * s, p,
-                                                                                                                     s, d_k);
-            launch_code_kernel(h, d_k, m, n, reinterpret_cast<unsigned long long *>(d_e1), (uint32_t)(E / 8), &d_sc->bad);
+        if (ns) {
+            azb_grow_decode_kernel<<<(uint32_t)((ns + 255) / 256), 256, 0, h->stream>>>(d_lv, (uint32_t)ns, s, d_lp);
             h->launches += 1;
             CK(cudaGetLastError());
-            CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_e1, d_e2, m, AzbGrowByCode{}, lo_bit, 128, h->stream));
-            CK(cub::DeviceSelect::Unique(d_tmp, tmp_bytes, d_e2, d_e1, &d_sc->n_sel, m, h->stream));
-            uint32_t u = 0, kept = 0;
-            CK(cudaMemcpyAsync(&u, &d_sc->n_sel, 4, cudaMemcpyDeviceToHost, h->stream));
-            CK(cudaStreamSynchronize(h->stream));
-            azb_grow_decode_kernel<<<(u + 255) / 256, 256, 0, h->stream>>>(d_e1, u, n, d_k);
-            launch_cost_n(h, d_k, u, n, d_l1, d_mu, d_c, &d_sc->err);
-            CK(cudaMemsetAsync(&d_sc->n_keep, 0, 4, h->stream));
-            azb_grow_keep_kernel<<<(u + 255) / 256, 256, 0, h->stream>>>(d_e1, d_l1, d_mu, u, thr, d_a + nacc, &d_sc->n_keep);
-            h->launches += 2;
-            CK(cudaGetLastError());
-            CK(cudaMemcpyAsync(&kept, &d_sc->n_keep, 4, cudaMemcpyDeviceToHost, h->stream));
-            CK(cudaStreamSynchronize(h->stream));
-            nacc += kept;
-            children += m;
-            evaluated += u;
-            done += p;
-            if (nacc && (nacc + kc > acap || done == ns)) {  // one entry per class, sorted by code
-                uint32_t nu = 0;
-                CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_a, d_b, (uint32_t)nacc, AzbGrowByCode{}, lo_bit, 128, h->stream));
-                CK(cub::DeviceSelect::Unique(d_tmp, tmp_bytes, d_b, d_a, &d_sc->n_sel, (uint32_t)nacc, h->stream));
-                CK(cudaMemcpyAsync(&nu, &d_sc->n_sel, 4, cudaMemcpyDeviceToHost, h->stream));
-                CK(cudaStreamSynchronize(h->stream));
-                nacc = nu;
-                if (nacc > cap_level)
-                    return fail(h, AZB_ERR_CAPACITY,
-                                "azb_trees_within: level %u (trees on %u vertices) holds more than %llu classes (at least %llu found; "
-                                "max_level %llu, room on the device for %llu)",
-                                n, n, (unsigned long long)cap_level, (unsigned long long)nacc, (unsigned long long)max_level,
-                                (unsigned long long)fit);
-            }
         }
+        const double thr = last ? bound : bound + AZB_GROW_EPS;
+        uint64_t children = 0, evaluated = 0, sent = 0, received = 0, merged = 0;  // merged: the list's size at its last merge
+        bool dirty = false;  // classes kept since that merge
+        nacc = 0;
+        // one entry per class, sorted by code; alone, a list over the cap ends the call here, sharded at the next record
+        auto merge = [&]() -> int {
+            uint32_t nu = 0;
+            CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_a, d_b, (uint32_t)nacc, AzbGrowByCode{}, lo_bit, 128, h->stream));
+            CK(cub::DeviceSelect::Unique(d_tmp, tmp_bytes, d_b, d_a, &d_sc->n_sel, (uint32_t)nacc, h->stream));
+            CK(cudaMemcpyAsync(&nu, &d_sc->n_sel, 4, cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+            nacc = merged = nu;
+            dirty = false;
+            if (nacc > cap_level && !sharded)
+                return fail(h, AZB_ERR_CAPACITY,
+                            "azb_trees_within: level %u (trees on %u vertices) holds more than %llu classes (at least %llu found; "
+                            "max_level %llu, room on the device for %llu)",
+                            n, n, (unsigned long long)cap_level, (unsigned long long)nacc, (unsigned long long)max_level,
+                            (unsigned long long)fit);
+            return AZB_OK;
+        };
+        // sharded: route the u classes at d_e1 to their owners, all-gather the records, stop if they say so, exchange the
+        // runs; *got = the distinct classes received, at d_r1
+        auto exchange = [&](uint32_t u, uint32_t *got) -> int {
+            unsigned long long *mine = d_rec + R * world;
+            CK(cudaMemsetAsync(mine, 0, R * 8, h->stream));
+            if (u) {
+                const uint32_t blocks = std::min((u + 255) / 256, 1184u);
+                CK(cudaMemsetAsync(d_cursor, 0, (size_t)world * 8, h->stream));
+                azb_grow_count_kernel<<<blocks, 256, 4 * world, h->stream>>>(d_e1, u, world, mine);
+                azb_grow_route_kernel<<<blocks, 256, 20 * world, h->stream>>>(d_e1, u, world, mine, d_cursor, d_send);
+                h->launches += 2;
+                CK(cudaGetLastError());
+            }
+            const unsigned long long tail[2] = {merged, cap_level};
+            CK(cudaMemcpyAsync(mine + world + WR_SHARE, tail, sizeof(tail), cudaMemcpyHostToDevice, h->stream));
+            CK(cudaMemcpyAsync(mine + world + WR_ERR, &d_sc->err, 4, cudaMemcpyDeviceToDevice, h->stream));
+            int rc2 = comm_allgather(h, mine, d_rec, R);
+            if (rc2) return rc2;
+            CK(cudaMemcpyAsync(rec.data(), d_rec, R * world * 8, cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+            rc2 = within_agreed_stop(h, rec, world, n, max_level);
+            if (rc2) return rc2;
+            ulonglong2 *recv = reinterpret_cast<ulonglong2 *>(d_r2);
+            rc2 = comm_exchange(h, d_send, rec.data(), recv);
+            if (rc2) return rc2;
+            uint64_t nr = 0;
+            for (uint32_t r = 0; r < world; ++r) {
+                nr += rec[R * r + me];
+                if (r != me) sent += rec[R * me + r], received += rec[R * r + me];
+            }
+            *got = 0;
+            if (nr == 0) return AZB_OK;
+            CK(cudaMemcpy2DAsync(d_r1, E, recv, 16, 16, nr, cudaMemcpyDeviceToDevice, h->stream));
+            CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_r1, d_r2, (uint32_t)nr, AzbGrowByCode{}, lo_bit, 128, h->stream));
+            CK(cub::DeviceSelect::Unique(d_tmp, tmp_bytes, d_r2, d_r1, &d_sc->n_sel, (uint32_t)nr, h->stream));
+            CK(cudaMemcpyAsync(got, &d_sc->n_sel, 4, cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+            return AZB_OK;
+        };
+        uint64_t done = 0;
+        for (uint32_t round = 0; round < rounds; ++round) {
+            const uint32_t p = (uint32_t)std::min<uint64_t>(pc, ns - done), m = p * s;
+            uint32_t u = 0;
+            if (p) {
+                azb_grow_expand_kernel<<<(uint32_t)std::min<size_t>(((size_t)m * n + 255) / 256, 8192), 256, 0, h->stream>>>(d_lp + done * s,
+                                                                                                                         p, s, d_k);
+                launch_code_kernel(h, d_k, m, n, reinterpret_cast<unsigned long long *>(d_e1), (uint32_t)(E / 8), &d_sc->bad);
+                h->launches += 1;
+                CK(cudaGetLastError());
+                CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_e1, d_e2, m, AzbGrowByCode{}, lo_bit, 128, h->stream));
+                CK(cub::DeviceSelect::Unique(d_tmp, tmp_bytes, d_e2, d_e1, &d_sc->n_sel, m, h->stream));
+                CK(cudaMemcpyAsync(&u, &d_sc->n_sel, 4, cudaMemcpyDeviceToHost, h->stream));
+                CK(cudaStreamSynchronize(h->stream));
+            }
+            const AzbGrowEnt *fresh = d_e1;  // the distinct classes this rank evaluates in this round
+            if (sharded) {
+                rc = exchange(u, &u);
+                if (rc) return rc;
+                fresh = d_r1;
+            }
+            // decode, cost and keep, in pieces of at most one chunk (alone: the chunk, in one piece)
+            for (uint32_t off = 0; off < u && merged <= cap_level; off += kc) {
+                const uint32_t q = std::min(kc, u - off);
+                uint32_t kept = 0;
+                azb_grow_decode_kernel<<<(q + 255) / 256, 256, 0, h->stream>>>(fresh + off, q, n, d_k);
+                launch_cost_n(h, d_k, q, n, d_l1, d_mu, d_c, &d_sc->err);
+                CK(cudaMemsetAsync(&d_sc->n_keep, 0, 4, h->stream));
+                azb_grow_keep_kernel<<<(q + 255) / 256, 256, 0, h->stream>>>(fresh + off, d_l1, d_mu, q, thr, d_a + nacc, &d_sc->n_keep);
+                h->launches += 2;
+                CK(cudaGetLastError());
+                CK(cudaMemcpyAsync(&kept, &d_sc->n_keep, 4, cudaMemcpyDeviceToHost, h->stream));
+                CK(cudaStreamSynchronize(h->stream));
+                nacc += kept;
+                evaluated += q;
+                dirty = dirty || kept;
+                if (dirty && nacc + kc > acap) {
+                    rc = merge();
+                    if (rc) return rc;
+                }
+            }
+            children += m;
+            done += p;
+        }
+        if (dirty) {
+            rc = merge();
+            if (rc) return rc;
+        }
+        if (sharded) {  // the level's closing record: every rank's share of it
+            uint32_t none = 0;
+            rc = exchange(0, &none);
+            if (rc) return rc;
+            for (uint32_t r = 0; r < world; ++r) share[r] = rec[R * r + world + WR_SHARE];
+        } else {
+            share[0] = nacc;
+        }
+        total = 0;
+        for (uint64_t c : share) total += c;
         uint32_t err = 0;
         CK(cudaMemcpyAsync(&err, &d_sc->err, 4, cudaMemcpyDeviceToHost, h->stream));
         lvl.resize(last ? 0 : nacc);
         if (!last && nacc) CK(cudaMemcpyAsync(lvl.data(), d_a, nacc * E, cudaMemcpyDeviceToHost, h->stream));
         CK(cudaStreamSynchronize(h->stream));
         if (err) return fail(h, AZB_ERR_LAMBDA, "%s", azb_strerror(AZB_ERR_LAMBDA));
-        if (trace)
+        const double level_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+        if (trace && !sharded)
             fprintf(stderr, "azb_trees_within: N %u level %u: %llu classes, %llu children, %llu evaluated, %.3f ms\n", N, n,
-                    (unsigned long long)nacc, (unsigned long long)children, (unsigned long long)evaluated,
-                    std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
-        if (nacc == 0) break;  // no tree on more vertices is within the bound either
+                    (unsigned long long)nacc, (unsigned long long)children, (unsigned long long)evaluated, level_ms);
+        if (trace && sharded)
+            fprintf(stderr,
+                    "azb_comm_trees_within: N %u level %u rank %u: %llu classes owned, %llu global, %llu children, %llu codes sent, "
+                    "%llu received, %llu evaluated, %.3f ms\n",
+                    N, n, me, (unsigned long long)nacc, (unsigned long long)total, (unsigned long long)children,
+                    (unsigned long long)sent, (unsigned long long)received, (unsigned long long)evaluated, level_ms);
+        if (total == 0) break;  // no tree on more vertices is within the bound either
     }
     // the last level, by (key bits, code): count the keys below the bound, and the first k through the cost kernel of
-    // azb_eval_costs on their canonical parent arrays
-    const uint32_t nres = (uint32_t)std::min<uint64_t>(k, nacc);
+    // azb_eval_costs on their canonical parent arrays.  Sharded, each rank sorts its share and the first k of every share
+    // are merged on every rank's host, so all ranks cost the same entries.
+    const uint32_t nres = (uint32_t)std::min<uint64_t>(k, total);
     std::vector<AzbGrowEnt> res(nres);
     unsigned long long below = 0;
     uint32_t cerr = 0;
     if (nres) {
-        CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_a, d_b, (uint32_t)nacc, AzbGrowByKey{}, h->stream));
-        azb_grow_below_kernel<<<(uint32_t)((nacc + 255) / 256), 256, 0, h->stream>>>(d_b, (uint32_t)nacc, bound, &d_sc->below);
+        if (nacc) {
+            CK(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_a, d_b, (uint32_t)nacc, AzbGrowByKey{}, h->stream));
+            azb_grow_below_kernel<<<(uint32_t)((nacc + 255) / 256), 256, 0, h->stream>>>(d_b, (uint32_t)nacc, bound, &d_sc->below);
+            h->launches += 1;
+            CK(cudaGetLastError());
+        }
+        if (sharded) {
+            const unsigned long long mk = std::min<uint64_t>(k, nacc);
+            unsigned long long *mine = d_top + tw * world;
+            CK(cudaMemcpyAsync(mine, &mk, 8, cudaMemcpyHostToDevice, h->stream));
+            CK(cudaMemcpyAsync(mine + 1, &d_sc->below, 8, cudaMemcpyDeviceToDevice, h->stream));
+            if (mk) CK(cudaMemcpyAsync(mine + 2, d_b, mk * E, cudaMemcpyDeviceToDevice, h->stream));
+            rc = comm_allgather(h, mine, d_top, tw);
+            if (rc) return rc;
+            std::vector<unsigned long long> top(tw * world);
+            CK(cudaMemcpyAsync(top.data(), d_top, top.size() * 8, cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+            std::vector<AzbGrowEnt> all;
+            for (uint32_t r = 0; r < world; ++r) {
+                const unsigned long long *tr = top.data() + tw * r;
+                below += tr[1];
+                for (unsigned long long i = 0; i < tr[0]; ++i) all.push_back(AzbGrowEnt{tr[2 + 3 * i], tr[3 + 3 * i], tr[4 + 3 * i]});
+            }
+            std::sort(all.begin(), all.end(), [](const AzbGrowEnt &a, const AzbGrowEnt &b) {
+                return std::tie(a.key, a.hi, a.lo) < std::tie(b.key, b.hi, b.lo);
+            });
+            CK(cudaMemcpyAsync(d_b, all.data(), (size_t)nres * E, cudaMemcpyHostToDevice, h->stream));
+        }
         azb_grow_decode_kernel<<<(nres + 255) / 256, 256, 0, h->stream>>>(d_b, nres, N, d_res);
-        h->launches += 2;
+        h->launches += 1;
         CK(cudaGetLastError());
         rc = cost_tail(h, d_res, nres, N, d_res_cost, nullptr, h->ev1, parents, lambda1, mu, eval, &cerr);
         if (rc) return rc;
         CK(cudaMemcpyAsync(res.data(), d_b, (size_t)nres * E, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaMemcpyAsync(&below, &d_sc->below, 8, cudaMemcpyDeviceToHost, h->stream));
+        if (!sharded) CK(cudaMemcpyAsync(&below, &d_sc->below, 8, cudaMemcpyDeviceToHost, h->stream));
     } else {
         CK(cudaEventRecord(h->ev1, h->stream));
     }
@@ -2348,9 +2570,28 @@ extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_
             codes[2 * i + 1] = res[i].lo;
         }
     if (n_out) *n_out = nres;
-    if (n_within) *n_within = nacc;
+    if (n_within) *n_within = total;
     if (n_below) *n_below = below;
     return AZB_OK;
+}
+
+extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out, uint64_t *n_within,
+                                uint64_t *n_below, uint64_t *codes, uint8_t *parents, double *lambda1, uint32_t *mu, float *eval,
+                                float *ms) {
+    if (!h) return AZB_ERR_INVALID;
+    if (k == 0 || k > AZB_BEST_MAX_K) return fail(h, AZB_ERR_INVALID, "k must be in 1..%u, got %u", AZB_BEST_MAX_K, k);
+    if (std::isnan(bound)) return fail(h, AZB_ERR_INVALID, "azb_trees_within: the bound is NaN");
+    return trees_within(h, false, bound, k, max_level, n_out, n_within, n_below, codes, parents, lambda1, mu, eval, ms);
+}
+
+extern "C" int azb_comm_trees_within(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out,
+                                     uint64_t *n_within, uint64_t *n_below, uint64_t *codes, uint8_t *parents, double *lambda1,
+                                     uint32_t *mu, float *eval, float *ms) {
+    if (!h) return AZB_ERR_INVALID;
+    if (!h->nccl_comm) return fail(h, AZB_ERR_STATE, "azb_comm_init has not been called");
+    if (h->comm_world > AZB_GROW_MAX_WORLD)
+        return fail(h, AZB_ERR_INVALID, "azb_comm_trees_within: %d ranks, at most %u", h->comm_world, AZB_GROW_MAX_WORLD);
+    return trees_within(h, true, bound, k, max_level, n_out, n_within, n_below, codes, parents, lambda1, mu, eval, ms);
 }
 
 // cascade waves that outgrew the shared-memory work list and continued in global scratch since azb_create (diagnostic;
@@ -2426,7 +2667,10 @@ typedef int (*nccl_allreduce_fn)(const void *, void *, size_t, int, int, void *,
 typedef int (*nccl_allgather_fn)(const void *, void *, size_t, int, void *, cudaStream_t);
 typedef int (*nccl_destroy_fn)(void *);
 typedef const char *(*nccl_errstr_fn)(int);
-enum { AZB_NCCL_UINT32 = 3, AZB_NCCL_FLOAT32 = 7, AZB_NCCL_FLOAT64 = 8, AZB_NCCL_SUM = 0 };  // nccl.h: ncclDataType_t / ncclRedOp_t
+typedef int (*nccl_send_fn)(const void *, size_t, int, int, void *, cudaStream_t);  // ncclSend / ncclRecv: buffer, count, type, peer
+typedef int (*nccl_recv_fn)(void *, size_t, int, int, void *, cudaStream_t);
+typedef int (*nccl_group_fn)(void);
+enum { AZB_NCCL_UINT32 = 3, AZB_NCCL_UINT64 = 5, AZB_NCCL_FLOAT32 = 7, AZB_NCCL_FLOAT64 = 8, AZB_NCCL_SUM = 0 };  // nccl.h: ncclDataType_t / ncclRedOp_t
 
 static void *nccl_open(void) {
     static void *lib = nullptr;
@@ -2457,6 +2701,45 @@ static int comm_allreduce(azb_handle *h, void *buf, size_t count, int dtype) {
     auto ar = (nccl_allreduce_fn)dlsym(h->nccl_lib, "ncclAllReduce");
     if (!ar) return fail(h, AZB_ERR_CUDA, "ncclAllReduce not found");
     NCCLCK(ar(buf, buf, count, dtype, AZB_NCCL_SUM, h->nccl_comm, h->stream));
+    return AZB_OK;
+}
+
+// azb_comm_trees_within: an all-gather of `count` u64 words per rank
+static int comm_allgather(azb_handle *h, const unsigned long long *send, unsigned long long *recv, size_t count) {
+    auto ag = (nccl_allgather_fn)dlsym(h->nccl_lib, "ncclAllGather");
+    if (!ag) return fail(h, AZB_ERR_CUDA, "ncclAllGather not found");
+    NCCLCK(ag(send, recv, count, AZB_NCCL_UINT64, h->nccl_comm, h->stream));
+    return AZB_OK;
+}
+
+// azb_comm_trees_within: the runs of one round.  rec = the round's all-gathered records; this rank's run for rank d
+// (rec[me][d] codes, runs in rank order at send) goes to d, and d's run for this rank lands at recv in rank order.  The
+// own run is a device copy.
+static int comm_exchange(azb_handle *h, const ulonglong2 *send, const unsigned long long *rec, ulonglong2 *recv) {
+    const uint32_t world = (uint32_t)h->comm_world, me = (uint32_t)h->comm_rank;
+    const size_t R = world + WR_WORDS;
+    auto snd = (nccl_send_fn)dlsym(h->nccl_lib, "ncclSend");
+    auto rcv = (nccl_recv_fn)dlsym(h->nccl_lib, "ncclRecv");
+    auto gstart = (nccl_group_fn)dlsym(h->nccl_lib, "ncclGroupStart");
+    auto gend = (nccl_group_fn)dlsym(h->nccl_lib, "ncclGroupEnd");
+    if (!snd || !rcv || !gstart || !gend) return fail(h, AZB_ERR_CUDA, "ncclSend, ncclRecv, ncclGroupStart or ncclGroupEnd not found");
+    unsigned long long so = 0, ro = 0, self_so = 0, self_ro = 0;
+    NCCLCK(gstart());
+    for (uint32_t d = 0; d < world; ++d) {
+        const unsigned long long ns = rec[R * me + d], nr = rec[R * d + me];
+        if (d == me) {
+            self_so = so;
+            self_ro = ro;
+        } else {
+            if (ns) NCCLCK(snd(send + so, 2 * ns, AZB_NCCL_UINT64, (int)d, h->nccl_comm, h->stream));
+            if (nr) NCCLCK(rcv(recv + ro, 2 * nr, AZB_NCCL_UINT64, (int)d, h->nccl_comm, h->stream));
+        }
+        so += ns;
+        ro += nr;
+    }
+    NCCLCK(gend());
+    const unsigned long long own = rec[R * me + me];
+    if (own) CK(cudaMemcpyAsync(recv + self_ro, send + self_so, own * 16, cudaMemcpyDeviceToDevice, h->stream));
     return AZB_OK;
 }
 

@@ -12,6 +12,11 @@
 //   keep               the classes with key <= the level's threshold, appended to the level's list
 // The list is sorted and made unique by code whenever it could overflow and at the end of the level; it is the next
 // level.  At the last level it is sorted by (key bits, code) and the first k are the result.
+//
+// Over several ranks (azb_comm_trees_within) each class has one owner, azb_grow_owner, and a rank holds only the classes
+// it owns.  Between unique and decode a round routes the chunk's classes to their owners: count and route below write
+// them as per-owner runs of 16-byte codes, the host exchanges the runs, and each rank sorts and makes unique what it
+// received before it decodes, costs and keeps it.
 #pragma once
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_select.cuh>
@@ -21,6 +26,7 @@
 
 #define AZB_GROW_CHUNK (1u << 22)  // children per chunk
 #define AZB_GROW_EPS 1e-9          // slack of the levels below N (absolute, on the key)
+#define AZB_GROW_MAX_WORLD 256u    // ranks azb_comm_trees_within takes: one round's codes stay below 2^31
 
 struct AzbGrowEnt {            // one class: its code and, once evaluated, the bits of its key (> 0: they order like values)
     unsigned long long hi, lo;  // the code, as azb_tree_codes writes it (hi, lo = string bits 0..63, 64..127)
@@ -94,4 +100,60 @@ __global__ void __launch_bounds__(256) azb_grow_below_kernel(const AzbGrowEnt *_
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     const int c = __syncthreads_count(t < m && __longlong_as_double((long long)ent[t].key) < bound);
     if (threadIdx.x == 0 && c) atomicAdd(below, (unsigned long long)c);
+}
+
+// the rank that holds a class when the growth is split over `world` ranks (include/azb.h)
+__host__ __device__ __forceinline__ uint32_t azb_grow_owner(unsigned long long hi, unsigned long long lo, uint32_t world) {
+    return (uint32_t)(azb_mix64(hi ^ azb_mix64(lo)) % world);
+}
+
+// counts[d] += the entries of ent[0, m) that rank d owns.  Dynamic shared memory: 4 * world bytes.
+__global__ void __launch_bounds__(256) azb_grow_count_kernel(const AzbGrowEnt *__restrict__ ent, uint32_t m, uint32_t world,
+                                                             unsigned long long *__restrict__ counts) {
+    extern __shared__ uint32_t s_cnt[];
+    for (uint32_t d = threadIdx.x; d < world; d += blockDim.x) s_cnt[d] = 0;
+    __syncthreads();
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += gridDim.x * blockDim.x)
+        atomicAdd(&s_cnt[azb_grow_owner(ent[i].hi, ent[i].lo, world)], 1u);
+    __syncthreads();
+    for (uint32_t d = threadIdx.x; d < world; d += blockDim.x)
+        if (s_cnt[d]) atomicAdd(&counts[d], (unsigned long long)s_cnt[d]);
+}
+
+// The codes of ent[0, m) as contiguous runs by owner: rank d's run starts at counts[0] + .. + counts[d - 1] (what
+// azb_grow_count_kernel gave), and cursor[d] (zeroed before the launch) is the part of it taken so far.  Each block takes
+// its slots of a run with one atomic per owner per tile of 256 entries; the order within a run is arbitrary, the
+// receiver sorts.  Dynamic shared memory: 20 * world bytes.
+__global__ void __launch_bounds__(256) azb_grow_route_kernel(const AzbGrowEnt *__restrict__ ent, uint32_t m, uint32_t world,
+                                                             const unsigned long long *__restrict__ counts,
+                                                             unsigned long long *__restrict__ cursor, ulonglong2 *__restrict__ out) {
+    extern __shared__ unsigned long long s_run[];  // [world] run starts | [world] this tile's bases | [world] u32 counts
+    unsigned long long *s_base = s_run + world;
+    uint32_t *s_cnt = reinterpret_cast<uint32_t *>(s_base + world);
+    if (threadIdx.x == 0) {
+        unsigned long long run = 0;
+        for (uint32_t d = 0; d < world; ++d) {
+            s_run[d] = run;
+            run += counts[d];
+        }
+    }
+    for (uint32_t tile = blockIdx.x * blockDim.x; tile < m; tile += gridDim.x * blockDim.x) {
+        for (uint32_t d = threadIdx.x; d < world; d += blockDim.x) s_cnt[d] = 0;
+        __syncthreads();
+        const uint32_t i = tile + threadIdx.x;
+        unsigned long long hi = 0, lo = 0;
+        uint32_t d = 0, slot = 0;
+        if (i < m) {
+            hi = ent[i].hi;
+            lo = ent[i].lo;
+            d = azb_grow_owner(hi, lo, world);
+            slot = atomicAdd(&s_cnt[d], 1u);
+        }
+        __syncthreads();
+        for (uint32_t r = threadIdx.x; r < world; r += blockDim.x)
+            s_base[r] = s_run[r] + (s_cnt[r] ? atomicAdd(&cursor[r], (unsigned long long)s_cnt[r]) : 0ull);
+        __syncthreads();
+        if (i < m) out[s_base[d] + slot] = make_ulonglong2(hi, lo);
+        __syncthreads();
+    }
 }

@@ -363,7 +363,8 @@ int azb_exhaustive_best(azb_handle *h, uint64_t start, uint64_t count, uint32_t 
  * classes (0: as many as fit in the device's free memory, which also bounds a larger max_level); azb_last_error names the
  * level and the classes found so far, and no output is written.  AZB_ERR_LAMBDA as azb_eval_costs.  The call works
  * before azb_init_trees, runs on the library stream, changes no tree, walker, counter, argmin, model or RNG state, and
- * its scratch counts in azb_device_bytes. */
+ * its scratch counts in azb_device_bytes.  It uses this handle's GPU alone, with or without a communicator;
+ * azb_comm_trees_within (below) splits the same call over the communicator's ranks. */
 int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out, uint64_t *n_within,
                      uint64_t *n_below, uint64_t *codes /*[k*2]*/, uint8_t *parents /*[k*N]*/, double *lambda1 /*[k]*/,
                      uint32_t *mu /*[k]*/, float *eval /*[k]*/, float *ms);
@@ -444,6 +445,33 @@ int azb_comm_destroy(azb_handle *h);
  * azb_get_argmin plus the owning rank; the lowest rank wins ties */
 int azb_comm_argmin(azb_handle *h, uint8_t *parents, uint32_t *permitted, double *lambda1, uint32_t *mu, float *eval,
                     int *owner_rank);
+/* azb_trees_within split over the ranks of the communicator: collective (every rank calls it), with the same arguments
+ * and outputs.  Every rank returns the same outputs, bit for bit what azb_trees_within returns on one handle of the same
+ * N for the same bound and k, whatever the world size and each rank's chunk size: every class is costed on its
+ * canonical labelling, so its key does not depend on the rank that costs it.  azb_trees_within itself stays local.
+ * Ownership: a class (code hi, lo) belongs to rank mix64(hi ^ mix64(lo)) mod world (mix64 as in the checkpoint digest
+ * above); a rank holds only the classes of each level it owns, the path and the star on 4 vertices start with theirs.
+ * A level runs in R rounds on every rank, R = the most chunks of parents any rank has at that level (a rank with none
+ * left takes part with an empty chunk).  A round: expand, code, sort and unique by code the rank's chunk; route the
+ * classes by owner into per-rank runs of 16-byte codes; all-gather a record per rank (its send counts to every rank, its
+ * kept-list size, its cap and its cost error word); exchange the runs with grouped NCCL sends and receives (the own run
+ * is a device copy); sort and unique the received codes, then decode, cost and keep them in pieces of at most one
+ * chunk.  The kept list is sorted and made unique by code as in azb_trees_within, and one more record closes the level:
+ * the level's size is the sum of the kept lists, and at 0 every rank stops.  At the last level each rank sorts its
+ * share by (key bits, code); n_within and n_below are sums over ranks, each rank's first min(k, share) are all-gathered
+ * and merged by (key bits, code), and every rank costs the global first min(k, n_within) as azb_trees_within does.
+ * Errors are agreed: the first collective all-gathers every rank's (N, bound bits, k, max_level), and every rank returns
+ * AZB_ERR_INVALID (azb_last_error names the rank and the field) for k == 0, k > 65536 or a NaN bound on any rank, and
+ * for an N, bound, k or max_level that differs between ranks.  AZB_ERR_CAPACITY on every rank, in the same round, when
+ * the sum of the kept lists exceeds max_level or a rank's share exceeds what its device has room for (the message
+ * names the level; with the same max_level this is the level where azb_trees_within stops).  AZB_ERR_LAMBDA on every
+ * rank when any rank saw it.  A CUDA or NCCL failure is reported by the rank that saw it.  After an agreed refusal the
+ * communicator stays usable.  AZB_ERR_STATE without azb_comm_init, AZB_ERR_INVALID on more than 256 ranks.  Works
+ * before azb_init_trees, runs all NCCL work on the library stream, changes no tree, walker, counter, argmin, model or
+ * RNG state; the exchange buffers come from the handle's scratch and count in azb_device_bytes. */
+int azb_comm_trees_within(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out, uint64_t *n_within,
+                          uint64_t *n_below, uint64_t *codes /*[k*2]*/, uint8_t *parents /*[k*N]*/, double *lambda1 /*[k]*/,
+                          uint32_t *mu /*[k]*/, float *eval /*[k]*/, float *ms);
 
 /* measurement helper: `reps` NCCL all-reduces of the gradient buffer (azb_mlp_num_params floats), timed with events on
  * the library's stream; *ms = milliseconds per all-reduce */

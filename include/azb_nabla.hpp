@@ -248,6 +248,17 @@ class NablaOptimizer {
     // (azb_trees_within); max_level caps the classes of a level (0: what fits in device memory)
     std::vector<TreeWithin> trees_within(double bound = -1.0, uint32_t k = 100, uint64_t max_level = 0, uint64_t *n_within = nullptr,
                                          uint64_t *n_below = nullptr) {
+        return trees_within_with(azb_trees_within, bound, k, max_level, n_within, n_below);
+    }
+    // trees_within split over the ranks of the attached communicator (azb_comm_trees_within): collective, every rank calls
+    // it with the same arguments and gets the same result, bit for bit trees_within's on one handle
+    std::vector<TreeWithin> comm_trees_within(double bound = -1.0, uint32_t k = 100, uint64_t max_level = 0,
+                                              uint64_t *n_within = nullptr, uint64_t *n_below = nullptr) {
+        return trees_within_with(azb_comm_trees_within, bound, k, max_level, n_within, n_below);
+    }
+    template <class Fn>
+    std::vector<TreeWithin> trees_within_with(Fn fn, double bound, uint32_t k, uint64_t max_level, uint64_t *n_within,
+                                              uint64_t *n_below) {
         const size_t n_v = cfg_.n_vertices, kk = k ? k : 1;
         std::vector<uint64_t> codes(kk * 2);
         std::vector<uint8_t> parents(kk * n_v);
@@ -255,8 +266,8 @@ class NablaOptimizer {
         std::vector<uint32_t> mu(kk);
         std::vector<float> eval(kk);
         uint32_t n = 0;
-        ck(azb_trees_within(h_, bound, k, max_level, &n, n_within, n_below, codes.data(), parents.data(), l1.data(), mu.data(),
-                            eval.data(), nullptr));
+        ck(fn(h_, bound, k, max_level, &n, n_within, n_below, codes.data(), parents.data(), l1.data(), mu.data(), eval.data(),
+              nullptr));
         std::vector<TreeWithin> out(n);
         for (uint32_t i = 0; i < n; ++i) {
             out[i].code[0] = codes[2 * i];

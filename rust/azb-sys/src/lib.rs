@@ -129,6 +129,7 @@ extern "C" {
     pub fn azb_free_trees(h: *mut azb_handle, start: u64, m: u32, parents: *mut u8) -> c_int;
     pub fn azb_exhaustive_best(h: *mut azb_handle, start: u64, count: u64, k: u32, bound: f64, n_out: *mut u32, n_below: *mut u64, index: *mut u64, parents: *mut u8, lambda1: *mut f64, mu: *mut u32, eval: *mut f32, ms: *mut f32) -> c_int;
     pub fn azb_trees_within(h: *mut azb_handle, bound: f64, k: u32, max_level: u64, n_out: *mut u32, n_within: *mut u64, n_below: *mut u64, codes: *mut u64, parents: *mut u8, lambda1: *mut f64, mu: *mut u32, eval: *mut f32, ms: *mut f32) -> c_int;
+    pub fn azb_comm_trees_within(h: *mut azb_handle, bound: f64, k: u32, max_level: u64, n_out: *mut u32, n_within: *mut u64, n_below: *mut u64, codes: *mut u64, parents: *mut u8, lambda1: *mut f64, mu: *mut u32, eval: *mut f32, ms: *mut f32) -> c_int;
     pub fn azb_checkpoint_size(h: *mut azb_handle, bytes: *mut u64) -> c_int;
     pub fn azb_checkpoint_save(h: *mut azb_handle, buf: *mut c_void, size: u64, written: *mut u64) -> c_int;
     pub fn azb_checkpoint_load(h: *mut azb_handle, blobs: *const *const c_void, sizes: *const u64, n_blobs: u32) -> c_int;
