@@ -95,6 +95,10 @@ SIGNATURES = {
                                       C.POINTER(C.c_uint64), u8p, f64p, u32p, f32p, f32p]),
     "azb_trees_within": (C.c_int, [C.c_void_p, C.c_double, C.c_uint32, C.c_uint64, u32p, C.POINTER(C.c_uint64),
                                    C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), u8p, f64p, u32p, f32p, f32p]),
+    "azb_trees_within_proof": (C.c_int, [C.c_void_p, C.c_double, C.c_uint32, C.c_uint64, u32p, C.POINTER(C.c_uint64),
+                                         C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), u8p, f64p, u32p, f32p,
+                                         C.POINTER(C.c_uint64), f32p]),
+    "azb_certify_keys": (C.c_int, [C.c_void_p, u8p, C.c_uint32, C.c_double, f64p, f64p, u32p, C.POINTER(C.c_int8), f32p]),
     "azb_comm_trees_within": (C.c_int, [C.c_void_p, C.c_double, C.c_uint32, C.c_uint64, u32p, C.POINTER(C.c_uint64),
                                         C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), u8p, f64p, u32p, f32p, f32p]),
     "azb_checkpoint_size": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
@@ -577,11 +581,15 @@ class Handle:
         res.update(n_below=int(below.value), ms=float(ms.value))
         return res
 
-    def trees_within(self, bound=None, k: int = 100, max_level: int = 0):
+    def trees_within(self, bound=None, k: int = 100, max_level: int = 0, prove: bool = False):
         """Every isomorphism class on N vertices with key = mu + lambda1 <= bound (azb_trees_within; default: the star's
         key), the first k ascending by (key, code): dict of arrays code u64[., 2], parents u8[., N] (canonical labelling),
         lambda1 f64, mu u32, eval f32, plus n_within, n_below (key < bound) and ms (device time).  max_level caps the
-        classes of any level (0: what fits in device memory); beyond it AzbError with ERR_CAPACITY."""
+        classes of any level (0: what fits in device memory); beyond it AzbError with ERR_CAPACITY.  prove=True runs
+        azb_trees_within_proof (default bound: sqrt(N - 1) + 1 exactly) and adds proof = dict(below, equal, above, open,
+        unproven_pruned) (include/azb.h)."""
+        if prove:
+            return self._trees_within(self._L.azb_trees_within_proof, bound, k, max_level, prove=True)
         return self._trees_within(self._L.azb_trees_within, bound, k, max_level)
 
     def comm_trees_within(self, bound=None, k: int = 100, max_level: int = 0):
@@ -589,17 +597,38 @@ class Handle:
         calls it with the same arguments and gets the same dict, bit for bit what trees_within gives on one handle."""
         return self._trees_within(self._L.azb_comm_trees_within, bound, k, max_level)
 
-    def _trees_within(self, fn, bound, k, max_level):
+    def _trees_within(self, fn, bound, k, max_level, prove=False):
         kk = max(int(k), 1)
         out = dict(code=np.zeros((kk, 2), dtype=np.uint64), parents=np.zeros((kk, self.n), dtype=np.uint8),
                    lambda1=np.zeros(kk, dtype=np.float64), mu=np.zeros(kk, dtype=np.uint32), eval=np.zeros(kk, dtype=np.float32))
         n, within, below, ms = C.c_uint32(), C.c_uint64(), C.c_uint64(), C.c_float()
+        proof = np.zeros(5, dtype=np.uint64)
         self._ck(fn(self._h, -1.0 if bound is None else float(bound), k, max_level, C.byref(n), C.byref(within), C.byref(below),
                     _p(out["code"], C.c_uint64), _p(out["parents"], C.c_uint8), _p(out["lambda1"], C.c_double),
-                    _p(out["mu"], C.c_uint32), _p(out["eval"], C.c_float), C.byref(ms)))
+                    _p(out["mu"], C.c_uint32), _p(out["eval"], C.c_float), *([_p(proof, C.c_uint64)] if prove else []),
+                    C.byref(ms)))
         res = {name: a[:n.value] for name, a in out.items()}
         res.update(n_within=int(within.value), n_below=int(below.value), ms=float(ms.value))
+        if prove:
+            res["proof"] = dict(zip(("below", "equal", "above", "open", "unproven_pruned"), (int(x) for x in proof)))
         return res
+
+    def certify_keys(self, parents, bound=None):
+        """Certificates of the keys mu + lambda1 of trees u8[M, N] against bound (azb_certify_keys; default: sqrt(N - 1) + 1
+        exactly): dict lambda1_lo, lambda1_hi (f64, lambda1_lo < lambda1 < lambda1_hi, NaN where not enclosed), mu (u32,
+        greedy matching), verdict (i8: -1 key < bound, 0 key == bound, +1 key > bound, all proven; 2 open), ms."""
+        p = np.ascontiguousarray(parents, dtype=np.uint8)
+        m = p.shape[0]
+        if p.shape != (m, self.n):
+            raise ValueError("parent rows")
+        out = dict(lambda1_lo=np.zeros(m, dtype=np.float64), lambda1_hi=np.zeros(m, dtype=np.float64),
+                   mu=np.zeros(m, dtype=np.uint32), verdict=np.zeros(m, dtype=np.int8))
+        ms = C.c_float()
+        self._ck(self._L.azb_certify_keys(self._h, _p(p, C.c_uint8), m, -1.0 if bound is None else float(bound),
+                                          _p(out["lambda1_lo"], C.c_double), _p(out["lambda1_hi"], C.c_double),
+                                          _p(out["mu"], C.c_uint32), _p(out["verdict"], C.c_int8), C.byref(ms)))
+        out["ms"] = float(ms.value)
+        return out
 
     def comm_allreduce_bench(self, reps: int = 20) -> float:
         ms = C.c_float()

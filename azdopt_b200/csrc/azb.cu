@@ -31,6 +31,7 @@
 #include "azb_ckpt.cuh"
 #include "azb_enum.cuh"
 #include "azb_grow.cuh"
+#include "azb_certify.cuh"
 
 #include <dlfcn.h>
 
@@ -1529,6 +1530,78 @@ int azb_eval_costs(azb_handle *h, const uint8_t *parents, uint32_t m, double *la
     CK(cudaSetDevice(h->cfg.device));
     return eval_costs_dev(h, parents, m, lambda1, mu, c, ms);
 }
+}  // extern "C"
+
+// ---- certificates of c21 keys against a bound (azb_certify.cuh) ----
+// the bound of azb_certify_keys and azb_trees_within_proof as the kernels take it, for trees on N vertices
+static AzbCertBound cert_bound(double bound, uint32_t N) {
+    AzbCertBound b{bound, N, bound < 0.0 ? 1 : 0, 0};
+    uint32_t s = 0;
+    while ((s + 1) * (s + 1) <= N - 1) ++s;
+    // (bound - 1)^2 = N - 1 for a bound >= 0 needs N - 1 = s^2 and bound = s + 1
+    b.tie = b.dflt || (s * s == N - 1 && bound == (double)(s + 1));
+    return b;
+}
+
+template <class Kernel>
+static int cert_smem(azb_handle *h, Kernel kernel, uint32_t n) {
+    const size_t smem = azb_certify_smem(n);
+    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    return AZB_OK;
+}
+
+// azb_certify_kernel on m device parent arrays of n vertices with their lambda_1 from the cost kernel
+static int launch_certify(azb_handle *h, const uint8_t *d_par, uint32_t m, uint32_t n, const double *d_l1, const AzbCertBound &b,
+                          double *lo, double *hi, uint32_t *mu, int8_t *verdict, unsigned long long *tally) {
+    int rc = cert_smem(h, azb_certify_kernel, n);
+    if (rc) return rc;
+    azb_certify_kernel<<<(m + AZB_CERT_THREADS - 1) / AZB_CERT_THREADS, AZB_CERT_THREADS, azb_certify_smem(n), h->stream>>>(
+        d_par, m, n, d_l1, b, lo, hi, mu, verdict, tally);
+    h->launches += 1;
+    CK(cudaGetLastError());
+    return AZB_OK;
+}
+
+extern "C" int azb_certify_keys(azb_handle *h, const uint8_t *parents, uint32_t m, double bound, double *lambda1_lo,
+                                double *lambda1_hi, uint32_t *mu, int8_t *verdict, float *ms) {
+    if (!h || !parents || m == 0) return AZB_ERR_INVALID;
+    if (std::isnan(bound)) return fail(h, AZB_ERR_INVALID, "azb_certify_keys: the bound is NaN");
+    const uint32_t N = h->N;
+    for (uint32_t i = 0; i < m; ++i)
+        for (uint32_t v = 1; v < N; ++v)
+            if (parents[(size_t)i * N + v] >= v) return fail(h, AZB_ERR_INVALID, "tree %u: parents[%u] is not < %u", i, v, v);
+    CK(cudaSetDevice(h->cfg.device));
+    uint8_t *d_par = nullptr;
+    CostOut d;
+    double *d_lo = nullptr, *d_hi = nullptr;
+    uint32_t *d_mu = nullptr;
+    int8_t *d_v = nullptr;
+    int rc = scratch(h, [&](Carve &cv) {
+        d_par = cv.take<uint8_t>((size_t)m * N);
+        d.take(cv, m);
+        d_lo = cv.take<double>(m);
+        d_hi = cv.take<double>(m);
+        d_mu = cv.take<uint32_t>(m);
+        d_v = cv.take<int8_t>(m);
+    });
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(d_par, parents, (size_t)m * N, cudaMemcpyHostToDevice, h->stream));
+    uint32_t err = 0;
+    rc = cost_tail(h, d_par, m, N, d, h->ev0, nullptr, nullptr, nullptr, nullptr, nullptr, &err);
+    if (rc) return rc;
+    rc = launch_certify(h, d_par, m, N, d.l1, cert_bound(bound, N), d_lo, d_hi, d_mu, d_v, nullptr);
+    if (rc) return rc;
+    CK(cudaEventRecord(h->ev1, h->stream));
+    if (lambda1_lo) CK(cudaMemcpyAsync(lambda1_lo, d_lo, (size_t)m * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (lambda1_hi) CK(cudaMemcpyAsync(lambda1_hi, d_hi, (size_t)m * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (mu) CK(cudaMemcpyAsync(mu, d_mu, (size_t)m * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (verdict) CK(cudaMemcpyAsync(verdict, d_v, m, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (ms) CK(cudaEventElapsedTime(ms, h->ev0, h->ev1));
+    if (err) return fail(h, (int)err, "%s", azb_strerror((int)err));
+    return AZB_OK;
+}
+extern "C" {
 
 // ---- stand-alone cost + action kinds of connected bitset graphs (SURVEY 8(f) row 3) ----
 }  // extern "C"
@@ -2244,10 +2317,11 @@ static int within_agreed_stop(azb_handle *h, const std::vector<unsigned long lon
     return AZB_OK;
 }
 
-// azb_trees_within (sharded = false: this handle alone, no collective) and azb_comm_trees_within (sharded = true)
+// azb_trees_within (sharded = false: this handle alone, no collective) and azb_comm_trees_within (sharded = true);
+// proof != null (azb_trees_within_proof, alone only): the same outputs and the five proof words
 static int trees_within(azb_handle *h, bool sharded, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out,
                         uint64_t *n_within, uint64_t *n_below, uint64_t *codes, uint8_t *parents, double *lambda1, uint32_t *mu,
-                        float *eval, float *ms) {
+                        float *eval, uint64_t *proof, float *ms) {
     CK(cudaSetDevice(h->cfg.device));
     const uint32_t N = h->N, chunk = h->grow_chunk ? h->grow_chunk : AZB_GROW_CHUNK;
     const uint32_t world = sharded ? (uint32_t)h->comm_world : 1u, me = sharded ? (uint32_t)h->comm_rank : 0u;
@@ -2259,6 +2333,8 @@ static int trees_within(azb_handle *h, bool sharded, double bound, uint32_t k, u
         rc = within_agree_args(h, bound, k, max_level, chunk, chunks);
         if (rc) return rc;
     }
+    const AzbCertBound cb = cert_bound(bound, N);  // before the default bound becomes the star's computed key
+    uint64_t pw[5] = {0, 0, 0, 0, 0};             // the proof words so far
     CK(cudaEventRecord(h->ev0, h->stream));
     if (bound < 0.0) {  // the star's key on its canonical labelling: every vertex under vertex 0
         uint8_t *d_star = nullptr;
@@ -2347,7 +2423,7 @@ static int trees_within(azb_handle *h, bool sharded, double bound, uint32_t k, u
         uint32_t *d_mu = nullptr;
         float *d_c = nullptr;
         ulonglong2 *d_send = nullptr;
-        unsigned long long *d_rec = nullptr, *d_cursor = nullptr;
+        unsigned long long *d_rec = nullptr, *d_cursor = nullptr, *d_proof = nullptr;
         rc = scratch(h, [&](Carve &cv) {
             d_lv = cv.take<AzbGrowEnt>(ns);
             d_lp = cv.take<uint8_t>(ns * s);
@@ -2370,10 +2446,16 @@ static int trees_within(azb_handle *h, bool sharded, double bound, uint32_t k, u
             d_rec = cv.take<unsigned long long>(sharded ? R * (world + 1) : 0);
             d_cursor = cv.take<unsigned long long>(sharded ? world : 0);
             d_top = cv.take<unsigned long long>(sharded && last ? tw * (world + 1) : 0);  // count, below, first k entries
+            d_proof = cv.take<unsigned long long>(proof ? 5 : 0);  // this level's proof words
         });
         if (rc) return rc;
         CK(cudaMemcpyAsync(d_lv, lvl.data(), ns * E, cudaMemcpyHostToDevice, h->stream));
         CK(cudaMemsetAsync(d_sc, 0, sizeof(AzbGrowScalars), h->stream));
+        if (proof) {
+            CK(cudaMemsetAsync(d_proof, 0, 5 * 8, h->stream));
+            rc = cert_smem(h, azb_certify_pruned_kernel, n);
+            if (rc) return rc;
+        }
         if (ns) {
             azb_grow_decode_kernel<<<(uint32_t)((ns + 255) / 256), 256, 0, h->stream>>>(d_lv, (uint32_t)ns, s, d_lp);
             h->launches += 1;
@@ -2470,6 +2552,12 @@ static int trees_within(azb_handle *h, bool sharded, double bound, uint32_t k, u
                 azb_grow_keep_kernel<<<(q + 255) / 256, 256, 0, h->stream>>>(fresh + off, d_l1, d_mu, q, thr, d_a + nacc, &d_sc->n_keep);
                 h->launches += 2;
                 CK(cudaGetLastError());
+                if (proof) {  // the classes keep dropped: key > bound proven, or proof[4]
+                    azb_certify_pruned_kernel<<<(q + AZB_CERT_THREADS - 1) / AZB_CERT_THREADS, AZB_CERT_THREADS, azb_certify_smem(n),
+                                                h->stream>>>(d_k, q, n, d_l1, d_mu, thr, cb, &d_proof[4]);
+                    h->launches += 1;
+                    CK(cudaGetLastError());
+                }
                 CK(cudaMemcpyAsync(&kept, &d_sc->n_keep, 4, cudaMemcpyDeviceToHost, h->stream));
                 CK(cudaStreamSynchronize(h->stream));
                 nacc += kept;
@@ -2487,6 +2575,17 @@ static int trees_within(azb_handle *h, bool sharded, double bound, uint32_t k, u
             rc = merge();
             if (rc) return rc;
         }
+        // proof, last level: the verdict of every result class, once each (a class can be kept in several chunks, so
+        // the chunks cannot count them), on its canonical labelling as the level costed it
+        for (uint32_t off = 0; proof && last && off < nacc; off += kc) {
+            const uint32_t q = (uint32_t)std::min<uint64_t>(kc, nacc - off);
+            azb_grow_decode_kernel<<<(q + 255) / 256, 256, 0, h->stream>>>(d_a + off, q, n, d_k);
+            launch_cost_n(h, d_k, q, n, d_l1, d_mu, d_c, &d_sc->err);
+            h->launches += 1;
+            CK(cudaGetLastError());
+            rc = launch_certify(h, d_k, q, n, d_l1, cb, nullptr, nullptr, nullptr, nullptr, d_proof);
+            if (rc) return rc;
+        }
         if (sharded) {  // the level's closing record: every rank's share of it
             uint32_t none = 0;
             rc = exchange(0, &none);
@@ -2498,11 +2597,14 @@ static int trees_within(azb_handle *h, bool sharded, double bound, uint32_t k, u
         total = 0;
         for (uint64_t c : share) total += c;
         uint32_t err = 0;
+        unsigned long long lp[5] = {0, 0, 0, 0, 0};
         CK(cudaMemcpyAsync(&err, &d_sc->err, 4, cudaMemcpyDeviceToHost, h->stream));
+        if (proof) CK(cudaMemcpyAsync(lp, d_proof, sizeof(lp), cudaMemcpyDeviceToHost, h->stream));
         lvl.resize(last ? 0 : nacc);
         if (!last && nacc) CK(cudaMemcpyAsync(lvl.data(), d_a, nacc * E, cudaMemcpyDeviceToHost, h->stream));
         CK(cudaStreamSynchronize(h->stream));
         if (err) return fail(h, AZB_ERR_LAMBDA, "%s", azb_strerror(AZB_ERR_LAMBDA));
+        for (int w = 0; w < 5; ++w) pw[w] += lp[w];
         const double level_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
         if (trace && !sharded)
             fprintf(stderr, "azb_trees_within: N %u level %u: %llu classes, %llu children, %llu evaluated, %.3f ms\n", N, n,
@@ -2572,6 +2674,7 @@ static int trees_within(azb_handle *h, bool sharded, double bound, uint32_t k, u
     if (n_out) *n_out = nres;
     if (n_within) *n_within = total;
     if (n_below) *n_below = below;
+    if (proof) memcpy(proof, pw, sizeof(pw));
     return AZB_OK;
 }
 
@@ -2581,7 +2684,18 @@ extern "C" int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_
     if (!h) return AZB_ERR_INVALID;
     if (k == 0 || k > AZB_BEST_MAX_K) return fail(h, AZB_ERR_INVALID, "k must be in 1..%u, got %u", AZB_BEST_MAX_K, k);
     if (std::isnan(bound)) return fail(h, AZB_ERR_INVALID, "azb_trees_within: the bound is NaN");
-    return trees_within(h, false, bound, k, max_level, n_out, n_within, n_below, codes, parents, lambda1, mu, eval, ms);
+    return trees_within(h, false, bound, k, max_level, n_out, n_within, n_below, codes, parents, lambda1, mu, eval, nullptr, ms);
+}
+
+extern "C" int azb_trees_within_proof(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out,
+                                      uint64_t *n_within, uint64_t *n_below, uint64_t *codes, uint8_t *parents, double *lambda1,
+                                      uint32_t *mu, float *eval, uint64_t *proof, float *ms) {
+    if (!h) return AZB_ERR_INVALID;
+    if (k == 0 || k > AZB_BEST_MAX_K) return fail(h, AZB_ERR_INVALID, "k must be in 1..%u, got %u", AZB_BEST_MAX_K, k);
+    if (std::isnan(bound)) return fail(h, AZB_ERR_INVALID, "azb_trees_within_proof: the bound is NaN");
+    uint64_t pw[5];
+    return trees_within(h, false, bound, k, max_level, n_out, n_within, n_below, codes, parents, lambda1, mu, eval,
+                        proof ? proof : pw, ms);
 }
 
 extern "C" int azb_comm_trees_within(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out,
@@ -2591,7 +2705,7 @@ extern "C" int azb_comm_trees_within(azb_handle *h, double bound, uint32_t k, ui
     if (!h->nccl_comm) return fail(h, AZB_ERR_STATE, "azb_comm_init has not been called");
     if (h->comm_world > AZB_GROW_MAX_WORLD)
         return fail(h, AZB_ERR_INVALID, "azb_comm_trees_within: %d ranks, at most %u", h->comm_world, AZB_GROW_MAX_WORLD);
-    return trees_within(h, true, bound, k, max_level, n_out, n_within, n_below, codes, parents, lambda1, mu, eval, ms);
+    return trees_within(h, true, bound, k, max_level, n_out, n_within, n_below, codes, parents, lambda1, mu, eval, nullptr, ms);
 }
 
 // cascade waves that outgrew the shared-memory work list and continued in global scratch since azb_create (diagnostic;

@@ -119,6 +119,10 @@ def main():
     with open(os.path.join(args.out, "best.g6"), "wb") as g:
         g.write(opt.argmin_graph6() + b"\n")
     print("best tree (graph6):", opt.argmin_graph6().decode())
+    cert = opt.h.certify_keys(opt.argmin_data().parents[None])   # proven against sqrt(N - 1) + 1, or open
+    verdict = {-1: "proven below", 0: "proven equal to", 1: "proven above", 2: "open against"}[int(cert["verdict"][0])]
+    print(f"best tree's key mu + lambda_1 (lambda_1 in ({cert['lambda1_lo'][0]!r}, {cert['lambda1_hi'][0]!r}), "
+          f"mu = {cert['mu'][0]}): {verdict} sqrt(N - 1) + 1")
     if best:
         with open(os.path.join(args.out, "best_trees.g6"), "wb") as g:
             for t in best.result():

@@ -368,6 +368,45 @@ int azb_exhaustive_best(azb_handle *h, uint64_t start, uint64_t count, uint32_t 
 int azb_trees_within(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out, uint64_t *n_within,
                      uint64_t *n_below, uint64_t *codes /*[k*2]*/, uint8_t *parents /*[k*N]*/, double *lambda1 /*[k]*/,
                      uint32_t *mu /*[k]*/, float *eval /*[k]*/, float *ms);
+/* ---- extension (no reference item): certificates of c21 keys against a bound, with directed rounding.
+ * rd / ru: one IEEE binary64 operation rounded down / up, no contraction.
+ * Interval inertia count JT(T, x) for a tree T (parents[v] < v) and a binary64 point x: every vertex starts with the
+ * interval [-x, -x].  For v = n-1 down to 1 the interval [l_v, u_v] of v is final when it is reached; if it contains 0
+ * (or has a NaN end) the result is undecided, otherwise r_lo = rd(1/u_v), r_hi = ru(1/l_v), and then for p = parents[v]
+ * l_p = rd(l_p - r_hi), u_p = ru(u_p - r_lo).  Vertex 0 is undecided if its interval contains 0.  Otherwise the count is
+ * the number of v with l_v > 0.  Every exact Jacobs-Trevisan value lies in its interval and none is 0, so a decided
+ * count is the number of eigenvalues of A above x: 0 proves lambda1 < x, >= 1 proves lambda1 > x.
+ * mu: greedy leaf matching, v = n-1 down to 1 is matched with parents[v] when both are unmatched (exact for trees).
+ * Enclosure of lambda1 from c = the cost kernel's lambda1 (a starting point only; nothing relies on it being right):
+ * with d_j = 4^j ulp(c), j = 0 .. 11, lambda1_lo = rd(c - d_j) for the first j at which JT is decided with a count >= 1,
+ * lambda1_hi = ru(c + d_j) for the first j at which JT is decided with a count of 0; both NaN if either is not found
+ * (or c is outside [1, 2^1000)).  So lambda1_lo < lambda1 < lambda1_hi.
+ * The bound as a real number: a bound >= 0 is that binary64 value; a bound < 0 is sqrt(N - 1) + 1 exactly (the star's
+ * true key, not its rounded value).  t = bound - mu is enclosed in [t_lo, t_hi]: t_lo = rd(b_lo - mu), t_hi = ru(b_hi -
+ * mu) with b_lo = b_hi = bound, or for the default bound b_lo = rd(rd_sqrt(N - 1) + 1), b_hi = ru(ru_sqrt(N - 1) + 1).
+ * Verdict (int8): 0 = key == bound proven, only for a star (mu = 1) against the default bound or against a bound >= 0
+ * with (bound - 1)^2 = N - 1; else -1 = key < bound proven (lambda1_hi <= t_lo, or JT at t_lo decided with a count of
+ * 0); else +1 = key > bound proven (lambda1_lo >= t_hi, or JT at t_hi decided with a count >= 1); else 2 = open (any
+ * other exact tie, or intervals too wide to decide).  Never a guess.
+ * azb_certify_keys: for m trees on the handle's N vertices, the cost kernel of azb_eval_costs and then the certificate
+ * of each: lambda1_lo, lambda1_hi, the greedy mu and the verdict against bound.  ms = device time of the call.  Any
+ * output pointer may be NULL.  AZB_ERR_INVALID as azb_eval_costs (azb_last_error names the first bad tree) and for a
+ * NaN bound; AZB_ERR_LAMBDA as azb_eval_costs.  Works before azb_init_trees, runs on the library stream, changes no
+ * state, and its scratch counts in azb_device_bytes. */
+int azb_certify_keys(azb_handle *h, const uint8_t *parents /*[m*N]*/, uint32_t m, double bound, double *lambda1_lo /*[m]*/,
+                     double *lambda1_hi /*[m]*/, uint32_t *mu /*[m]*/, int8_t *verdict /*[m]*/, float *ms);
+/* azb_trees_within_proof: azb_trees_within with the certificate above run on its way; every output but proof is bit for
+ * bit what azb_trees_within gives (ms includes the certificates).  proof[5]:
+ *   [0] result classes proven below the bound, [1] proven equal to it (the star), [2] proven above it (the binary64
+ *   filter let them in), [3] open; these sum to n_within and are counted once per class, after the last level's merge;
+ *   [4] classes dropped at any level (key not <= the level's threshold) for which key > bound was not proven: JT at t_hi
+ *   counts >= 1, or else JT counts >= 1 at one of the points rd(c - 4^j ulp(c)), j = 0 .. 11, above t_hi.  A class met
+ *   in several chunks of one level counts once for each, so [4] is 0 exactly when every dropped class is proven.
+ * When proof[3] = proof[4] = 0 this is a theorem (DESIGN.md §4.12): exactly n_within - proof[2] trees on N vertices have
+ * key <= bound, and proof[0] of them have key < bound.  Errors and state as azb_trees_within; proof may be NULL. */
+int azb_trees_within_proof(azb_handle *h, double bound, uint32_t k, uint64_t max_level, uint32_t *n_out, uint64_t *n_within,
+                           uint64_t *n_below, uint64_t *codes /*[k*2]*/, uint8_t *parents /*[k*N]*/, double *lambda1 /*[k]*/,
+                           uint32_t *mu /*[k]*/, float *eval /*[k]*/, uint64_t *proof /*[5]*/, float *ms);
 /* persistent walker state: states, paths, last_positions (optimizer/mod.rs:10-14) */
 int azb_get_walkers(azb_handle *h, uint8_t *parents, uint32_t *permitted, uint32_t *path, uint32_t *pos,
                     uint32_t *path_len);

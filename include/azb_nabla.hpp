@@ -256,6 +256,35 @@ class NablaOptimizer {
                                               uint64_t *n_within = nullptr, uint64_t *n_below = nullptr) {
         return trees_within_with(azb_comm_trees_within, bound, k, max_level, n_within, n_below);
     }
+    // trees_within with its certificate (azb_trees_within_proof): proof[5] = result classes proven below, equal, above the
+    // bound (< 0: sqrt(N - 1) + 1 exactly), open, and dropped classes not proven above it; the rest as trees_within
+    std::vector<TreeWithin> trees_within_proof(uint64_t proof[5], double bound = -1.0, uint32_t k = 100, uint64_t max_level = 0,
+                                               uint64_t *n_within = nullptr, uint64_t *n_below = nullptr) {
+        return trees_within_with(
+            [proof](azb_handle *h, double b, uint32_t kk, uint64_t ml, uint32_t *n, uint64_t *nw, uint64_t *nb, uint64_t *c,
+                    uint8_t *p, double *l1, uint32_t *mu, float *ev, float *ms) {
+                return azb_trees_within_proof(h, b, kk, ml, n, nw, nb, c, p, l1, mu, ev, proof, ms);
+            },
+            bound, k, max_level, n_within, n_below);
+    }
+    // certificates of the keys of m trees (parents: m * N bytes) against bound (< 0: sqrt(N - 1) + 1 exactly)
+    // (azb_certify_keys): verdict -1 / 0 / +1 = key below / equal to / above the bound, proven; 2 = open
+    struct KeyCertificates {
+        std::vector<double> lambda_1_lo, lambda_1_hi;
+        std::vector<uint32_t> mu;
+        std::vector<int8_t> verdict;
+    };
+    KeyCertificates certify_keys(const std::vector<uint8_t> &parents, double bound = -1.0) {
+        const uint32_t m = (uint32_t)(parents.size() / cfg_.n_vertices);
+        KeyCertificates out;
+        out.lambda_1_lo.resize(m);
+        out.lambda_1_hi.resize(m);
+        out.mu.resize(m);
+        out.verdict.resize(m);
+        ck(azb_certify_keys(h_, parents.data(), m, bound, out.lambda_1_lo.data(), out.lambda_1_hi.data(), out.mu.data(),
+                            out.verdict.data(), nullptr));
+        return out;
+    }
     template <class Fn>
     std::vector<TreeWithin> trees_within_with(Fn fn, double bound, uint32_t k, uint64_t max_level, uint64_t *n_within,
                                               uint64_t *n_below) {

@@ -129,6 +129,8 @@ extern "C" {
     pub fn azb_free_trees(h: *mut azb_handle, start: u64, m: u32, parents: *mut u8) -> c_int;
     pub fn azb_exhaustive_best(h: *mut azb_handle, start: u64, count: u64, k: u32, bound: f64, n_out: *mut u32, n_below: *mut u64, index: *mut u64, parents: *mut u8, lambda1: *mut f64, mu: *mut u32, eval: *mut f32, ms: *mut f32) -> c_int;
     pub fn azb_trees_within(h: *mut azb_handle, bound: f64, k: u32, max_level: u64, n_out: *mut u32, n_within: *mut u64, n_below: *mut u64, codes: *mut u64, parents: *mut u8, lambda1: *mut f64, mu: *mut u32, eval: *mut f32, ms: *mut f32) -> c_int;
+    pub fn azb_trees_within_proof(h: *mut azb_handle, bound: f64, k: u32, max_level: u64, n_out: *mut u32, n_within: *mut u64, n_below: *mut u64, codes: *mut u64, parents: *mut u8, lambda1: *mut f64, mu: *mut u32, eval: *mut f32, proof: *mut u64, ms: *mut f32) -> c_int;
+    pub fn azb_certify_keys(h: *mut azb_handle, parents: *const u8, m: u32, bound: f64, lambda1_lo: *mut f64, lambda1_hi: *mut f64, mu: *mut u32, verdict: *mut i8, ms: *mut f32) -> c_int;
     pub fn azb_comm_trees_within(h: *mut azb_handle, bound: f64, k: u32, max_level: u64, n_out: *mut u32, n_within: *mut u64, n_below: *mut u64, codes: *mut u64, parents: *mut u8, lambda1: *mut f64, mu: *mut u32, eval: *mut f32, ms: *mut f32) -> c_int;
     pub fn azb_checkpoint_size(h: *mut azb_handle, bytes: *mut u64) -> c_int;
     pub fn azb_checkpoint_save(h: *mut azb_handle, buf: *mut c_void, size: u64, written: *mut u64) -> c_int;
